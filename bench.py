@@ -2,7 +2,7 @@
 """bench.py — force evaluations per second of the genome-wide MultiMM model on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload gw|chrom|region|stress] [--decompose]
+                    [--workload gw|chrom|region|stress] [--decompose] [--dump-outputs DIR]
 
 Metric (BASELINE.json: "genome-wide minimization wall-time; force evals/s; ensemble
 structures/hour"): the headline `value` is metric 2, combined energy+force evaluations per second
@@ -25,6 +25,9 @@ MultiMM.add_* -> engine (C-ABI).  Metrics 1 and 3 ride on the same line:
 `ensemble`: metric 3 — every rank runs ONE ensemble member through the driver's own per-replica
            pipeline (run.run_replica: loaders, init CIF/PSF, force field, minimisation, minimised
            CIF, per-chromosome CIFs, tar.gz) on its GPU; structures/hour = ranks x 3600 / slowest.
+--dump-outputs DIR: what the last timed evaluation returned, DIR/energy_terms.npy (10,) kJ/mol and
+           DIR/forces.npy (N, 3) kJ/mol/nm, float64 (rank 0).  The inputs are seeded, so two builds run
+           with the same arguments can be compared array for array.
 `decomposed` (N > 1): the N = 2e6 stress system with its pair work shared by the ranks
            (mmm_dist.cu): ms per evaluation, pair-kernel share, ms in the exchange step.
 `cpu_baseline`: the CPU oracle (FP64 restatement of the OpenMM Reference semantics, OpenMP, thread
@@ -376,6 +379,14 @@ def ensemble_members(workload: str, rank: int, world: int, device: int, tmp: str
     return dict(wall_seconds=wall, members=reps)
 
 
+def dump_outputs(path: str, e_terms: np.ndarray, forces: np.ndarray) -> None:
+    """The arrays a caller of the evaluation receives, as float64 .npy (N = 2e6, the largest
+    workload, makes 48 MB of forces)."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "energy_terms.npy"), np.asarray(e_terms, dtype=np.float64))
+    np.save(os.path.join(path, "forces.npy"), np.asarray(forces, dtype=np.float64))
+
+
 def run_ours(opt):
     import torch
     import torch.distributed as dist
@@ -427,6 +438,8 @@ def run_ours(opt):
             barrier()
             clk.mark_end()
         launches = eng.launch_count - launches0
+        if opt.dump_outputs and rank == 0:
+            dump_outputs(opt.dump_outputs, *eng.last_result())
         coll_ms = eng.last_collective_ms if decomposed else 0.0
         total_ms, pair_ms_max, coll_ms = max_over_ranks([total_ms, pair_ms, coll_ms], device=dev)
         value = whole_job_rate(1 if decomposed else world, K, total_ms)
@@ -697,7 +710,11 @@ def main():
     ap.add_argument("--decomposed-steps", type=int, default=5)
     ap.add_argument("--no-ref-full", action="store_true", help="reference arm: skip the one real full-size evaluation")
     ap.add_argument("--openmm-minimize-cap", type=float, default=120.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the energies and forces of the last timed evaluation to DIR/<name>.npy")
     opt = ap.parse_args()
+    if opt.dump_outputs and opt.impl != "ours":
+        ap.error("--dump-outputs writes what the engine computed: it needs --impl ours")
     if opt.impl == "reference":
         run_reference(opt)
     else:

@@ -167,6 +167,13 @@ int mmm_evaluate_n(mmm_handle h, int n);
  * the timed region.  total_ms: all n evaluations (flushes included); pair_ms: sum of the n pair
  * kernel launches alone (per-launch events). Either output may be NULL. */
 int mmm_evaluate_timed(mmm_handle h, int n, int flush_l2, float *total_ms, float *pair_ms);
+/* What the most recent evaluation (mmm_energy_forces, mmm_evaluate_n, mmm_evaluate_timed)
+ * computed, without evaluating again: per-term energies and forces (N x 3, = -dE/dx), as
+ * mmm_energy_forces returns them, for the positions and parameters that evaluation ran with
+ * (setting new ones does not recompute them). mmm_minimize and mmm_md_run reuse these buffers:
+ * after either, MMM_ERR_STATE until the next evaluation, as before the first. Either output may
+ * be NULL. */
+int mmm_last_result(mmm_handle h, double *e_terms, double *forces);
 
 /* ---- minimisation (Simulation.minimizeEnergy(), model.py:886) -------------------- */
 /* L-BFGS (m = 6, strong-Wolfe backtracking) until the per-particle RMS-force rule of

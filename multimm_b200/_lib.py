@@ -31,7 +31,8 @@ EXPORTS = (
     "mmm_set_pair_term", "mmm_set_external_term", "mmm_set_cutoff",
     "mmm_set_positions", "mmm_get_positions", "mmm_set_positions_device", "mmm_get_positions_device",
     "mmm_hilbert_init", "mmm_hilbert_points",
-    "mmm_energy_forces", "mmm_energy_forces_device", "mmm_evaluate_n", "mmm_evaluate_timed", "mmm_minimize",
+    "mmm_energy_forces", "mmm_energy_forces_device", "mmm_evaluate_n", "mmm_evaluate_timed", "mmm_last_result",
+    "mmm_minimize",
     "mmm_launch_count", "mmm_set_graph", "mmm_set_chb_surrogate", "mmm_set_pair_kernel", "mmm_pair_kernel_in_use", "mmm_last_pair_kernel_ms", "mmm_get_cell_list", "mmm_get_cell_grid", "mmm_measure_fp32_peak",
     "mmm_dist_unique_id", "mmm_dist_init", "mmm_dist_emulate", "mmm_dist_last_exchange_ms", "mmm_dist_queue_mode",
     "mmm_mean_pair_distance", "mmm_contact_map", "mmm_md_configure", "mmm_md_set_amd", "mmm_set_velocities_to_temperature", "mmm_set_velocities", "mmm_get_velocities", "mmm_md_run",
@@ -98,6 +99,7 @@ def load():
         "mmm_energy_forces_device": (i32, [vp, vp, vp]),
         "mmm_evaluate_n": (i32, [vp, i32]),
         "mmm_evaluate_timed": (i32, [vp, i32, i32, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
+        "mmm_last_result": (i32, [vp, vp, vp]),
         "mmm_minimize": (i32, [vp, dbl, i64, C.POINTER(MinReport)]),
         "mmm_launch_count": (i64, [vp]),
         "mmm_set_pair_kernel": (i32, [vp, i32]),

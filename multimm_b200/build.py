@@ -24,11 +24,12 @@ NVCC_FLAGS = [
 ]
 
 
-def _nvcc() -> str:
-    for cand in (shutil.which("nvcc"), "/usr/local/cuda/bin/nvcc"):
+def cuda_tool(name: str) -> str:
+    """A CUDA toolkit program (nvcc, cuobjdump): from PATH, else the toolkit's default location."""
+    for cand in (shutil.which(name), os.path.join("/usr/local/cuda/bin", name)):
         if cand and os.path.exists(cand):
             return cand
-    raise RuntimeError("nvcc not found; libmultimm_b200.so cannot be built")
+    raise RuntimeError(f"{name} not found (neither on PATH nor in /usr/local/cuda/bin)")
 
 
 def sources() -> list[str]:
@@ -50,7 +51,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     # link into a private name and rename: a concurrent reader (another test worker, an ensemble
     # worker) sees either the old library or the complete new one, never a half-written file
     tmp = f"{LIB_PATH}.{os.getpid()}.tmp"
-    cmd = [_nvcc(), *NVCC_FLAGS, *os.environ.get("MMM_EXTRA_NVCC_FLAGS", "").split(), "-o", tmp, *sources()]
+    cmd = [cuda_tool("nvcc"), *NVCC_FLAGS, *os.environ.get("MMM_EXTRA_NVCC_FLAGS", "").split(), "-o", tmp, *sources()]
     if verbose:
         cmd[1:1] = ["-Xptxas", "-v"]
     try:

@@ -623,19 +623,33 @@ int mmm_energy_forces_device(mmm_handle h, double* e_terms, double* d_forces) {
   return MMM_OK;
 }
 
+// d_g holds the gradient: negated on the device, not by a host pass over 24 N bytes
+static int copy_forces_to_host(mmm_system* h, double* forces) {
+  if (!h->d_fout) MMM_CUDA(h, cudaMalloc((void**)&h->d_fout, sizeof(double) * 3 * (size_t)h->n));
+  k_negate<<<(unsigned)((3 * h->n + 255) / 256), 256, 0, h->stream>>>(3 * h->n, h->d_g, h->d_fout);
+  h->launches++;
+  MMM_CUDA(h, cudaGetLastError());
+  MMM_CUDA(h, cudaMemcpyAsync(forces, h->d_fout, sizeof(double) * 3 * h->n, cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MMM_OK;
+}
+
 int mmm_energy_forces(mmm_handle h, double* e_terms, double* forces) {
   if (!h) return MMM_ERR_ARG;
   int rc = mmm_energy_forces_device(h, e_terms, nullptr);
   if (rc) return rc;
-  if (forces) {  // d_g holds the gradient: negated on the device, not by a host pass over 24 N bytes
-    if (!h->d_fout) MMM_CUDA(h, cudaMalloc((void**)&h->d_fout, sizeof(double) * 3 * (size_t)h->n));
-    k_negate<<<(unsigned)((3 * h->n + 255) / 256), 256, 0, h->stream>>>(3 * h->n, h->d_g, h->d_fout);
-    h->launches++;
-    MMM_CUDA(h, cudaGetLastError());
-    MMM_CUDA(h, cudaMemcpyAsync(forces, h->d_fout, sizeof(double) * 3 * h->n, cudaMemcpyDeviceToHost, h->stream));
+  return forces ? copy_forces_to_host(h, forces) : MMM_OK;
+}
+
+int mmm_last_result(mmm_handle h, double* e_terms, double* forces) {
+  if (!h) return MMM_ERR_ARG;
+  if (!h->have_result) return mmm_fail(h, MMM_ERR_STATE, "mmm_last_result: no result to read (nothing evaluated since creation, mmm_minimize or mmm_md_run)");
+  cudaSetDevice(h->device);
+  if (e_terms) {
+    MMM_CUDA(h, cudaMemcpyAsync(e_terms, h->d_eterms, sizeof(double) * MMM_NUM_TERMS, cudaMemcpyDeviceToHost, h->stream));
     MMM_CUDA(h, cudaStreamSynchronize(h->stream));
   }
-  return MMM_OK;
+  return forces ? copy_forces_to_host(h, forces) : MMM_OK;
 }
 
 int mmm_evaluate_n(mmm_handle h, int n) {
@@ -707,6 +721,7 @@ int mmm_minimize(mmm_handle h, double tol, int64_t max_iter, mmm_min_report* out
     if ((rc = dev_alloc(h, &h->d_S, n3 * MMM_LBFGS_M))) return rc;
     if ((rc = dev_alloc(h, &h->d_Y, n3 * MMM_LBFGS_M))) return rc;
   }
+  h->have_result = false;  // the line search leaves trial-point state in d_g / d_eterms
   return mmm_run_minimize(h, tol, max_iter, out);
 }
 

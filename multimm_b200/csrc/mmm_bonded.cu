@@ -354,5 +354,6 @@ int mmm_launch_finalize_energy(mmm_system* h) {
                                              h->d_eterms);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
+  h->have_result = true;
   return MMM_OK;
 }

@@ -181,6 +181,7 @@ struct mmm_system {
   double* d_epart = nullptr;     // [n_red_blocks][6] external+bonded energy partials
   double* d_dpart = nullptr;     // [n_red_blocks][MMM_NDOT] dot partials
   double* d_eterms = nullptr;    // [MMM_NUM_TERMS] result of the last evaluation
+  bool have_result = false;      // d_eterms / d_g hold a finished stand-alone evaluation (mmm_last_result)
 
   // L-BFGS
   LbfgsState* d_lb = nullptr;

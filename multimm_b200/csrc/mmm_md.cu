@@ -213,6 +213,7 @@ int mmm_md_run(mmm_handle h, int64_t n_steps, mmm_md_report* out) {
   cudaSetDevice(h->device);
   int rc = ensure_velocities(h);
   if (rc) return rc;
+  h->have_result = false;  // the integrator reuses d_g / d_eterms
   MdArgs A;
   A.integrator = h->md_integrator;
   A.dt = h->md_dt;

@@ -158,6 +158,14 @@ class Engine:
         self._ck(self._lib.mmm_evaluate_timed(self._h, int(n), int(bool(flush_l2)), C.byref(tot), C.byref(pair)))
         return float(tot.value), float(pair.value)
 
+    def last_result(self):
+        """Per-term energies (10,) and forces (N,3) of the most recent evaluation, read back
+        without evaluating again (e.g. the last of ``evaluate_timed``'s evaluations)."""
+        e = np.zeros(NUM_TERMS)
+        f = np.empty((self.n, 3))
+        self._ck(self._lib.mmm_last_result(self._h, _p(e), _p(f)))
+        return e, f
+
     def minimize(self, tol: float = 10.0, max_iter: int = 0) -> dict:
         """L-BFGS to OpenMM's default tolerance (10 kJ/mol/nm RMS force), unlimited iterations."""
         rep = MinReport()

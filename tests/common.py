@@ -13,6 +13,17 @@ if ROOT not in sys.path:
 
 from oracle import oracle as O  # noqa: E402
 
+# Root of a checkout of the original MultiMM (github.com/SFGLab/MultiMM).  The tests that run its code
+# live need one and skip without it; the outputs it gave are frozen under tests/golden and run everywhere.
+REFERENCE = os.environ.get("MULTIMM_REFERENCE", "")
+NO_REFERENCE = "no checkout of the original MultiMM named by MULTIMM_REFERENCE"
+
+
+def reference_file(rel: str) -> str | None:
+    """Path of `rel` inside the MULTIMM_REFERENCE checkout, None where there is no such file."""
+    path = os.path.join(REFERENCE, rel) if REFERENCE else None
+    return path if path and os.path.exists(path) else None
+
 # reference defaults (config.py:188-246)
 DEF = dict(
     bond_r0=0.1, bond_k=3.0e5, angle_t0=np.pi, angle_k=100.0, loop_r0=0.1, loop_k=3.0e4,

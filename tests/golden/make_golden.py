@@ -1,7 +1,7 @@
 """Generates tests/golden/*.npz by running the REFERENCE's own loaders
-(/root/reference/src/multimm/utils.py: import_bed, import_mns_from_bedpe) on synthetic input
-files written by multimm_b200.synthetic.  Run in the build container only (the reference tree
-does not travel to the GPU box); the inputs and outputs are committed.
+($MULTIMM_REFERENCE/src/multimm/utils.py: import_bed, import_mns_from_bedpe) on synthetic input
+files written by multimm_b200.synthetic.  Run only with MULTIMM_REFERENCE set; the inputs and
+outputs are committed.
 
     python tests/golden/make_golden.py
 
@@ -19,8 +19,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF_UTILS = "/root/reference/src/multimm/utils.py"
-REF_FIXTURE = "/root/reference/tests/fixtures/ENCFF045MJY_simple.bedpe"
+REFERENCE = os.environ["MULTIMM_REFERENCE"]  # a checkout of the original MultiMM
+REF_UTILS = os.path.join(REFERENCE, "src", "multimm", "utils.py")
+REF_FIXTURE = os.path.join(REFERENCE, "tests", "fixtures", "ENCFF045MJY_simple.bedpe")
 
 
 def load_reference_utils():

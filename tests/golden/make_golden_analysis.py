@@ -1,5 +1,5 @@
 """Generates tests/golden/analysis_*_report.txt by running the REFERENCE's own analyze_structure
-(/root/reference/src/multimm/plots.py:630-829) on two small structures.  Build container only.
+($MULTIMM_REFERENCE/src/multimm/plots.py:630-829) on two small structures.  Needs MULTIMM_REFERENCE.
 plots.py imports matplotlib, pyvista, seaborn, mpl_toolkits at the top and draws figures at the
 end of analyze_structure; those modules are absent here and are replaced by MagicMock objects — the
 numeric report (the part re-hosted in multimm_b200/analysis.py) does not depend on them.
@@ -19,7 +19,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/src/multimm"
+REF = os.path.join(os.environ["MULTIMM_REFERENCE"], "src", "multimm")  # a checkout of the original MultiMM
 
 
 def load_plots():

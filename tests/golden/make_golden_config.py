@@ -1,9 +1,9 @@
 """Generates tests/golden/config_golden.json by running the REFERENCE's own config model, MODELLING_LEVEL
-presets and cross-field checks (/root/reference/src/multimm/config.py: SimulationConfig;
+presets and cross-field checks ($MULTIMM_REFERENCE/src/multimm/config.py: SimulationConfig;
 run.py: ArgumentChanger.convenient_argument_changer, args_tests) on a matrix of inputs.
 `openmm.unit` (absent) is replaced by this repo's units module, which is what the reference's
 parse_quantity evaluates unit expressions against; every other absent import is a MagicMock.
-Build container only.     python tests/golden/make_golden_config.py
+Needs MULTIMM_REFERENCE.     python tests/golden/make_golden_config.py
 """
 import importlib.util
 import json
@@ -16,7 +16,7 @@ from unittest.mock import MagicMock
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/src/multimm"
+REF = os.path.join(os.environ["MULTIMM_REFERENCE"], "src", "multimm")  # a checkout of the original MultiMM
 
 from multimm_b200 import units  # noqa: E402
 

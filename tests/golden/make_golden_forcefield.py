@@ -1,5 +1,5 @@
 """Generates tests/golden/forcefield_golden.npz / .json by executing the REFERENCE's own force-field
-builder (/root/reference/src/multimm/model.py: set_radiuses and the ten add_* methods, unmodified)
+builder ($MULTIMM_REFERENCE/src/multimm/model.py: set_radiuses and the ten add_* methods, unmodified)
 against a RECORDING stand-in for the `openmm` module, and then evaluating the energy expressions
 the reference handed to it — its own Lepton strings, global and per-particle parameters, bond /
 angle / loop lists — with a small Lepton-to-numpy evaluator in FP64.
@@ -12,7 +12,7 @@ by the evaluator are the documented ones: HarmonicBondForce 1/2 k (r-r0)^2, Harm
 1/2 k (theta-theta0)^2, CustomNonbondedForce NoCutoff = sum over i<j with particle 1 = lower index,
 delta(x) = [x == 0], step(x) = [x >= 0].
 
-Build container only (needs /root/reference).   python tests/golden/make_golden_forcefield.py
+Needs MULTIMM_REFERENCE.   python tests/golden/make_golden_forcefield.py
 """
 import importlib.util
 import json
@@ -27,7 +27,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/src/multimm"
+REF = os.path.join(os.environ["MULTIMM_REFERENCE"], "src", "multimm")  # a checkout of the original MultiMM
 
 from multimm_b200 import units  # noqa: E402
 from multimm_b200.config import SimulationConfig  # noqa: E402

@@ -1,7 +1,7 @@
 """Generates tests/golden/model_init_golden.npz by running the REFERENCE's own MultiMM.__init__
-(/root/reference/src/multimm/model.py:24-162: input ingestion, chromosome spins and strengths, gene
+($MULTIMM_REFERENCE/src/multimm/model.py:24-162: input ingestion, chromosome spins and strengths, gene
 window) with its own loaders on the synthetic inputs of tests/golden.  Absent modules are stand-ins
-(see make_golden_forcefield.py); nothing in __init__ touches OpenMM.  Build container only.
+(see make_golden_forcefield.py); nothing in __init__ touches OpenMM.  Needs MULTIMM_REFERENCE.
 
     python tests/golden/make_golden_model_init.py
 """

@@ -1,8 +1,8 @@
 """Generates tests/golden/structures_golden.npz and tests/golden/cif_*.txt by running the
 REFERENCE's own structure generators and file writers
-(/root/reference/src/multimm/initial_structure_tools.py: polymer_circle, helix_structure,
+($MULTIMM_REFERENCE/src/multimm/initial_structure_tools.py: polymer_circle, helix_structure,
 spiral_structure, sphere_surface_structure, trefoil_knot_structure, build_init_mmcif, write_mmcif,
-write_mmcif_chrom, generate_psf; utils.get_coordinates_cif).  Build container only; outputs are
+write_mmcif_chrom, generate_psf; utils.get_coordinates_cif).  Needs MULTIMM_REFERENCE; outputs are
 committed.  The module imports matplotlib, hilbertcurve, scipy.interpolate, tqdm and (through
 .utils) pyBigWig / openmm.unit at the top; none is used by the functions called here, the absent
 ones are stubbed.  The Hilbert curve itself cannot be generated (hilbertcurve is not installed):
@@ -19,7 +19,7 @@ import types
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference/src/multimm"
+REF = os.path.join(os.environ["MULTIMM_REFERENCE"], "src", "multimm")  # a checkout of the original MultiMM
 
 
 def load_reference():

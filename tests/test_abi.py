@@ -8,6 +8,7 @@ import subprocess
 import pytest
 
 from multimm_b200 import _lib
+from multimm_b200.build import cuda_tool
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "multimm_b200.h")
@@ -31,7 +32,7 @@ def test_library_exports_every_declared_symbol(built_lib):
 
 
 def test_library_is_sm100a_only_and_has_no_undefined_nccl_dependency(built_lib):
-    out = subprocess.run(["cuobjdump", "--list-elf", built_lib], capture_output=True, text=True).stdout
+    out = subprocess.run([cuda_tool("cuobjdump"), "--list-elf", built_lib], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
     # NCCL is opened with dlopen (single-GPU users and this CPU box need no libnccl at load time)
@@ -70,7 +71,7 @@ def test_pair_kernel_resources_allow_two_ctas_per_sm(built_lib):
     """The Newton-3 kernel is designed for two resident 256-thread CTAs per SM (DESIGN.md 4.1):
     <= 128 registers per thread, static shared memory within the 48 KB that needs no opt-in, and the
     hot variant on packed f32x2 arithmetic.  A change that silently breaks one of these costs ~2x."""
-    out = subprocess.run(["cuobjdump", "--dump-resource-usage", built_lib], capture_output=True, text=True).stdout
+    out = subprocess.run([cuda_tool("cuobjdump"), "--dump-resource-usage", built_lib], capture_output=True, text=True).stdout
     rows = re.findall(r"Function (\S*k_pair_n3\S*):\s*\n\s*REG:(\d+) STACK:(\d+) SHARED:(\d+)", out)
     assert len(rows) >= 16, len(rows)
     for name, reg, stack, shared in rows:
@@ -82,7 +83,7 @@ def test_pair_kernel_resources_allow_two_ctas_per_sm(built_lib):
         assert int(stack) <= 192, (name, stack)  # spilled words live in the rare variants' prologues, never in a pair loop
     gw = [n for n, *_ in rows if "k_pair_n3ILi6ELi1ELb1" in n]
     assert len(gw) == 1
-    sass = subprocess.run(["cuobjdump", "-sass", "-fun", gw[0], built_lib], capture_output=True, text=True).stdout
+    sass = subprocess.run([cuda_tool("cuobjdump"), "-sass", "-fun", gw[0], built_lib], capture_output=True, text=True).stdout
     assert sass.count("FFMA2") >= 100 and "FMUL2" in sass and "FADD2" in sass
     assert "REDG.E.ADD.64" in sass  # the 64-bit fixed-point force accumulation
     # no pair loop (a backward branch around >= 100 packed FMAs) touches local memory: spills stay outside

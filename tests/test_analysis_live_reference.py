@@ -1,6 +1,6 @@
 """Randomised differential test of the structure report against the REFERENCE's own
-analyze_structure (/root/reference/src/multimm/plots.py:630-829), run live: the report text must be
-identical.  Only where the reference checkout exists (the build container)."""
+analyze_structure ($MULTIMM_REFERENCE/src/multimm/plots.py:630-829), run live: the report text must be
+identical.  Only where the reference checkout exists (MULTIMM_REFERENCE)."""
 import importlib.util
 import os
 import sys
@@ -8,11 +8,11 @@ import sys
 import numpy as np
 import pytest
 
+from common import NO_REFERENCE, reference_file
 from multimm_b200 import analysis, structures
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.exists("/root/reference/src/multimm/plots.py"),
-                                reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(reference_file("src/multimm/plots.py") is None, reason=NO_REFERENCE)
 
 
 @pytest.fixture(scope="module")

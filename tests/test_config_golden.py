@@ -1,5 +1,5 @@
 """config.ini semantics against the REFERENCE's own config model, presets and cross-field checks
-(tests/golden/make_golden_config.py ran /root/reference/src/multimm/config.py and run.py): same
+(tests/golden/make_golden_config.py ran $MULTIMM_REFERENCE/src/multimm/config.py and run.py): same
 coercions, same defaults for every field the two models share, same MODELLING_LEVEL overrides,
 same accept / reject decisions."""
 import json
@@ -66,12 +66,21 @@ def test_same_outcome_as_the_reference(name):
     assert got == ref["checks"], (name, got, ref["checks"])
 
 
-def test_cli_precedence_matches_the_reference_get_config():
-    """defaults < ini (all sections, keys case-folded) < CLI, then the presets: run.py:349-395."""
-    argv = [a if not a.endswith("sample_config.ini") else a for a in GOLD["cli_argv"]]
+def test_cli_precedence_matches_the_reference_get_config(tmp_path):
+    """defaults < ini (all sections, keys case-folded) < CLI, then the presets: run.py:349-395.
+    get_config writes metadata/config_auto.ini under OUT_PATH, so the ini is run from a copy whose
+    OUT_PATH points into tmp_path; the reference kept the ini's OUT_PATH as written."""
+    ref_out = GOLD["cli_reference"]["OUT_PATH"]
+    text = open(os.path.join(ROOT, "tests", "golden", "sample_config.ini")).read()
+    assert f"OUT_PATH = {ref_out}\n" in text
+    ini = tmp_path / "sample_config.ini"
+    out = str(tmp_path / "out")
+    ini.write_text(text.replace(f"OUT_PATH = {ref_out}\n", f"OUT_PATH = {out}\n"))
+    argv = [str(ini) if a.endswith("sample_config.ini") else a for a in GOLD["cli_argv"]]
     args, _ = run.get_config(argv)
     ours = {k: plain(v) for k, v in args.model_dump().items()}
-    for field, want in GOLD["cli_reference"].items():
+    assert os.path.exists(os.path.join(out, "metadata", "config_auto.ini"))
+    for field, want in dict(GOLD["cli_reference"], OUT_PATH=out).items():
         if field not in DIFFERENT:
             assert same(want, ours[field]), (field, want, ours[field])
     assert ours["N_BEADS"] == 5000 and ours["EV_POWER"] == 5.0  # the region preset wins over the CLI's n_beads

@@ -1,9 +1,9 @@
 """Randomised differential test of the config model against the REFERENCE's own
-(/root/reference/src/multimm/config.py: SimulationConfig; run.py: ArgumentChanger, args_tests), run
+($MULTIMM_REFERENCE/src/multimm/config.py: SimulationConfig; run.py: ArgumentChanger, args_tests), run
 live: random subsets of fields given as the strings an ini file would hold (booleans in every
 accepted spelling, numbers, quantities with units, enum values, chromosome names, the occasional
 malformed value).  Same accept / reject decision at each stage, same field values before and after
-the MODELLING_LEVEL presets.  Only where the reference checkout exists (the build container)."""
+the MODELLING_LEVEL presets.  Only where the reference checkout exists (MULTIMM_REFERENCE)."""
 import importlib.util
 import os
 import sys
@@ -11,13 +11,13 @@ import sys
 import numpy as np
 import pytest
 
+from common import NO_REFERENCE, reference_file
 from multimm_b200 import run
 from multimm_b200.config import SimulationConfig
 from test_config_golden import DIFFERENT, plain, same
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.exists("/root/reference/src/multimm/config.py"),
-                                reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(reference_file("src/multimm/config.py") is None, reason=NO_REFERENCE)
 BEDPE = "tests/golden/synthetic_loops.bedpe"
 BED = "tests/golden/synthetic_subcompartments.bed"
 
@@ -105,8 +105,8 @@ def test_reference_example_inis_load_unmodified(name, tmp_path):
     the authors' absolute data paths are pointed at this repo's fixtures (they do not exist anywhere)."""
     from multimm_b200.model import resolve_platform
 
-    path = f"/root/reference/examples/{name}"
-    if not os.path.exists(path):
+    path = reference_file(f"examples/{name}")
+    if path is None:
         pytest.skip("example not shipped in this checkout")
     raw = run.read_ini(path)
     assert raw["PLATFORM"] == "OpenCL"

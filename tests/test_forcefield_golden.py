@@ -1,7 +1,7 @@
 """The force field against the REFERENCE's own builder.
 
 tests/golden/make_golden_forcefield.py executed the unmodified add_* methods of
-/root/reference/src/multimm/model.py against a recording stand-in for `openmm` and evaluated the
+$MULTIMM_REFERENCE/src/multimm/model.py against a recording stand-in for `openmm` and evaluated the
 Lepton strings, parameters and bond/angle lists they produced (FP64).  Here the same inputs go
 through THIS repo's chain — host mirror (multimm_b200/model.py) -> the calls it would make on the
 C-ABI -> CPU oracle — and every per-term energy must agree.  This pins, for every functional form:

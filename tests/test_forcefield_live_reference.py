@@ -1,11 +1,11 @@
 """Randomised differential test of the force-field builder against the REFERENCE's own add_*
-methods, run live (/root/reference/src/multimm/model.py:164-720 executed unmodified against the
+methods, run live ($MULTIMM_REFERENCE/src/multimm/model.py:164-720 executed unmodified against the
 recording `openmm` stand-in of tests/golden/make_golden_forcefield.py, their Lepton strings
 evaluated in FP64).  Every numeric config field that feeds a term is drawn at random, together with
 the functional forms, the geometry, the chromosome layout and the loops; this repo's chain (host
 mirror -> the calls it makes on the C-ABI -> CPU oracle) must give the same ten energies.  Only
-where the reference checkout exists (the build container); the frozen cases of
-test_forcefield_golden.py travel to the GPU box instead."""
+where the reference checkout exists (MULTIMM_REFERENCE); the frozen cases of
+test_forcefield_golden.py run everywhere."""
 import importlib.util
 import os
 import sys
@@ -13,13 +13,12 @@ import sys
 import numpy as np
 import pytest
 
-from common import O
+from common import NO_REFERENCE, O, reference_file
 from multimm_b200 import model
 from multimm_b200.config import SimulationConfig
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.exists("/root/reference/src/multimm/model.py"),
-                                reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(reference_file("src/multimm/model.py") is None, reason=NO_REFERENCE)
 
 FORMS = dict(EV_FORCE_TYPE=("powerlaw", "gaussian_core"), COB_FORCE_TYPE=("gaussian", "yukawa", "theta"),
              SCB_FORCE_TYPE=("gaussian", "yukawa", "theta"), CHB_FORCE_TYPE=("polynomial", "gaussian", "saturating"),

@@ -147,6 +147,27 @@ def test_determinism_and_newton(built_lib):
     eng.close()
 
 
+def test_last_result_reads_back_the_last_timed_evaluation(built_lib):
+    """bench.py --dump-outputs: what the last of evaluate_timed's evaluations computed, without another one."""
+    from multimm_b200.engine import Error
+
+    case = make_case(5000, n_chrom=4, seed=9)
+    eng = to_engine(case)
+    with pytest.raises(Error, match="no result to read"):
+        eng.last_result()
+    e0, f0 = eng.energy_forces()
+    eng.set_positions(case["x"] * 1.01)
+    eng.evaluate_timed(2, flush_l2=True)
+    e_t, f_t = eng.last_result()
+    e1, f1 = eng.energy_forces()
+    assert np.array_equal(e_t, e1) and np.array_equal(f_t, f1)
+    assert not np.array_equal(f_t, f0)
+    eng.minimize(tol=10.0, max_iter=3)  # the minimiser reuses the result buffers: nothing to read back
+    with pytest.raises(Error, match="no result to read"):
+        eng.last_result()
+    eng.close()
+
+
 @pytest.mark.parametrize("n,n_chrom,terms", [
     (700, 1, ("EV",)),
     (5000, 4, ("EV", "SCB", "CHB")),
@@ -293,12 +314,15 @@ def test_sharded_pair_work_is_bit_identical(built_lib, world):
     eng.close()
     eng = to_engine(case)
     eng.dist_emulate(world)
+    eng.evaluate_timed(2, flush_l2=False)
+    e_t, f_t = eng.last_result()  # what bench.py --dump-outputs writes when the pair work is sharded
     e2, f2 = eng.energy_forces()
     assert eng.pair_kernel_in_use == 2
     rep2 = eng.minimize(tol=10.0, max_iter=12)
     x2 = eng.get_positions()
     eng.close()
     assert np.array_equal(e1, e2) and np.array_equal(f1, f2)
+    assert np.array_equal(e1, e_t) and np.array_equal(f1, f_t)
     assert rep1["e_final"] == rep2["e_final"] and rep1["evaluations"] == rep2["evaluations"]
     assert np.array_equal(x1, x2)
 

@@ -1,18 +1,19 @@
 """Host loaders against golden outputs of the REFERENCE's own functions
 (tests/golden/loaders_golden.npz, produced by tests/golden/make_golden.py importing
-/root/reference/src/multimm/utils.py).  Integer arrays must match exactly."""
+$MULTIMM_REFERENCE/src/multimm/utils.py).  Integer arrays must match exactly."""
 import os
 
 import numpy as np
 import pytest
 
+from common import NO_REFERENCE, reference_file
 from multimm_b200 import loaders
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 G = np.load(os.path.join(GOLD, "loaders_golden.npz"))
 BEDPE = os.path.join(GOLD, "synthetic_loops.bedpe")
 BED = os.path.join(GOLD, "synthetic_subcompartments.bed")
-REF_FIXTURE = "/root/reference/tests/fixtures/ENCFF045MJY_simple.bedpe"
+REF_FIXTURE = reference_file("tests/fixtures/ENCFF045MJY_simple.bedpe")
 
 CASES = {
     "gw_20k": dict(N_beads=20000, chrom=None, coords=None, shuffle=False, seed=0),
@@ -61,7 +62,7 @@ def test_chrom_strength_table():
     assert loaders.CHROM_STRENGTH[0] == 0.0 and loaders.CHROM_STRENGTH[20] == 1.0  # chr1, chr21
 
 
-@pytest.mark.skipif(not os.path.exists(REF_FIXTURE), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(REF_FIXTURE is None, reason=NO_REFERENCE)
 @pytest.mark.parametrize("n_beads,chrom,coords", [(1000, None, None), (200000, None, None),
                                                   (10000, "chr1", [0, 248387328])])
 def test_reference_fixture(n_beads, chrom, coords):

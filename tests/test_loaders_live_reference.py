@@ -1,7 +1,7 @@
 """Randomised differential test of the host loaders against the REFERENCE's own functions, run live
-(/root/reference/src/multimm/utils.py: import_mns_from_bedpe :425, import_bed :220).  Only where the
-reference checkout exists (the build container); the frozen cases of test_loaders.py travel to the
-GPU box instead.  Integer outputs must be identical, distances equal to the last bit or two."""
+($MULTIMM_REFERENCE/src/multimm/utils.py: import_mns_from_bedpe :425, import_bed :220).  Only where the
+reference checkout exists (MULTIMM_REFERENCE); the frozen cases of test_loaders.py run
+everywhere.  Integer outputs must be identical, distances equal to the last bit or two."""
 import importlib.util
 import os
 import sys
@@ -9,11 +9,11 @@ import sys
 import numpy as np
 import pytest
 
+from common import NO_REFERENCE, reference_file
 from multimm_b200 import loaders, synthetic
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_UTILS = "/root/reference/src/multimm/utils.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_UTILS), reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(reference_file("src/multimm/utils.py") is None, reason=NO_REFERENCE)
 
 
 @pytest.fixture(scope="module")

@@ -1,7 +1,7 @@
 """Randomised differential test of MultiMM.__init__ (input ingestion, chromosome ends / ids /
-spins / strengths, gene window; /root/reference/src/multimm/model.py:24-162) against the
+spins / strengths, gene window; $MULTIMM_REFERENCE/src/multimm/model.py:24-162) against the
 REFERENCE's own __init__, run live on freshly drawn synthetic inputs.  Only where the reference
-checkout exists (the build container); the frozen cases of test_model_init_golden.py travel."""
+checkout exists (MULTIMM_REFERENCE); the frozen cases of test_model_init_golden.py run everywhere."""
 import importlib.util
 import os
 import sys
@@ -9,12 +9,12 @@ import sys
 import numpy as np
 import pytest
 
+from common import NO_REFERENCE, reference_file
 from multimm_b200 import loaders, model, synthetic
 from multimm_b200.config import SimulationConfig
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.exists("/root/reference/src/multimm/model.py"),
-                                reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(reference_file("src/multimm/model.py") is None, reason=NO_REFERENCE)
 GENES = ("gene_id\tgene_name\tchromosome\tstart\tend\nENSG01\tAAA\tchr1\t30000000\t30600000\n"
          "ENSG02\tBBB\tchr2\t50000000\t50090000\nENSG03\tCCC\tchr17\t7000000\t7020000\n")
 ATTRS = ("ms", "ns", "chr_ends", "chrom_idxs", "Cs", "chrom_spin", "gene_start", "gene_end")

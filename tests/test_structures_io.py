@@ -1,6 +1,6 @@
 """Structure generators and structure files against golden outputs of the REFERENCE's own code
 (tests/golden/make_golden_structures.py ran initial_structure_tools.py / utils.py from
-/root/reference): the .cif / .psf files are part of the contract (north star: "keeps ... structure
+$MULTIMM_REFERENCE): the .cif / .psf files are part of the contract (north star: "keeps ... structure
 outputs"), so the text must match byte for byte."""
 import os
 

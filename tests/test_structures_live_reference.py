@@ -1,8 +1,8 @@
 """Randomised differential test of the structure files and start curves against the REFERENCE's
-own writers and generators, run live (/root/reference/src/multimm/initial_structure_tools.py:
+own writers and generators, run live ($MULTIMM_REFERENCE/src/multimm/initial_structure_tools.py:
 build_init_mmcif, write_mmcif, write_mmcif_chrom, generate_psf, compute_init_struct;
 utils.get_coordinates_cif).  Text must match byte for byte.  Only where the reference checkout
-exists (the build container); the frozen files of test_structures_io.py travel to the GPU box."""
+exists (MULTIMM_REFERENCE); the frozen files of test_structures_io.py run everywhere."""
 import importlib.util
 import os
 import sys
@@ -10,11 +10,11 @@ import sys
 import numpy as np
 import pytest
 
+from common import NO_REFERENCE, reference_file
 from multimm_b200 import cif, structures
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.exists("/root/reference/src/multimm/initial_structure_tools.py"),
-                                reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(reference_file("src/multimm/initial_structure_tools.py") is None, reason=NO_REFERENCE)
 
 
 @pytest.fixture(scope="module")
