@@ -219,6 +219,30 @@ int mmm_mean_pair_distance(mmm_handle h, double *mean_out);
 int mmm_contact_map(int device, const double *xyz, int64_t n, int bins, int log_scale, double *map_out,
                     double *mean_dist_out);
 
+/* ---- contact frequencies (simulated Hi-C; not in the reference, whose genome-wide runs return before
+ * any contact analysis, model.py:1069-1213) ----------------------------------------------------------- */
+/* Contacts at the current positions: every unordered bead pair i < j with d2 < rc^2, where
+ * d2 = (dx*dx + dy*dy) + dz*dz (dx = x_i - x_j, ...) and rc^2 = rc*rc are evaluated in FP64 on the master
+ * positions, operation by operation without FMA contraction, so that any IEEE evaluation of the same
+ * expression in the same order agrees pair for pair.  Counts, all uint64 and exact:
+ *   map_out   (n_bins x n_bins, row-major; may be NULL): contacts between bins p and q of bin_of_bead
+ *             (int32[N], -1 = the bead is left out of the map); symmetric: an off-diagonal pair adds 1 to
+ *             (p, q) and to (q, p), a pair within one bin adds 1 to (p, p).  bin_of_bead may be NULL when
+ *             map_out is NULL;
+ *   sep_out   (uint64[N]; may be NULL): sep_out[s] = contacts with j - i = s whose beads carry the same
+ *             chromosome id (mmm_set_bead_params; NULL ids = one chromosome); sep_out[0] = 0;
+ *   pairs_out (may be NULL): all contacts, whatever their bins.
+ * 1 <= n_bins <= 4096 (a dense map of 128 MB).  MMM_ERR_ARG for rc <= 0 or not finite, n_bins outside
+ * that range, a bin id outside [-1, n_bins); MMM_ERR_STATE before positions are set.  Changes no state an
+ * evaluation, a minimisation or mmm_last_result reads; the scratch (bin table, map) is allocated on the
+ * first call, and again only when a larger map is asked for. */
+int mmm_contacts(mmm_handle h, double rc_nm, const int32_t *bin_of_bead, int32_t n_bins, uint64_t *map_out,
+                 uint64_t *sep_out, int64_t *pairs_out);
+/* Of the last mmm_contacts call: the bead pairs it tested in FP64 (those its box culling kept; contacts over
+ * candidates is its hit rate) and the device time of its kernels in ms (CUDA events on the handle's stream,
+ * from the FP32 copy to the last count; the copies of the results excluded).  Either output may be NULL. */
+int mmm_contacts_stats(mmm_handle h, int64_t *candidates_out, float *device_ms_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

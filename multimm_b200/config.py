@@ -20,7 +20,7 @@ import os
 from enum import Enum
 from typing import Any, Optional
 
-from pydantic import BaseModel, BeforeValidator, WithJsonSchema, create_model, model_validator
+from pydantic import BaseModel, BeforeValidator, TypeAdapter, WithJsonSchema, create_model, model_validator
 from typing_extensions import Annotated
 
 from .units import Quantity, parse_quantity
@@ -181,6 +181,23 @@ _FIELDS: dict[str, tuple[Any, Any]] = {
     "MIN_MAX_ITERATIONS": (int, 0),       # 0 = until converged (OpenMM default)
 }
 
+# Contact-map settings (multimm_b200.contacts; not in the reference).  They are accepted from the ini and
+# the command line like the fields above and validated the same way, but kept as model extras that exist
+# only when given: a config without them has exactly the reference's field set plus the engine knobs above,
+# and dumps (config_auto.ini, parameters.txt) exactly as before.  Read them with contact_setting().
+CONTACT_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_CONTACTS": (B, False),          # count contacts of the minimised structure (analysis/contacts.npz; ensembles: ensemble_contacts.npz)
+    "CONTACT_RADIUS": (float, 0.2),       # nm; a bead pair closer than this is a contact (2 x the default bond length)
+    "CONTACT_RESOLUTION": (int, 0),       # bp per bin of the contact map; 0 = about 1000 bins over the modelled genome or region
+}
+_CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in CONTACT_FIELDS.items()}
+
+
+def contact_setting(args, name: str):
+    """Value of a CONTACT_FIELDS setting of `args`, its default where it was not given."""
+    extra = getattr(args, "__pydantic_extra__", None) or {}
+    return extra.get(name, CONTACT_FIELDS[name][1])
+
 
 class _Base(BaseModel):
     model_config = {
@@ -188,6 +205,7 @@ class _Base(BaseModel):
         "populate_by_name": True,
         "validate_assignment": True,
         "validate_default": True,
+        "extra": "allow",  # for CONTACT_FIELDS only: every other unknown key is dropped in _blank_to_none
     }
 
     @model_validator(mode="before")
@@ -199,6 +217,12 @@ class _Base(BaseModel):
             return data
         out = {}
         for key, val in data.items():
+            if key in CONTACT_FIELDS:
+                if val is not None:  # given: validated like a field (ValueError -> ValidationError)
+                    out[key] = _CONTACT_ADAPTERS[key].validate_python(val)
+                continue
+            if key not in _FIELDS:  # unknown keys are ignored, as pydantic's default does
+                continue
             if isinstance(val, str) and val.strip().lower() in ("", "none"):
                 ftype = _FIELDS.get(key, (str, None))[0]
                 nullable = type(None) in getattr(ftype, "__args__", ()) or ftype is Chrom

@@ -244,6 +244,17 @@ struct mmm_system {
   void* d_flush = nullptr;           // 256 MiB L2-flush scratch (bench only)
   double* d_fout = nullptr;          // [3n] forces (= -gradient) staged for mmm_energy_forces' host copy
   float last_pair_ms = 0.f;
+
+  // contact counting (mmm_contacts.cu): scratch kept for the handle's lifetime
+  int* d_ct_bin = nullptr;                 // [n] bin of every bead
+  unsigned long long* d_ct_map = nullptr;  // [ct_map_cap] dense bin x bin counts
+  size_t ct_map_cap = 0;
+  unsigned long long* d_ct_sep = nullptr;  // [n] same-chromosome contacts by index separation
+  TileInfo* d_ct_stage = nullptr;          // [stages] boxes of the chain-order 256-bead stages
+  unsigned long long* d_ct_cnt = nullptr;  // [2] contacts, candidate pairs tested
+  int64_t ct_candidates = 0;               // candidate pairs the last call tested in FP64
+  float ct_ms = 0.f;                       // device time of the last call's kernels (events below)
+  cudaEvent_t ct_ev0 = nullptr, ct_ev1 = nullptr;
 };
 
 // ---------------------------------------------------------------------------------------
@@ -289,6 +300,8 @@ int mmm_launch_chb_clusters(mmm_system* h, const int* d_skip);
 // mmm_cells.cu
 int mmm_launch_pair_cutoff(mmm_system* h, const int* d_skip);
 int64_t mmm_cells_energy_slots(const mmm_system* h);
+// mmm_contacts.cu
+void mmm_contacts_free(mmm_system* h);
 // mmm_bonded.cu
 int mmm_upload_topology(mmm_system* h);
 int mmm_upload_angles(mmm_system* h, const int32_t* ai, const int32_t* aj, const int32_t* ak,

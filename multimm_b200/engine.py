@@ -178,6 +178,30 @@ class Engine:
         self._ck(self._lib.mmm_mean_pair_distance(self._h, C.byref(out)))
         return float(out.value)
 
+    def contacts(self, rc_nm: float, bin_of_bead=None, n_bins: int = 1, want_sep: bool = True):
+        """Contacts (FP64 d2 < rc^2, see mmm_contacts) at the current positions, counted on the device.
+        Returns (map, sep, pairs): map (n_bins, n_bins) uint64, symmetric, of the contacts between the bins
+        of ``bin_of_bead`` (int[N], -1 = left out), or None without ``bin_of_bead``; sep (N,) uint64,
+        same-chromosome contacts by index separation j - i, or None if not ``want_sep``; pairs, all contacts."""
+        n_bins = int(n_bins)
+        bins = None
+        if bin_of_bead is not None:
+            bins = _arr(bin_of_bead, np.int32)
+            if bins.shape != (self.n,):
+                raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        cmap = np.empty((n_bins, n_bins), dtype=np.uint64) if bins is not None and 1 <= n_bins <= 4096 else None
+        sep = np.empty(self.n, dtype=np.uint64) if want_sep else None
+        pairs = C.c_int64()
+        self._ck(self._lib.mmm_contacts(self._h, float(rc_nm), _p(bins), n_bins, _p(cmap), _p(sep), C.byref(pairs)))
+        return cmap, sep, int(pairs.value)
+
+    def contacts_stats(self) -> dict:
+        """Of the last contacts() call: bead pairs tested in FP64 (those that survived box culling) and the
+        device time of its kernels in ms (CUDA events on the engine's stream)."""
+        cand, ms = C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_contacts_stats(self._h, C.byref(cand), C.byref(ms)))
+        return dict(candidates=int(cand.value), device_ms=float(ms.value))
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

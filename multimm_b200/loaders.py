@@ -128,8 +128,14 @@ def import_bed(bed_file, N_beads, coords=None, chrom=None, save_path="", shuffle
 
 
 def import_mns_from_bedpe(bedpe_file, N_beads, coords=None, chrom=None, threshold=0, min_loop_dist=2, path="",
-                          down_prob=1.0, shuffle=False, seed=0, n_chroms=22):
-    """Loop track -> (ms int[L], ns int[L], ds float[L], chr_ends int[C+1], chrom_idxs int[C])."""
+                          down_prob=1.0, shuffle=False, seed=0, n_chroms=22, layout=None):
+    """Loop track -> (ms int[L], ns int[L], ds float[L], chr_ends int[C+1], chrom_idxs int[C]).
+
+    ``layout``: an optional dict that receives the bead-to-genome mapping this call used (it changes
+    neither the return value nor the draws from numpy's random stream): ``resolution`` (bp per bead),
+    ``ends`` (bp offset of every block in the concatenated coordinate), ``chr_ends``, ``chrom_idxs`` and
+    ``start_bp`` / ``stop_bp`` (the modelled region, or 0 / None genome-wide).  Bead i of block k then sits
+    at bp ``start_bp + i * resolution + resolution // 2 - ends[k]`` of chromosome ``chrom_idxs[k]``."""
     np.random.seed(seed)
     df = pd.read_csv(bedpe_file, header=None, sep="\t")
     idxs, ends = _chrom_layout(chrom, shuffle, n_chroms)
@@ -187,6 +193,10 @@ def import_mns_from_bedpe(bedpe_file, N_beads, coords=None, chrom=None, threshol
             np.save(os.path.join(meta, "ns.npy"), ns)
             np.save(os.path.join(meta, "ds.npy"), ds)
     logger.info(f"Number of loops is {len(ms)}")
+    if layout is not None:
+        layout.update(resolution=int(resolution), ends=ends.astype(np.int64), chr_ends=chr_ends.astype(np.int64),
+                      chrom_idxs=idxs.astype(np.int64), start_bp=int(coords[0]) if chrom is not None else 0,
+                      stop_bp=int(coords[1]) if chrom is not None else None)
     return ms.astype(int), ns.astype(int), ds, chr_ends.astype(int), idxs.astype(int)
 
 

@@ -19,6 +19,7 @@ import time
 import numpy as np
 
 from . import _lib, analysis, cif, loaders, structures
+from .config import contact_setting
 from .engine import Engine
 from .units import Quantity
 
@@ -118,10 +119,15 @@ class MultiMM:
                 flip_prob=args.COMPARTMENT_FLIP_PROB, noise_strength=args.COMPARTMENT_NOISE_STD)
         if not str(args.LOOPS_PATH).lower().endswith(".bedpe"):
             raise ValueError("You did not provide appropriate loop file. Loop .bedpe file is obligatory.")
-        # chr_ends / chrom_idxs of the bed loader are overwritten here (appendix A, Q4)
+        # chr_ends / chrom_idxs of the bed loader are overwritten here (appendix A, Q4); the loop loader's
+        # bead-to-genome mapping is what places beads in genomic coordinates (contacts.genome_bins)
+        self.layout = {}
         self.ms, self.ns, self.ds, self.chr_ends, self.chrom_idxs = loaders.import_mns_from_bedpe(
             bedpe_file=args.LOOPS_PATH, N_beads=args.N_BEADS, coords=coords, chrom=chrom, path=self.save_path,
-            shuffle=args.SHUFFLE_CHROMS, seed=args.SHUFFLING_SEED, down_prob=args.DOWNSAMPLING_PROB)
+            shuffle=args.SHUFFLE_CHROMS, seed=args.SHUFFLING_SEED, down_prob=args.DOWNSAMPLING_PROB,
+            layout=self.layout)
+        self.contacts = None        # counts of the minimised structure (SAVE_CONTACTS)
+        self.contacts_file = None   # where finish() writes them; the ensemble driver points it outside run_<i>
 
         # chrom_spin: chromosome id per bead; chrom_strength: indexed by POSITION in the (possibly
         # shuffled) order, not by chromosome id (model.py:158-162; appendix A, Q8)
@@ -443,8 +449,23 @@ class MultiMM:
     def compute(self):
         """The GPU-bound stage: minimisation, MD relaxation if configured.  No structure files except MD's."""
         self.min_energy(write_files=False)
+        if contact_setting(self.args, "SAVE_CONTACTS"):
+            self.count_contacts()
         if self.args.SIM_RUN_MD:
             self.run_md()
+
+    def count_contacts(self):
+        """Contacts of the minimised structure (SAVE_CONTACTS), counted by this member's own engine at the
+        positions the minimisation left on the device, binned in canonical genomic coordinates."""
+        from . import contacts
+
+        t0 = time.time()
+        a = self.args
+        gb = contacts.genome_bins(self.layout, int(contact_setting(a, "CONTACT_RESOLUTION")), n_beads=a.N_BEADS)
+        rc = float(contact_setting(a, "CONTACT_RADIUS"))
+        cmap, sep, pairs = self.engine.contacts(rc, gb.bins, gb.n_bins)
+        self.contacts = contacts.result(cmap, sep, pairs, rc, gb, contacts.sep_pairs(self.chrom_spin))
+        self.timings["contacts_s"] = time.time() - t0
 
     def finish(self):
         """Structure files, per-chromosome files, reports, parameters.  Host work (the report's device
@@ -454,6 +475,13 @@ class MultiMM:
             self.save_chromosomes()  # the minimised structure, as model.py:1222-1224 (before MD)
         if self.args.SAVE_PLOTS:
             self.make_reports()
+        if self.contacts is not None:
+            from . import contacts
+
+            if self.contacts_file is None:
+                contacts.save_dense(os.path.join(self.save_path, "analysis", "contacts.npz"), self.contacts)
+            else:
+                contacts.save_member(self.contacts_file, self.contacts)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

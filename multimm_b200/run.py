@@ -56,7 +56,7 @@ def _early_cuda_start():
 _WARMUP = _early_cuda_start()
 
 from . import loaders  # noqa: E402
-from .config import SimulationConfig  # noqa: E402
+from .config import CONTACT_FIELDS, SimulationConfig, contact_setting  # noqa: E402
 from .units import Quantity  # noqa: E402
 
 logger = logging.getLogger("multimm_b200")
@@ -199,6 +199,36 @@ def args_tests(args):
         # that asks for one this engine does not have must not run a whole minimisation first
         raise ValueError(f"SIM_INTEGRATOR_TYPE={args.SIM_INTEGRATOR_TYPE!r} is not available "
                          f"(supported: {', '.join(_lib.MD_INTEGRATORS)})")
+    check_contact_fields(args)
+
+
+def check_contact_fields(args):
+    """CONTACT_RADIUS finite and > 0; CONTACT_RESOLUTION >= 0 and, where the modelled stretch is known from
+    the config alone (not for gene-level runs), at most contacts.MAX_BINS bins."""
+    import math
+
+    from . import contacts
+
+    rc = float(contact_setting(args, "CONTACT_RADIUS"))
+    if not (math.isfinite(rc) and rc > 0.0):
+        raise ValueError(f"CONTACT_RADIUS={rc!r} must be a finite distance > 0 (nm)")
+    res = int(contact_setting(args, "CONTACT_RESOLUTION"))
+    if res < 0:
+        raise ValueError(f"CONTACT_RESOLUTION={res} must be >= 0 (0 = automatic)")
+    if res == 0 or str(args.MODELLING_LEVEL or "").lower() == "gene":
+        return
+    if args.CHROM is None:
+        sp = contacts.spans(range(22))
+    elif args.LOC_START is not None and args.LOC_END is not None:
+        sp = contacts.spans([loaders._chrom_index(args.CHROM)], int(args.LOC_START), int(args.LOC_END))
+    elif args.CHROM in loaders.CHROM_SIZES:
+        sp = contacts.spans([loaders._chrom_index(args.CHROM)], 0, loaders.CHROM_SIZES[args.CHROM])
+    else:
+        return
+    nb = contacts.bin_count(sp, res)
+    if nb > contacts.MAX_BINS:
+        raise ValueError(f"CONTACT_RESOLUTION={res} bp gives {nb} contact-map bins; at most {contacts.MAX_BINS} "
+                         "are supported (0 = automatic)")
 
 
 def read_ini(path: str) -> dict:
@@ -220,7 +250,7 @@ def get_config(argv=None):
     ap.add_argument("-c", "--config_file", metavar="FILE", help="config file (ini format)")
     ap.add_argument("--gpus", default=None, help="comma-separated CUDA device indices for ensemble workers "
                                                  "(default: DEVICE, or every visible GPU for ensembles)")
-    for name in SimulationConfig.model_fields:
+    for name in (*SimulationConfig.model_fields, *CONTACT_FIELDS):
         ap.add_argument(f"--{name.lower()}")
     ns = vars(ap.parse_args(argv))
     raw = read_ini(ns["config_file"]) if ns.get("config_file") else {}
@@ -333,8 +363,31 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     os.makedirs(run_path, exist_ok=True)
     t0 = time.time()
     md = MultiMM(cfg, device=device)
+    # outside run_<i>, so that archiving does not take it away; summed by run_ensemble
+    md.contacts_file = member_contacts_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
+
+
+def member_contacts_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "contacts", f"member_{i}.npz")
+
+
+def write_ensemble_contacts(args, results: list[dict]) -> str | None:
+    """SAVE_CONTACTS: OUT_PATH/ensemble_contacts.npz, the sum of the contact files of the members that
+    succeeded (exact integer sums: the same bits whichever GPU ran which member)."""
+    if not contact_setting(args, "SAVE_CONTACTS") or not results:
+        return None
+    from . import contacts
+
+    paths = [member_contacts_path(args.OUT_PATH, r["replica"]) for r in sorted(results, key=lambda r: r["replica"])]
+    agg = contacts.aggregate(paths)
+    out = os.path.join(args.OUT_PATH, "ensemble_contacts.npz")
+    contacts.save_dense(out, agg)
+    logger.info(f"ensemble contacts: {int(agg['members'])} members, {agg['counts'].shape[0]} bins at "
+                f"{int(agg['resolution_bp'])} bp, {int(agg['pairs'])} contacts (rc = {float(agg['radius_nm'])} nm) "
+                f"-> {out}")
+    return out
 
 
 def prepare_replica(params: dict, i: int, run_path: str, device: int):
@@ -535,9 +588,10 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         got = []
         run_replicas_on_device(params, paths, list(range(n)), devices[0], archive, got.append)
         errors = [p for kind, p in got if kind != "ok"]
+        results = [p for kind, p in got if kind == "ok"]
+        write_ensemble_contacts(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
-        results = [p for kind, p in got if kind == "ok"]
         check_archives(results)
         return results
     ctx = mp.get_context("spawn")  # CUDA contexts must not be forked
@@ -571,6 +625,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
             if p.is_alive():
                 p.terminate()  # exact processes we started
                 p.join()
+    write_ensemble_contacts(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
