@@ -238,9 +238,32 @@ int mmm_contact_map(int device, const double *xyz, int64_t n, int bins, int log_
  * first call, and again only when a larger map is asked for. */
 int mmm_contacts(mmm_handle h, double rc_nm, const int32_t *bin_of_bead, int32_t n_bins, uint64_t *map_out,
                  uint64_t *sep_out, int64_t *pairs_out);
-/* Of the last mmm_contacts call: the bead pairs it tested in FP64 (those its box culling kept; contacts over
- * candidates is its hit rate) and the device time of its kernels in ms (CUDA events on the handle's stream,
- * from the FP32 copy to the last count; the copies of the results excluded).  Either output may be NULL. */
+/* Sparse contact map at the current positions (model.py:1069-1213 has only the dense heat map): the same
+ * contact test as mmm_contacts, over the same culled candidates; bins int32, any count (1 <= n_bins <=
+ * 2^31 - 1).  The entry (p, q), p <= q, counts the contacts with one bead in bin p and the other in bin q;
+ * a pair inside one bin adds 1 to (p, p) once; beads with bin -1 are left out.  So the dense map of
+ * mmm_contacts at the same positions and bins has M[p, q] = M[q, p] = v.  n_entries_out: the number of
+ * nonzero entries; pairs_out: all contacts, whatever their bins (either may be NULL).  The entries stay on
+ * the device for mmm_contacts_sparse_read; they are built there as the key p * n_bins + q of every binned
+ * contact, radix-sorted and run-length reduced, so they are bit-identical however the work is scheduled.
+ * MMM_ERR_ARG for rc <= 0 or not finite, n_bins < 1, bin_of_bead NULL or a bin id outside [-1, n_bins);
+ * MMM_ERR_STATE before positions are set.  Changes no state an evaluation, a minimisation or
+ * mmm_last_result reads.  Scratch: 16 B per binned contact plus 0.5 B per binned contact of sort table
+ * and O(N), allocated on the first call and again only when a call has more binned contacts than any
+ * before it. */
+int mmm_contacts_sparse(mmm_handle h, double rc_nm, const int32_t *bin_of_bead, int32_t n_bins,
+                        int64_t *n_entries_out, int64_t *pairs_out);
+/* The entries of the last mmm_contacts_sparse call, sorted by (row, col), row <= col, vals > 0:
+ * rows_out, cols_out int32[n_entries], vals_out uint64[n_entries]; any may be NULL, and n_entries = 0
+ * succeeds.  Rows and cols are split from the keys on the device.  May be called again; MMM_ERR_STATE
+ * before any successful mmm_contacts_sparse call. */
+int mmm_contacts_sparse_read(mmm_handle h, int32_t *rows_out, int32_t *cols_out, uint64_t *vals_out);
+/* Of the last mmm_contacts or mmm_contacts_sparse call, whichever ran last: the bead pairs it tested in
+ * FP64 (those its box culling kept; contacts over candidates is its hit rate; the sparse call tests them
+ * twice, counting then writing keys, and reports them once) and the device time of its kernels in ms (CUDA
+ * events on the handle's stream, from the FP32 copy to the last count, the sparse call's sort and run
+ * count included; the copies of the results and mmm_contacts_sparse_read excluded).  Either output may
+ * be NULL. */
 int mmm_contacts_stats(mmm_handle h, int64_t *candidates_out, float *device_ms_out);
 
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */

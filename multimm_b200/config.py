@@ -190,13 +190,18 @@ CONTACT_FIELDS: dict[str, tuple[Any, Any]] = {
     "CONTACT_RADIUS": (float, 0.2),       # nm; a bead pair closer than this is a contact (2 x the default bond length)
     "CONTACT_RESOLUTION": (int, 0),       # bp per bin of the contact map; 0 = about 1000 bins over the modelled genome or region
 }
-_CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in CONTACT_FIELDS.items()}
+# The fine (sparse) contact map, kept the same way; effective only with SAVE_CONTACTS.
+CONTACT_FINE_FIELDS: dict[str, tuple[Any, Any]] = {
+    "CONTACT_FINE_RESOLUTION": (int, 0),  # bp per bin of the sparse map (contacts_fine.npz); 0 = off
+}
+EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS}
+_CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
-    """Value of a CONTACT_FIELDS setting of `args`, its default where it was not given."""
+    """Value of a CONTACT_FIELDS or CONTACT_FINE_FIELDS setting of `args`, its default where it was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
-    return extra.get(name, CONTACT_FIELDS[name][1])
+    return extra.get(name, EXTRA_FIELDS[name][1])
 
 
 class _Base(BaseModel):
@@ -205,7 +210,7 @@ class _Base(BaseModel):
         "populate_by_name": True,
         "validate_assignment": True,
         "validate_default": True,
-        "extra": "allow",  # for CONTACT_FIELDS only: every other unknown key is dropped in _blank_to_none
+        "extra": "allow",  # for EXTRA_FIELDS only: every other unknown key is dropped in _blank_to_none
     }
 
     @model_validator(mode="before")
@@ -217,7 +222,7 @@ class _Base(BaseModel):
             return data
         out = {}
         for key, val in data.items():
-            if key in CONTACT_FIELDS:
+            if key in EXTRA_FIELDS:
                 if val is not None:  # given: validated like a field (ValueError -> ValidationError)
                     out[key] = _CONTACT_ADAPTERS[key].validate_python(val)
                 continue

@@ -14,7 +14,13 @@ Files (numpy ``.npz``):
   P(s) = sep_contacts / sep_pairs), ``pairs`` (all contacts);
 * ``contacts/member_<i>.npz`` of an ensemble member: the same, with the map as the sparse upper triangle
   (``rows``, ``cols``, ``vals``) and ``n_bins``.  Integer sums do not depend on order, so the ensemble file
-  is the same bit for bit whichever GPU ran which member.
+  is the same bit for bit whichever GPU ran which member;
+* the fine map (``CONTACT_FINE_RESOLUTION``, ``Engine.contacts_sparse``): ``analysis/contacts_fine.npz`` of a
+  single run, ``contacts/member_<i>_fine.npz`` of an ensemble member and ``ensemble_contacts_fine.npz`` of an
+  ensemble.  Always sparse, never a dense ``counts`` (a 5 kb genome-wide map has ~6e5 bins): ``rows``,
+  ``cols`` (int32), ``vals`` (uint64), the nonzero upper triangle sorted by (row, col) with rows <= cols;
+  ``n_bins``, ``bin_chrom``, ``bin_start_bp``, ``resolution_bp``, ``radius_nm``, ``members``, ``pairs``.
+  Read it with ``load_fine``; ``coarsen`` and ``fine_block`` give dense views of it.
 """
 from __future__ import annotations
 
@@ -26,6 +32,9 @@ import numpy as np
 from . import loaders
 
 MAX_BINS = 4096     # dense map cap of mmm_contacts (128 MB of uint64)
+MAX_FINE_BINS = 2**31 - 1  # sparse map (mmm_contacts_sparse): bins are int32
+FINE_KEYS = ("rows", "cols", "vals", "n_bins", "bin_chrom", "bin_start_bp", "resolution_bp", "radius_nm",
+             "members", "pairs")
 AUTO_BINS = 1000    # CONTACT_RESOLUTION = 0: about this many bins over the modelled genome or region
 
 
@@ -63,16 +72,18 @@ def bin_count(sp, resolution_bp: int) -> int:
     return int(sum(-(-(hi - lo) // resolution_bp) for _, lo, hi in sp))
 
 
-def genome_bins(layout: dict, resolution_bp: int = 0, n_beads: int | None = None) -> GenomeBins:
+def genome_bins(layout: dict, resolution_bp: int = 0, n_beads: int | None = None,
+                max_bins: int = MAX_BINS) -> GenomeBins:
     """Canonical bin of every bead of a run whose bead-to-genome mapping is ``layout`` (what
     loaders.import_mns_from_bedpe fills; MultiMM.layout).  Bead i of block k sits at bp
     ``start_bp + i * res + res // 2 - ends[k]`` of chromosome ``chrom_idxs[k]``, clamped to the modelled
-    stretch of that chromosome.  resolution_bp 0: automatic (auto_resolution).  ValueError beyond MAX_BINS."""
+    stretch of that chromosome.  resolution_bp 0: automatic (auto_resolution).  ValueError beyond max_bins
+    (MAX_BINS for the dense map, MAX_FINE_BINS for the sparse one)."""
     sp = spans(layout["chrom_idxs"], int(layout.get("start_bp", 0)), layout.get("stop_bp"))
     r = int(resolution_bp) if resolution_bp and resolution_bp > 0 else auto_resolution(sp)
     nb = bin_count(sp, r)
-    if nb > MAX_BINS:
-        raise ValueError(f"CONTACT_RESOLUTION={r} bp gives {nb} bins; at most {MAX_BINS} are supported")
+    if nb > max_bins:
+        raise ValueError(f"CONTACT_RESOLUTION={r} bp gives {nb} bins; at most {max_bins} are supported")
     first = np.zeros(len(loaders.CHROM_LENGTHS), np.int64)
     lo_of = np.zeros(len(loaders.CHROM_LENGTHS), np.int64)
     bin_chrom, bin_start = [], []
@@ -155,9 +166,11 @@ def save_member(path: str, d: dict):
 
 
 def load(path: str) -> dict:
-    """A contacts file of any kind, with the map dense."""
+    """A dense or member contacts file, with the map dense.  ValueError for a fine file (load_fine)."""
     with np.load(path) as z:
         d = {k: z[k] for k in z.files}
+    if "sep_contacts" not in d:
+        raise ValueError(f"{path} is a fine (sparse) contacts file; read it with contacts.load_fine")
     if "counts" not in d:
         b = int(d.pop("n_bins"))
         rows, cols, vals = d.pop("rows"), d.pop("cols"), d.pop("vals")
@@ -188,6 +201,110 @@ def aggregate(paths) -> dict:
         acc["members"] = np.int64(acc["members"] + int(d.get("members", 1)))
         acc["pairs"] = np.int64(acc["pairs"] + int(d["pairs"]))
     return acc
+
+
+def fine_result(rows, cols, vals, pairs, radius_nm, gb: GenomeBins, members: int = 1) -> dict:
+    """The in-memory form of a fine contacts file (what Engine.contacts_sparse returns, with its bins)."""
+    return dict(rows=np.asarray(rows, np.int32), cols=np.asarray(cols, np.int32), vals=np.asarray(vals, np.uint64),
+                n_bins=np.int64(gb.n_bins), bin_chrom=np.asarray(gb.bin_chrom, np.int32),
+                bin_start_bp=np.asarray(gb.bin_start_bp, np.int64), resolution_bp=np.int64(gb.resolution_bp),
+                radius_nm=np.float64(radius_nm), members=np.int64(members), pairs=np.int64(pairs))
+
+
+def save_fine(path: str, d: dict):
+    _write(path, {k: d[k] for k in FINE_KEYS})
+
+
+def load_fine(path: str) -> dict:
+    """A fine contacts file, sparse as stored."""
+    with np.load(path) as z:
+        if "rows" not in z.files or "sep_contacts" in z.files:
+            raise ValueError(f"{path} is not a fine contacts file")
+        return {k: z[k] for k in FINE_KEYS}
+
+
+def _merge(rows, cols, vals, r2, c2, v2, n_bins: int):
+    """Sum of two sorted sparse upper triangles, sorted (exact uint64; merged, never densified)."""
+    k1 = rows.astype(np.int64) * n_bins + cols
+    k2 = r2.astype(np.int64) * n_bins + c2
+    keys = np.concatenate([k1, k2])
+    v = np.concatenate([vals, v2])
+    order = np.argsort(keys, kind="stable")
+    keys, v = keys[order], v[order]
+    head = np.ones(len(keys), bool)
+    head[1:] = keys[1:] != keys[:-1]
+    starts = np.flatnonzero(head)
+    out_v = np.add.reduceat(v, starts) if len(starts) else v[:0]
+    k = keys[starts]
+    return (k // n_bins).astype(np.int32), (k % n_bins).astype(np.int32), out_v.astype(np.uint64)
+
+
+def aggregate_fine(paths) -> dict:
+    """Sum of fine member files: exact uint64, the same bytes in any member order (sorted merge of sparse
+    entries); the bins, radius and resolution must agree."""
+    paths = list(paths)
+    if not paths:
+        raise ValueError("no fine contact files to aggregate")
+    acc = None
+    for p in paths:
+        d = load_fine(p)
+        if acc is None:
+            acc = dict(d)
+            continue
+        for k in ("n_bins", "bin_chrom", "bin_start_bp", "radius_nm", "resolution_bp"):
+            if not np.array_equal(acc[k], d[k]):
+                raise ValueError(f"{p}: {k} differs from the other members")
+        acc["rows"], acc["cols"], acc["vals"] = _merge(acc["rows"], acc["cols"], acc["vals"], d["rows"], d["cols"],
+                                                       d["vals"], int(acc["n_bins"]))
+        acc["members"] = np.int64(acc["members"] + int(d["members"]))
+        acc["pairs"] = np.int64(acc["pairs"] + int(d["pairs"]))
+    return acc
+
+
+def coarsen(fine: dict, resolution_bp: int) -> np.ndarray:
+    """Dense symmetric uint64 map of a fine map at ``resolution_bp``, a multiple of its resolution giving at
+    most MAX_BINS bins.  Both grids start at each chromosome's ``lo``, so coarse bin = fine bin // k within
+    a chromosome and the sums are exact; the coarse grid is what genome_bins makes at resolution_bp."""
+    r = int(fine["resolution_bp"])
+    if resolution_bp <= 0 or resolution_bp % r:
+        raise ValueError(f"resolution_bp={resolution_bp} is not a multiple of the fine resolution {r} bp")
+    k = resolution_bp // r
+    chrom = np.asarray(fine["bin_chrom"])
+    starts = np.flatnonzero(np.concatenate([[True], chrom[1:] != chrom[:-1]]))  # a chromosome's bins are contiguous
+    ends = np.append(starts[1:], len(chrom))
+    cmap = np.empty(len(chrom), np.int64)
+    nb = 0
+    for a, b in zip(starts, ends):
+        cmap[a:b] = nb + np.arange(b - a) // k
+        nb += -(-(b - a) // k)
+    if nb > MAX_BINS:
+        raise ValueError(f"resolution_bp={resolution_bp} gives {nb} bins; at most {MAX_BINS} are supported")
+    out = np.zeros((nb, nb), np.uint64)
+    p, q = cmap[fine["rows"]], cmap[fine["cols"]]
+    vals = np.asarray(fine["vals"], np.uint64)
+    np.add.at(out, (p, q), vals)
+    off = p != q
+    np.add.at(out, (q[off], p[off]), vals[off])
+    return out
+
+
+def fine_block(fine: dict, chrom: str | int, start_bp: int, end_bp: int) -> tuple[np.ndarray, np.ndarray]:
+    """(counts, bin_start_bp): the dense symmetric uint64 sub-matrix of the fine map over the bins of
+    chromosome ``chrom`` (name or CHROM_NAMES index) that overlap [start_bp, end_bp), and their first bps."""
+    c = {v: i for i, v in loaders.CHROM_NAMES.items()}[chrom] if isinstance(chrom, str) else int(chrom)
+    r = int(fine["resolution_bp"])
+    start = np.asarray(fine["bin_start_bp"], np.int64)
+    sel = np.flatnonzero((np.asarray(fine["bin_chrom"]) == c) & (start < end_bp) & (start + r > start_bp))
+    if len(sel) == 0:
+        return np.zeros((0, 0), np.uint64), start[:0]
+    lo, hi = int(sel[0]), int(sel[-1]) + 1   # a chromosome's bins are contiguous
+    rows, cols = np.asarray(fine["rows"]), np.asarray(fine["cols"])
+    m = (rows >= lo) & (rows < hi) & (cols >= lo) & (cols < hi)
+    p, q, v = rows[m] - lo, cols[m] - lo, np.asarray(fine["vals"], np.uint64)[m]
+    out = np.zeros((hi - lo, hi - lo), np.uint64)
+    out[p, q] = v
+    out[q, p] = v
+    return out, start[lo:hi]
 
 
 def contact_counts(V, rc_nm: float, bins=None, n_bins: int = 1, chrom=None, device: int = 0):

@@ -2,9 +2,11 @@
 //   every unordered bead pair i < j with d2 < rc^2, decided in FP64 on the master positions d_x with
 //   d2 = (dx*dx + dy*dy) + dz*dz rounded operation by operation (no FMA contraction), so that a numpy
 //   evaluation of the same expression gives the same verdict for every pair, the boundary included.
-// Contacts are counted three ways with integer atomics (bit-identical however the work is scheduled):
+// mmm_contacts counts them three ways with integer atomics (bit-identical however the work is scheduled):
 // per (bin_i, bin_j) in a dense symmetric map, per index separation j - i for same-chromosome pairs
-// (P(s)), and in total.
+// (P(s)), and in total.  mmm_contacts_sparse stores the map sparse, for any int32 number of bins: the
+// same kernel (k_contacts, sink kKeys) writes the key p * n_bins + q (p <= q) of every binned contact,
+// an LSD radix sort over the significant bits orders them, and runs of equal keys become the entries.
 //
 // Culling is two-level over the chain-order tiles mmm_launch_prepare builds (32 beads, FP32 boxes of
 // the centred copy): one warp per i-tile tests its box against 256-bead stage boxes, 32 stages at a time,
@@ -12,7 +14,19 @@
 // 32 x 32 beads of every tile pair that survives.  The cut-off mode's Morton order is not used: rebuilding
 // it at rc would change the handle's sorted state.  The pass writes only the FP32 copy (d_pos4, d_soa,
 // d_tiles, which every evaluation rewrites from d_x before reading) and its own scratch.
+//
+// Sparse pass, per call (M = binned contacts, E = entries):
+//   k_contacts<kTileCount>  binned contacts of every i-tile -> exclusive scan -> each warp's key offset
+//   k_contacts<kKeys>       keys of warp a at [off_a, off_a+1): no atomics, deterministic order
+//   k_rs_hist / scan / k_rs_scatter   LSD radix sort, 8-bit digits, ceil(log2(n_bins^2)) bits
+//   k_rle<kCount>           heads (first key of a run) per 4096-key chunk -> scan -> E
+// and in mmm_contacts_sparse_read, into the other sort buffer: k_rle<kVals> (run lengths), then
+// k_rle<kSplit> (row = key / n_bins, col = key % n_bins of every head).
+// Scratch: 2 x 8 B per binned contact (the two sort buffers; the read reuses the free one), a digit x
+// chunk table of 8 B x 256 per 4096 keys, and O(N) for the per-tile offsets.
 #include <math.h>
+
+#include <algorithm>
 
 #include "mmm_internal.cuh"
 
@@ -21,6 +35,12 @@ namespace {
 constexpr int CT_WARPS = 8;                              // i-tiles per CTA
 constexpr int CT_TILES_PER_STAGE = MMM_STAGE / MMM_TILE;  // 8
 constexpr int CT_MAX_BINS = 4096;
+constexpr int CS_THREADS = 256, CS_PER = 16, CS_CHUNK = CS_THREADS * CS_PER;  // sort / scan / run blocks: 4096 keys
+constexpr int CS_DIGIT_BITS = 8, CS_DIGITS = 1 << CS_DIGIT_BITS;
+
+// what k_contacts does with a contact: the dense map + P(s) + totals; the binned-contact count of the
+// i-tile (sparse pass 1); the key of every binned contact at the tile's offset (sparse pass 2) + totals
+enum CtSink { kDense, kTileCount, kKeys };
 
 // Gap between [lo_a, hi_a] and [lo_b, hi_b], shrunk by 2^-20 of the largest coordinate involved.  An FP32
 // coordinate of the centred copy is within 2^-24 |p| of the FP64 one and the subtraction adds 2^-24 of
@@ -57,13 +77,16 @@ __global__ void __launch_bounds__(256) k_ct_stage_boxes(const TileInfo* __restri
 }
 
 // One warp per i-tile a; j-tiles b >= a.  Lane l holds bead i = 32 a + l; the beads of the current j-tile
-// are staged in shared memory and read as broadcasts.  Map increments are aggregated over the lanes that
-// hit the same bin pair in the same step (consecutive i-beads mostly share a bin).
+// are staged in shared memory and read as broadcasts.  kDense: map increments are aggregated over the lanes
+// that hit the same bin pair in the same step (consecutive i-beads mostly share a bin).  kTileCount /
+// kKeys see the same candidates in the same order, so pass 2 writes exactly the keys pass 1 counted.
+template <CtSink kSink>
 __global__ void __launch_bounds__(CT_WARPS * 32) k_contacts(
     const double* __restrict__ x, const int* __restrict__ type, const int* __restrict__ bin,
     const TileInfo* __restrict__ tiles, const TileInfo* __restrict__ stages, int n, int ntr, int nst, double rc2,
     float rcm2, int nbins, unsigned long long* __restrict__ map, unsigned long long* __restrict__ sep,
-    unsigned long long* __restrict__ counts) {
+    unsigned long long* __restrict__ counts, long long* __restrict__ tile_keys,
+    unsigned long long* __restrict__ keys) {
   __shared__ double s_x[CT_WARPS][3][32];
   __shared__ int s_bin[CT_WARPS][32], s_chr[CT_WARPS][32];
   const unsigned full = 0xffffffffu;
@@ -81,6 +104,7 @@ __global__ void __launch_bounds__(CT_WARPS * 32) k_contacts(
   }
   const TileInfo A = tiles[a];
   unsigned long long npairs = 0, ncand = 0;
+  long long kpos = kSink == kKeys ? tile_keys[a] : 0;  // next key slot of this warp (warp-uniform)
   for (int t0 = a / CT_TILES_PER_STAGE; t0 < nst; t0 += 32) {
     const int t = t0 + lane;
     unsigned sm = __ballot_sync(full, t < nst && ct_near(A, stages[t], rcm2));
@@ -99,7 +123,7 @@ __global__ void __launch_bounds__(CT_WARPS * 32) k_contacts(
           s_x[w][1][lane] = x[3 * (size_t)j + 1];
           s_x[w][2][lane] = x[3 * (size_t)j + 2];
           s_bin[w][lane] = bin ? bin[j] : -1;
-          s_chr[w][lane] = (type[j] >> 8) & 0xFFFF;
+          if (kSink == kDense) s_chr[w][lane] = (type[j] >> 8) & 0xFFFF;
         }
         __syncwarp();
         const int jn = min(MMM_TILE, n - tb * MMM_TILE);
@@ -113,32 +137,231 @@ __global__ void __launch_bounds__(CT_WARPS * 32) k_contacts(
           const bool hit = ireal && jj >= jstart && d2 < rc2;
           if (!__any_sync(full, hit)) continue;
           const int bj = s_bin[w][jj];
-          if (hit) {
-            ++npairs;
-            if (sep && ci == s_chr[w][jj]) atomicAdd(&sep[tb * MMM_TILE + jj - i], 1ull);
-          }
-          if (map) {
-            const int key = hit && bi >= 0 && bj >= 0 ? bi * nbins + bj : -1;
-            const unsigned grp = __match_any_sync(full, key);
-            if (key >= 0 && lane == __ffs(grp) - 1) {
-              const unsigned long long c = (unsigned long long)__popc(grp);
-              atomicAdd(&map[(size_t)key], c);
-              if (bi != bj) atomicAdd(&map[(size_t)bj * nbins + bi], c);
+          if constexpr (kSink == kDense) {
+            if (hit) {
+              ++npairs;
+              if (sep && ci == s_chr[w][jj]) atomicAdd(&sep[tb * MMM_TILE + jj - i], 1ull);
             }
+            if (map) {
+              const int key = hit && bi >= 0 && bj >= 0 ? bi * nbins + bj : -1;
+              const unsigned grp = __match_any_sync(full, key);
+              if (key >= 0 && lane == __ffs(grp) - 1) {
+                const unsigned long long c = (unsigned long long)__popc(grp);
+                atomicAdd(&map[(size_t)key], c);
+                if (bi != bj) atomicAdd(&map[(size_t)bj * nbins + bi], c);
+              }
+            }
+          } else {
+            if (hit) ++npairs;
+            const bool binned = hit && bi >= 0 && bj >= 0;
+            const unsigned em = __ballot_sync(full, binned);
+            if (kSink == kKeys && binned) {
+              const unsigned p = (unsigned)min(bi, bj), q = (unsigned)max(bi, bj);
+              keys[kpos + __popc(em & ((1u << lane) - 1u))] = (unsigned long long)p * (unsigned)nbins + q;
+            }
+            kpos += __popc(em);
           }
         }
       }
     }
   }
+  if constexpr (kSink == kTileCount) {
+    if (lane == 0) tile_keys[a] = kpos;
+  } else {
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    npairs += __shfl_xor_sync(full, npairs, o);
-    ncand += __shfl_xor_sync(full, ncand, o);
+    for (int o = 16; o > 0; o >>= 1) {
+      npairs += __shfl_xor_sync(full, npairs, o);
+      ncand += __shfl_xor_sync(full, ncand, o);
+    }
+    if (lane == 0) {
+      atomicAdd(&counts[0], npairs);
+      atomicAdd(&counts[1], ncand);
+    }
   }
-  if (lane == 0) {
-    atomicAdd(&counts[0], npairs);
-    atomicAdd(&counts[1], ncand);
+}
+
+// ---- exclusive scan of an int64 array of any length, in place; the total lands in part[nparts] ----------
+// (nparts = ceil(len / CS_CHUNK); part holds nparts + 1 entries)
+__device__ __forceinline__ long long cs_block_exclusive(long long v, long long* s_warp, long long* total) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  long long inc = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const long long u = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += u;
   }
+  if (lane == 31) s_warp[w] = inc;
+  __syncthreads();
+  long long before = 0, all = 0;
+  for (int k = 0; k < CS_THREADS / 32; ++k) {
+    if (k < w) before += s_warp[k];
+    all += s_warp[k];
+  }
+  __syncthreads();  // s_warp is reused by the next call
+  *total = all;
+  return before + inc - v;
+}
+
+__global__ void __launch_bounds__(CS_THREADS) k_scan_parts(const long long* __restrict__ a, long long len,
+                                                           long long* __restrict__ part) {
+  __shared__ long long s_warp[CS_THREADS / 32];
+  const long long base = (long long)blockIdx.x * CS_CHUNK + (long long)threadIdx.x * CS_PER;
+  long long v = 0;
+  for (int k = 0; k < CS_PER; ++k)
+    if (base + k < len) v += a[base + k];
+  long long total;
+  cs_block_exclusive(v, s_warp, &total);
+  if (threadIdx.x == 0) part[blockIdx.x] = total;
+}
+
+__global__ void __launch_bounds__(CS_THREADS) k_scan_top(long long* __restrict__ part, int nparts) {
+  __shared__ long long s_warp[CS_THREADS / 32];
+  long long carry = 0;
+  for (int b0 = 0; b0 < nparts; b0 += CS_THREADS) {
+    const int b = b0 + threadIdx.x;
+    const long long v = b < nparts ? part[b] : 0;
+    long long total;
+    const long long ex = cs_block_exclusive(v, s_warp, &total);
+    if (b < nparts) part[b] = carry + ex;
+    carry += total;
+  }
+  if (threadIdx.x == 0) part[nparts] = carry;
+}
+
+__global__ void __launch_bounds__(CS_THREADS) k_scan_apply(long long* __restrict__ a, long long len,
+                                                           const long long* __restrict__ part) {
+  __shared__ long long s_warp[CS_THREADS / 32];
+  const long long base = (long long)blockIdx.x * CS_CHUNK + (long long)threadIdx.x * CS_PER;
+  long long v[CS_PER], sum = 0;
+#pragma unroll
+  for (int k = 0; k < CS_PER; ++k) {
+    v[k] = base + k < len ? a[base + k] : 0;
+    sum += v[k];
+  }
+  long long total;
+  long long run = part[blockIdx.x] + cs_block_exclusive(sum, s_warp, &total);
+#pragma unroll
+  for (int k = 0; k < CS_PER; ++k) {
+    if (base + k < len) a[base + k] = run;
+    run += v[k];
+  }
+}
+
+// ---- LSD radix sort of 64-bit keys, one pass = hist + scan + scatter ------------------------------------
+// The table is digit-major (table[d * nblocks + b]), so that one flat exclusive scan gives every (digit,
+// block) its first output slot.
+__global__ void __launch_bounds__(CS_THREADS) k_rs_hist(const unsigned long long* __restrict__ keys, long long n,
+                                                        int shift, long long* __restrict__ table, int nblocks) {
+  __shared__ int s_cnt[CS_DIGITS];
+  for (int d = threadIdx.x; d < CS_DIGITS; d += CS_THREADS) s_cnt[d] = 0;
+  __syncthreads();
+  const long long base = (long long)blockIdx.x * CS_CHUNK;
+  for (int q = threadIdx.x; q < CS_CHUNK; q += CS_THREADS) {  // whole warps every round: match_any below
+    const long long e = base + q;
+    const int d = e < n ? (int)((keys[e] >> shift) & (CS_DIGITS - 1)) : -1;
+    const unsigned peers = __match_any_sync(0xffffffffu, d);
+    if (d >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&s_cnt[d], __popc(peers));
+  }
+  __syncthreads();
+  for (int d = threadIdx.x; d < CS_DIGITS; d += CS_THREADS) table[(size_t)d * nblocks + blockIdx.x] = s_cnt[d];
+}
+
+// Stable scatter.  Warp w owns keys [w * 512, (w + 1) * 512) of the block's chunk and visits them in 16
+// rounds of 32 consecutive keys, so (round, lane) order is the key order.  Per round the lanes with equal
+// digits find each other with match_any; the lowest of them advances the warp's counter of that digit.
+__global__ void __launch_bounds__(CS_THREADS) k_rs_scatter(const unsigned long long* __restrict__ keys_in, long long n,
+                                                           int shift, const long long* __restrict__ table, int nblocks,
+                                                           unsigned long long* __restrict__ keys_out) {
+  constexpr int kWarps = CS_THREADS / 32;
+  __shared__ int s_cnt[kWarps][CS_DIGITS];
+  __shared__ long long s_base[CS_DIGITS];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int d = threadIdx.x; d < kWarps * CS_DIGITS; d += CS_THREADS) (&s_cnt[0][0])[d] = 0;
+  __syncthreads();
+  const long long base = (long long)blockIdx.x * CS_CHUNK + warp * (CS_CHUNK / kWarps);
+  unsigned long long key[CS_PER];
+  int rank[CS_PER];
+#pragma unroll
+  for (int r = 0; r < CS_PER; ++r) {
+    const long long e = base + r * 32 + lane;
+    const bool have = e < n;
+    key[r] = have ? keys_in[e] : 0ull;
+    const int d = have ? (int)((key[r] >> shift) & (CS_DIGITS - 1)) : -1;
+    const unsigned peers = __match_any_sync(0xffffffffu, d);
+    const int before = __popc(peers & ((1u << lane) - 1u));
+    int old = 0;
+    if (have && before == 0) {
+      old = s_cnt[warp][d];
+      s_cnt[warp][d] = old + __popc(peers);
+    }
+    old = __shfl_sync(0xffffffffu, old, __ffs(peers) - 1);
+    rank[r] = have ? old + before : -1;
+    __syncwarp();
+  }
+  __syncthreads();
+  for (int d = threadIdx.x; d < CS_DIGITS; d += CS_THREADS) {  // exclusive prefix over the warps, per digit
+    int run = 0;
+#pragma unroll
+    for (int w = 0; w < kWarps; ++w) {
+      const int c = s_cnt[w][d];
+      s_cnt[w][d] = run;
+      run += c;
+    }
+    s_base[d] = table[(size_t)d * nblocks + blockIdx.x];
+  }
+  __syncthreads();
+#pragma unroll
+  for (int r = 0; r < CS_PER; ++r) {
+    if (rank[r] < 0) continue;
+    const int d = (int)((key[r] >> shift) & (CS_DIGITS - 1));
+    keys_out[s_base[d] + s_cnt[warp][d] + rank[r]] = key[r];
+  }
+}
+
+// ---- runs of equal sorted keys -> entries -------------------------------------------------------------
+// Thread t of block b owns keys [b * 4096 + 16 t, + 16); a head is a key unlike its predecessor, and entry
+// e(k) of key k = (heads at or before k) - 1.  kCount: heads of the chunk -> cnt[b].  kVals: vals[e] +=
+// the length of every piece of a run the thread holds (integer atomics: exact in any order; vals zeroed).
+// kSplit: rows[e] = key / n_bins, cols[e] = key % n_bins at every head.  off = the scanned kCount output.
+enum RleMode { kCount, kVals, kSplit };
+template <RleMode kMode>
+__global__ void __launch_bounds__(CS_THREADS) k_rle(const unsigned long long* __restrict__ keys, long long n,
+                                                    long long* __restrict__ cnt, const long long* __restrict__ off,
+                                                    unsigned nbins, unsigned long long* __restrict__ vals,
+                                                    int* __restrict__ rows, int* __restrict__ cols) {
+  __shared__ long long s_warp[CS_THREADS / 32];
+  const long long base = (long long)blockIdx.x * CS_CHUNK + (long long)threadIdx.x * CS_PER;
+  unsigned long long prev = base > 0 && base - 1 < n ? keys[base - 1] : ~0ull;  // no key is ~0 (< 2^62)
+  unsigned long long k[CS_PER];
+  long long heads = 0;
+#pragma unroll
+  for (int q = 0; q < CS_PER; ++q) {
+    k[q] = base + q < n ? keys[base + q] : prev;  // past the end: a repeat, never a head
+    heads += (base + q < n && k[q] != (q ? k[q - 1] : prev)) ? 1 : 0;
+  }
+  long long total;
+  const long long before = cs_block_exclusive(heads, s_warp, &total);
+  if constexpr (kMode == kCount) {
+    if (threadIdx.x == 0) cnt[blockIdx.x] = total;
+    return;
+  }
+  long long e = off[blockIdx.x] + before - 1;  // entry of the key before this thread's first
+  unsigned long long len = 0;
+#pragma unroll
+  for (int q = 0; q < CS_PER; ++q) {
+    if (base + q >= n) break;
+    if (k[q] != (q ? k[q - 1] : prev)) {
+      if (kMode == kVals && len) atomicAdd(&vals[e], len);
+      ++e;
+      len = 0;
+      if (kMode == kSplit) {
+        rows[e] = (int)(k[q] / nbins);
+        cols[e] = (int)(k[q] % nbins);
+      }
+    }
+    ++len;
+  }
+  if (kMode == kVals && len) atomicAdd(&vals[e], len);
 }
 
 // scratch that lives as long as the handle: allocated on the first call (the map when a larger one is
@@ -154,12 +377,45 @@ int ct_alloc(mmm_system* h, T** p, size_t count) {
   return MMM_OK;
 }
 
+// exclusive scan of a[0, len) in place; part: ceil(len / CS_CHUNK) + 1 entries, the last receives the total
+void cs_scan(mmm_system* h, long long* a, long long len, long long* part) {
+  const int nparts = (int)std::max<long long>(1, (len + CS_CHUNK - 1) / CS_CHUNK);
+  k_scan_parts<<<nparts, CS_THREADS, 0, h->stream>>>(a, len, part);
+  k_scan_top<<<1, CS_THREADS, 0, h->stream>>>(part, nparts);
+  k_scan_apply<<<nparts, CS_THREADS, 0, h->stream>>>(a, len, part);
+  h->launches += 3;
+}
+
+long long cs_blocks(long long nkeys) { return std::max<long long>(1, (nkeys + CS_CHUNK - 1) / CS_CHUNK); }
+// sort table (digit x chunk) followed by the partial sums of its scan
+size_t cs_table_len(long long nkeys) { return (size_t)(CS_DIGITS * cs_blocks(nkeys)) * 17 / 16 + 2; }
+
+// the argument checks of mmm_contacts and mmm_contacts_sparse (max_bins: 4096 for the dense map)
+int ct_check_args(mmm_system* h, const char* who, double rc_nm, const int32_t* bin_of_bead, int32_t n_bins, int max_bins,
+             bool need_bins) {
+  if (!(rc_nm > 0.0) || !isfinite(rc_nm)) return mmm_fail(h, MMM_ERR_ARG, std::string(who) + ": rc must be finite and > 0");
+  if (n_bins < 1 || n_bins > max_bins)
+    return mmm_fail(h, MMM_ERR_ARG, std::string(who) + (max_bins == CT_MAX_BINS ? ": n_bins must be in [1, 4096]"
+                                                                              : ": n_bins must be >= 1"));
+  if (need_bins && !bin_of_bead) return mmm_fail(h, MMM_ERR_ARG, std::string(who) + ": a map needs bin_of_bead");
+  if (bin_of_bead)
+    for (int64_t i = 0; i < h->n; ++i)
+      if (bin_of_bead[i] < -1 || bin_of_bead[i] >= n_bins)
+        return mmm_fail(h, MMM_ERR_ARG, std::string(who) + ": bin id outside [-1, n_bins)");
+  if (!h->positions_set) return mmm_fail(h, MMM_ERR_STATE, "positions were never set");
+  return MMM_OK;
+}
+
 }  // namespace
 
 void mmm_contacts_free(mmm_system* h) {
-  void* ptrs[] = {h->d_ct_bin, h->d_ct_map, h->d_ct_sep, h->d_ct_stage, h->d_ct_cnt};
+  void* ptrs[] = {h->d_ct_bin, h->d_ct_map, h->d_ct_sep, h->d_ct_stage, h->d_ct_cnt,
+                  h->d_cs_tile, h->d_cs_keys[0], h->d_cs_keys[1], h->d_cs_table};
   for (void* p : ptrs)
     if (p) cudaFree(p);
+  h->d_cs_tile = nullptr; h->d_cs_keys[0] = h->d_cs_keys[1] = nullptr; h->d_cs_table = nullptr;
+  h->cs_key_cap = 0;
+  h->cs_valid = false;
   if (h->ct_ev0) cudaEventDestroy(h->ct_ev0);
   if (h->ct_ev1) cudaEventDestroy(h->ct_ev1);
   h->ct_ev0 = h->ct_ev1 = nullptr;
@@ -170,22 +426,14 @@ void mmm_contacts_free(mmm_system* h) {
 extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_bead, int32_t n_bins, uint64_t* map_out,
                             uint64_t* sep_out, int64_t* pairs_out) {
   if (!h) return MMM_ERR_ARG;
-  if (!(rc_nm > 0.0) || !isfinite(rc_nm)) return mmm_fail(h, MMM_ERR_ARG, "mmm_contacts: rc must be finite and > 0");
-  if (n_bins < 1 || n_bins > CT_MAX_BINS)
-    return mmm_fail(h, MMM_ERR_ARG, "mmm_contacts: n_bins must be in [1, 4096]");
-  if (map_out && !bin_of_bead) return mmm_fail(h, MMM_ERR_ARG, "mmm_contacts: a map needs bin_of_bead");
-  if (bin_of_bead)
-    for (int64_t i = 0; i < h->n; ++i)
-      if (bin_of_bead[i] < -1 || bin_of_bead[i] >= n_bins)
-        return mmm_fail(h, MMM_ERR_ARG, "mmm_contacts: bin id outside [-1, n_bins)");
-  if (!h->positions_set) return mmm_fail(h, MMM_ERR_STATE, "positions were never set");
+  int rc;
+  if ((rc = ct_check_args(h, "mmm_contacts", rc_nm, bin_of_bead, n_bins, CT_MAX_BINS, map_out != nullptr))) return rc;
   cudaSetDevice(h->device);
   const int n = (int)h->n;
   const int ntr = (n + MMM_TILE - 1) / MMM_TILE;                    // tiles holding a real bead
   const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;  // stages holding a real tile
   const bool want_map = map_out != nullptr;
   const size_t cells = (size_t)n_bins * (size_t)n_bins;
-  int rc;
   if ((rc = ct_alloc(h, &h->d_ct_bin, (size_t)n))) return rc;
   if ((rc = ct_alloc(h, &h->d_ct_sep, (size_t)n))) return rc;
   if ((rc = ct_alloc(h, &h->d_ct_stage, (size_t)nst))) return rc;
@@ -213,9 +461,9 @@ extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_be
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
   const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
-  k_contacts<<<(ntr + CT_WARPS - 1) / CT_WARPS, CT_WARPS * 32, 0, h->stream>>>(
+  k_contacts<kDense><<<(ntr + CT_WARPS - 1) / CT_WARPS, CT_WARPS * 32, 0, h->stream>>>(
       h->d_x, h->d_type, want_map ? h->d_ct_bin : nullptr, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2,
-      n_bins, want_map ? h->d_ct_map : nullptr, sep_out ? h->d_ct_sep : nullptr, h->d_ct_cnt);
+      n_bins, want_map ? h->d_ct_map : nullptr, sep_out ? h->d_ct_sep : nullptr, h->d_ct_cnt, nullptr, nullptr);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
   MMM_CUDA(h, cudaEventRecord(h->ct_ev1, h->stream));
@@ -229,6 +477,132 @@ extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_be
   if (pairs_out) *pairs_out = (int64_t)cnt[0];
   h->ct_candidates = (int64_t)cnt[1];
   cudaEventElapsedTime(&h->ct_ms, h->ct_ev0, h->ct_ev1);
+  return MMM_OK;
+}
+
+extern "C" int mmm_contacts_sparse(mmm_handle h, double rc_nm, const int32_t* bin_of_bead, int32_t n_bins,
+                                   int64_t* n_entries_out, int64_t* pairs_out) {
+  if (!h) return MMM_ERR_ARG;
+  int rc;
+  if ((rc = ct_check_args(h, "mmm_contacts_sparse", rc_nm, bin_of_bead, n_bins, INT32_MAX, true))) return rc;
+  cudaSetDevice(h->device);
+  h->cs_valid = false;
+  const int n = (int)h->n;
+  const int ntr = (n + MMM_TILE - 1) / MMM_TILE;
+  const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;
+  if ((rc = ct_alloc(h, &h->d_ct_bin, (size_t)n))) return rc;
+  if ((rc = ct_alloc(h, &h->d_ct_stage, (size_t)nst))) return rc;
+  if ((rc = ct_alloc(h, &h->d_ct_cnt, 2))) return rc;
+  if ((rc = ct_alloc(h, &h->d_cs_tile, (size_t)ntr + cs_blocks(ntr) + 1))) return rc;  // counts, then scan parts
+  if (!h->ct_ev0) MMM_CUDA(h, cudaEventCreate(&h->ct_ev0));
+  if (!h->ct_ev1) MMM_CUDA(h, cudaEventCreate(&h->ct_ev1));
+  long long* tile = h->d_cs_tile;
+  long long* tile_part = tile + ntr;
+  MMM_CUDA(h, cudaMemcpyAsync(h->d_ct_bin, bin_of_bead, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
+  MMM_CUDA(h, cudaMemsetAsync(h->d_ct_cnt, 0, sizeof(unsigned long long) * 2, h->stream));
+  MMM_CUDA(h, cudaEventRecord(h->ct_ev0, h->stream));
+  if ((rc = mmm_launch_prepare(h, nullptr))) return rc;
+  k_ct_stage_boxes<<<(nst + 255) / 256, 256, 0, h->stream>>>(h->d_tiles, ntr, nst, h->d_ct_stage);
+  const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
+  const int ctas = (ntr + CT_WARPS - 1) / CT_WARPS;
+  k_contacts<kTileCount><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
+      h->d_x, h->d_type, h->d_ct_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
+      nullptr, nullptr, h->d_cs_tile, nullptr);
+  h->launches += 2;
+  cs_scan(h, tile, ntr, tile_part);
+  MMM_CUDA(h, cudaGetLastError());
+  long long m = 0;  // binned contacts = keys
+  MMM_CUDA(h, cudaMemcpyAsync(&m, tile_part + cs_blocks(ntr), sizeof(m), cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  if ((size_t)m > h->cs_key_cap) {  // grow: exactly this call's keys (the stream is idle: synchronised above)
+    void* old[] = {h->d_cs_keys[0], h->d_cs_keys[1], h->d_cs_table};
+    for (void* p : old)
+      if (p) cudaFree(p);
+    h->d_cs_keys[0] = h->d_cs_keys[1] = nullptr;
+    h->d_cs_table = nullptr;
+    h->cs_key_cap = 0;
+    if ((rc = ct_alloc(h, &h->d_cs_keys[0], (size_t)m))) return rc;
+    if ((rc = ct_alloc(h, &h->d_cs_keys[1], (size_t)m))) return rc;
+    if ((rc = ct_alloc(h, &h->d_cs_table, cs_table_len(m)))) return rc;
+    h->cs_key_cap = (size_t)m;
+  }
+  if (!h->d_cs_table && (rc = ct_alloc(h, &h->d_cs_table, cs_table_len(0)))) return rc;  // m = 0 on the first call
+  long long* table = reinterpret_cast<long long*>(h->d_cs_table);
+  const int nblocks = (int)cs_blocks(m);
+  long long* table_part = table + (size_t)CS_DIGITS * nblocks;
+  k_contacts<kKeys><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
+      h->d_x, h->d_type, h->d_ct_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
+      nullptr, h->d_ct_cnt, h->d_cs_tile, h->d_cs_keys[0]);
+  h->launches++;
+  // keys < n_bins^2: sort on ceil(log2(n_bins^2)) bits, 8 per pass
+  int bits = 0;
+  const unsigned long long kmax = (unsigned long long)n_bins * (unsigned long long)n_bins - 1ull;
+  while (bits < 64 && (kmax >> bits)) ++bits;
+  int src = 0;
+  if (m > 0) {
+    for (int shift = 0; shift < bits; shift += CS_DIGIT_BITS) {
+      k_rs_hist<<<nblocks, CS_THREADS, 0, h->stream>>>(h->d_cs_keys[src], m, shift, table, nblocks);
+      cs_scan(h, table, (long long)CS_DIGITS * nblocks, table_part);
+      k_rs_scatter<<<nblocks, CS_THREADS, 0, h->stream>>>(h->d_cs_keys[src], m, shift, table, nblocks,
+                                                          h->d_cs_keys[1 - src]);
+      h->launches += 2;
+      src = 1 - src;
+    }
+    // entries: heads per chunk -> offsets (the first nblocks slots of the table, kept for the read)
+    k_rle<kCount><<<nblocks, CS_THREADS, 0, h->stream>>>(h->d_cs_keys[src], m, table, nullptr, 0u, nullptr, nullptr,
+                                                         nullptr);
+    h->launches++;
+    cs_scan(h, table, nblocks, table + nblocks);
+  }
+  MMM_CUDA(h, cudaGetLastError());
+  MMM_CUDA(h, cudaEventRecord(h->ct_ev1, h->stream));
+  unsigned long long cnt[2];
+  long long entries = 0;
+  MMM_CUDA(h, cudaMemcpyAsync(cnt, h->d_ct_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, h->stream));
+  if (m > 0)
+    MMM_CUDA(h, cudaMemcpyAsync(&entries, table + nblocks + cs_blocks(nblocks), sizeof(entries),
+                                cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  h->cs_keys = m;
+  h->cs_entries = entries;
+  h->cs_src = src;
+  h->cs_nbins = n_bins;
+  h->cs_valid = true;
+  if (n_entries_out) *n_entries_out = entries;
+  if (pairs_out) *pairs_out = (int64_t)cnt[0];
+  h->ct_candidates = (int64_t)cnt[1];
+  cudaEventElapsedTime(&h->ct_ms, h->ct_ev0, h->ct_ev1);
+  return MMM_OK;
+}
+
+extern "C" int mmm_contacts_sparse_read(mmm_handle h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out) {
+  if (!h) return MMM_ERR_ARG;
+  if (!h->cs_valid) return mmm_fail(h, MMM_ERR_STATE, "mmm_contacts_sparse_read: no mmm_contacts_sparse call to read");
+  const long long m = h->cs_keys, e = h->cs_entries;
+  if (e == 0) return MMM_OK;
+  cudaSetDevice(h->device);
+  const int nblocks = (int)cs_blocks(m);
+  const unsigned long long* keys = h->d_cs_keys[h->cs_src];
+  unsigned long long* spare = h->d_cs_keys[1 - h->cs_src];  // free after the sort; m >= e slots
+  const long long* off = h->d_cs_table;
+  if (vals_out) {
+    MMM_CUDA(h, cudaMemsetAsync(spare, 0, sizeof(unsigned long long) * (size_t)e, h->stream));
+    k_rle<kVals><<<nblocks, CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, 0u, spare, nullptr, nullptr);
+    h->launches++;
+    MMM_CUDA(h, cudaGetLastError());
+    MMM_CUDA(h, cudaMemcpyAsync(vals_out, spare, sizeof(uint64_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));
+  }
+  if (rows_out || cols_out) {  // rows then cols as int32 in the same spare buffer (8 B per entry)
+    int* rows = reinterpret_cast<int*>(spare);
+    int* cols = rows + e;
+    k_rle<kSplit><<<nblocks, CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, (unsigned)h->cs_nbins, nullptr, rows,
+                                                         cols);
+    h->launches++;
+    MMM_CUDA(h, cudaGetLastError());
+    if (rows_out) MMM_CUDA(h, cudaMemcpyAsync(rows_out, rows, sizeof(int32_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));
+    if (cols_out) MMM_CUDA(h, cudaMemcpyAsync(cols_out, cols, sizeof(int32_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));
+  }
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
   return MMM_OK;
 }
 

@@ -255,6 +255,15 @@ struct mmm_system {
   int64_t ct_candidates = 0;               // candidate pairs the last call tested in FP64
   float ct_ms = 0.f;                       // device time of the last call's kernels (events below)
   cudaEvent_t ct_ev0 = nullptr, ct_ev1 = nullptr;
+  // sparse map (mmm_contacts_sparse): grown to the binned contacts of the largest call so far
+  long long* d_cs_tile = nullptr;                       // [tiles + scan parts] int64 key counts -> offsets
+  unsigned long long* d_cs_keys[2] = {nullptr, nullptr};  // [cs_key_cap] each: the radix sort's buffers
+  long long* d_cs_table = nullptr;                      // digit x chunk table + scan parts; then run offsets
+  size_t cs_key_cap = 0;
+  int64_t cs_keys = 0, cs_entries = 0;                  // of the last call: binned contacts, entries
+  int cs_src = 0;                                       // which d_cs_keys holds the sorted keys
+  int32_t cs_nbins = 0;
+  bool cs_valid = false;                                // a call succeeded; mmm_contacts_sparse_read may run
 };
 
 // ---------------------------------------------------------------------------------------

@@ -195,8 +195,24 @@ class Engine:
         self._ck(self._lib.mmm_contacts(self._h, float(rc_nm), _p(bins), n_bins, _p(cmap), _p(sep), C.byref(pairs)))
         return cmap, sep, int(pairs.value)
 
+    def contacts_sparse(self, rc_nm: float, bin_of_bead, n_bins: int):
+        """The contact map of ``contacts`` stored sparse, for any int32 number of bins (mmm_contacts_sparse).
+        Returns (rows int32, cols int32, vals uint64, pairs): the nonzero entries of the upper triangle
+        sorted by (row, col), row <= col, counting the contacts between bins row and col of ``bin_of_bead``
+        (int[N], -1 = left out); pairs, all contacts."""
+        bins = _arr(bin_of_bead, np.int32)
+        if bins.shape != (self.n,):
+            raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        n_entries, pairs = C.c_int64(), C.c_int64()
+        self._ck(self._lib.mmm_contacts_sparse(self._h, float(rc_nm), _p(bins), int(n_bins), C.byref(n_entries),
+                                               C.byref(pairs)))
+        e = int(n_entries.value)
+        rows, cols, vals = np.empty(e, np.int32), np.empty(e, np.int32), np.empty(e, np.uint64)
+        self._ck(self._lib.mmm_contacts_sparse_read(self._h, _p(rows), _p(cols), _p(vals)))
+        return rows, cols, vals, int(pairs.value)
+
     def contacts_stats(self) -> dict:
-        """Of the last contacts() call: bead pairs tested in FP64 (those that survived box culling) and the
+        """Of the last contacts() or contacts_sparse() call: bead pairs tested in FP64 (those that survived box culling) and the
         device time of its kernels in ms (CUDA events on the engine's stream)."""
         cand, ms = C.c_int64(), C.c_float()
         self._ck(self._lib.mmm_contacts_stats(self._h, C.byref(cand), C.byref(ms)))

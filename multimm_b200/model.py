@@ -128,6 +128,8 @@ class MultiMM:
             layout=self.layout)
         self.contacts = None        # counts of the minimised structure (SAVE_CONTACTS)
         self.contacts_file = None   # where finish() writes them; the ensemble driver points it outside run_<i>
+        self.contacts_fine = None   # sparse map of the same contacts (CONTACT_FINE_RESOLUTION)
+        self.contacts_fine_file = None
 
         # chrom_spin: chromosome id per bead; chrom_strength: indexed by POSITION in the (possibly
         # shuffled) order, not by chromosome id (model.py:158-162; appendix A, Q8)
@@ -466,6 +468,13 @@ class MultiMM:
         cmap, sep, pairs = self.engine.contacts(rc, gb.bins, gb.n_bins)
         self.contacts = contacts.result(cmap, sep, pairs, rc, gb, contacts.sep_pairs(self.chrom_spin))
         self.timings["contacts_s"] = time.time() - t0
+        fine_res = int(contact_setting(a, "CONTACT_FINE_RESOLUTION"))
+        if fine_res > 0:
+            t0 = time.time()
+            fb = contacts.genome_bins(self.layout, fine_res, n_beads=a.N_BEADS, max_bins=contacts.MAX_FINE_BINS)
+            rows, cols, vals, pairs = self.engine.contacts_sparse(rc, fb.bins, fb.n_bins)
+            self.contacts_fine = contacts.fine_result(rows, cols, vals, pairs, rc, fb)
+            self.timings["contacts_fine_s"] = time.time() - t0
 
     def finish(self):
         """Structure files, per-chromosome files, reports, parameters.  Host work (the report's device
@@ -482,6 +491,11 @@ class MultiMM:
                 contacts.save_dense(os.path.join(self.save_path, "analysis", "contacts.npz"), self.contacts)
             else:
                 contacts.save_member(self.contacts_file, self.contacts)
+        if self.contacts_fine is not None:
+            from . import contacts
+
+            path = self.contacts_fine_file or os.path.join(self.save_path, "analysis", "contacts_fine.npz")
+            contacts.save_fine(path, self.contacts_fine)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

@@ -56,7 +56,7 @@ def _early_cuda_start():
 _WARMUP = _early_cuda_start()
 
 from . import loaders  # noqa: E402
-from .config import CONTACT_FIELDS, SimulationConfig, contact_setting  # noqa: E402
+from .config import EXTRA_FIELDS, SimulationConfig, contact_setting  # noqa: E402
 from .units import Quantity  # noqa: E402
 
 logger = logging.getLogger("multimm_b200")
@@ -203,8 +203,9 @@ def args_tests(args):
 
 
 def check_contact_fields(args):
-    """CONTACT_RADIUS finite and > 0; CONTACT_RESOLUTION >= 0 and, where the modelled stretch is known from
-    the config alone (not for gene-level runs), at most contacts.MAX_BINS bins."""
+    """CONTACT_RADIUS finite and > 0; CONTACT_RESOLUTION >= 0 and CONTACT_FINE_RESOLUTION >= 0 and, where the
+    modelled stretch is known from the config alone (not for gene-level runs), at most contacts.MAX_BINS
+    and contacts.MAX_FINE_BINS bins."""
     import math
 
     from . import contacts
@@ -215,20 +216,37 @@ def check_contact_fields(args):
     res = int(contact_setting(args, "CONTACT_RESOLUTION"))
     if res < 0:
         raise ValueError(f"CONTACT_RESOLUTION={res} must be >= 0 (0 = automatic)")
-    if res == 0 or str(args.MODELLING_LEVEL or "").lower() == "gene":
+    fine = int(contact_setting(args, "CONTACT_FINE_RESOLUTION"))
+    if fine < 0:
+        raise ValueError(f"CONTACT_FINE_RESOLUTION={fine} must be >= 0 (0 = no fine map)")
+    sp = _modelled_spans(args)
+    if sp is None:
         return
+    if res > 0:
+        nb = contacts.bin_count(sp, res)
+        if nb > contacts.MAX_BINS:
+            raise ValueError(f"CONTACT_RESOLUTION={res} bp gives {nb} contact-map bins; at most {contacts.MAX_BINS} "
+                             "are supported (0 = automatic)")
+    if fine > 0:
+        nb = contacts.bin_count(sp, fine)
+        if nb > contacts.MAX_FINE_BINS:
+            raise ValueError(f"CONTACT_FINE_RESOLUTION={fine} bp gives {nb} fine contact-map bins; at most "
+                             f"{contacts.MAX_FINE_BINS} are supported")
+
+
+def _modelled_spans(args):
+    """contacts.spans of the modelled stretch where the config alone determines it, else None."""
+    from . import contacts
+
+    if str(args.MODELLING_LEVEL or "").lower() == "gene":
+        return None
     if args.CHROM is None:
-        sp = contacts.spans(range(22))
-    elif args.LOC_START is not None and args.LOC_END is not None:
-        sp = contacts.spans([loaders._chrom_index(args.CHROM)], int(args.LOC_START), int(args.LOC_END))
-    elif args.CHROM in loaders.CHROM_SIZES:
-        sp = contacts.spans([loaders._chrom_index(args.CHROM)], 0, loaders.CHROM_SIZES[args.CHROM])
-    else:
-        return
-    nb = contacts.bin_count(sp, res)
-    if nb > contacts.MAX_BINS:
-        raise ValueError(f"CONTACT_RESOLUTION={res} bp gives {nb} contact-map bins; at most {contacts.MAX_BINS} "
-                         "are supported (0 = automatic)")
+        return contacts.spans(range(22))
+    if args.LOC_START is not None and args.LOC_END is not None:
+        return contacts.spans([loaders._chrom_index(args.CHROM)], int(args.LOC_START), int(args.LOC_END))
+    if args.CHROM in loaders.CHROM_SIZES:
+        return contacts.spans([loaders._chrom_index(args.CHROM)], 0, loaders.CHROM_SIZES[args.CHROM])
+    return None
 
 
 def read_ini(path: str) -> dict:
@@ -250,7 +268,7 @@ def get_config(argv=None):
     ap.add_argument("-c", "--config_file", metavar="FILE", help="config file (ini format)")
     ap.add_argument("--gpus", default=None, help="comma-separated CUDA device indices for ensemble workers "
                                                  "(default: DEVICE, or every visible GPU for ensembles)")
-    for name in (*SimulationConfig.model_fields, *CONTACT_FIELDS):
+    for name in (*SimulationConfig.model_fields, *EXTRA_FIELDS):
         ap.add_argument(f"--{name.lower()}")
     ns = vars(ap.parse_args(argv))
     raw = read_ini(ns["config_file"]) if ns.get("config_file") else {}
@@ -365,12 +383,17 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     md = MultiMM(cfg, device=device)
     # outside run_<i>, so that archiving does not take it away; summed by run_ensemble
     md.contacts_file = member_contacts_path(params["OUT_PATH"], i)
+    md.contacts_fine_file = member_contacts_fine_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
 
 def member_contacts_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "contacts", f"member_{i}.npz")
+
+
+def member_contacts_fine_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "contacts", f"member_{i}_fine.npz")
 
 
 def write_ensemble_contacts(args, results: list[dict]) -> str | None:
@@ -387,6 +410,15 @@ def write_ensemble_contacts(args, results: list[dict]) -> str | None:
     logger.info(f"ensemble contacts: {int(agg['members'])} members, {agg['counts'].shape[0]} bins at "
                 f"{int(agg['resolution_bp'])} bp, {int(agg['pairs'])} contacts (rc = {float(agg['radius_nm'])} nm) "
                 f"-> {out}")
+    if int(contact_setting(args, "CONTACT_FINE_RESOLUTION")) > 0:
+        paths = [member_contacts_fine_path(args.OUT_PATH, r["replica"])
+                 for r in sorted(results, key=lambda r: r["replica"])]
+        fine = contacts.aggregate_fine(paths)
+        out_fine = os.path.join(args.OUT_PATH, "ensemble_contacts_fine.npz")
+        contacts.save_fine(out_fine, fine)
+        logger.info(f"ensemble fine contacts: {int(fine['members'])} members, {int(fine['n_bins'])} bins at "
+                    f"{int(fine['resolution_bp'])} bp, {len(fine['vals'])} entries, {int(fine['pairs'])} contacts "
+                    f"-> {out_fine}")
     return out
 
 
