@@ -266,6 +266,26 @@ int mmm_contacts_sparse_read(mmm_handle h, int32_t *rows_out, int32_t *cols_out,
  * be NULL. */
 int mmm_contacts_stats(mmm_handle h, int64_t *candidates_out, float *device_ms_out);
 
+/* ---- mean-distance maps (simulated chromatin tracing; not in the reference, whose model.py:1069-1213
+ * analyses only per-structure bead-index blocks) ------------------------------------------------------ */
+/* Sums of the distance and of its square over every unordered bead pair i < j whose beads both have a bin
+ * (bin_of_bead int32[N], -1 = the bead is left out), at the current positions.  Per pair, in FP64 on the
+ * master positions: d2 = (dx*dx + dy*dy) + dz*dz rounded operation by operation as in mmm_contacts,
+ * d = sqrt(d2) correctly rounded, each quantised on its own with Q = 2^-24 (round half to even):
+ * qd = rint(d * 2^24), qd2 = rint(d2 * 2^24).  They are added to dense symmetric maps (n_bins x n_bins,
+ * row-major, uint64): at (p, q) and, when p != q, at (q, p).  Integer sums, so the maps are bit-identical
+ * however the work is scheduled and any IEEE restatement gives the same integers; maps of the same bins add
+ * up exactly.  dist_sum_out, dist2_sum_out may be NULL; device_ms_out (may be NULL): device time of the
+ * pass (CUDA events on the handle's stream, from clearing the maps to the last sum).  All pairs, no
+ * culling.  1 <= n_bins <= 4096.  MMM_ERR_ARG for n_bins outside that range, bin_of_bead NULL, a bin id
+ * outside [-1, n_bins), positions that are not finite, or sums that could overflow int64: (bead pairs of
+ * the fullest bin pair) x ceil(2^24 D^2) >= 2^63 with D the diagonal of the beads' bounding box, padded for
+ * rounding.  MMM_ERR_STATE before positions are set.  Changes no state an evaluation, a minimisation or
+ * mmm_last_result reads; the scratch (bin table, both maps) is allocated on the first call, and again only
+ * when a larger map is asked for. */
+int mmm_distance_map(mmm_handle h, const int32_t *bin_of_bead, int32_t n_bins, uint64_t *dist_sum_out,
+                     uint64_t *dist2_sum_out, float *device_ms_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

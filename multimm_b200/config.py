@@ -194,12 +194,18 @@ CONTACT_FIELDS: dict[str, tuple[Any, Any]] = {
 CONTACT_FINE_FIELDS: dict[str, tuple[Any, Any]] = {
     "CONTACT_FINE_RESOLUTION": (int, 0),  # bp per bin of the sparse map (contacts_fine.npz); 0 = off
 }
-EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS}
+# Mean-distance maps and radial profiles (multimm_b200.distances), kept the same way.
+DISTANCE_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_DISTANCES": (B, False),         # distance sums of the minimised structure (analysis/distances.npz; ensembles: ensemble_distances.npz)
+    "DISTANCE_RESOLUTION": (int, 0),      # bp per bin of the distance map; 0 = about 1000 bins, at most 4096 bins
+}
+EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
-    """Value of a CONTACT_FIELDS or CONTACT_FINE_FIELDS setting of `args`, its default where it was not given."""
+    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS or DISTANCE_FIELDS setting of `args`, its default where
+    it was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

@@ -138,6 +138,7 @@ int mmm_destroy(mmm_handle h) {
   for (void* p : ptrs)
     if (p) cudaFree(p);
   mmm_contacts_free(h);
+  mmm_distances_free(h);
   mmm_dist_destroy(h);
   if (h->ev_c0) cudaEventDestroy(h->ev_c0);
   if (h->ev_c1) cudaEventDestroy(h->ev_c1);

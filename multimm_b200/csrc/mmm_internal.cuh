@@ -264,6 +264,13 @@ struct mmm_system {
   int cs_src = 0;                                       // which d_cs_keys holds the sorted keys
   int32_t cs_nbins = 0;
   bool cs_valid = false;                                // a call succeeded; mmm_contacts_sparse_read may run
+
+  // mean-distance maps (mmm_distances.cu): scratch kept for the handle's lifetime
+  int* d_dm_bin = nullptr;                 // [n] bin of every bead
+  unsigned long long* d_dm_map = nullptr;  // [2][dm_map_cap] quantised distance sums, then squared-distance sums
+  size_t dm_map_cap = 0;
+  double* d_dm_box = nullptr;              // per-block bounding boxes of the beads (overflow guard)
+  cudaEvent_t dm_ev0 = nullptr, dm_ev1 = nullptr;
 };
 
 // ---------------------------------------------------------------------------------------
@@ -311,6 +318,8 @@ int mmm_launch_pair_cutoff(mmm_system* h, const int* d_skip);
 int64_t mmm_cells_energy_slots(const mmm_system* h);
 // mmm_contacts.cu
 void mmm_contacts_free(mmm_system* h);
+// mmm_distances.cu
+void mmm_distances_free(mmm_system* h);
 // mmm_bonded.cu
 int mmm_upload_topology(mmm_system* h);
 int mmm_upload_angles(mmm_system* h, const int32_t* ai, const int32_t* aj, const int32_t* ak,

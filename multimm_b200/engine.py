@@ -218,6 +218,26 @@ class Engine:
         self._ck(self._lib.mmm_contacts_stats(self._h, C.byref(cand), C.byref(ms)))
         return dict(candidates=int(cand.value), device_ms=float(ms.value))
 
+    def distance_map(self, bin_of_bead, n_bins: int):
+        """Sums of the quantised distance and squared distance over every bead pair i < j, binned by
+        ``bin_of_bead`` (int[N], -1 = left out), at the current positions (mmm_distance_map).  Returns
+        (dist_sum, dist2_sum): uint64 (n_bins, n_bins), symmetric, in units of Q = 2^-24 nm and nm^2."""
+        n_bins = int(n_bins)
+        bins = _arr(bin_of_bead, np.int32)
+        if bins is None or bins.shape != (self.n,):
+            raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        shape = (n_bins, n_bins) if 1 <= n_bins <= 4096 else (0, 0)
+        dsum, d2sum = np.empty(shape, np.uint64), np.empty(shape, np.uint64)
+        ms = C.c_float()
+        self._ck(self._lib.mmm_distance_map(self._h, _p(bins), n_bins, _p(dsum), _p(d2sum), C.byref(ms)))
+        self._distance_ms = float(ms.value)
+        return dsum, d2sum
+
+    def distance_stats(self) -> dict:
+        """Of the last distance_map() call: the device time of its pass in ms (CUDA events on the engine's
+        stream)."""
+        return dict(device_ms=getattr(self, "_distance_ms", 0.0))
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

@@ -130,6 +130,8 @@ class MultiMM:
         self.contacts_file = None   # where finish() writes them; the ensemble driver points it outside run_<i>
         self.contacts_fine = None   # sparse map of the same contacts (CONTACT_FINE_RESOLUTION)
         self.contacts_fine_file = None
+        self.distances = None       # distance sums of the minimised structure (SAVE_DISTANCES)
+        self.distances_file = None  # where finish() writes them; the ensemble driver points it outside run_<i>
 
         # chrom_spin: chromosome id per bead; chrom_strength: indexed by POSITION in the (possibly
         # shuffled) order, not by chromosome id (model.py:158-162; appendix A, Q8)
@@ -453,6 +455,8 @@ class MultiMM:
         self.min_energy(write_files=False)
         if contact_setting(self.args, "SAVE_CONTACTS"):
             self.count_contacts()
+        if contact_setting(self.args, "SAVE_DISTANCES"):
+            self.count_distances()
         if self.args.SIM_RUN_MD:
             self.run_md()
 
@@ -476,6 +480,23 @@ class MultiMM:
             self.contacts_fine = contacts.fine_result(rows, cols, vals, pairs, rc, fb)
             self.timings["contacts_fine_s"] = time.time() - t0
 
+    def count_distances(self):
+        """Distance sums of the minimised structure (SAVE_DISTANCES): the all-pairs map summed by this member's
+        own engine at the positions the minimisation left on the device, and the radial sums about the
+        container centre on the host, binned in canonical genomic coordinates."""
+        from . import contacts, distances
+
+        t0 = time.time()
+        a = self.args
+        res = int(contact_setting(a, "DISTANCE_RESOLUTION"))
+        try:
+            gb = contacts.genome_bins(self.layout, res, n_beads=a.N_BEADS, max_bins=distances.MAX_BINS)
+        except ValueError as e:
+            raise ValueError(f"DISTANCE_RESOLUTION={res}: {e}") from None
+        dsum, d2sum = self.engine.distance_map(gb.bins, gb.n_bins)
+        self.distances = distances.result(dsum, d2sum, gb, self.engine.get_positions(), self.mass_center)
+        self.timings["distances_s"] = time.time() - t0
+
     def finish(self):
         """Structure files, per-chromosome files, reports, parameters.  Host work (the report's device
         pass takes the device index, not this member's engine)."""
@@ -496,6 +517,11 @@ class MultiMM:
 
             path = self.contacts_fine_file or os.path.join(self.save_path, "analysis", "contacts_fine.npz")
             contacts.save_fine(path, self.contacts_fine)
+        if self.distances is not None:
+            from . import distances
+
+            distances.save(self.distances_file or os.path.join(self.save_path, "analysis", "distances.npz"),
+                           self.distances)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

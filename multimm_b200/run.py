@@ -200,6 +200,23 @@ def args_tests(args):
         raise ValueError(f"SIM_INTEGRATOR_TYPE={args.SIM_INTEGRATOR_TYPE!r} is not available "
                          f"(supported: {', '.join(_lib.MD_INTEGRATORS)})")
     check_contact_fields(args)
+    check_distance_fields(args)
+
+
+def check_distance_fields(args):
+    """DISTANCE_RESOLUTION >= 0 and, where the modelled stretch is known from the config alone, at most
+    distances.MAX_BINS bins."""
+    from . import contacts, distances
+
+    res = int(contact_setting(args, "DISTANCE_RESOLUTION"))
+    if res < 0:
+        raise ValueError(f"DISTANCE_RESOLUTION={res} must be >= 0 (0 = automatic)")
+    sp = _modelled_spans(args)
+    if res > 0 and sp is not None:
+        nb = contacts.bin_count(sp, res)
+        if nb > distances.MAX_BINS:
+            raise ValueError(f"DISTANCE_RESOLUTION={res} bp gives {nb} distance-map bins; at most {distances.MAX_BINS} "
+                             "are supported (0 = automatic)")
 
 
 def check_contact_fields(args):
@@ -384,6 +401,7 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     # outside run_<i>, so that archiving does not take it away; summed by run_ensemble
     md.contacts_file = member_contacts_path(params["OUT_PATH"], i)
     md.contacts_fine_file = member_contacts_fine_path(params["OUT_PATH"], i)
+    md.distances_file = member_distances_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
@@ -394,6 +412,26 @@ def member_contacts_path(out_path: str, i: int) -> str:
 
 def member_contacts_fine_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "contacts", f"member_{i}_fine.npz")
+
+
+def member_distances_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "distances", f"member_{i}.npz")
+
+
+def write_ensemble_distances(args, results: list[dict]) -> str | None:
+    """SAVE_DISTANCES: OUT_PATH/ensemble_distances.npz, the sum of the distance files of the members that
+    succeeded (exact integer sums: the same bits whichever GPU ran which member)."""
+    if not contact_setting(args, "SAVE_DISTANCES") or not results:
+        return None
+    from . import distances
+
+    paths = [member_distances_path(args.OUT_PATH, r["replica"]) for r in sorted(results, key=lambda r: r["replica"])]
+    agg = distances.aggregate(paths)
+    out = os.path.join(args.OUT_PATH, "ensemble_distances.npz")
+    distances.save(out, agg)
+    logger.info(f"ensemble distances: {int(agg['members'])} members, {len(agg['bin_beads'])} bins at "
+                f"{int(agg['resolution_bp'])} bp -> {out}")
+    return out
 
 
 def write_ensemble_contacts(args, results: list[dict]) -> str | None:
@@ -622,6 +660,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         errors = [p for kind, p in got if kind != "ok"]
         results = [p for kind, p in got if kind == "ok"]
         write_ensemble_contacts(args, results)
+        write_ensemble_distances(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
         check_archives(results)
@@ -658,6 +697,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
                 p.terminate()  # exact processes we started
                 p.join()
     write_ensemble_contacts(args, [r for r in results if r.get("replica", -1) >= 0])
+    write_ensemble_distances(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
