@@ -6,13 +6,15 @@
 // as an explicit extension: plain truncation (OpenMM CutoffNonPeriodic semantics, no shift, no
 // switch) of EV / COB / SCB at r < rc; the oracle applies the same truncation with the same FP32
 // inclusion test, so cell contents, sorted order and the number of pairs inside the cut-off are
-// bit-exact (tests/test_gpu_parity.py).  CHB's polynomial grows with r and cannot be truncated:
+// bit-exact (tests/test_gpu_parity.py; grid, keys and order against the numpy restatement
+// tests/cells_ref.py, every form and the cell-boundary edge in tests/test_gpu_cutoff_reference.py).  CHB's polynomial grows with r and cannot be truncated:
 // when CHB is on, an exact all-pairs pass restricted to CHB runs beside the cell-list pass.
 //
 // Per evaluation (all hand-written; the sort is a counting sort by cell, which the cell structure
 // gives for free, followed by an id-rank inside each cell so that the order is exactly (key, id) —
 // the oracle's stable sort — whatever order the atomics landed in):
-//   k_cell_grid   (1 block)  bounding box of the real tiles -> origin, cell edge (>= rc), dim <= 64
+//   k_cell_grid   (1 block)  bounding box of the real tiles -> origin, cell edge rc (1 + 2^-12) or
+//                            coarser, dim <= 64 (the margin keeps every in-cut pair in neighbouring cells)
 //   k_cell_keys   30-bit Morton key of the bead's cell + histogram (RED.ADD per bead)      16 B read,  4 B written per bead
 //   k_cell_scan   (1 block)  exclusive scan of the 8^bits cell counts in use -> [start, end) per cell
 //   k_cell_place  unstable placement: slot = start[key] + atomic cursor                    8 B written per bead
@@ -33,6 +35,7 @@ using namespace pairmath;
 constexpr int kMaxDim = 64;
 constexpr int kMaxCodes = kMaxDim * kMaxDim * kMaxDim;  // 8^6
 constexpr int kCellWarps = 8;
+constexpr float kCellMargin = 0x1p-12f;  // cell edge = rc * (1 + kCellMargin): see k_cell_grid
 
 struct CellGrid {
   float origin, cell;
@@ -77,12 +80,20 @@ __global__ void __launch_bounds__(256) k_cell_grid(const TileInfo* __restrict__ 
     }
     __syncthreads();
   }
+  // The cell edge is strictly larger than rc, so that every pair the FP32 test accepts lies in
+  // neighbouring cells.  A pair with fmaf(dz, dz, fmaf(dy, dy, dx * dx)) < fl(rc * rc) has, on every axis,
+  // |fl(x_i - x_j)| < rc (1 + 2^-23), so |x_i - x_j| < rc (1 + 2^-22), which is below (1 - 2^-13) cells of
+  // rc (1 + 2^-12).  The cell coordinate floorf(__fdiv_rn(x - origin, cell)) rounds twice, each time by
+  // at most 2^-24 of a value below 64 cells, so it moves by less than 2^-17 cells per bead; the two
+  // beads' coordinates then differ by less than 1 - 2^-13 + 2^-16 < 1 cell, and their cells by at most
+  // one.  (With an edge of exactly rc, pairs on cell boundaries — any lattice of rc / k — land two
+  // cells apart and the 27-cell walk never meets them.)  The coarse branch has even more room.
   if (threadIdx.x == 0) {
     const float origin = s_lo[0];
     const float extent = fmaxf(s_hi[0] - origin, 0.0f);
-    float cell = rc;
+    float cell = rc * (1.0f + kCellMargin);
     int dim = (int)floorf(__fdiv_rn(extent, cell)) + 1;
-    if (dim > kMaxDim) {  // coarser cells are still correct (cell >= rc); keys are clamped anyway
+    if (dim > kMaxDim) {  // coarser cells are still correct (cell > rc); keys are clamped anyway
       cell = __fdiv_rn(extent, (float)(kMaxDim - 1));
       dim = kMaxDim;
     }
