@@ -96,31 +96,24 @@ extern "C" int mmm_contact_map(int device, const double* xyz, int64_t n, int bin
   std::vector<long long> edges((size_t)bins + 1);
   const double step = (double)n / (double)bins;
   for (int k = 0; k <= bins; ++k) edges[(size_t)k] = (long long)(k == bins ? (double)n : (double)k * step);
-  double *d_x = nullptr, *d_map = nullptr, *d_part = nullptr;
-  long long* d_edges = nullptr;
   const long long nblocks = (long long)bins * (bins + 1) / 2;
   if (nblocks > 2147483647LL) return MMM_ERR_ARG;
-  int rc = MMM_OK;
-  auto ok = [&](cudaError_t e) { if (e != cudaSuccess && rc == MMM_OK) rc = MMM_ERR_CUDA; return e == cudaSuccess; };
-  ok(cudaMalloc((void**)&d_x, sizeof(double) * 3 * (size_t)n));
-  ok(cudaMalloc((void**)&d_map, sizeof(double) * (size_t)bins * bins));
-  ok(cudaMalloc((void**)&d_part, sizeof(double) * (size_t)nblocks));
-  ok(cudaMalloc((void**)&d_edges, sizeof(long long) * edges.size()));
-  std::vector<double> part;
-  if (rc == MMM_OK) {
-    ok(cudaMemcpy(d_x, xyz, sizeof(double) * 3 * (size_t)n, cudaMemcpyHostToDevice));
-    ok(cudaMemcpy(d_edges, edges.data(), sizeof(long long) * edges.size(), cudaMemcpyHostToDevice));
-    k_contact_bins<<<(unsigned)nblocks, 256>>>(d_x, d_edges, bins, log_scale, d_map, d_part);
-    ok(cudaGetLastError());
-    ok(cudaMemcpy(map_out, d_map, sizeof(double) * (size_t)bins * bins, cudaMemcpyDeviceToHost));
-    if (mean_dist_out) {
-      part.resize((size_t)nblocks);
-      ok(cudaMemcpy(part.data(), d_part, sizeof(double) * (size_t)nblocks, cudaMemcpyDeviceToHost));
-    }
-  }
-  cudaFree(d_x); cudaFree(d_map); cudaFree(d_part); cudaFree(d_edges);
-  if (rc != MMM_OK) return mmm_fail(nullptr, rc, "CUDA error: contact-map pass failed");
+  DevBuf<double> d_x, d_map, d_part;
+  DevBuf<long long> d_edges;
+  int rc;
+  if ((rc = mmm_reserve(nullptr, d_x, 3 * (size_t)n, "contact-map coordinates")) ||
+      (rc = mmm_reserve(nullptr, d_map, (size_t)bins * bins, "contact map")) ||
+      (rc = mmm_reserve(nullptr, d_part, (size_t)nblocks, "contact-map partial sums")) ||
+      (rc = mmm_reserve(nullptr, d_edges, edges.size(), "contact-map bin edges")))
+    return rc;
+  MMM_CUDA(nullptr, cudaMemcpy(d_x, xyz, sizeof(double) * 3 * (size_t)n, cudaMemcpyHostToDevice));
+  MMM_CUDA(nullptr, cudaMemcpy(d_edges, edges.data(), sizeof(long long) * edges.size(), cudaMemcpyHostToDevice));
+  k_contact_bins<<<(unsigned)nblocks, 256>>>(d_x, d_edges, bins, log_scale, d_map, d_part);
+  MMM_CUDA(nullptr, cudaGetLastError());
+  MMM_CUDA(nullptr, cudaMemcpy(map_out, d_map, sizeof(double) * (size_t)bins * bins, cudaMemcpyDeviceToHost));
   if (mean_dist_out) {
+    std::vector<double> part((size_t)nblocks);
+    MMM_CUDA(nullptr, cudaMemcpy(part.data(), d_part, sizeof(double) * (size_t)nblocks, cudaMemcpyDeviceToHost));
     double s = 0.0;
     for (double v : part) s += v;
     *mean_dist_out = s / ((double)n * (double)n);  // zero diagonal included, as np.mean(cdist(V, V))
@@ -135,15 +128,13 @@ extern "C" int mmm_mean_pair_distance(mmm_handle h, double* mean_out) {
   int rc = mmm_launch_prepare(h, nullptr);  // d_x -> centred FP32 copy
   if (rc) return rc;
   const int blocks = (int)((h->n + 255) / 256);
-  double* d_part = nullptr;
-  MMM_CUDA(h, cudaMalloc((void**)&d_part, sizeof(double) * blocks));
+  DevBuf<double> d_part;
+  if ((rc = mmm_reserve(h, d_part, (size_t)blocks, "mean-distance partial sums"))) return rc;
   k_sum_distances<<<blocks, 256, 0, h->stream>>>(h->d_pos4, h->n, h->npad, d_part);
   h->launches++;
   std::vector<double> part((size_t)blocks);
-  cudaError_t e = cudaMemcpyAsync(part.data(), d_part, sizeof(double) * blocks, cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  cudaFree(d_part);
-  if (e != cudaSuccess) return mmm_fail(h, MMM_ERR_CUDA, std::string("CUDA error: ") + cudaGetErrorString(e));
+  MMM_CUDA(h, cudaMemcpyAsync(part.data(), d_part, sizeof(double) * blocks, cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
   double s = 0.0;
   for (double p : part) s += p;
   // np.mean over the full N x N matrix, zero diagonal included (plots.py:664)

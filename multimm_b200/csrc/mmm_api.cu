@@ -22,16 +22,6 @@ int mmm_fail(mmm_system* h, int code, const std::string& msg) {
 #define REQUIRE(h, cond, msg) \
   do { if (!(cond)) return mmm_fail((h), MMM_ERR_ARG, (msg)); } while (0)
 
-template <typename T>
-static int dev_alloc(mmm_system* h, T** p, size_t count) {
-  if (*p) { cudaFree(*p); *p = nullptr; }
-  if (count == 0) return MMM_OK;
-  cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-  if (e != cudaSuccess)
-    return mmm_fail(h, MMM_ERR_NOMEM, std::string("CUDA error: ") + cudaGetErrorString(e) + " (cudaMalloc)");
-  return MMM_OK;
-}
-
 static void derive_pair_params(mmm_system* h) {
   PairParams& p = h->pp;
   p.ev_pref = p.ev_form == MMM_EV_POWERLAW ? p.ev_eps * powf(p.ev_sigma, p.ev_power) : 0.0f;
@@ -93,20 +83,21 @@ int mmm_create(int device, int64_t n_beads, mmm_handle* out) {
   cudaEventCreate(&h->ev_a);
   cudaEventCreate(&h->ev_b);
   const size_t n3 = 3 * (size_t)n_beads;
-  if ((rc = dev_alloc(h, &h->d_type, (size_t)h->npad))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_cstr, (size_t)n_beads))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_s, (size_t)n_beads))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_x, n3))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_center, 3))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_pos4, (size_t)h->npad))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_soa, 3 * (size_t)h->npad))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_tiles, (size_t)h->ntiles))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_g, n3))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_counter, 4))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_epart, (size_t)h->n_red_blocks * 6))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_dpart, (size_t)h->n_red_blocks * MMM_NDOT))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_eterms, MMM_NUM_TERMS))) return fail(rc);
-  if ((rc = dev_alloc(h, &h->d_lb, 1))) return fail(rc);
+  if ((rc = mmm_reserve(h, h->d_type, (size_t)h->npad, "bead types")) ||
+      (rc = mmm_reserve(h, h->d_cstr, (size_t)n_beads, "chromosome strengths")) ||
+      (rc = mmm_reserve(h, h->d_s, (size_t)n_beads, "compartment labels")) ||
+      (rc = mmm_reserve(h, h->d_x, n3, "positions")) ||
+      (rc = mmm_reserve(h, h->d_center, 3, "centre")) ||
+      (rc = mmm_reserve(h, h->d_pos4, (size_t)h->npad, "FP32 positions")) ||
+      (rc = mmm_reserve(h, h->d_soa, 3 * (size_t)h->npad, "FP32 coordinate planes")) ||
+      (rc = mmm_reserve(h, h->d_tiles, (size_t)h->ntiles, "tile boxes")) ||
+      (rc = mmm_reserve(h, h->d_g, n3, "gradient")) ||
+      (rc = mmm_reserve(h, h->d_counter, 4, "work counters")) ||
+      (rc = mmm_reserve(h, h->d_epart, (size_t)h->n_red_blocks * 6, "energy partials")) ||
+      (rc = mmm_reserve(h, h->d_dpart, (size_t)h->n_red_blocks * MMM_NDOT, "dot partials")) ||
+      (rc = mmm_reserve(h, h->d_eterms, MMM_NUM_TERMS, "energy terms")) ||
+      (rc = mmm_reserve(h, h->d_lb, 1, "L-BFGS state")))
+    return fail(rc);
   if (cudaMallocHost((void**)&h->h_done, 64) != cudaSuccess)
     return fail(mmm_fail(h, MMM_ERR_NOMEM, "CUDA error: cudaMallocHost"));
   cudaMemsetAsync(h->d_cstr, 0, sizeof(double) * n_beads, h->stream);
@@ -127,29 +118,13 @@ int mmm_destroy(mmm_handle h) {
   if (!h) return MMM_OK;
   cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
-  void* ptrs[] = {h->d_type, h->d_cstr, h->d_s, h->d_bl_ptr, h->d_bl_partner, h->d_bl_flags, h->d_bl_r0, h->d_bl_k,
-                  h->d_an_ptr, h->d_an_ijk, h->d_an_par, h->d_x, h->d_center, h->d_pos4, h->d_soa, h->d_tiles, h->d_g,
-                  h->d_fpair, h->epair_aliased ? nullptr : h->d_epair, h->d_facc, h->d_items, h->d_counter, h->d_epart, h->d_dpart, h->d_eterms, h->d_lb, h->d_xp,
-                  h->d_gp, h->d_d, h->d_S, h->d_Y, h->d_keys, h->d_order, h->d_keys_tmp, h->d_order_tmp,
-                  h->d_pos4_sorted, h->d_cell_start, h->d_sort_tmp, h->d_cell_grid, h->d_cell_npairs, h->d_v,
-                  h->d_cl_start, h->d_cl_of_bead, h->d_cl_by_chrom, h->d_cl_range, h->d_cl_cen, h->d_cl_force,
-                  h->d_soa_sorted, h->d_tiles_sorted, h->d_stage_boxes, h->d_sort_table, h->d_items_cut, h->d_cut_npairs,
-                  h->d_cut_eacc};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  mmm_contacts_free(h);
-  mmm_distances_free(h);
   mmm_dist_destroy(h);
-  if (h->ev_c0) cudaEventDestroy(h->ev_c0);
-  if (h->ev_c1) cudaEventDestroy(h->ev_c1);
   if (h->h_done) cudaFreeHost(h->h_done);
   for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
-  if (h->d_flush) cudaFree(h->d_flush);
-  if (h->d_fout) cudaFree(h->d_fout);
-  if (h->ev_a) cudaEventDestroy(h->ev_a);
-  if (h->ev_b) cudaEventDestroy(h->ev_b);
+  for (cudaEvent_t e : {h->ev_a, h->ev_b, h->ev_c0, h->ev_c1, h->ct_ev0, h->ct_ev1, h->dm_ev0, h->dm_ev1})
+    if (e) cudaEventDestroy(e);
   if (h->stream) cudaStreamDestroy(h->stream);
-  delete h;
+  delete h;  // the device buffers free themselves
   return MMM_OK;
 }
 
@@ -405,16 +380,13 @@ int mmm_hilbert_points(mmm_handle h, int p, int32_t* ijk_out) {
   REQUIRE(h, p >= 1 && p <= 10, "mmm_hilbert_points: order p must be in [1, 10]");
   REQUIRE(h, h->n <= ((int64_t)1 << (3 * p)), "mmm_hilbert_points: N exceeds the 2^(3p) points of the curve");
   cudaSetDevice(h->device);
-  int32_t* d_ijk = nullptr;
-  MMM_CUDA(h, cudaMalloc((void**)&d_ijk, sizeof(int32_t) * 3 * h->n));
-  int rc = mmm_launch_hilbert(h, p, 0.0, d_ijk);
-  if (!rc) {
-    cudaError_t e = cudaMemcpyAsync(ijk_out, d_ijk, sizeof(int32_t) * 3 * h->n, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) rc = mmm_fail(h, MMM_ERR_CUDA, std::string("CUDA error: ") + cudaGetErrorString(e));
-  }
-  cudaFree(d_ijk);
-  return rc;
+  DevBuf<int32_t> d_ijk;
+  int rc;
+  if ((rc = mmm_reserve(h, d_ijk, 3 * (size_t)h->n, "Hilbert points")) || (rc = mmm_launch_hilbert(h, p, 0.0, d_ijk)))
+    return rc;
+  MMM_CUDA(h, cudaMemcpyAsync(ijk_out, d_ijk, sizeof(int32_t) * 3 * h->n, cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MMM_OK;
 }
 
 }  // extern "C"
@@ -434,15 +406,14 @@ static int wanted_pair_mode(const mmm_system* h) {
 
 static void free_scratch(mmm_system* h) {
   cudaStreamSynchronize(h->stream);
-  if (h->d_fpair) { cudaFree(h->d_fpair); h->d_fpair = nullptr; }
-  if (h->d_epair && !h->epair_aliased) cudaFree(h->d_epair);
+  h->d_fpair.reset();
+  h->d_epair_buf.reset();
   h->d_epair = nullptr;
-  h->epair_aliased = false;
-  if (h->d_facc) { cudaFree(h->d_facc); h->d_facc = nullptr; }
-  if (h->d_items) { cudaFree(h->d_items); h->d_items = nullptr; }
-  if (h->d_items_cut) { cudaFree(h->d_items_cut); h->d_items_cut = nullptr; }
-  if (h->d_cut_npairs) { cudaFree(h->d_cut_npairs); h->d_cut_npairs = nullptr; }
-  if (h->d_cut_eacc) { cudaFree(h->d_cut_eacc); h->d_cut_eacc = nullptr; }
+  h->d_facc.reset();
+  h->d_items.reset();
+  h->d_items_cut.reset();
+  h->d_cut_npairs.reset();
+  h->d_cut_eacc.reset();
   h->scratch_sig = -1;
 }
 
@@ -488,15 +459,13 @@ static int ensure_scratch(mmm_system* h) {
     h->n3_items = (int)items.size();
     h->n3_chb_only = chb_n3;
     h->n_items = h->n3_items;
-    if ((rc = dev_alloc(h, &h->d_items, items.size()))) return rc;
-    MMM_CUDA(h, cudaMemcpyAsync(h->d_items, items.data(), items.size() * sizeof(int2), cudaMemcpyHostToDevice, h->stream));
-    MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+    if ((rc = mmm_upload(h, h->d_items, items, "Newton-3 work items"))) return rc;
   }
   if (mode == 2 || chb_n3 || cut_n3) {
     // several GPUs: the per-item energy slots live behind the force planes in the same allocation,
     // so that ONE all-reduce (uint64 sum) covers both (mmm_dist.cu)
     const size_t tail = h->nccl_comm ? 4 * ((size_t)h->n3_items + (size_t)h->n_cut_slots) : 0;
-    if ((rc = dev_alloc(h, &h->d_facc, 3 * (size_t)h->npad + tail))) return rc;
+    if ((rc = mmm_reserve(h, h->d_facc, 3 * (size_t)h->npad + tail, "force accumulator"))) return rc;
     MMM_CUDA(h, cudaMemsetAsync(h->d_facc, 0, sizeof(unsigned long long) * (3 * (size_t)h->npad + tail), h->stream));
   }
   if (mode == 1 || chb_gather) {
@@ -520,13 +489,11 @@ static int ensure_scratch(mmm_system* h) {
     h->n_items_cut = (int)items.size();
     h->h_cut_iblk.resize(items.size());
     for (size_t q = 0; q < items.size(); ++q) h->h_cut_iblk[q] = items[q].x;
-    if ((rc = dev_alloc(h, &h->d_items_cut, items.size()))) return rc;
-    MMM_CUDA(h, cudaMemcpyAsync(h->d_items_cut, items.data(), items.size() * sizeof(int2), cudaMemcpyHostToDevice, h->stream));
-    MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-    if ((rc = dev_alloc(h, &h->d_cut_npairs, (size_t)h->n_cut_slots))) return rc;
+    if ((rc = mmm_upload(h, h->d_items_cut, items, "cut-off work items"))) return rc;
+    if ((rc = mmm_reserve(h, h->d_cut_npairs, (size_t)h->n_cut_slots, "cut-off pair counts"))) return rc;
     MMM_CUDA(h, cudaMemsetAsync(h->d_cut_npairs, 0, sizeof(double) * (size_t)h->n_cut_slots, h->stream));
     if (cut_warp) {
-      if ((rc = dev_alloc(h, &h->d_cut_eacc, 4))) return rc;
+      if ((rc = mmm_reserve(h, h->d_cut_eacc, 4, "cut-off energy accumulator"))) return rc;
       MMM_CUDA(h, cudaMemsetAsync(h->d_cut_eacc, 0, sizeof(unsigned long long) * 4, h->stream));
     }
     h->cells_item0 = h->n_items;
@@ -545,7 +512,7 @@ static int ensure_scratch(mmm_system* h) {
   if (h->n_items == 0) h->n_items = 1;
   if (h->n_planes > 0) {
     const size_t cnt = (size_t)h->n_planes * 3 * (size_t)h->npad;
-    if ((rc = dev_alloc(h, &h->d_fpair, cnt))) return rc;
+    if ((rc = mmm_reserve(h, h->d_fpair, cnt, "force planes"))) return rc;
     MMM_CUDA(h, cudaMemsetAsync(h->d_fpair, 0, sizeof(double) * cnt, h->stream));
   }
   if (h->nccl_comm) {
@@ -553,9 +520,9 @@ static int ensure_scratch(mmm_system* h) {
     if (!(mode == 2 || (cut_n3 && chb_ok)))
       return mmm_fail(h, MMM_ERR_STATE, "the multi-GPU path needs the Newton-3 kernel (in cut-off mode: default functional forms, EV on)");
     h->d_epair = reinterpret_cast<double*>(h->d_facc + 3 * (size_t)h->npad);
-    h->epair_aliased = true;
   } else {
-    if ((rc = dev_alloc(h, &h->d_epair, (size_t)h->n_items * 4))) return rc;
+    if ((rc = mmm_reserve(h, h->d_epair_buf, (size_t)h->n_items * 4, "energy slots"))) return rc;
+    h->d_epair = h->d_epair_buf;
     MMM_CUDA(h, cudaMemsetAsync(h->d_epair, 0, sizeof(double) * (size_t)h->n_items * 4, h->stream));
   }
   h->scratch_sig = sig;
@@ -627,7 +594,8 @@ int mmm_energy_forces_device(mmm_handle h, double* e_terms, double* d_forces) {
 
 // d_g holds the gradient: negated on the device, not by a host pass over 24 N bytes
 static int copy_forces_to_host(mmm_system* h, double* forces) {
-  if (!h->d_fout) MMM_CUDA(h, cudaMalloc((void**)&h->d_fout, sizeof(double) * 3 * (size_t)h->n));
+  int rc = mmm_reserve(h, h->d_fout, 3 * (size_t)h->n, "force copy");
+  if (rc) return rc;
   k_negate<<<(unsigned)((3 * h->n + 255) / 256), 256, 0, h->stream>>>(3 * h->n, h->d_g, h->d_fout);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
@@ -675,7 +643,7 @@ int mmm_evaluate_timed(mmm_handle h, int n, int flush_l2, float* total_ms, float
   if (rc) return rc;
   cudaSetDevice(h->device);
   const size_t flush_bytes = (size_t)256 << 20;
-  if (flush_l2 && !h->d_flush) MMM_CUDA(h, cudaMalloc(&h->d_flush, flush_bytes));
+  if (flush_l2 && (rc = mmm_reserve(h, h->d_flush, flush_bytes, "L2-flush scratch"))) return rc;
   while (h->ev_pool.size() < (size_t)2 * n + 2) {
     cudaEvent_t e;
     MMM_CUDA(h, cudaEventCreate(&e));
@@ -716,13 +684,11 @@ int mmm_minimize(mmm_handle h, double tol, int64_t max_iter, mmm_min_report* out
   if (rc) return rc;
   cudaSetDevice(h->device);
   const size_t n3 = 3 * (size_t)h->n;
-  if (!h->d_xp) {
-    if ((rc = dev_alloc(h, &h->d_xp, n3))) return rc;
-    if ((rc = dev_alloc(h, &h->d_gp, n3))) return rc;
-    if ((rc = dev_alloc(h, &h->d_d, n3))) return rc;
-    if ((rc = dev_alloc(h, &h->d_S, n3 * MMM_LBFGS_M))) return rc;
-    if ((rc = dev_alloc(h, &h->d_Y, n3 * MMM_LBFGS_M))) return rc;
-  }
+  if ((rc = mmm_reserve(h, h->d_xp, n3, "L-BFGS x")) || (rc = mmm_reserve(h, h->d_gp, n3, "L-BFGS g")) ||
+      (rc = mmm_reserve(h, h->d_d, n3, "L-BFGS direction")) ||
+      (rc = mmm_reserve(h, h->d_S, n3 * MMM_LBFGS_M, "L-BFGS s history")) ||
+      (rc = mmm_reserve(h, h->d_Y, n3 * MMM_LBFGS_M, "L-BFGS y history")))
+    return rc;
   h->have_result = false;  // the line search leaves trial-point state in d_g / d_eterms
   return mmm_run_minimize(h, tol, max_iter, out);
 }

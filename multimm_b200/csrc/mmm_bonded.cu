@@ -246,16 +246,6 @@ __global__ void __launch_bounds__(256) k_finalize_energy(const double* __restric
   }
 }
 
-template <typename T>
-int upload(mmm_system* h, T** dptr, const std::vector<T>& v) {
-  if (*dptr) { cudaFree(*dptr); *dptr = nullptr; }
-  if (v.empty()) return MMM_OK;
-  MMM_CUDA(h, cudaMalloc((void**)dptr, v.size() * sizeof(T)));
-  MMM_CUDA(h, cudaMemcpyAsync(*dptr, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream));
-  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  return MMM_OK;
-}
-
 }  // namespace
 
 // Build the per-bead gather lists from the bond / loop arrays held on the host side of the handle.
@@ -282,16 +272,13 @@ int mmm_upload_topology(mmm_system* h) {
     put(h->h_loop_i[b], h->h_loop_j[b], lk | 1, h->h_loop_r0[b], h->h_loop_k[b]);
     put(h->h_loop_j[b], h->h_loop_i[b], lk, h->h_loop_r0[b], h->h_loop_k[b]);
   }
+  if (ne == 0) ptr.clear();  // d_bl_ptr NULL: no bonds
   int rc;
-  if (ne == 0) {
-    if (h->d_bl_ptr) { cudaFree(h->d_bl_ptr); h->d_bl_ptr = nullptr; }
-  } else {
-    if ((rc = upload(h, &h->d_bl_ptr, ptr))) return rc;
-  }
-  if ((rc = upload(h, &h->d_bl_partner, partner))) return rc;
-  if ((rc = upload(h, &h->d_bl_flags, flags))) return rc;
-  if ((rc = upload(h, &h->d_bl_r0, r0))) return rc;
-  if ((rc = upload(h, &h->d_bl_k, kk))) return rc;
+  if ((rc = mmm_upload(h, h->d_bl_ptr, ptr, "bond list offsets")) ||
+      (rc = mmm_upload(h, h->d_bl_partner, partner, "bond partners")) ||
+      (rc = mmm_upload(h, h->d_bl_flags, flags, "bond flags")) || (rc = mmm_upload(h, h->d_bl_r0, r0, "bond lengths")) ||
+      (rc = mmm_upload(h, h->d_bl_k, kk, "bond constants")))
+    return rc;
   h->topo_dirty = false;
   return MMM_OK;
 }
@@ -313,14 +300,11 @@ int mmm_upload_angles(mmm_system* h, const int32_t* ai, const int32_t* aj, const
       par[q] = make_double2(t0[a], kt[a]);
     }
   }
+  if (na == 0) ptr.clear();  // d_an_ptr NULL: no angles
   int rc;
-  if (na == 0) {
-    if (h->d_an_ptr) { cudaFree(h->d_an_ptr); h->d_an_ptr = nullptr; }
-  } else {
-    if ((rc = upload(h, &h->d_an_ptr, ptr))) return rc;
-  }
-  if ((rc = upload(h, &h->d_an_ijk, ijk))) return rc;
-  if ((rc = upload(h, &h->d_an_par, par))) return rc;
+  if ((rc = mmm_upload(h, h->d_an_ptr, ptr, "angle list offsets")) ||
+      (rc = mmm_upload(h, h->d_an_ijk, ijk, "angle beads")) || (rc = mmm_upload(h, h->d_an_par, par, "angle parameters")))
+    return rc;
   h->n_angles = na;
   return MMM_OK;
 }
@@ -328,8 +312,8 @@ int mmm_upload_angles(mmm_system* h, const int32_t* ai, const int32_t* aj, const
 int mmm_launch_assemble(mmm_system* h, const int* d_skip) {
   AsmArgs A;
   A.x = h->d_x;
-  A.fpair = (h->pair_mode == 1 || (h->pair_mode == 3 && !h->cut_n3)) ? h->d_fpair : nullptr;
-  A.facc = (h->pair_mode == 2 || (h->pair_mode == 3 && (h->cut_n3 || (h->n3_items > 0 && h->n3_chb_only)))) ? h->d_facc : nullptr;
+  A.fpair = (h->pair_mode == 1 || (h->pair_mode == 3 && !h->cut_n3)) ? h->d_fpair.get() : nullptr;
+  A.facc = (h->pair_mode == 2 || (h->pair_mode == 3 && (h->cut_n3 || (h->n3_items > 0 && h->n3_chb_only)))) ? h->d_facc.get() : nullptr;
   A.nchunk = h->n_planes;
   A.n = h->n;
   A.npad = h->npad;
@@ -337,7 +321,7 @@ int mmm_launch_assemble(mmm_system* h, const int* d_skip) {
   A.bl_r0 = h->d_bl_r0; A.bl_k = h->d_bl_k;
   A.an_ptr = h->d_an_ptr; A.an_ijk = h->d_an_ijk; A.an_par = h->d_an_par;
   A.s = h->d_s; A.cstr = h->d_cstr;
-  A.cl_force = (h->pair_mode == 3 && h->chb_clusters) ? h->d_cl_force : nullptr;
+  A.cl_force = (h->pair_mode == 3 && h->chb_clusters) ? h->d_cl_force.get() : nullptr;
   A.cl_of_bead = h->d_cl_of_bead;
   A.ep = h->ep;
   A.g = h->d_g;

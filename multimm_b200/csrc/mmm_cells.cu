@@ -37,11 +37,6 @@ constexpr int kMaxCodes = kMaxDim * kMaxDim * kMaxDim;  // 8^6
 constexpr int kCellWarps = 8;
 constexpr float kCellMargin = 0x1p-12f;  // cell edge = rc * (1 + kCellMargin): see k_cell_grid
 
-struct CellGrid {
-  float origin, cell;
-  int dim, bits;
-};
-
 __host__ __device__ inline uint32_t spread3(uint32_t v) {
   v &= 0x3ff;
   v = (v | (v << 16)) & 0x030000FF;
@@ -367,26 +362,19 @@ void launch_cells_evp(const CellArgs& A, int gk, int blocks, cudaStream_t st) {
 
 int64_t mmm_cells_energy_slots(const mmm_system* h) { return (h->n + kCellWarps * 32 - 1) / (kCellWarps * 32); }
 
-int mmm_cells_alloc(mmm_system* h) {
-  // every buffer on its own: some are shared with mmm_cutoff.cu (which may have run first on this handle)
-  const size_t n = (size_t)h->npad;  // npad: the shared order covers the pads
-  auto need = [&](void** p, size_t bytes) -> int {
-    if (*p) return MMM_OK;
-    MMM_CUDA(h, cudaMalloc(p, bytes));
-    return MMM_OK;
-  };
+static int mmm_cells_alloc(mmm_system* h) {
+  const size_t npad = (size_t)h->npad;
   int rc;
-  if ((rc = need((void**)&h->d_keys, n * sizeof(uint32_t)))) return rc;
-  if ((rc = need((void**)&h->d_keys_tmp, n * sizeof(uint32_t)))) return rc;
-  if ((rc = need((void**)&h->d_order, n * sizeof(int)))) return rc;
-  if ((rc = need((void**)&h->d_order_tmp, n * sizeof(int)))) return rc;
-  if ((rc = need((void**)&h->d_pos4_sorted, n * sizeof(float4)))) return rc;
-  if ((rc = need((void**)&h->d_cell_start, (size_t)2 * kMaxCodes * sizeof(int)))) return rc;
-  if ((rc = need((void**)&h->d_cell_grid, sizeof(CellGrid)))) return rc;
-  if ((rc = need((void**)&h->d_cell_npairs, (size_t)mmm_cells_energy_slots(h) * sizeof(unsigned long long)))) return rc;
-  // per-cell histogram + placement cursor
-  h->sort_tmp_bytes = (size_t)2 * kMaxCodes * sizeof(int);
-  if ((rc = need(&h->d_sort_tmp, h->sort_tmp_bytes))) return rc;
+  // keys, order, sorted positions and grid are shared with mmm_cutoff.cu: both reserve npad (the most either uses)
+  if ((rc = mmm_reserve(h, h->d_keys, npad, "cell keys")) || (rc = mmm_reserve(h, h->d_keys_tmp, npad, "cell keys")) ||
+      (rc = mmm_reserve(h, h->d_order, npad, "sorted order")) ||
+      (rc = mmm_reserve(h, h->d_order_tmp, npad, "sorted order")) ||
+      (rc = mmm_reserve(h, h->d_pos4_sorted, npad, "sorted positions")) ||
+      (rc = mmm_reserve(h, h->d_cell_grid, 1, "cell grid")) ||
+      (rc = mmm_reserve(h, h->d_cell_start, (size_t)2 * kMaxCodes, "cell ranges")) ||
+      (rc = mmm_reserve(h, h->d_cell_npairs, (size_t)mmm_cells_energy_slots(h), "cell pair counts")) ||
+      (rc = mmm_reserve(h, h->d_sort_tmp, (size_t)2 * kMaxCodes, "cell histogram")))
+    return rc;
   return MMM_OK;
 }
 
@@ -397,7 +385,7 @@ int mmm_launch_pair_cutoff(mmm_system* h, const int* d_skip) {
   if ((rc = mmm_cells_alloc(h))) return rc;
   const int n = (int)h->n;
   const int blocks = (n + 255) / 256;
-  CellGrid* grid = reinterpret_cast<CellGrid*>(h->d_cell_grid);
+  CellGrid* grid = h->d_cell_grid;
   int* cstart = h->d_cell_start;
   int* cend = h->d_cell_start + kMaxCodes;
 
@@ -407,9 +395,9 @@ int mmm_launch_pair_cutoff(mmm_system* h, const int* d_skip) {
   if (collect) h->ev_cursor++;
   if (!h->capturing) MMM_CUDA(h, cudaEventRecord(ea, h->stream));
 
-  int* count = reinterpret_cast<int*>(h->d_sort_tmp);
+  int* count = h->d_sort_tmp;  // per-cell histogram, then placement cursor
   int* cursor = count + kMaxCodes;
-  MMM_CUDA(h, cudaMemsetAsync(h->d_sort_tmp, 0, h->sort_tmp_bytes, h->stream));
+  MMM_CUDA(h, cudaMemsetAsync(count, 0, sizeof(int) * 2 * kMaxCodes, h->stream));
   k_cell_grid<<<1, 256, 0, h->stream>>>(h->d_tiles, (int)h->ntiles, (float)h->cutoff, grid, d_skip);
   k_cell_keys<<<blocks, 256, 0, h->stream>>>(h->d_pos4, h->n, grid, h->d_keys_tmp, count, d_skip);
   k_cell_scan<<<1, 1024, 0, h->stream>>>(grid, count, cstart, cend, d_skip);
@@ -465,9 +453,13 @@ int mmm_get_cell_grid(mmm_handle h, float* cell_out, int32_t* dim_out, float* or
   if (h->pair_mode != 3 || !h->d_keys)
     return mmm_fail(h, MMM_ERR_STATE, "mmm_get_cell_grid: no cut-off evaluation has run on this handle");
   cudaSetDevice(h->device);
+  CellGrid g;
+  MMM_CUDA(h, cudaMemcpyAsync(&g, h->d_cell_grid, sizeof(g), cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (cell_out) *cell_out = g.cell;
+  if (dim_out) *dim_out = g.dim;
+  if (origin_out) *origin_out = g.origin;
   if (h->cut_n3) {
-    int rc = mmm_cutoff_read_grid(h, cell_out, dim_out, origin_out);
-    if (rc) return rc;
     if (pairs_in_cutoff) {
       std::vector<double> per_item((size_t)h->n_cut_slots);
       MMM_CUDA(h, cudaMemcpyAsync(per_item.data(), h->d_cut_npairs, per_item.size() * sizeof(double),
@@ -479,16 +471,11 @@ int mmm_get_cell_grid(mmm_handle h, float* cell_out, int32_t* dim_out, float* or
     }
     return MMM_OK;
   }
-  CellGrid g;
-  std::vector<unsigned long long> cnt((size_t)mmm_cells_energy_slots(h));
-  MMM_CUDA(h, cudaMemcpyAsync(&g, h->d_cell_grid, sizeof(g), cudaMemcpyDeviceToHost, h->stream));
-  MMM_CUDA(h, cudaMemcpyAsync(cnt.data(), h->d_cell_npairs, cnt.size() * sizeof(unsigned long long),
-                              cudaMemcpyDeviceToHost, h->stream));
-  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  if (cell_out) *cell_out = g.cell;
-  if (dim_out) *dim_out = g.dim;
-  if (origin_out) *origin_out = g.origin;
   if (pairs_in_cutoff) {
+    std::vector<unsigned long long> cnt((size_t)mmm_cells_energy_slots(h));
+    MMM_CUDA(h, cudaMemcpyAsync(cnt.data(), h->d_cell_npairs, cnt.size() * sizeof(unsigned long long),
+                                cudaMemcpyDeviceToHost, h->stream));
+    MMM_CUDA(h, cudaStreamSynchronize(h->stream));
     unsigned long long s = 0;
     for (unsigned long long v : cnt) s += v;
     *pairs_in_cutoff = (int64_t)(s / 2);  // the gather kernel sees each unordered pair twice

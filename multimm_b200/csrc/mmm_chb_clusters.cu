@@ -150,16 +150,6 @@ __global__ void __launch_bounds__(256) k_cl_forces(const FarArgs A) {
   }
 }
 
-template <typename T>
-int upload_vec(mmm_system* h, T** dptr, const std::vector<T>& v) {
-  if (*dptr) { cudaFree(*dptr); *dptr = nullptr; }
-  if (v.empty()) return MMM_OK;
-  MMM_CUDA(h, cudaMalloc((void**)dptr, v.size() * sizeof(T)));
-  MMM_CUDA(h, cudaMemcpyAsync(*dptr, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream));
-  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  return MMM_OK;
-}
-
 }  // namespace
 
 int mmm_chb_clusters_blocks(const mmm_system* h) { return h->n_clusters; }  // one energy slot per cluster
@@ -177,13 +167,12 @@ int mmm_chb_clusters_build(mmm_system* h) {
   start.push_back(n);
   h->n_clusters = ncl;
   int rc;
-  if ((rc = upload_vec(h, &h->d_cl_start, start))) return rc;
-  if ((rc = upload_vec(h, &h->d_cl_of_bead, of_bead))) return rc;
-  if ((rc = upload_vec(h, &h->d_cl_by_chrom, chrom))) return rc;  // chromosome id of every cluster
-  if (h->d_cl_cen) { cudaFree(h->d_cl_cen); h->d_cl_cen = nullptr; }
-  if (h->d_cl_force) { cudaFree(h->d_cl_force); h->d_cl_force = nullptr; }
-  MMM_CUDA(h, cudaMalloc((void**)&h->d_cl_cen, sizeof(double) * 4 * (size_t)ncl));
-  MMM_CUDA(h, cudaMalloc((void**)&h->d_cl_force, sizeof(double) * 3 * (size_t)ncl));
+  if ((rc = mmm_upload(h, h->d_cl_start, start, "cluster starts")) ||
+      (rc = mmm_upload(h, h->d_cl_of_bead, of_bead, "cluster of every bead")) ||
+      (rc = mmm_upload(h, h->d_cl_by_chrom, chrom, "cluster chromosomes")) ||  // chromosome id of every cluster
+      (rc = mmm_reserve(h, h->d_cl_cen, 4 * (size_t)ncl, "cluster centroids")) ||
+      (rc = mmm_reserve(h, h->d_cl_force, 3 * (size_t)ncl, "cluster forces")))
+    return rc;
   return MMM_OK;
 }
 

@@ -364,19 +364,6 @@ __global__ void __launch_bounds__(CS_THREADS) k_rle(const unsigned long long* __
   if (kMode == kVals && len) atomicAdd(&vals[e], len);
 }
 
-// scratch that lives as long as the handle: allocated on the first call (the map when a larger one is
-// needed), so that a call does not synchronise the device while another handle minimises beside it
-template <typename T>
-int ct_alloc(mmm_system* h, T** p, size_t count) {
-  if (*p) return MMM_OK;
-  cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-  if (e != cudaSuccess) {
-    *p = nullptr;
-    return mmm_fail(h, MMM_ERR_NOMEM, std::string("CUDA error: ") + cudaGetErrorString(e) + " (cudaMalloc, contacts)");
-  }
-  return MMM_OK;
-}
-
 // exclusive scan of a[0, len) in place; part: ceil(len / CS_CHUNK) + 1 entries, the last receives the total
 void cs_scan(mmm_system* h, long long* a, long long len, long long* part) {
   const int nparts = (int)std::max<long long>(1, (len + CS_CHUNK - 1) / CS_CHUNK);
@@ -408,21 +395,6 @@ int ct_check_args(mmm_system* h, const char* who, double rc_nm, const int32_t* b
 
 }  // namespace
 
-void mmm_contacts_free(mmm_system* h) {
-  void* ptrs[] = {h->d_ct_bin, h->d_ct_map, h->d_ct_sep, h->d_ct_stage, h->d_ct_cnt,
-                  h->d_cs_tile, h->d_cs_keys[0], h->d_cs_keys[1], h->d_cs_table};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  h->d_cs_tile = nullptr; h->d_cs_keys[0] = h->d_cs_keys[1] = nullptr; h->d_cs_table = nullptr;
-  h->cs_key_cap = 0;
-  h->cs_valid = false;
-  if (h->ct_ev0) cudaEventDestroy(h->ct_ev0);
-  if (h->ct_ev1) cudaEventDestroy(h->ct_ev1);
-  h->ct_ev0 = h->ct_ev1 = nullptr;
-  h->d_ct_bin = nullptr; h->d_ct_map = nullptr; h->d_ct_sep = nullptr; h->d_ct_stage = nullptr; h->d_ct_cnt = nullptr;
-  h->ct_map_cap = 0;
-}
-
 extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_bead, int32_t n_bins, uint64_t* map_out,
                             uint64_t* sep_out, int64_t* pairs_out) {
   if (!h) return MMM_ERR_ARG;
@@ -434,21 +406,16 @@ extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_be
   const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;  // stages holding a real tile
   const bool want_map = map_out != nullptr;
   const size_t cells = (size_t)n_bins * (size_t)n_bins;
-  if ((rc = ct_alloc(h, &h->d_ct_bin, (size_t)n))) return rc;
-  if ((rc = ct_alloc(h, &h->d_ct_sep, (size_t)n))) return rc;
-  if ((rc = ct_alloc(h, &h->d_ct_stage, (size_t)nst))) return rc;
-  if ((rc = ct_alloc(h, &h->d_ct_cnt, 2))) return rc;
+  // scratch lives as long as the handle and only grows (the map when a call needs a larger one), so
+  // that a call does not synchronise the device while another handle minimises beside it
+  if ((rc = mmm_reserve(h, h->d_ct_bin, (size_t)n, "contact bins")) ||
+      (rc = mmm_reserve(h, h->d_ct_sep, (size_t)n, "contacts by separation")) ||
+      (rc = mmm_reserve(h, h->d_ct_stage, (size_t)nst, "contact stage boxes")) ||
+      (rc = mmm_reserve(h, h->d_ct_cnt, 2, "contact counters")) ||
+      (want_map && (rc = mmm_reserve(h, h->d_ct_map, cells, "contact map"))))
+    return rc;
   if (!h->ct_ev0) MMM_CUDA(h, cudaEventCreate(&h->ct_ev0));
   if (!h->ct_ev1) MMM_CUDA(h, cudaEventCreate(&h->ct_ev1));
-  if (want_map && h->ct_map_cap < cells) {
-    if (h->d_ct_map) {
-      MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-      cudaFree(h->d_ct_map);
-      h->d_ct_map = nullptr;
-    }
-    if ((rc = ct_alloc(h, &h->d_ct_map, cells))) return rc;
-    h->ct_map_cap = cells;
-  }
   if (want_map) {
     MMM_CUDA(h, cudaMemcpyAsync(h->d_ct_bin, bin_of_bead, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
     MMM_CUDA(h, cudaMemsetAsync(h->d_ct_map, 0, sizeof(unsigned long long) * cells, h->stream));
@@ -462,8 +429,8 @@ extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_be
   MMM_CUDA(h, cudaGetLastError());
   const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
   k_contacts<kDense><<<(ntr + CT_WARPS - 1) / CT_WARPS, CT_WARPS * 32, 0, h->stream>>>(
-      h->d_x, h->d_type, want_map ? h->d_ct_bin : nullptr, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2,
-      n_bins, want_map ? h->d_ct_map : nullptr, sep_out ? h->d_ct_sep : nullptr, h->d_ct_cnt, nullptr, nullptr);
+      h->d_x, h->d_type, want_map ? h->d_ct_bin.get() : nullptr, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2,
+      n_bins, want_map ? h->d_ct_map.get() : nullptr, sep_out ? h->d_ct_sep.get() : nullptr, h->d_ct_cnt, nullptr, nullptr);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
   MMM_CUDA(h, cudaEventRecord(h->ct_ev1, h->stream));
@@ -490,10 +457,11 @@ extern "C" int mmm_contacts_sparse(mmm_handle h, double rc_nm, const int32_t* bi
   const int n = (int)h->n;
   const int ntr = (n + MMM_TILE - 1) / MMM_TILE;
   const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;
-  if ((rc = ct_alloc(h, &h->d_ct_bin, (size_t)n))) return rc;
-  if ((rc = ct_alloc(h, &h->d_ct_stage, (size_t)nst))) return rc;
-  if ((rc = ct_alloc(h, &h->d_ct_cnt, 2))) return rc;
-  if ((rc = ct_alloc(h, &h->d_cs_tile, (size_t)ntr + cs_blocks(ntr) + 1))) return rc;  // counts, then scan parts
+  if ((rc = mmm_reserve(h, h->d_ct_bin, (size_t)n, "contact bins")) ||
+      (rc = mmm_reserve(h, h->d_ct_stage, (size_t)nst, "contact stage boxes")) ||
+      (rc = mmm_reserve(h, h->d_ct_cnt, 2, "contact counters")) ||
+      (rc = mmm_reserve(h, h->d_cs_tile, (size_t)ntr + cs_blocks(ntr) + 1, "contact tile counts")))  // counts, then scan parts
+    return rc;
   if (!h->ct_ev0) MMM_CUDA(h, cudaEventCreate(&h->ct_ev0));
   if (!h->ct_ev1) MMM_CUDA(h, cudaEventCreate(&h->ct_ev1));
   long long* tile = h->d_cs_tile;
@@ -514,20 +482,12 @@ extern "C" int mmm_contacts_sparse(mmm_handle h, double rc_nm, const int32_t* bi
   long long m = 0;  // binned contacts = keys
   MMM_CUDA(h, cudaMemcpyAsync(&m, tile_part + cs_blocks(ntr), sizeof(m), cudaMemcpyDeviceToHost, h->stream));
   MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  if ((size_t)m > h->cs_key_cap) {  // grow: exactly this call's keys (the stream is idle: synchronised above)
-    void* old[] = {h->d_cs_keys[0], h->d_cs_keys[1], h->d_cs_table};
-    for (void* p : old)
-      if (p) cudaFree(p);
-    h->d_cs_keys[0] = h->d_cs_keys[1] = nullptr;
-    h->d_cs_table = nullptr;
-    h->cs_key_cap = 0;
-    if ((rc = ct_alloc(h, &h->d_cs_keys[0], (size_t)m))) return rc;
-    if ((rc = ct_alloc(h, &h->d_cs_keys[1], (size_t)m))) return rc;
-    if ((rc = ct_alloc(h, &h->d_cs_table, cs_table_len(m)))) return rc;
-    h->cs_key_cap = (size_t)m;
-  }
-  if (!h->d_cs_table && (rc = ct_alloc(h, &h->d_cs_table, cs_table_len(0)))) return rc;  // m = 0 on the first call
-  long long* table = reinterpret_cast<long long*>(h->d_cs_table);
+  // grown to exactly this call's keys when they do not fit
+  if ((rc = mmm_reserve(h, h->d_cs_keys[0], (size_t)m, "contact keys")) ||
+      (rc = mmm_reserve(h, h->d_cs_keys[1], (size_t)m, "contact keys")) ||
+      (rc = mmm_reserve(h, h->d_cs_table, cs_table_len(m), "contact sort table")))
+    return rc;
+  long long* table = h->d_cs_table;
   const int nblocks = (int)cs_blocks(m);
   long long* table_part = table + (size_t)CS_DIGITS * nblocks;
   k_contacts<kKeys><<<ctas, CT_WARPS * 32, 0, h->stream>>>(

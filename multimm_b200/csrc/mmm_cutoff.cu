@@ -30,11 +30,6 @@
 
 namespace {
 
-struct CutGrid {  // same layout as the CellGrid of mmm_cells.cu (read back by mmm_get_cell_grid)
-  float origin, cell;
-  int dim, bits;
-};
-
 constexpr int kMaxDim = 1024;
 constexpr int kDigitBits = 10, kDigits = 1 << kDigitBits, kPasses = 3;
 constexpr int kSortThreads = 256, kSortPer = 8, kSortChunk = kSortThreads * kSortPer;  // 2048 keys per block
@@ -55,7 +50,7 @@ __host__ __device__ inline uint32_t spread3(uint32_t v) {
 }
 
 __global__ void __launch_bounds__(256) k_cut_grid(const TileInfo* __restrict__ tiles, int ntiles, float rc,
-                                                  CutGrid* __restrict__ g, const int* __restrict__ skip) {
+                                                  CellGrid* __restrict__ g, const int* __restrict__ skip) {
   if (skip && *skip) return;
   __shared__ float s_lo[256], s_hi[256];
   float lo = 3.0e38f, hi = -3.0e38f;
@@ -89,20 +84,20 @@ __global__ void __launch_bounds__(256) k_cut_grid(const TileInfo* __restrict__ t
   }
 }
 
-__device__ __forceinline__ uint32_t cell_coord(float x, const CutGrid& g) {
+__device__ __forceinline__ uint32_t cell_coord(float x, const CellGrid& g) {
   int v = (int)floorf(__fdiv_rn(x - g.origin, g.cell));
   v = v < 0 ? 0 : v;
   v = v > g.dim - 1 ? g.dim - 1 : v;  // beads beyond 1024 cells share the edge cell (a contraction)
   return (uint32_t)v;
 }
 
-__global__ void __launch_bounds__(256) k_cut_keys(const float4* __restrict__ pos4, int n, const CutGrid* __restrict__ gp,
+__global__ void __launch_bounds__(256) k_cut_keys(const float4* __restrict__ pos4, int n, const CellGrid* __restrict__ gp,
                                                   uint32_t* __restrict__ keys, int* __restrict__ ids,
                                                   const int* __restrict__ skip) {
   if (skip && *skip) return;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const CutGrid g = *gp;
+  const CellGrid g = *gp;
   const float4 p = pos4[i];
   keys[i] = spread3(cell_coord(p.x, g)) | (spread3(cell_coord(p.y, g)) << 1) | (spread3(cell_coord(p.z, g)) << 2);
   ids[i] = i;
@@ -283,29 +278,23 @@ __global__ void __launch_bounds__(256) k_stage_boxes(const TileInfo* __restrict_
   stages[s] = b;  // cmin == MMM_PAD_CHROM: nothing real in the stage
 }
 
-template <typename T>
-int alloc_once(mmm_system* h, T** p, size_t count) {
-  if (*p) return MMM_OK;
-  MMM_CUDA(h, cudaMalloc((void**)p, count * sizeof(T)));
-  return MMM_OK;
-}
-
 }  // namespace
 
-int mmm_cutoff_alloc(mmm_system* h) {
+static int mmm_cutoff_alloc(mmm_system* h) {
   const size_t n = (size_t)h->n, npad = (size_t)h->npad;
   const int nblocks = (int)((n + kSortChunk - 1) / kSortChunk);
   int rc;
-  if ((rc = alloc_once(h, &h->d_keys, n))) return rc;
-  if ((rc = alloc_once(h, &h->d_keys_tmp, n))) return rc;
-  if ((rc = alloc_once(h, &h->d_order, npad))) return rc;
-  if ((rc = alloc_once(h, &h->d_order_tmp, npad))) return rc;
-  if ((rc = alloc_once(h, &h->d_pos4_sorted, npad))) return rc;
-  if ((rc = alloc_once(h, &h->d_soa_sorted, 3 * npad))) return rc;
-  if ((rc = alloc_once(h, &h->d_tiles_sorted, npad / MMM_TILE))) return rc;
-  if ((rc = alloc_once(h, &h->d_stage_boxes, npad / MMM_STAGE))) return rc;
-  if ((rc = alloc_once(h, (CutGrid**)&h->d_cell_grid, 1))) return rc;
-  if ((rc = alloc_once(h, &h->d_sort_table, (size_t)kDigits * nblocks))) return rc;
+  // keys, order, sorted positions and grid are shared with mmm_cells.cu: both reserve npad (the most either uses)
+  if ((rc = mmm_reserve(h, h->d_keys, npad, "cell keys")) || (rc = mmm_reserve(h, h->d_keys_tmp, npad, "cell keys")) ||
+      (rc = mmm_reserve(h, h->d_order, npad, "sorted order")) ||
+      (rc = mmm_reserve(h, h->d_order_tmp, npad, "sorted order")) ||
+      (rc = mmm_reserve(h, h->d_pos4_sorted, npad, "sorted positions")) ||
+      (rc = mmm_reserve(h, h->d_cell_grid, 1, "cell grid")) ||
+      (rc = mmm_reserve(h, h->d_soa_sorted, 3 * npad, "sorted coordinate planes")) ||
+      (rc = mmm_reserve(h, h->d_tiles_sorted, npad / MMM_TILE, "sorted tile boxes")) ||
+      (rc = mmm_reserve(h, h->d_stage_boxes, npad / MMM_STAGE, "sorted stage boxes")) ||
+      (rc = mmm_reserve(h, h->d_sort_table, (size_t)kDigits * nblocks, "radix-sort table")))
+    return rc;
   return MMM_OK;
 }
 
@@ -313,7 +302,7 @@ int mmm_cutoff_alloc(mmm_system* h) {
 static int rebuild_order(mmm_system* h, const int* d_skip) {
   const int n = (int)h->n, npad = (int)h->npad;
   const int nblocks = (n + kSortChunk - 1) / kSortChunk;
-  CutGrid* grid = reinterpret_cast<CutGrid*>(h->d_cell_grid);
+  CellGrid* grid = h->d_cell_grid;
   k_cut_grid<<<1, 256, 0, h->stream>>>(h->d_tiles, (int)h->ntiles, (float)h->cutoff, grid, d_skip);
   k_cut_keys<<<(n + 255) / 256, 256, 0, h->stream>>>(h->d_pos4, n, grid, h->d_keys_tmp, h->d_order_tmp, d_skip);
   uint32_t* kin = h->d_keys_tmp; uint32_t* kout = h->d_keys;
@@ -364,13 +353,3 @@ int mmm_launch_pair_cutoff_n3(mmm_system* h, const int* d_skip) {
 }
 
 int mmm_cutoff_resort_period() { return kResortEvery; }
-
-int mmm_cutoff_read_grid(mmm_system* h, float* cell, int32_t* dim, float* origin) {
-  CutGrid g;
-  MMM_CUDA(h, cudaMemcpyAsync(&g, h->d_cell_grid, sizeof(g), cudaMemcpyDeviceToHost, h->stream));
-  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  if (cell) *cell = g.cell;
-  if (dim) *dim = g.dim;
-  if (origin) *origin = g.origin;
-  return MMM_OK;
-}

@@ -88,10 +88,10 @@ static int setup_global_queue(mmm_system* h, NcclApi* a) {
   ncclComm_t comm = (ncclComm_t)h->nccl_comm;
   cudaIpcMemHandle_t handle;
   memset(&handle, 0, sizeof(handle));
-  int* mine = nullptr;
+  DevBuf<int> mine;  // rank 0: the counters, handed to h->d_gqueue when every rank can reach them
   int ok = 1;
   if (h->dist_rank == 0) {
-    if (cudaMalloc((void**)&mine, 2 * sizeof(int)) != cudaSuccess || cudaMemset(mine, 0, 2 * sizeof(int)) != cudaSuccess ||
+    if (mmm_reserve(h, mine, 2, "work-queue counters") != MMM_OK || cudaMemset(mine, 0, 2 * sizeof(int)) != cudaSuccess ||
         cudaIpcGetMemHandle(&handle, mine) != cudaSuccess) {
       cudaGetLastError();
       ok = 0;
@@ -101,14 +101,14 @@ static int setup_global_queue(mmm_system* h, NcclApi* a) {
   struct Msg { int ok; cudaIpcMemHandle_t handle; } msg;
   msg.ok = ok;
   msg.handle = handle;
-  Msg* d_msg = nullptr;
-  MMM_CUDA(h, cudaMalloc((void**)&d_msg, sizeof(Msg)));
+  DevBuf<Msg> d_msg;
+  int rc;
+  if ((rc = mmm_reserve(h, d_msg, 1, "work-queue handle"))) return rc;
   MMM_CUDA(h, cudaMemcpyAsync(d_msg, &msg, sizeof(Msg), cudaMemcpyHostToDevice, h->stream));
   ncclResult_t r = a->Broadcast(d_msg, d_msg, sizeof(Msg), ncclChar, 0, comm, h->stream);
-  if (r != ncclSuccess) { cudaFree(d_msg); return nccl_fail(h, a, r, "broadcast of the work-queue handle"); }
+  if (r != ncclSuccess) return nccl_fail(h, a, r, "broadcast of the work-queue handle");
   MMM_CUDA(h, cudaMemcpyAsync(&msg, d_msg, sizeof(Msg), cudaMemcpyDeviceToHost, h->stream));
   MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  cudaFree(d_msg);
   // every rank reports whether it can reach the counters; the queue is used only if all can
   int can = msg.ok;
   int* ptr = mine;
@@ -120,25 +120,21 @@ static int setup_global_queue(mmm_system* h, NcclApi* a) {
     }
     ptr = (int*)p;
   }
-  unsigned long long* d_votes = nullptr;
-  MMM_CUDA(h, cudaMalloc((void**)&d_votes, sizeof(unsigned long long)));
+  DevBuf<unsigned long long> d_votes;
+  if ((rc = mmm_reserve(h, d_votes, 1, "work-queue votes"))) return rc;
   const unsigned long long vote = can ? 1ull : 0ull;
   MMM_CUDA(h, cudaMemcpyAsync(d_votes, &vote, sizeof(vote), cudaMemcpyHostToDevice, h->stream));
   r = a->AllReduce(d_votes, d_votes, 1, ncclUint64, ncclSum, comm, h->stream);
-  unsigned long long votes = 0;
-  if (r == ncclSuccess) {
-    cudaMemcpyAsync(&votes, d_votes, sizeof(votes), cudaMemcpyDeviceToHost, h->stream);
-    cudaStreamSynchronize(h->stream);
-  }
-  cudaFree(d_votes);
   if (r != ncclSuccess) return nccl_fail(h, a, r, "all-reduce of the work-queue votes");
+  unsigned long long votes = 0;
+  MMM_CUDA(h, cudaMemcpyAsync(&votes, d_votes, sizeof(votes), cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
   if (votes == (unsigned long long)h->dist_world) {
-    h->d_gqueue = ptr;
+    h->d_gqueue = h->dist_rank == 0 ? mine.release() : ptr;
     h->gqueue_owner = h->dist_rank == 0;
     h->gqueue_eval = 0;
-  } else {  // somebody cannot: everybody falls back to static dealing
-    if (h->dist_rank == 0) { if (mine) cudaFree(mine); }
-    else if (can && ptr) cudaIpcCloseMemHandle(ptr);
+  } else if (h->dist_rank != 0 && can && ptr) {  // somebody cannot: everybody falls back to static dealing
+    cudaIpcCloseMemHandle(ptr);
   }
   return MMM_OK;
 }

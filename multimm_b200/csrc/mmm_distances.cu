@@ -168,31 +168,7 @@ __global__ void __launch_bounds__(256) k_dm_bbox(const double* __restrict__ x, i
   }
 }
 
-template <typename T>
-int dm_alloc(mmm_system* h, T** p, size_t count) {
-  if (*p) return MMM_OK;
-  cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-  if (e != cudaSuccess) {
-    *p = nullptr;
-    return mmm_fail(h, MMM_ERR_NOMEM, std::string("CUDA error: ") + cudaGetErrorString(e) + " (cudaMalloc, distance map)");
-  }
-  return MMM_OK;
-}
-
 }  // namespace
-
-void mmm_distances_free(mmm_system* h) {
-  void* ptrs[] = {h->d_dm_bin, h->d_dm_map, h->d_dm_box};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  h->d_dm_bin = nullptr;
-  h->d_dm_map = nullptr;
-  h->d_dm_box = nullptr;
-  h->dm_map_cap = 0;
-  if (h->dm_ev0) cudaEventDestroy(h->dm_ev0);
-  if (h->dm_ev1) cudaEventDestroy(h->dm_ev1);
-  h->dm_ev0 = h->dm_ev1 = nullptr;
-}
 
 extern "C" int mmm_distance_map(mmm_handle h, const int32_t* bin_of_bead, int32_t n_bins, uint64_t* dist_sum_out,
                                 uint64_t* dist2_sum_out, float* device_ms_out) {
@@ -210,19 +186,12 @@ extern "C" int mmm_distance_map(mmm_handle h, const int32_t* bin_of_bead, int32_
   cudaSetDevice(h->device);
   int rc;
   const size_t cells = (size_t)n_bins * (size_t)n_bins;
-  if ((rc = dm_alloc(h, &h->d_dm_bin, (size_t)std::max(n, 1)))) return rc;
-  if ((rc = dm_alloc(h, &h->d_dm_box, (size_t)DM_BOX_BLOCKS * 6))) return rc;
+  if ((rc = mmm_reserve(h, h->d_dm_bin, (size_t)std::max(n, 1), "distance-map bins")) ||
+      (rc = mmm_reserve(h, h->d_dm_box, (size_t)DM_BOX_BLOCKS * 6, "distance-map boxes")) ||
+      (rc = mmm_reserve(h, h->d_dm_map, 2 * cells, "distance map")))
+    return rc;
   if (!h->dm_ev0) MMM_CUDA(h, cudaEventCreate(&h->dm_ev0));
   if (!h->dm_ev1) MMM_CUDA(h, cudaEventCreate(&h->dm_ev1));
-  if (h->dm_map_cap < cells) {
-    if (h->d_dm_map) {
-      MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-      cudaFree(h->d_dm_map);
-      h->d_dm_map = nullptr;
-    }
-    if ((rc = dm_alloc(h, &h->d_dm_map, 2 * cells))) return rc;
-    h->dm_map_cap = cells;
-  }
   unsigned long long* dmap = h->d_dm_map;
   unsigned long long* d2map = h->d_dm_map + cells;
 

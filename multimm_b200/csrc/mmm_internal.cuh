@@ -96,6 +96,50 @@ struct LbfgsState {
 
 enum ApplyFlag { APPLY_NONE = 0, APPLY_INIT = 1, APPLY_RETRY = 2, APPLY_ACCEPT = 3, APPLY_RESTORE = 4 };
 
+// Grid of the cut-off mode's cell keys, written on the device by k_cut_grid (mmm_cutoff.cu) or
+// k_cell_grid (mmm_cells.cu) into the one d_cell_grid of the handle, and read back by mmm_get_cell_grid.
+struct CellGrid {
+  float origin, cell;  // lower corner (every axis) and edge of a cubic cell
+  int dim, bits;       // cells per axis, key bits per axis
+};
+
+// ---------------------------------------------------------------------------------------
+// device memory
+// ---------------------------------------------------------------------------------------
+template <class T> class DevBuf;
+template <class T> int mmm_reserve(mmm_system* h, DevBuf<T>& buf, size_t count, const char* what);
+
+// An owning device buffer of up to cap_ elements of T.  It converts to T*, so kernel arguments and
+// pointer arithmetic read as for a raw pointer.  It grows only through mmm_reserve; the destructor
+// and reset() free it.
+template <class T>
+class DevBuf {
+ public:
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { reset(); }
+  operator T*() const { return p_; }
+  T* get() const { return p_; }  // for a conditional expression or a cast
+  T* operator->() const { return p_; }
+  void reset() {
+    if (p_) cudaFree(p_);
+    p_ = nullptr;
+    cap_ = 0;
+  }
+  T* release() {  // the caller frees what it gets
+    T* p = p_;
+    p_ = nullptr;
+    cap_ = 0;
+    return p;
+  }
+
+ private:
+  friend int mmm_reserve<T>(mmm_system* h, DevBuf<T>& buf, size_t count, const char* what);
+  T* p_ = nullptr;
+  size_t cap_ = 0;
+};
+
 // ---------------------------------------------------------------------------------------
 // the handle
 // ---------------------------------------------------------------------------------------
@@ -120,48 +164,49 @@ struct mmm_system {
   bool types_dirty = true;
 
   // per-bead parameters
-  int* d_type = nullptr;         // packed type bits [npad]
-  double* d_cstr = nullptr;      // chrom_strength [n]
-  signed char* d_s = nullptr;    // compartment label [n]
+  DevBuf<int> d_type;            // packed type bits [npad]
+  DevBuf<double> d_cstr;         // chrom_strength [n]
+  DevBuf<signed char> d_s;       // compartment label [n]
 
   // topology in gather (CSR) form
   int64_t n_bonds = 0, n_loops = 0, n_angles = 0;
   int loop_form = 0;
-  int* d_bl_ptr = nullptr;       // [n+1]
-  int* d_bl_partner = nullptr;   // [2*(nb+nl)]
-  int* d_bl_flags = nullptr;     // bit0: entry owns the energy; bits 1-2: 0 backbone bond, else 1 + loop form
-  double* d_bl_r0 = nullptr;
-  double* d_bl_k = nullptr;
-  int* d_an_ptr = nullptr;       // [n+1]
-  int4* d_an_ijk = nullptr;      // [3*na] (i, j, k, role)
-  double2* d_an_par = nullptr;   // [3*na] (theta0, k)
+  DevBuf<int> d_bl_ptr;          // [n+1]
+  DevBuf<int> d_bl_partner;      // [2*(nb+nl)]
+  DevBuf<int> d_bl_flags;        // bit0: entry owns the energy; bits 1-2: 0 backbone bond, else 1 + loop form
+  DevBuf<double> d_bl_r0;
+  DevBuf<double> d_bl_k;
+  DevBuf<int> d_an_ptr;          // [n+1]
+  DevBuf<int4> d_an_ijk;         // [3*na] (i, j, k, role)
+  DevBuf<double2> d_an_par;      // [3*na] (theta0, k)
   std::vector<int32_t> h_bond_i, h_bond_j, h_loop_i, h_loop_j;
   std::vector<double> h_bond_r0, h_bond_k, h_loop_r0, h_loop_k;
   bool topo_dirty = true;
 
   // state
-  double* d_x = nullptr;         // [3n] master positions (nm), row-major N x 3
-  double* d_center = nullptr;    // [3] centre used for the FP32 copy
-  float4* d_pos4 = nullptr;      // [npad] centred FP32 xyz + type bits
-  float* d_soa = nullptr;        // [3][npad] the same coordinates as planes
-  TileInfo* d_tiles = nullptr;   // [ntiles]
-  double* d_g = nullptr;         // [3n] gradient (= -force)
+  DevBuf<double> d_x;            // [3n] master positions (nm), row-major N x 3
+  DevBuf<double> d_center;       // [3] centre used for the FP32 copy
+  DevBuf<float4> d_pos4;         // [npad] centred FP32 xyz + type bits
+  DevBuf<float> d_soa;           // [3][npad] the same coordinates as planes
+  DevBuf<TileInfo> d_tiles;      // [ntiles]
+  DevBuf<double> d_g;            // [3n] gradient (= -force)
 
   // pair-kernel scratch
   int nchunk = 1;
   int n_planes = 0;              // planes of d_fpair the assemble pass sums (gather chunks + cell-list plane)
   int chunk_tiles = 0;           // j-tiles per chunk (a whole number of stages)
   int scratch_sig = -1;
-  double* d_fpair = nullptr;     // [nchunk][3][npad]
-  double* d_epair = nullptr;     // [items][4]
+  DevBuf<double> d_fpair;        // [nchunk][3][npad]
+  DevBuf<double> d_epair_buf;    // [items][4] energy slots (single GPU)
+  double* d_epair = nullptr;     // d_epair_buf; several GPUs: the tail of d_facc (one all-reduce covers both)
   int64_t n_items = 0;
-  int* d_counter = nullptr;      // dynamic work counter
+  DevBuf<int> d_counter;         // dynamic work counter
   // pair_mode: which kernel the scratch is sized for. 0 none, 1 gather (mmm_pair.cu),
   // 2 Newton-3 (mmm_pair_n3.cu), 3 cut-off cell list (mmm_cells.cu)
   int pair_mode = 0;
   int pair_kernel_pref = 0;      // 0 auto, 1 force the gather kernel (tests / A-B timing)
-  unsigned long long* d_facc = nullptr;  // [3][npad] fixed-point force accumulator (Newton-3, cells)
-  int2* d_items = nullptr;       // Newton-3 work items
+  DevBuf<unsigned long long> d_facc;  // [3][npad] fixed-point force accumulator (Newton-3, cells)
+  DevBuf<int2> d_items;          // Newton-3 work items
   // several GPUs, one system (mmm_dist.cu): Newton-3 items are dealt round-robin to the ranks
   int dist_rank = 0, dist_world = 1;
   bool dist_emulate = false;     // run every rank's share on this GPU, one after another (tests)
@@ -169,7 +214,6 @@ struct mmm_system {
   int* d_gqueue = nullptr;       // two ticket counters in rank 0's memory (CUDA IPC): one work queue for all GPUs
   bool gqueue_owner = false;
   int64_t gqueue_eval = 0;       // evaluations drawn from the queue so far (selects the counter)
-  bool epair_aliased = false;    // dist: d_epair is the tail of the d_facc allocation (one all-reduce covers both)
   cudaEvent_t ev_c0 = nullptr, ev_c1 = nullptr;  // around the exchange step of the last evaluation (dist)
   int n3_items = 0;              // number of Newton-3 work items (their energy slots come first in d_epair)
   bool n3_chb_only = false;      // the item list is the cut-off mode's CHB-only list
@@ -178,19 +222,19 @@ struct mmm_system {
   // reductions
   int n_red_blocks = 0;
   int n_dot_blocks = 0;
-  double* d_epart = nullptr;     // [n_red_blocks][6] external+bonded energy partials
-  double* d_dpart = nullptr;     // [n_red_blocks][MMM_NDOT] dot partials
-  double* d_eterms = nullptr;    // [MMM_NUM_TERMS] result of the last evaluation
+  DevBuf<double> d_epart;        // [n_red_blocks][6] external+bonded energy partials
+  DevBuf<double> d_dpart;        // [n_red_blocks][MMM_NDOT] dot partials
+  DevBuf<double> d_eterms;       // [MMM_NUM_TERMS] result of the last evaluation
   bool have_result = false;      // d_eterms / d_g hold a finished stand-alone evaluation (mmm_last_result)
 
   // L-BFGS
-  LbfgsState* d_lb = nullptr;
-  double *d_xp = nullptr, *d_gp = nullptr, *d_d = nullptr;
-  double *d_S = nullptr, *d_Y = nullptr;  // [m][3n]
+  DevBuf<LbfgsState> d_lb;
+  DevBuf<double> d_xp, d_gp, d_d;
+  DevBuf<double> d_S, d_Y;       // [m][3n]
   int* h_done = nullptr;         // pinned mirror of LbfgsState::done / counters
 
   // MD relaxation (mmm_md.cu)
-  double* d_v = nullptr;         // [3n] velocities, nm/ps
+  DevBuf<double> d_v;            // [3n] velocities, nm/ps
   bool md_configured = false;
   int md_integrator = 0;
   double md_dt = 0.001, md_temperature = 310.0, md_gamma = 0.5, md_mass = 16427.889;
@@ -199,40 +243,38 @@ struct mmm_system {
   int64_t md_step = 0;
 
   // cell list (cutoff mode)
-  uint32_t* d_keys = nullptr;    // [n] sorted keys
-  int* d_order = nullptr;        // [n] sorted bead order
-  uint32_t* d_keys_tmp = nullptr;
-  int* d_order_tmp = nullptr;
-  float4* d_pos4_sorted = nullptr;
-  int* d_cell_start = nullptr;   // [ncells+1]
-  void* d_sort_tmp = nullptr;
-  size_t sort_tmp_bytes = 0;
-  void* d_cell_grid = nullptr;   // device CellGrid {origin, cell, dim, bits}
-  unsigned long long* d_cell_npairs = nullptr;  // ordered pairs inside the cut-off, per CTA
+  DevBuf<uint32_t> d_keys;       // [n] sorted keys
+  DevBuf<int> d_order;           // [n] sorted bead order
+  DevBuf<uint32_t> d_keys_tmp;
+  DevBuf<int> d_order_tmp;
+  DevBuf<float4> d_pos4_sorted;
+  DevBuf<int> d_cell_start;      // [ncells+1]
+  DevBuf<int> d_sort_tmp;        // [2][cells] per-cell histogram, placement cursor
+  DevBuf<CellGrid> d_cell_grid;
+  DevBuf<unsigned long long> d_cell_npairs;  // ordered pairs inside the cut-off, per CTA
   // cut-off mode on the Newton-3 machinery (mmm_cutoff.cu; default functional forms)
   bool cut_n3 = false;           // the cut-off pass runs the CUT variant of k_pair_n3 (else k_pair_cells)
-  float* d_soa_sorted = nullptr;       // [3][npad] coordinate planes in Morton-sorted order
-  TileInfo* d_tiles_sorted = nullptr;  // [npad / 32] boxes of the sorted tiles
-  TileInfo* d_stage_boxes = nullptr;   // [npad / 256] boxes of the sorted stages
-  int* d_sort_table = nullptr;         // radix-sort digit x block table
-  int2* d_items_cut = nullptr;         // all-pairs item table the CUT kernel culls from
+  DevBuf<float> d_soa_sorted;          // [3][npad] coordinate planes in Morton-sorted order
+  DevBuf<TileInfo> d_tiles_sorted;     // [npad / 32] boxes of the sorted tiles
+  DevBuf<TileInfo> d_stage_boxes;      // [npad / 256] boxes of the sorted stages
+  DevBuf<int> d_sort_table;            // radix-sort digit x block table
+  DevBuf<int2> d_items_cut;            // all-pairs item table the CUT kernel culls from
   int n_items_cut = 0;
   std::vector<int32_t> h_cut_iblk;     // i-block of every item of d_items_cut (slab boundaries of the sharded mode)
-  double* d_cut_npairs = nullptr;      // [n_items_cut] pairs inside the cut-off (warp kernel: one per rank)
+  DevBuf<double> d_cut_npairs;         // [n_items_cut] pairs inside the cut-off (warp kernel: one per rank)
   bool cut_warp = false;               // the one-warp-per-item kernel serves the cut-off pass (else the CTA-level CUT variant)
   int n_cut_slots = 0;                 // energy slots of the cut-off pass
-  unsigned long long* d_cut_eacc = nullptr;  // [4] fixed-point energies + pair count (warp kernel)
+  DevBuf<unsigned long long> d_cut_eacc;  // [4] fixed-point energies + pair count (warp kernel)
   int sort_age = 0;                    // evaluations since the Morton order was rebuilt (0: rebuild now)
   // CHB on cluster centroids (mmm_chb_clusters.cu): coarse-stage surrogate, cut-off mode only
   bool chb_surrogate = false;    // requested (mmm_set_chb_surrogate)
   bool chb_clusters = false;     // in force for the current scratch
   int n_clusters = 0;
-  int* d_cl_start = nullptr;     // [n_clusters + 1] first bead of every cluster
-  int* d_cl_of_bead = nullptr;   // [n] cluster of every bead
-  int* d_cl_by_chrom = nullptr;  // [n_clusters] clusters sorted by chromosome id
-  int2* d_cl_range = nullptr;    // [n_clusters] slots of by_chrom that hold the same chromosome
-  double* d_cl_cen = nullptr;    // [n_clusters][4] centroid, bead count
-  double* d_cl_force = nullptr;  // [n_clusters][3] force on every bead of the cluster
+  DevBuf<int> d_cl_start;        // [n_clusters + 1] first bead of every cluster
+  DevBuf<int> d_cl_of_bead;      // [n] cluster of every bead
+  DevBuf<int> d_cl_by_chrom;     // [n_clusters] clusters sorted by chromosome id
+  DevBuf<double> d_cl_cen;       // [n_clusters][4] centroid, bead count
+  DevBuf<double> d_cl_force;     // [n_clusters][3] force on every bead of the cluster
   int64_t cl_item0 = 0;          // first d_epair item of the cluster pass
   int cells_plane = 0;           // plane of d_fpair the cell-list pass writes
   int64_t cells_item0 = 0;       // first d_epair item of the cell-list pass
@@ -241,35 +283,32 @@ struct mmm_system {
   cudaEvent_t ev_a = nullptr, ev_b = nullptr;
   std::vector<cudaEvent_t> ev_pool;  // per-launch event pairs while a timed batch runs
   int ev_cursor = -1;                // -1: not collecting
-  void* d_flush = nullptr;           // 256 MiB L2-flush scratch (bench only)
-  double* d_fout = nullptr;          // [3n] forces (= -gradient) staged for mmm_energy_forces' host copy
+  DevBuf<unsigned char> d_flush;     // 256 MiB L2-flush scratch (bench only)
+  DevBuf<double> d_fout;             // [3n] forces (= -gradient) staged for mmm_energy_forces' host copy
   float last_pair_ms = 0.f;
 
   // contact counting (mmm_contacts.cu): scratch kept for the handle's lifetime
-  int* d_ct_bin = nullptr;                 // [n] bin of every bead
-  unsigned long long* d_ct_map = nullptr;  // [ct_map_cap] dense bin x bin counts
-  size_t ct_map_cap = 0;
-  unsigned long long* d_ct_sep = nullptr;  // [n] same-chromosome contacts by index separation
-  TileInfo* d_ct_stage = nullptr;          // [stages] boxes of the chain-order 256-bead stages
-  unsigned long long* d_ct_cnt = nullptr;  // [2] contacts, candidate pairs tested
+  DevBuf<int> d_ct_bin;                    // [n] bin of every bead
+  DevBuf<unsigned long long> d_ct_map;     // [n_bins^2] dense bin x bin counts
+  DevBuf<unsigned long long> d_ct_sep;     // [n] same-chromosome contacts by index separation
+  DevBuf<TileInfo> d_ct_stage;             // [stages] boxes of the chain-order 256-bead stages
+  DevBuf<unsigned long long> d_ct_cnt;     // [2] contacts, candidate pairs tested
   int64_t ct_candidates = 0;               // candidate pairs the last call tested in FP64
   float ct_ms = 0.f;                       // device time of the last call's kernels (events below)
   cudaEvent_t ct_ev0 = nullptr, ct_ev1 = nullptr;
   // sparse map (mmm_contacts_sparse): grown to the binned contacts of the largest call so far
-  long long* d_cs_tile = nullptr;                       // [tiles + scan parts] int64 key counts -> offsets
-  unsigned long long* d_cs_keys[2] = {nullptr, nullptr};  // [cs_key_cap] each: the radix sort's buffers
-  long long* d_cs_table = nullptr;                      // digit x chunk table + scan parts; then run offsets
-  size_t cs_key_cap = 0;
+  DevBuf<long long> d_cs_tile;                          // [tiles + scan parts] int64 key counts -> offsets
+  DevBuf<unsigned long long> d_cs_keys[2];              // [keys] each: the radix sort's buffers
+  DevBuf<long long> d_cs_table;                         // digit x chunk table + scan parts; then run offsets
   int64_t cs_keys = 0, cs_entries = 0;                  // of the last call: binned contacts, entries
   int cs_src = 0;                                       // which d_cs_keys holds the sorted keys
   int32_t cs_nbins = 0;
   bool cs_valid = false;                                // a call succeeded; mmm_contacts_sparse_read may run
 
   // mean-distance maps (mmm_distances.cu): scratch kept for the handle's lifetime
-  int* d_dm_bin = nullptr;                 // [n] bin of every bead
-  unsigned long long* d_dm_map = nullptr;  // [2][dm_map_cap] quantised distance sums, then squared-distance sums
-  size_t dm_map_cap = 0;
-  double* d_dm_box = nullptr;              // per-block bounding boxes of the beads (overflow guard)
+  DevBuf<int> d_dm_bin;                    // [n] bin of every bead
+  DevBuf<unsigned long long> d_dm_map;     // [2][n_bins^2] quantised distance sums, then squared-distance sums
+  DevBuf<double> d_dm_box;                 // per-block bounding boxes of the beads (overflow guard)
   cudaEvent_t dm_ev0 = nullptr, dm_ev1 = nullptr;
 };
 
@@ -284,6 +323,40 @@ int mmm_fail(mmm_system* h, int code, const std::string& msg);
       return mmm_fail((h), MMM_ERR_CUDA,                                                   \
                       std::string("CUDA error: ") + cudaGetErrorString(_e) + " at " #call); \
   } while (0)
+
+// Make buf hold at least count elements.  A buffer that is large enough is left alone (same
+// pointer: captured graphs and earlier views stay valid); otherwise it is replaced by exactly
+// count elements, after the handle's stream is done with the old one.  Nothing allocates while a
+// graph is captured.  h may be NULL for a temporary of a call without a handle.
+template <class T>
+int mmm_reserve(mmm_system* h, DevBuf<T>& buf, size_t count, const char* what) {
+  if (count <= buf.cap_) return MMM_OK;
+  if (h && h->capturing)
+    return mmm_fail(h, MMM_ERR_STATE, std::string("allocation of ") + what + " while a CUDA graph is captured");
+  if (h && buf.p_) cudaStreamSynchronize(h->stream);
+  buf.reset();
+  cudaError_t e = cudaMalloc((void**)&buf.p_, count * sizeof(T));
+  if (e != cudaSuccess) {
+    buf.p_ = nullptr;
+    return mmm_fail(h, MMM_ERR_NOMEM, std::string("CUDA error: ") + cudaGetErrorString(e) + " (cudaMalloc, " + what + ")");
+  }
+  buf.cap_ = count;
+  return MMM_OK;
+}
+
+// Reserve and copy v from the host; an empty v leaves buf NULL.
+template <class T>
+int mmm_upload(mmm_system* h, DevBuf<T>& buf, const std::vector<T>& v, const char* what) {
+  if (v.empty()) {
+    buf.reset();
+    return MMM_OK;
+  }
+  int rc = mmm_reserve(h, buf, v.size(), what);
+  if (rc) return rc;
+  MMM_CUDA(h, cudaMemcpyAsync(buf, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MMM_OK;
+}
 
 // ---------------------------------------------------------------------------------------
 // kernel launchers (defined in the other .cu files)
@@ -307,7 +380,6 @@ int mmm_launch_pair_n3_cut(mmm_system* h, const int* d_skip);
 int mmm_cut_warp_build_items(mmm_system* h, std::vector<int2>& items);  // sorted arrays -> d_facc, d_epair (cut-off mode)
 // mmm_cutoff.cu
 int mmm_launch_pair_cutoff_n3(mmm_system* h, const int* d_skip);
-int mmm_cutoff_read_grid(mmm_system* h, float* cell, int32_t* dim, float* origin);
 int mmm_cutoff_resort_period();
 // mmm_chb_clusters.cu
 int mmm_chb_clusters_build(mmm_system* h);
@@ -316,10 +388,6 @@ int mmm_launch_chb_clusters(mmm_system* h, const int* d_skip);
 // mmm_cells.cu
 int mmm_launch_pair_cutoff(mmm_system* h, const int* d_skip);
 int64_t mmm_cells_energy_slots(const mmm_system* h);
-// mmm_contacts.cu
-void mmm_contacts_free(mmm_system* h);
-// mmm_distances.cu
-void mmm_distances_free(mmm_system* h);
 // mmm_bonded.cu
 int mmm_upload_topology(mmm_system* h);
 int mmm_upload_angles(mmm_system* h, const int32_t* ai, const int32_t* aj, const int32_t* ak,

@@ -129,9 +129,11 @@ __global__ void __launch_bounds__(256) k_md_v2(int64_t n3, const double* __restr
   if (threadIdx.x == 0) part[blockIdx.x] = s[0];
 }
 
+// velocities are zero until something sets them
 int ensure_velocities(mmm_system* h) {
   if (h->d_v) return MMM_OK;
-  MMM_CUDA(h, cudaMalloc((void**)&h->d_v, sizeof(double) * 3 * (size_t)h->n));
+  int rc = mmm_reserve(h, h->d_v, 3 * (size_t)h->n, "velocities");
+  if (rc) return rc;
   MMM_CUDA(h, cudaMemsetAsync(h->d_v, 0, sizeof(double) * 3 * (size_t)h->n, h->stream));
   return MMM_OK;
 }

@@ -45,8 +45,9 @@ extern "C" int mmm_measure_fp32_peak(int device, double* tflops_out, double* muf
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return MMM_ERR_CUDA;
   const int blocks = prop.multiProcessorCount * 8, threads = 256;
-  float* d_out = nullptr;
-  if (cudaMalloc((void**)&d_out, sizeof(float) * blocks * threads) != cudaSuccess) return MMM_ERR_NOMEM;
+  DevBuf<float> d_out;
+  int rc = mmm_reserve(nullptr, d_out, (size_t)blocks * threads, "peak-rate output");
+  if (rc) return rc;
   cudaEvent_t a, b;
   cudaEventCreate(&a);
   cudaEventCreate(&b);
@@ -71,7 +72,6 @@ extern "C" int mmm_measure_fp32_peak(int device, double* tflops_out, double* muf
   cudaError_t e = cudaGetLastError();
   cudaEventDestroy(a);
   cudaEventDestroy(b);
-  cudaFree(d_out);
   if (e != cudaSuccess) return MMM_ERR_CUDA;
   if (tflops_out) *tflops_out = best_f;
   if (mufu_tops_out) *mufu_tops_out = best_m;

@@ -1269,7 +1269,7 @@ int mmm_launch_pair_cut_warp(mmm_system* h, const int* d_skip) {
   A.stage_boxes = h->d_stage_boxes;
   A.perm = h->d_order;
   A.facc = h->d_facc;
-  A.eacc = reinterpret_cast<long long*>(h->d_cut_eacc);
+  A.eacc = reinterpret_cast<long long*>(h->d_cut_eacc.get());
   A.items = h->d_items_cut;
   A.counter = h->d_counter + 1;
   A.skip = d_skip;

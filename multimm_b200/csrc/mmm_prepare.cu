@@ -134,7 +134,7 @@ __global__ void __launch_bounds__(256) k_hilbert(int64_t n, int p, double spacin
 
 int mmm_launch_hilbert(mmm_system* h, int p, double spacing, int32_t* d_ijk) {
   const int64_t blocks = (h->n + 255) / 256;
-  k_hilbert<<<(unsigned)blocks, 256, 0, h->stream>>>(h->n, p, spacing, d_ijk ? nullptr : h->d_x, d_ijk);
+  k_hilbert<<<(unsigned)blocks, 256, 0, h->stream>>>(h->n, p, spacing, d_ijk ? nullptr : h->d_x.get(), d_ijk);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
   return MMM_OK;
