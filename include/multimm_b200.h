@@ -286,6 +286,45 @@ int mmm_contacts_stats(mmm_handle h, int64_t *candidates_out, float *device_ms_o
 int mmm_distance_map(mmm_handle h, const int32_t *bin_of_bead, int32_t n_bins, uint64_t *dist_sum_out,
                      uint64_t *dist2_sum_out, float *device_ms_out);
 
+/* ---- trajectory maps (contact and distance maps summed over many structures, e.g. the states of an MD
+ * run; not in the reference) ----------------------------------------------------------------------------- */
+/* Sets up the sampler of this handle and clears its sums: the contact radius and the bin tables (int32[N],
+ * -1 = the bead is left out), uploaded once.  A NULL table switches that map off:
+ *   contact_bins  (1 <= n_contact_bins <= 4096): the dense map, sep and pairs of mmm_contacts;
+ *   fine_bins     (1 <= n_fine_bins <= 2^31 - 1; needs contact_bins): the sparse map of mmm_contacts_sparse;
+ *   distance_bins (1 <= n_distance_bins <= 4096): dist_sum and dist2_sum of mmm_distance_map.
+ * MMM_ERR_ARG for both contact_bins and distance_bins NULL, fine_bins without contact_bins, rc <= 0 or not
+ * finite (with contact_bins), an n_bins outside its range or a bin id outside [-1, n_bins).  The sampler's
+ * buffers are its own (allocated here and as the fine map grows, freed with the handle). */
+int mmm_sampler_configure(mmm_handle h, double rc_nm, const int32_t *contact_bins, int32_t n_contact_bins,
+                          const int32_t *fine_bins, int32_t n_fine_bins, const int32_t *distance_bins,
+                          int32_t n_distance_bins);
+/* Adds the structure at the current positions to every configured map.  After K calls every output of
+ * mmm_sampler_read / mmm_sampler_read_fine equals, bit for bit, the sum of what the one-shot calls return at
+ * the same K positions and bins (integer sums: exact and independent of order); the fine map is the sorted
+ * union of the K sparse maps with the counts of equal keys added, built on the device by a merge of each
+ * structure's entries into the accumulated ones (work and memory O(accumulated + new entries)).  The
+ * int64 guard of mmm_distance_map is cumulative: MMM_ERR_ARG, with every map left as it was, when the
+ * structure's bound would take the sum of the bounds of the structures already added to 2^63.
+ * MMM_ERR_STATE before mmm_sampler_configure or before positions are set.  After any other error the
+ * sampler must be configured again.  Changes no state an evaluation, a minimisation, an MD step,
+ * mmm_last_result, mmm_contacts_stats or mmm_contacts_sparse_read reads; synchronises with the host (twice
+ * more with the fine map on, for its key and entry counts). */
+int mmm_sample(mmm_handle h);
+/* The sums of the structures added since mmm_sampler_configure: samples_out, the number of structures;
+ * contact_map_out (uint64, n_contact_bins^2), sep_out (uint64[N]), pairs_out; fine_entries_out, the entries
+ * of the fine map (for mmm_sampler_read_fine); dist_sum_out, dist2_sum_out (uint64, n_distance_bins^2);
+ * device_ms_out, the device time of all mmm_sample calls (CUDA events on the handle's stream, from the first
+ * pass to the last, the fine map's host waits included).  Any output may be NULL; those of a map that is off
+ * are left untouched.  MMM_ERR_STATE as mmm_sample. */
+int mmm_sampler_read(mmm_handle h, int64_t *samples_out, uint64_t *contact_map_out, uint64_t *sep_out,
+                     int64_t *pairs_out, int64_t *fine_entries_out, uint64_t *dist_sum_out, uint64_t *dist2_sum_out,
+                     float *device_ms_out);
+/* The fine map's entries, sorted by (row, col), row <= col, vals > 0, as mmm_contacts_sparse_read:
+ * rows_out, cols_out int32[fine_entries], vals_out uint64[fine_entries]; any may be NULL, and 0 entries
+ * succeeds.  MMM_ERR_STATE as mmm_sample. */
+int mmm_sampler_read_fine(mmm_handle h, int32_t *rows_out, int32_t *cols_out, uint64_t *vals_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

@@ -199,13 +199,18 @@ DISTANCE_FIELDS: dict[str, tuple[Any, Any]] = {
     "SAVE_DISTANCES": (B, False),         # distance sums of the minimised structure (analysis/distances.npz; ensembles: ensemble_distances.npz)
     "DISTANCE_RESOLUTION": (int, 0),      # bp per bin of the distance map; 0 = about 1000 bins, at most 4096 bins
 }
-EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS}
+# Trajectory maps: the maps above summed over structures sampled during MD (files *_md.npz), kept the same way.
+# Which maps are sampled follows SAVE_CONTACTS, CONTACT_FINE_RESOLUTION and SAVE_DISTANCES.
+MD_SAMPLE_FIELDS: dict[str, tuple[Any, Any]] = {
+    "MD_SAMPLE_STEP": (int, 0),           # MD steps between two structures added to the trajectory maps; 0 = off
+}
+EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
-    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS or DISTANCE_FIELDS setting of `args`, its default where
-    it was not given."""
+    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS or MD_SAMPLE_FIELDS setting of `args`, its
+    default where it was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

@@ -20,7 +20,14 @@ Files (numpy ``.npz``):
   ensemble.  Always sparse, never a dense ``counts`` (a 5 kb genome-wide map has ~6e5 bins): ``rows``,
   ``cols`` (int32), ``vals`` (uint64), the nonzero upper triangle sorted by (row, col) with rows <= cols;
   ``n_bins``, ``bin_chrom``, ``bin_start_bp``, ``resolution_bp``, ``radius_nm``, ``members``, ``pairs``.
-  Read it with ``load_fine``; ``coarsen`` and ``fine_block`` give dense views of it.
+  Read it with ``load_fine``; ``coarsen`` and ``fine_block`` give dense views of it;
+* the trajectory maps (``MD_SAMPLE_STEP``, ``Engine.sampler_read``): the same maps summed over the structures
+  sampled during MD, in the same formats, named with ``_md`` before ``.npz``: ``analysis/contacts_md.npz`` and
+  ``analysis/contacts_fine_md.npz`` of a single run, ``contacts/member_<i>_md.npz`` and
+  ``contacts/member_<i>_fine_md.npz`` of an ensemble member, ``ensemble_contacts_md.npz`` and
+  ``ensemble_contacts_fine_md.npz`` of an ensemble.  A file of S sampled structures is their sum exactly as an
+  ensemble file is the sum of its members: ``members`` = S and ``sep_pairs`` S times one structure's, so
+  ``contact_probability``, ``aggregate``, ``aggregate_fine``, ``coarsen`` and ``fine_block`` read it unchanged.
 """
 from __future__ import annotations
 
@@ -142,6 +149,11 @@ def contact_probability(d: dict) -> np.ndarray:
     den = np.asarray(d["sep_pairs"], np.float64)
     with np.errstate(invalid="ignore", divide="ignore"):
         return np.where(den > 0, num / np.where(den > 0, den, 1.0), np.nan)
+
+
+def md_path(path: str) -> str:
+    """The trajectory-map file beside a structure's map file: ``_md`` before ``.npz``."""
+    return path[:-len(".npz")] + "_md.npz"
 
 
 def _write(path: str, arrays: dict):

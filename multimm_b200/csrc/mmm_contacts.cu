@@ -24,6 +24,12 @@
 // k_rle<kSplit> (row = key / n_bins, col = key % n_bins of every head).
 // Scratch: 2 x 8 B per binned contact (the two sort buffers; the read reuses the free one), a digit x
 // chunk table of 8 B x 256 per 4096 keys, and O(N) for the per-tile offsets.
+//
+// The trajectory sampler (mmm_sampler.cu) runs the dense pass and the sparse pass through the same functions
+// (mmm_contacts_dense_pass, mmm_contacts_sparse_pass) into its own buffers; its fine map adds
+//   k_rle<kKeyVals>         sorted keys -> unique (key, count) list of the structure
+//   k_merge_part, k_merge   merge-path merge with the accumulated (key, count) list
+//   k_rle<kCount>, scan, k_rle<kKeyVals>   equal keys (at most two, adjacent) -> one entry, counts added
 #include <math.h>
 
 #include <algorithm>
@@ -321,14 +327,18 @@ __global__ void __launch_bounds__(CS_THREADS) k_rs_scatter(const unsigned long l
 // ---- runs of equal sorted keys -> entries -------------------------------------------------------------
 // Thread t of block b owns keys [b * 4096 + 16 t, + 16); a head is a key unlike its predecessor, and entry
 // e(k) of key k = (heads at or before k) - 1.  kCount: heads of the chunk -> cnt[b].  kVals: vals[e] +=
-// the length of every piece of a run the thread holds (integer atomics: exact in any order; vals zeroed).
-// kSplit: rows[e] = key / n_bins, cols[e] = key % n_bins at every head.  off = the scanned kCount output.
-enum RleMode { kCount, kVals, kSplit };
+// the weight of every piece of a run the thread holds, a key weighing in_vals[k] (1 when in_vals is NULL;
+// integer atomics: exact in any order; vals zeroed).  kKeyVals: kVals, and out_keys[e] = key at every head
+// (a sorted, unique (key, value) list).  kSplit: rows[e] = key / n_bins, cols[e] = key % n_bins at every
+// head.  off = the scanned kCount output.
+enum RleMode { kCount, kVals, kKeyVals, kSplit };
 template <RleMode kMode>
 __global__ void __launch_bounds__(CS_THREADS) k_rle(const unsigned long long* __restrict__ keys, long long n,
                                                     long long* __restrict__ cnt, const long long* __restrict__ off,
-                                                    unsigned nbins, unsigned long long* __restrict__ vals,
-                                                    int* __restrict__ rows, int* __restrict__ cols) {
+                                                    unsigned nbins, const unsigned long long* __restrict__ in_vals,
+                                                    unsigned long long* __restrict__ vals,
+                                                    unsigned long long* __restrict__ out_keys, int* __restrict__ rows,
+                                                    int* __restrict__ cols) {
   __shared__ long long s_warp[CS_THREADS / 32];
   const long long base = (long long)blockIdx.x * CS_CHUNK + (long long)threadIdx.x * CS_PER;
   unsigned long long prev = base > 0 && base - 1 < n ? keys[base - 1] : ~0ull;  // no key is ~0 (< 2^62)
@@ -345,23 +355,80 @@ __global__ void __launch_bounds__(CS_THREADS) k_rle(const unsigned long long* __
     if (threadIdx.x == 0) cnt[blockIdx.x] = total;
     return;
   }
+  constexpr bool kSum = kMode == kVals || kMode == kKeyVals;
   long long e = off[blockIdx.x] + before - 1;  // entry of the key before this thread's first
   unsigned long long len = 0;
 #pragma unroll
   for (int q = 0; q < CS_PER; ++q) {
     if (base + q >= n) break;
     if (k[q] != (q ? k[q - 1] : prev)) {
-      if (kMode == kVals && len) atomicAdd(&vals[e], len);
+      if (kSum && len) atomicAdd(&vals[e], len);
       ++e;
       len = 0;
+      if (kMode == kKeyVals) out_keys[e] = k[q];
       if (kMode == kSplit) {
         rows[e] = (int)(k[q] / nbins);
         cols[e] = (int)(k[q] % nbins);
       }
     }
-    ++len;
+    if (kSum) len += in_vals ? in_vals[base + q] : 1ull;
   }
-  if (kMode == kVals && len) atomicAdd(&vals[e], len);
+  if (kSum && len) atomicAdd(&vals[e], len);
+}
+
+// ---- merge of two sorted (key, value) lists (the trajectory sampler's fine map) -------------------------
+// Merge path: output position d of the merge of A (na keys) and B (nb keys) takes i keys from A and d - i
+// from B, i the smallest with A[i] > B[d - 1 - i] (A first among equal keys).  k_merge_part finds i at the
+// first output of every CTA; k_merge stages the CTA's slices of A and B in shared memory, and each thread
+// finds its own diagonal there and merges MG_PER outputs.  Keys are unique within each list, so a key
+// appears at most twice in the output, adjacent; k_rle<kKeyVals> then adds the two values.
+constexpr int MG_THREADS = 256, MG_PER = 8, MG_TILE = MG_THREADS * MG_PER;
+
+__device__ __forceinline__ long long mg_diag(const unsigned long long* a, long long na, const unsigned long long* b,
+                                             long long nb, long long d) {
+  long long lo = d > nb ? d - nb : 0, hi = d < na ? d : na;
+  while (lo < hi) {
+    const long long mid = (lo + hi) >> 1;
+    if (a[mid] <= b[d - 1 - mid]) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(256) k_merge_part(const unsigned long long* __restrict__ a, long long na,
+                                                    const unsigned long long* __restrict__ b, long long nb, int nparts,
+                                                    long long* __restrict__ part) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p > nparts) return;
+  const long long d = (long long)p * MG_TILE;
+  part[p] = mg_diag(a, na, b, nb, d < na + nb ? d : na + nb);
+}
+
+__global__ void __launch_bounds__(MG_THREADS) k_merge(const unsigned long long* __restrict__ akey,
+                                                      const unsigned long long* __restrict__ aval, long long na,
+                                                      const unsigned long long* __restrict__ bkey,
+                                                      const unsigned long long* __restrict__ bval, long long nb,
+                                                      const long long* __restrict__ part,
+                                                      unsigned long long* __restrict__ okey,
+                                                      unsigned long long* __restrict__ oval) {
+  __shared__ unsigned long long s_key[MG_TILE], s_val[MG_TILE];
+  const long long d0 = (long long)blockIdx.x * MG_TILE, d1 = d0 + MG_TILE < na + nb ? d0 + MG_TILE : na + nb;
+  const long long a0 = part[blockIdx.x], a1 = part[blockIdx.x + 1];
+  const int la = (int)(a1 - a0), lb = (int)((d1 - a1) - (d0 - a0));
+  for (int t = threadIdx.x; t < la + lb; t += MG_THREADS) {  // A's slice, then B's
+    const long long g = t < la ? a0 + t : d0 - a0 + (t - la);
+    s_key[t] = t < la ? akey[g] : bkey[g];
+    s_val[t] = t < la ? aval[g] : bval[g];
+  }
+  __syncthreads();
+  const int d = min((int)threadIdx.x * MG_PER, la + lb);
+  int i = (int)mg_diag(s_key, la, s_key + la, lb, d), j = d - i;
+  for (int q = 0; q < MG_PER && d + q < la + lb; ++q) {
+    const bool take_a = i < la && (j >= lb || s_key[i] <= s_key[la + j]);
+    const int s = take_a ? i++ : la + j++;
+    okey[d0 + d + q] = s_key[s];
+    oval[d0 + d + q] = s_val[s];
+  }
 }
 
 // exclusive scan of a[0, len) in place; part: ceil(len / CS_CHUNK) + 1 entries, the last receives the total
@@ -395,6 +462,200 @@ int ct_check_args(mmm_system* h, const char* who, double rc_nm, const int32_t* b
 
 }  // namespace
 
+// The dense pass: contacts at the current positions added into map (n_bins^2; NULL: none, and then d_bin may
+// be NULL), sep (n) and cnt[2] (contacts, candidates), which are zeroed first when clear.  ev0 (may be NULL)
+// is recorded after the clearing.  mmm_contacts and the trajectory sampler run it.
+int mmm_contacts_dense_pass(mmm_system* h, double rc_nm, const int* d_bin, int32_t n_bins, unsigned long long* map,
+                            unsigned long long* sep, unsigned long long* cnt, bool clear, cudaEvent_t ev0) {
+  const int n = (int)h->n;
+  const int ntr = (n + MMM_TILE - 1) / MMM_TILE;                    // tiles holding a real bead
+  const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;  // stages holding a real tile
+  int rc;
+  if ((rc = mmm_reserve(h, h->d_ct_stage, (size_t)nst, "contact stage boxes"))) return rc;
+  if (clear) {
+    if (map)
+      MMM_CUDA(h, cudaMemsetAsync(map, 0, sizeof(unsigned long long) * (size_t)n_bins * (size_t)n_bins, h->stream));
+    if (sep) MMM_CUDA(h, cudaMemsetAsync(sep, 0, sizeof(unsigned long long) * (size_t)n, h->stream));
+    MMM_CUDA(h, cudaMemsetAsync(cnt, 0, sizeof(unsigned long long) * 2, h->stream));
+  }
+  if (ev0) MMM_CUDA(h, cudaEventRecord(ev0, h->stream));
+  if ((rc = mmm_launch_prepare(h, nullptr))) return rc;  // d_x -> FP32 copy and its tile boxes
+  k_ct_stage_boxes<<<(nst + 255) / 256, 256, 0, h->stream>>>(h->d_tiles, ntr, nst, h->d_ct_stage);
+  h->launches++;
+  MMM_CUDA(h, cudaGetLastError());
+  const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
+  k_contacts<kDense><<<(ntr + CT_WARPS - 1) / CT_WARPS, CT_WARPS * 32, 0, h->stream>>>(
+      h->d_x, h->d_type, map ? d_bin : nullptr, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, map,
+      sep, cnt, nullptr, nullptr);
+  h->launches++;
+  MMM_CUDA(h, cudaGetLastError());
+  return MMM_OK;
+}
+
+// The sparse pass up to the run count: the key of every binned contact, radix-sorted into keys[out->src], and
+// table[0, nblocks) = the first entry of every 4096-key chunk.  tile, keys and table are grown as needed;
+// cnt[2] (device) is cleared before ev0 and holds contacts and candidates after ev1 (either event may be NULL).  One host
+// synchronisation for the key count, one for the entry count.
+int mmm_contacts_sparse_pass(mmm_system* h, double rc_nm, const int* d_bin, int32_t n_bins, DevBuf<long long>& tile,
+                             DevBuf<unsigned long long>* keys, DevBuf<long long>& table, unsigned long long* cnt,
+                             cudaEvent_t ev0, cudaEvent_t ev1, CsSorted* out) {
+  const int n = (int)h->n;
+  const int ntr = (n + MMM_TILE - 1) / MMM_TILE;
+  const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;
+  int rc;
+  if ((rc = mmm_reserve(h, h->d_ct_stage, (size_t)nst, "contact stage boxes")) ||
+      (rc = mmm_reserve(h, tile, (size_t)ntr + cs_blocks(ntr) + 1, "contact tile counts")))  // counts, then scan parts
+    return rc;
+  long long* tile_part = tile + ntr;
+  MMM_CUDA(h, cudaMemsetAsync(cnt, 0, sizeof(unsigned long long) * 2, h->stream));
+  if (ev0) MMM_CUDA(h, cudaEventRecord(ev0, h->stream));
+  if ((rc = mmm_launch_prepare(h, nullptr))) return rc;
+  k_ct_stage_boxes<<<(nst + 255) / 256, 256, 0, h->stream>>>(h->d_tiles, ntr, nst, h->d_ct_stage);
+  const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
+  const int ctas = (ntr + CT_WARPS - 1) / CT_WARPS;
+  k_contacts<kTileCount><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
+      h->d_x, h->d_type, d_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
+      nullptr, nullptr, tile, nullptr);
+  h->launches += 2;
+  cs_scan(h, tile, ntr, tile_part);
+  MMM_CUDA(h, cudaGetLastError());
+  long long m = 0;  // binned contacts = keys
+  MMM_CUDA(h, cudaMemcpyAsync(&m, tile_part + cs_blocks(ntr), sizeof(m), cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  // grown to exactly this call's keys when they do not fit
+  if ((rc = mmm_reserve(h, keys[0], (size_t)m, "contact keys")) ||
+      (rc = mmm_reserve(h, keys[1], (size_t)m, "contact keys")) ||
+      (rc = mmm_reserve(h, table, cs_table_len(m), "contact sort table")))
+    return rc;
+  long long* tab = table;
+  const int nblocks = (int)cs_blocks(m);
+  long long* table_part = tab + (size_t)CS_DIGITS * nblocks;
+  k_contacts<kKeys><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
+      h->d_x, h->d_type, d_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
+      nullptr, cnt, tile, keys[0]);
+  h->launches++;
+  // keys < n_bins^2: sort on ceil(log2(n_bins^2)) bits, 8 per pass
+  int bits = 0;
+  const unsigned long long kmax = (unsigned long long)n_bins * (unsigned long long)n_bins - 1ull;
+  while (bits < 64 && (kmax >> bits)) ++bits;
+  int src = 0;
+  if (m > 0) {
+    for (int shift = 0; shift < bits; shift += CS_DIGIT_BITS) {
+      k_rs_hist<<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, shift, tab, nblocks);
+      cs_scan(h, tab, (long long)CS_DIGITS * nblocks, table_part);
+      k_rs_scatter<<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, shift, tab, nblocks, keys[1 - src]);
+      h->launches += 2;
+      src = 1 - src;
+    }
+    // entries: heads per chunk -> offsets (the first nblocks slots of the table, kept for the read)
+    k_rle<kCount><<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, tab, nullptr, 0u, nullptr, nullptr, nullptr,
+                                                         nullptr, nullptr);
+    h->launches++;
+    cs_scan(h, tab, nblocks, tab + nblocks);
+  }
+  MMM_CUDA(h, cudaGetLastError());
+  if (ev1) MMM_CUDA(h, cudaEventRecord(ev1, h->stream));
+  long long entries = 0;
+  MMM_CUDA(h, cudaMemcpyAsync(out->cnt, cnt, sizeof(out->cnt), cudaMemcpyDeviceToHost, h->stream));
+  if (m > 0)
+    MMM_CUDA(h, cudaMemcpyAsync(&entries, tab + nblocks + cs_blocks(nblocks), sizeof(entries), cudaMemcpyDeviceToHost,
+                                h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  out->keys = m;
+  out->entries = entries;
+  out->src = src;
+  return MMM_OK;
+}
+
+// Capacity for n entries of a list that grows by a few per cent a sample (the accumulated fine map): n rounded
+// up to the next of eight steps per power of two, so that the buffers are reallocated every ~12 % of growth
+// rather than at every sample.
+static size_t sp_capacity(long long n) {
+  size_t step = 1;
+  while (step * 16 <= (size_t)n) step <<= 1;
+  return ((size_t)n + step - 1) / step * step;
+}
+
+// The trajectory sampler's fine map: this structure's sparse map, reduced to a sorted unique (key, count) list
+// in the spare sort buffer and d_sp_sval, merged with the accumulated list d_sp_acc_*[0] into d_sp_acc_*[1],
+// and equal keys added back into d_sp_acc_*[0].  Work and memory O(accumulated + this structure's entries).
+int mmm_contacts_fine_accumulate(mmm_system* h) {
+  CsSorted srt;
+  int rc = mmm_contacts_sparse_pass(h, h->sp_rc, h->d_sp_fine_bin, h->sp_fine_bins, h->d_sp_tile, h->d_sp_keys,
+                                    h->d_sp_table, h->d_sp_cnt + 2, nullptr, nullptr, &srt);
+  if (rc) return rc;
+  const long long nb = srt.entries, na = h->sp_fine_n, nm = na + nb;
+  if (nb == 0) return MMM_OK;
+  unsigned long long* skey = h->d_sp_keys[1 - srt.src];  // free after the sort; keys >= entries slots
+  if ((rc = mmm_reserve(h, h->d_sp_sval, sp_capacity(nb), "sampler fine counts")) ||
+      (rc = mmm_reserve(h, h->d_sp_acc_key[1], sp_capacity(nm), "sampler fine keys")) ||
+      (rc = mmm_reserve(h, h->d_sp_acc_val[1], sp_capacity(nm), "sampler fine counts")))
+    return rc;
+  MMM_CUDA(h, cudaMemsetAsync(h->d_sp_sval, 0, sizeof(unsigned long long) * (size_t)nb, h->stream));
+  k_rle<kKeyVals><<<(int)cs_blocks(srt.keys), CS_THREADS, 0, h->stream>>>(
+      h->d_sp_keys[srt.src], srt.keys, nullptr, h->d_sp_table, 0u, nullptr, h->d_sp_sval, skey, nullptr, nullptr);
+  const int nparts = (int)((nm + MG_TILE - 1) / MG_TILE);
+  const long long nchunks = cs_blocks(nm);
+  if ((rc = mmm_reserve(h, h->d_sp_mpart, sp_capacity(std::max<long long>(nparts + 1, nchunks + cs_blocks(nchunks) + 1)),
+                        "sampler merge table")))
+    return rc;
+  long long* part = h->d_sp_mpart;
+  k_merge_part<<<(nparts + 1 + 255) / 256, 256, 0, h->stream>>>(h->d_sp_acc_key[0], na, skey, nb, nparts, part);
+  k_merge<<<nparts, MG_THREADS, 0, h->stream>>>(h->d_sp_acc_key[0], h->d_sp_acc_val[0], na, skey, h->d_sp_sval, nb,
+                                                part, h->d_sp_acc_key[1], h->d_sp_acc_val[1]);
+  // equal keys -> one entry: heads per chunk, their offsets, then keys and summed counts
+  k_rle<kCount><<<(int)nchunks, CS_THREADS, 0, h->stream>>>(h->d_sp_acc_key[1], nm, part, nullptr, 0u, nullptr, nullptr,
+                                                            nullptr, nullptr, nullptr);
+  h->launches += 4;
+  cs_scan(h, part, nchunks, part + nchunks);
+  MMM_CUDA(h, cudaGetLastError());
+  long long ne = 0;
+  MMM_CUDA(h, cudaMemcpyAsync(&ne, part + nchunks + cs_blocks(nchunks), sizeof(ne), cudaMemcpyDeviceToHost, h->stream));
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  if ((rc = mmm_reserve(h, h->d_sp_acc_key[0], sp_capacity(ne), "sampler fine keys")) ||
+      (rc = mmm_reserve(h, h->d_sp_acc_val[0], sp_capacity(ne), "sampler fine counts")))
+    return rc;
+  MMM_CUDA(h, cudaMemsetAsync(h->d_sp_acc_val[0], 0, sizeof(unsigned long long) * (size_t)ne, h->stream));
+  k_rle<kKeyVals><<<(int)nchunks, CS_THREADS, 0, h->stream>>>(h->d_sp_acc_key[1], nm, nullptr, part, 0u,
+                                                              h->d_sp_acc_val[1], h->d_sp_acc_val[0],
+                                                              h->d_sp_acc_key[0], nullptr, nullptr);
+  h->launches++;
+  MMM_CUDA(h, cudaGetLastError());
+  h->sp_fine_n = ne;
+  return MMM_OK;
+}
+
+namespace {
+// rows[e] = key / n_bins, cols[e] = key % n_bins of the sampler's fine entries
+__global__ void __launch_bounds__(256) k_split_keys(const unsigned long long* __restrict__ keys, long long n,
+                                                    unsigned nbins, int* __restrict__ rows, int* __restrict__ cols) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n) return;
+  rows[e] = (int)(keys[e] / nbins);
+  cols[e] = (int)(keys[e] % nbins);
+}
+}  // namespace
+
+int mmm_contacts_fine_read(mmm_system* h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out) {
+  const long long e = h->sp_fine_n;
+  if (e == 0) return MMM_OK;
+  if (vals_out)
+    MMM_CUDA(h, cudaMemcpyAsync(vals_out, h->d_sp_acc_val[0], sizeof(uint64_t) * (size_t)e, cudaMemcpyDeviceToHost,
+                                h->stream));
+  if (rows_out || cols_out) {  // rows then cols as int32 in the free merge buffer (>= e slots of 8 B)
+    int* rows = reinterpret_cast<int*>(h->d_sp_acc_key[1].get());
+    int* cols = rows + e;
+    k_split_keys<<<(unsigned)((e + 255) / 256), 256, 0, h->stream>>>(h->d_sp_acc_key[0], e, (unsigned)h->sp_fine_bins,
+                                                                      rows, cols);
+    h->launches++;
+    MMM_CUDA(h, cudaGetLastError());
+    if (rows_out) MMM_CUDA(h, cudaMemcpyAsync(rows_out, rows, sizeof(int32_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));
+    if (cols_out) MMM_CUDA(h, cudaMemcpyAsync(cols_out, cols, sizeof(int32_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));
+  }
+  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MMM_OK;
+}
+
 extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_bead, int32_t n_bins, uint64_t* map_out,
                             uint64_t* sep_out, int64_t* pairs_out) {
   if (!h) return MMM_ERR_ARG;
@@ -402,37 +663,22 @@ extern "C" int mmm_contacts(mmm_handle h, double rc_nm, const int32_t* bin_of_be
   if ((rc = ct_check_args(h, "mmm_contacts", rc_nm, bin_of_bead, n_bins, CT_MAX_BINS, map_out != nullptr))) return rc;
   cudaSetDevice(h->device);
   const int n = (int)h->n;
-  const int ntr = (n + MMM_TILE - 1) / MMM_TILE;                    // tiles holding a real bead
-  const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;  // stages holding a real tile
   const bool want_map = map_out != nullptr;
   const size_t cells = (size_t)n_bins * (size_t)n_bins;
   // scratch lives as long as the handle and only grows (the map when a call needs a larger one), so
   // that a call does not synchronise the device while another handle minimises beside it
   if ((rc = mmm_reserve(h, h->d_ct_bin, (size_t)n, "contact bins")) ||
       (rc = mmm_reserve(h, h->d_ct_sep, (size_t)n, "contacts by separation")) ||
-      (rc = mmm_reserve(h, h->d_ct_stage, (size_t)nst, "contact stage boxes")) ||
       (rc = mmm_reserve(h, h->d_ct_cnt, 2, "contact counters")) ||
       (want_map && (rc = mmm_reserve(h, h->d_ct_map, cells, "contact map"))))
     return rc;
   if (!h->ct_ev0) MMM_CUDA(h, cudaEventCreate(&h->ct_ev0));
   if (!h->ct_ev1) MMM_CUDA(h, cudaEventCreate(&h->ct_ev1));
-  if (want_map) {
+  if (want_map)
     MMM_CUDA(h, cudaMemcpyAsync(h->d_ct_bin, bin_of_bead, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
-    MMM_CUDA(h, cudaMemsetAsync(h->d_ct_map, 0, sizeof(unsigned long long) * cells, h->stream));
-  }
-  if (sep_out) MMM_CUDA(h, cudaMemsetAsync(h->d_ct_sep, 0, sizeof(unsigned long long) * (size_t)n, h->stream));
-  MMM_CUDA(h, cudaMemsetAsync(h->d_ct_cnt, 0, sizeof(unsigned long long) * 2, h->stream));
-  MMM_CUDA(h, cudaEventRecord(h->ct_ev0, h->stream));
-  if ((rc = mmm_launch_prepare(h, nullptr))) return rc;  // d_x -> FP32 copy and its tile boxes
-  k_ct_stage_boxes<<<(nst + 255) / 256, 256, 0, h->stream>>>(h->d_tiles, ntr, nst, h->d_ct_stage);
-  h->launches++;
-  MMM_CUDA(h, cudaGetLastError());
-  const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
-  k_contacts<kDense><<<(ntr + CT_WARPS - 1) / CT_WARPS, CT_WARPS * 32, 0, h->stream>>>(
-      h->d_x, h->d_type, want_map ? h->d_ct_bin.get() : nullptr, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2,
-      n_bins, want_map ? h->d_ct_map.get() : nullptr, sep_out ? h->d_ct_sep.get() : nullptr, h->d_ct_cnt, nullptr, nullptr);
-  h->launches++;
-  MMM_CUDA(h, cudaGetLastError());
+  if ((rc = mmm_contacts_dense_pass(h, rc_nm, h->d_ct_bin, n_bins, want_map ? h->d_ct_map.get() : nullptr,
+                                    sep_out ? h->d_ct_sep.get() : nullptr, h->d_ct_cnt, true, h->ct_ev0)))
+    return rc;
   MMM_CUDA(h, cudaEventRecord(h->ct_ev1, h->stream));
   unsigned long long cnt[2];
   MMM_CUDA(h, cudaMemcpyAsync(cnt, h->d_ct_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, h->stream));
@@ -455,82 +701,24 @@ extern "C" int mmm_contacts_sparse(mmm_handle h, double rc_nm, const int32_t* bi
   cudaSetDevice(h->device);
   h->cs_valid = false;
   const int n = (int)h->n;
-  const int ntr = (n + MMM_TILE - 1) / MMM_TILE;
-  const int nst = (ntr + CT_TILES_PER_STAGE - 1) / CT_TILES_PER_STAGE;
   if ((rc = mmm_reserve(h, h->d_ct_bin, (size_t)n, "contact bins")) ||
-      (rc = mmm_reserve(h, h->d_ct_stage, (size_t)nst, "contact stage boxes")) ||
-      (rc = mmm_reserve(h, h->d_ct_cnt, 2, "contact counters")) ||
-      (rc = mmm_reserve(h, h->d_cs_tile, (size_t)ntr + cs_blocks(ntr) + 1, "contact tile counts")))  // counts, then scan parts
+      (rc = mmm_reserve(h, h->d_ct_cnt, 2, "contact counters")))
     return rc;
   if (!h->ct_ev0) MMM_CUDA(h, cudaEventCreate(&h->ct_ev0));
   if (!h->ct_ev1) MMM_CUDA(h, cudaEventCreate(&h->ct_ev1));
-  long long* tile = h->d_cs_tile;
-  long long* tile_part = tile + ntr;
   MMM_CUDA(h, cudaMemcpyAsync(h->d_ct_bin, bin_of_bead, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
-  MMM_CUDA(h, cudaMemsetAsync(h->d_ct_cnt, 0, sizeof(unsigned long long) * 2, h->stream));
-  MMM_CUDA(h, cudaEventRecord(h->ct_ev0, h->stream));
-  if ((rc = mmm_launch_prepare(h, nullptr))) return rc;
-  k_ct_stage_boxes<<<(nst + 255) / 256, 256, 0, h->stream>>>(h->d_tiles, ntr, nst, h->d_ct_stage);
-  const float rcm2 = (float)(rc_nm * rc_nm) * (1.0f + 0x1p-16f);
-  const int ctas = (ntr + CT_WARPS - 1) / CT_WARPS;
-  k_contacts<kTileCount><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
-      h->d_x, h->d_type, h->d_ct_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
-      nullptr, nullptr, h->d_cs_tile, nullptr);
-  h->launches += 2;
-  cs_scan(h, tile, ntr, tile_part);
-  MMM_CUDA(h, cudaGetLastError());
-  long long m = 0;  // binned contacts = keys
-  MMM_CUDA(h, cudaMemcpyAsync(&m, tile_part + cs_blocks(ntr), sizeof(m), cudaMemcpyDeviceToHost, h->stream));
-  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  // grown to exactly this call's keys when they do not fit
-  if ((rc = mmm_reserve(h, h->d_cs_keys[0], (size_t)m, "contact keys")) ||
-      (rc = mmm_reserve(h, h->d_cs_keys[1], (size_t)m, "contact keys")) ||
-      (rc = mmm_reserve(h, h->d_cs_table, cs_table_len(m), "contact sort table")))
+  CsSorted srt;
+  if ((rc = mmm_contacts_sparse_pass(h, rc_nm, h->d_ct_bin, n_bins, h->d_cs_tile, h->d_cs_keys, h->d_cs_table,
+                                     h->d_ct_cnt, h->ct_ev0, h->ct_ev1, &srt)))
     return rc;
-  long long* table = h->d_cs_table;
-  const int nblocks = (int)cs_blocks(m);
-  long long* table_part = table + (size_t)CS_DIGITS * nblocks;
-  k_contacts<kKeys><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
-      h->d_x, h->d_type, h->d_ct_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
-      nullptr, h->d_ct_cnt, h->d_cs_tile, h->d_cs_keys[0]);
-  h->launches++;
-  // keys < n_bins^2: sort on ceil(log2(n_bins^2)) bits, 8 per pass
-  int bits = 0;
-  const unsigned long long kmax = (unsigned long long)n_bins * (unsigned long long)n_bins - 1ull;
-  while (bits < 64 && (kmax >> bits)) ++bits;
-  int src = 0;
-  if (m > 0) {
-    for (int shift = 0; shift < bits; shift += CS_DIGIT_BITS) {
-      k_rs_hist<<<nblocks, CS_THREADS, 0, h->stream>>>(h->d_cs_keys[src], m, shift, table, nblocks);
-      cs_scan(h, table, (long long)CS_DIGITS * nblocks, table_part);
-      k_rs_scatter<<<nblocks, CS_THREADS, 0, h->stream>>>(h->d_cs_keys[src], m, shift, table, nblocks,
-                                                          h->d_cs_keys[1 - src]);
-      h->launches += 2;
-      src = 1 - src;
-    }
-    // entries: heads per chunk -> offsets (the first nblocks slots of the table, kept for the read)
-    k_rle<kCount><<<nblocks, CS_THREADS, 0, h->stream>>>(h->d_cs_keys[src], m, table, nullptr, 0u, nullptr, nullptr,
-                                                         nullptr);
-    h->launches++;
-    cs_scan(h, table, nblocks, table + nblocks);
-  }
-  MMM_CUDA(h, cudaGetLastError());
-  MMM_CUDA(h, cudaEventRecord(h->ct_ev1, h->stream));
-  unsigned long long cnt[2];
-  long long entries = 0;
-  MMM_CUDA(h, cudaMemcpyAsync(cnt, h->d_ct_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, h->stream));
-  if (m > 0)
-    MMM_CUDA(h, cudaMemcpyAsync(&entries, table + nblocks + cs_blocks(nblocks), sizeof(entries),
-                                cudaMemcpyDeviceToHost, h->stream));
-  MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  h->cs_keys = m;
-  h->cs_entries = entries;
-  h->cs_src = src;
+  h->cs_keys = srt.keys;
+  h->cs_entries = srt.entries;
+  h->cs_src = srt.src;
   h->cs_nbins = n_bins;
   h->cs_valid = true;
-  if (n_entries_out) *n_entries_out = entries;
-  if (pairs_out) *pairs_out = (int64_t)cnt[0];
-  h->ct_candidates = (int64_t)cnt[1];
+  if (n_entries_out) *n_entries_out = srt.entries;
+  if (pairs_out) *pairs_out = (int64_t)srt.cnt[0];
+  h->ct_candidates = (int64_t)srt.cnt[1];
   cudaEventElapsedTime(&h->ct_ms, h->ct_ev0, h->ct_ev1);
   return MMM_OK;
 }
@@ -547,7 +735,8 @@ extern "C" int mmm_contacts_sparse_read(mmm_handle h, int32_t* rows_out, int32_t
   const long long* off = h->d_cs_table;
   if (vals_out) {
     MMM_CUDA(h, cudaMemsetAsync(spare, 0, sizeof(unsigned long long) * (size_t)e, h->stream));
-    k_rle<kVals><<<nblocks, CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, 0u, spare, nullptr, nullptr);
+    k_rle<kVals><<<nblocks, CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, 0u, nullptr, spare, nullptr, nullptr,
+                                                        nullptr);
     h->launches++;
     MMM_CUDA(h, cudaGetLastError());
     MMM_CUDA(h, cudaMemcpyAsync(vals_out, spare, sizeof(uint64_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));
@@ -555,8 +744,8 @@ extern "C" int mmm_contacts_sparse_read(mmm_handle h, int32_t* rows_out, int32_t
   if (rows_out || cols_out) {  // rows then cols as int32 in the same spare buffer (8 B per entry)
     int* rows = reinterpret_cast<int*>(spare);
     int* cols = rows + e;
-    k_rle<kSplit><<<nblocks, CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, (unsigned)h->cs_nbins, nullptr, rows,
-                                                         cols);
+    k_rle<kSplit><<<nblocks, CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, (unsigned)h->cs_nbins, nullptr, nullptr,
+                                                         nullptr, rows, cols);
     h->launches++;
     MMM_CUDA(h, cudaGetLastError());
     if (rows_out) MMM_CUDA(h, cudaMemcpyAsync(rows_out, rows, sizeof(int32_t) * (size_t)e, cudaMemcpyDeviceToHost, h->stream));

@@ -170,33 +170,15 @@ __global__ void __launch_bounds__(256) k_dm_bbox(const double* __restrict__ x, i
 
 }  // namespace
 
-extern "C" int mmm_distance_map(mmm_handle h, const int32_t* bin_of_bead, int32_t n_bins, uint64_t* dist_sum_out,
-                                uint64_t* dist2_sum_out, float* device_ms_out) {
-  if (!h) return MMM_ERR_ARG;
-  if (n_bins < 1 || n_bins > DM_MAX_BINS) return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: n_bins must be in [1, 4096]");
-  if (!bin_of_bead) return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: bin_of_bead is NULL");
+// Overflow guard of the distance sums: *bound = (pairs of the fullest bin pair) x (largest quantised value of
+// one pair), occ = beads per bin.  D bounds every pair distance: the diagonal of the beads' FP64 bounding box,
+// padded for rounding.  MMM_ERR_ARG (message prefixed by who) when the positions are not finite or when
+// prior + *bound reaches 2^63: the one-shot map passes prior = 0, the trajectory sampler the bounds of the
+// structures it has already summed.  Launches one kernel and synchronises; writes nothing else.
+int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t>& occ, double prior, double* bound) {
   const int n = (int)h->n;
-  std::vector<int64_t> occ((size_t)n_bins, 0);  // beads per bin: the largest bin pair bounds every sum
-  for (int i = 0; i < n; ++i) {
-    const int32_t b = bin_of_bead[i];
-    if (b < -1 || b >= n_bins) return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: bin id outside [-1, n_bins)");
-    if (b >= 0) ++occ[(size_t)b];
-  }
-  if (!h->positions_set) return mmm_fail(h, MMM_ERR_STATE, "positions were never set");
-  cudaSetDevice(h->device);
   int rc;
-  const size_t cells = (size_t)n_bins * (size_t)n_bins;
-  if ((rc = mmm_reserve(h, h->d_dm_bin, (size_t)std::max(n, 1), "distance-map bins")) ||
-      (rc = mmm_reserve(h, h->d_dm_box, (size_t)DM_BOX_BLOCKS * 6, "distance-map boxes")) ||
-      (rc = mmm_reserve(h, h->d_dm_map, 2 * cells, "distance map")))
-    return rc;
-  if (!h->dm_ev0) MMM_CUDA(h, cudaEventCreate(&h->dm_ev0));
-  if (!h->dm_ev1) MMM_CUDA(h, cudaEventCreate(&h->dm_ev1));
-  unsigned long long* dmap = h->d_dm_map;
-  unsigned long long* d2map = h->d_dm_map + cells;
-
-  // overflow guard: (pairs of the fullest bin pair) x (largest quantised value of one pair) must fit int64.
-  // D bounds every pair distance: the diagonal of the beads' FP64 bounding box, padded for rounding.
+  if ((rc = mmm_reserve(h, h->d_dm_box, (size_t)DM_BOX_BLOCKS * 6, "distance-map boxes"))) return rc;
   const int box_blocks = std::max(1, std::min(DM_BOX_BLOCKS, (n + 255) / 256));
   k_dm_bbox<<<box_blocks, 256, 0, h->stream>>>(h->d_x, n, h->d_dm_box);
   h->launches++;
@@ -216,7 +198,7 @@ extern "C" int mmm_distance_map(mmm_handle h, const int32_t* bin_of_bead, int32_
     d2max += ext * ext;
   }
   if (!std::isfinite(d2max))
-    return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: positions are not finite (no distance can be quantised)");
+    return mmm_fail(h, MMM_ERR_ARG, std::string(who) + ": positions are not finite (no distance can be quantised)");
   double pmax = 0.0, top1 = 0.0, top2 = 0.0;  // pairs of the fullest bin pair: a diagonal one or the two fullest bins
   for (int64_t c : occ) {
     const double v = (double)c;
@@ -231,26 +213,70 @@ extern "C" int mmm_distance_map(mmm_handle h, const int32_t* bin_of_bead, int32_
   pmax = std::max(pmax, top1 * top2);
   const double dpad = sqrt(d2max) * (1.0 + 0x1p-40) + 0x1p-60;  // D, padded for the rounding of d2 and d
   const double qmax = ceil(DM_SCALE * std::max(dpad * dpad, dpad)) + 1.0;  // bounds qd and qd2 of every pair
-  if (pmax * qmax >= 0x1p63)
+  *bound = pmax * qmax;
+  if (prior + *bound >= 0x1p63)
     return mmm_fail(h, MMM_ERR_ARG,
-                    "mmm_distance_map: the sums could overflow int64 (" + std::to_string((long long)pmax) +
+                    std::string(who) + ": the sums could overflow int64 (" + std::to_string((long long)pmax) +
                         " bead pairs in the fullest bin pair, distances up to " + std::to_string(dpad) +
-                        " nm at a quantum of 2^-24 nm); use more bins or a more compact structure");
+                        " nm at a quantum of 2^-24 nm" +
+                        (prior > 0.0 ? ", on top of the structures already summed" : "") +
+                        "); use more bins or a more compact structure");
+  return MMM_OK;
+}
 
-  MMM_CUDA(h, cudaMemcpyAsync(h->d_dm_bin, bin_of_bead, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
-  MMM_CUDA(h, cudaEventRecord(h->dm_ev0, h->stream));
-  MMM_CUDA(h, cudaMemsetAsync(h->d_dm_map, 0, sizeof(unsigned long long) * 2 * cells, h->stream));
+// The distance pass: sums at the current positions added into dmap and d2map (n_bins^2 each), zeroed first
+// when clear.  d_bin: the bin of every bead on the device.  mmm_distance_map and the sampler run it.
+int mmm_distance_pass(mmm_system* h, const int* d_bin, int32_t n_bins, unsigned long long* dmap,
+                      unsigned long long* d2map, bool clear) {
+  const int n = (int)h->n;
+  const size_t cells = (size_t)n_bins * (size_t)n_bins;
+  if (clear) {
+    MMM_CUDA(h, cudaMemsetAsync(dmap, 0, sizeof(unsigned long long) * cells, h->stream));
+    MMM_CUDA(h, cudaMemsetAsync(d2map, 0, sizeof(unsigned long long) * cells, h->stream));
+  }
   const int ntr = (n + MMM_TILE - 1) / MMM_TILE;
   const long long npairs_t = (long long)ntr * (ntr + 1) / 2;
   const long long nchunks = (npairs_t + DM_CHUNK - 1) / DM_CHUNK;
   if (nchunks > 0) {
     const long long want = (nchunks + DM_WARPS - 1) / DM_WARPS;
     const int ctas = (int)std::min<long long>(want, (long long)std::max(h->sm_count, 1) * 8);
-    k_distance_map<<<ctas, DM_WARPS * 32, 0, h->stream>>>(h->d_x, h->d_dm_bin, n, ntr, npairs_t, nchunks, n_bins, dmap,
+    k_distance_map<<<ctas, DM_WARPS * 32, 0, h->stream>>>(h->d_x, d_bin, n, ntr, npairs_t, nchunks, n_bins, dmap,
                                                           d2map);
     h->launches++;
     MMM_CUDA(h, cudaGetLastError());
   }
+  return MMM_OK;
+}
+
+extern "C" int mmm_distance_map(mmm_handle h, const int32_t* bin_of_bead, int32_t n_bins, uint64_t* dist_sum_out,
+                                uint64_t* dist2_sum_out, float* device_ms_out) {
+  if (!h) return MMM_ERR_ARG;
+  if (n_bins < 1 || n_bins > DM_MAX_BINS) return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: n_bins must be in [1, 4096]");
+  if (!bin_of_bead) return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: bin_of_bead is NULL");
+  const int n = (int)h->n;
+  std::vector<int64_t> occ((size_t)n_bins, 0);  // beads per bin: the largest bin pair bounds every sum
+  for (int i = 0; i < n; ++i) {
+    const int32_t b = bin_of_bead[i];
+    if (b < -1 || b >= n_bins) return mmm_fail(h, MMM_ERR_ARG, "mmm_distance_map: bin id outside [-1, n_bins)");
+    if (b >= 0) ++occ[(size_t)b];
+  }
+  if (!h->positions_set) return mmm_fail(h, MMM_ERR_STATE, "positions were never set");
+  cudaSetDevice(h->device);
+  int rc;
+  const size_t cells = (size_t)n_bins * (size_t)n_bins;
+  if ((rc = mmm_reserve(h, h->d_dm_bin, (size_t)std::max(n, 1), "distance-map bins")) ||
+      (rc = mmm_reserve(h, h->d_dm_map, 2 * cells, "distance map")))
+    return rc;
+  if (!h->dm_ev0) MMM_CUDA(h, cudaEventCreate(&h->dm_ev0));
+  if (!h->dm_ev1) MMM_CUDA(h, cudaEventCreate(&h->dm_ev1));
+  unsigned long long* dmap = h->d_dm_map;
+  unsigned long long* d2map = h->d_dm_map + cells;
+  double bound;
+  if ((rc = mmm_distance_guard(h, "mmm_distance_map", occ, 0.0, &bound))) return rc;
+
+  MMM_CUDA(h, cudaMemcpyAsync(h->d_dm_bin, bin_of_bead, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
+  MMM_CUDA(h, cudaEventRecord(h->dm_ev0, h->stream));
+  if ((rc = mmm_distance_pass(h, h->d_dm_bin, n_bins, dmap, d2map, true))) return rc;
   MMM_CUDA(h, cudaEventRecord(h->dm_ev1, h->stream));
   if (dist_sum_out)
     MMM_CUDA(h, cudaMemcpyAsync(dist_sum_out, dmap, sizeof(uint64_t) * cells, cudaMemcpyDeviceToHost, h->stream));

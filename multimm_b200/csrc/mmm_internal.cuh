@@ -310,6 +310,36 @@ struct mmm_system {
   DevBuf<unsigned long long> d_dm_map;     // [2][n_bins^2] quantised distance sums, then squared-distance sums
   DevBuf<double> d_dm_box;                 // per-block bounding boxes of the beads (overflow guard)
   cudaEvent_t dm_ev0 = nullptr, dm_ev1 = nullptr;
+
+  // trajectory sampler (mmm_sampler.cu): maps summed over many structures, on the device until read.  Its
+  // own buffers, so that sampling leaves the one-shot calls' results (mmm_contacts_sparse_read) alone
+  bool sp_configured = false;
+  double sp_rc = 0.0;
+  int32_t sp_ct_bins = 0, sp_fine_bins = 0, sp_dm_bins = 0;  // 0: that map is off
+  DevBuf<int> d_sp_ct_bin, d_sp_fine_bin, d_sp_dm_bin;      // [n] bins of every bead, uploaded once
+  std::vector<int64_t> sp_dm_occ;                          // beads per distance bin (overflow guard)
+  int64_t sp_samples = 0;
+  double sp_dm_bound = 0.0;                                // summed per-structure bounds of the distance sums
+  float sp_ms = 0.f;                                       // device time of all samples
+  cudaEvent_t sp_ev0 = nullptr, sp_ev1 = nullptr;
+  DevBuf<unsigned long long> d_sp_map;     // [n_bins^2] dense contact map
+  DevBuf<unsigned long long> d_sp_sep;     // [n] contacts by index separation
+  DevBuf<unsigned long long> d_sp_cnt;     // [4] contacts, candidates (summed); the fine pass's own two
+  DevBuf<unsigned long long> d_sp_dist;    // [2][n_bins^2] distance sums, squared-distance sums
+  // fine map: a sorted unique (key, count) list in d_sp_acc_*[0]; [1] receives the merge
+  DevBuf<long long> d_sp_tile, d_sp_table;             // the sparse pass's scratch (as d_cs_tile, d_cs_table)
+  DevBuf<unsigned long long> d_sp_keys[2];             // the sparse pass's sort buffers
+  DevBuf<unsigned long long> d_sp_sval;                // counts of one structure's entries
+  DevBuf<unsigned long long> d_sp_acc_key[2], d_sp_acc_val[2];
+  DevBuf<long long> d_sp_mpart;                        // merge partition, then run offsets of the merge
+  int64_t sp_fine_n = 0;                               // accumulated fine entries
+};
+
+// the sorted keys of one sparse pass (mmm_contacts_sparse_pass)
+struct CsSorted {
+  long long keys = 0, entries = 0;  // binned contacts, distinct keys
+  int src = 0;                      // which sort buffer holds the sorted keys
+  unsigned long long cnt[2] = {0, 0};  // contacts, candidates
 };
 
 // ---------------------------------------------------------------------------------------
@@ -396,6 +426,19 @@ int mmm_launch_assemble(mmm_system* h, const int* d_skip);  // -> d_g, d_epart
 int mmm_launch_finalize_energy(mmm_system* h);  // -> d_eterms (stand-alone evaluation)
 // mmm_lbfgs.cu
 int mmm_run_minimize(mmm_system* h, double tol, int64_t max_iter, mmm_min_report* out);
+
+// mmm_contacts.cu
+int mmm_contacts_dense_pass(mmm_system* h, double rc_nm, const int* d_bin, int32_t n_bins, unsigned long long* map,
+                            unsigned long long* sep, unsigned long long* cnt, bool clear, cudaEvent_t ev0);
+int mmm_contacts_sparse_pass(mmm_system* h, double rc_nm, const int* d_bin, int32_t n_bins, DevBuf<long long>& tile,
+                             DevBuf<unsigned long long>* keys, DevBuf<long long>& table, unsigned long long* cnt,
+                             cudaEvent_t ev0, cudaEvent_t ev1, CsSorted* out);
+int mmm_contacts_fine_accumulate(mmm_system* h);  // the sampler's fine map += the current structure's
+int mmm_contacts_fine_read(mmm_system* h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out);
+// mmm_distances.cu
+int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t>& occ, double prior, double* bound);
+int mmm_distance_pass(mmm_system* h, const int* d_bin, int32_t n_bins, unsigned long long* dmap,
+                      unsigned long long* d2map, bool clear);
 
 // one full evaluation at the positions in d_x: prepare -> pair -> assemble.  d_skip (may be
 // NULL) points at a device flag; when it is non-zero every kernel returns immediately.

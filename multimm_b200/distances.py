@@ -10,7 +10,11 @@ quantised and summed per bin the same way on the host.  Bins are the canonical g
 in any order.
 
 Files (numpy ``.npz``): ``analysis/distances.npz`` of a single run, ``distances/member_<i>.npz`` of an
-ensemble member and ``ensemble_distances.npz`` of an ensemble, all in one format:
+ensemble member and ``ensemble_distances.npz`` of an ensemble, all in one format.  With ``MD_SAMPLE_STEP``
+the same maps summed over the structures sampled during MD (``Engine.sampler_read``) go to
+``analysis/distances_md.npz``, ``distances/member_<i>_md.npz`` and ``ensemble_distances_md.npz``: a file of
+S sampled structures is their sum exactly as an ensemble file is the sum of its members (``members`` = S,
+pair and bead counts S times one structure's), so every function below reads it unchanged.
 
 * ``dist_sum``, ``dist2_sum``: uint64, the upper triangle p <= q of the B x B maps, flattened in
   ``np.triu_indices(B)`` order, in units of Q nm and Q nm^2 (every entry of a distance map is a sum over
@@ -64,16 +68,35 @@ def radial_sums(x, center, bins, n_bins: int) -> tuple[np.ndarray, np.ndarray]:
 def result(dist_sum, dist2_sum, gb: GenomeBins, x, center, members: int = 1) -> dict:
     """The in-memory form of a distances file (dense maps) of one structure: the device maps of
     Engine.distance_map at bins ``gb``, and the radial sums of its positions ``x`` about ``center``."""
+    rs, r2s = radial_sums(x, center, gb.bins, gb.n_bins)
+    pairs, n = _counts(gb)
+    return _result(dist_sum, dist2_sum, gb, pairs, n, rs, r2s, members)
+
+
+def sampled_result(dist_sum, dist2_sum, gb: GenomeBins, radial_sum, radial2_sum, samples: int) -> dict:
+    """The in-memory form of a distances file summed over ``samples`` structures of one run, all binned by
+    ``gb`` (Engine.sampler_read, radial sums added per structure): ``members`` = samples, and the pair and
+    bead counts are ``samples`` times one structure's, as in an ensemble file of that many members."""
+    pairs, n = _counts(gb)
+    s = np.uint64(samples)
+    return _result(dist_sum, dist2_sum, gb, pairs * s, n * s, radial_sum, radial2_sum, samples)
+
+
+def _counts(gb: GenomeBins) -> tuple[np.ndarray, np.ndarray]:
+    """(pair_count (B, B), bin_beads (B,)) of one structure binned by ``gb``."""
     bins = np.asarray(gb.bins, np.int64)
-    rs, r2s = radial_sums(x, center, bins, gb.n_bins)
     n = np.bincount(bins[bins >= 0], minlength=gb.n_bins).astype(np.uint64)
     pairs = np.outer(n, n)
     pairs[np.diag_indices(gb.n_bins)] = n * (n - np.uint64(1)) // np.uint64(2)  # 0 for an empty bin (wraps to 0 * ...)
+    return pairs, n
+
+
+def _result(dist_sum, dist2_sum, gb: GenomeBins, pairs, n, rs, r2s, members: int) -> dict:
     return dict(dist_sum=np.asarray(dist_sum, np.uint64), dist2_sum=np.asarray(dist2_sum, np.uint64),
-                pair_count=pairs, bin_beads=n, radial_sum=rs,
-                radial2_sum=r2s, members=np.int64(members), resolution_bp=np.int64(gb.resolution_bp),
-                bin_chrom=np.asarray(gb.bin_chrom, np.int32), bin_start_bp=np.asarray(gb.bin_start_bp, np.int64),
-                quantum_log2=np.int64(QUANTUM_LOG2))
+                pair_count=pairs, bin_beads=n, radial_sum=np.asarray(rs, np.uint64),
+                radial2_sum=np.asarray(r2s, np.uint64), members=np.int64(members),
+                resolution_bp=np.int64(gb.resolution_bp), bin_chrom=np.asarray(gb.bin_chrom, np.int32),
+                bin_start_bp=np.asarray(gb.bin_start_bp, np.int64), quantum_log2=np.int64(QUANTUM_LOG2))
 
 
 def save(path: str, d: dict):

@@ -238,6 +238,48 @@ class Engine:
         stream)."""
         return dict(device_ms=getattr(self, "_distance_ms", 0.0))
 
+    # -- trajectory maps (sums over many structures) --------------------------------------------------
+    def sampler_configure(self, rc_nm: float = 0.2, contact_bins=None, n_contact_bins: int = 0, fine_bins=None,
+                          n_fine_bins: int = 0, distance_bins=None, n_distance_bins: int = 0):
+        """Clear the sampler and set its maps (mmm_sampler_configure): the dense contact map, sep and pairs of
+        ``contacts`` over ``contact_bins``, the sparse map of ``contacts_sparse`` over ``fine_bins`` (needs
+        ``contact_bins``), the sums of ``distance_map`` over ``distance_bins``; None switches a map off."""
+        tabs = []
+        for bins in (contact_bins, fine_bins, distance_bins):
+            b = _arr(bins, np.int32)
+            if b is not None and b.shape != (self.n,):
+                raise ValueError(f"bin tables must have shape ({self.n},)")
+            tabs.append(b)
+        self._ck(self._lib.mmm_sampler_configure(self._h, float(rc_nm), _p(tabs[0]), int(n_contact_bins), _p(tabs[1]),
+                                                 int(n_fine_bins), _p(tabs[2]), int(n_distance_bins)))
+        self._sampler = (None if tabs[0] is None else int(n_contact_bins), None if tabs[1] is None else int(n_fine_bins),
+                         None if tabs[2] is None else int(n_distance_bins))
+
+    def sample(self):
+        """Add the structure at the current positions to every map of the sampler (mmm_sample)."""
+        self._ck(self._lib.mmm_sample(self._h))
+
+    def sampler_read(self) -> dict:
+        """The sampler's sums (mmm_sampler_read, mmm_sampler_read_fine): ``samples``; ``counts`` (B, B), ``sep``
+        (N,) uint64 and ``pairs``; the fine map ``rows``, ``cols`` int32, ``vals`` uint64 (sorted upper
+        triangle); ``dist_sum``, ``dist2_sum`` (B, B) uint64; ``device_ms`` of all samples.  The entries of a
+        map that is off are None."""
+        nc, nf, nd = getattr(self, "_sampler", (None, None, None))
+        counts = np.empty((nc, nc), np.uint64) if nc else None
+        sep = np.empty(self.n, np.uint64) if nc else None
+        dsum = np.empty((nd, nd), np.uint64) if nd else None
+        d2sum = np.empty((nd, nd), np.uint64) if nd else None
+        samples, pairs, entries, ms = C.c_int64(), C.c_int64(), C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_sampler_read(self._h, C.byref(samples), _p(counts), _p(sep), C.byref(pairs),
+                                            C.byref(entries), _p(dsum), _p(d2sum), C.byref(ms)))
+        out = dict(samples=int(samples.value), counts=counts, sep=sep, pairs=int(pairs.value) if nc else None,
+                   rows=None, cols=None, vals=None, dist_sum=dsum, dist2_sum=d2sum, device_ms=float(ms.value))
+        if nf:
+            e = int(entries.value)
+            out["rows"], out["cols"], out["vals"] = np.empty(e, np.int32), np.empty(e, np.int32), np.empty(e, np.uint64)
+            self._ck(self._lib.mmm_sampler_read_fine(self._h, _p(out["rows"]), _p(out["cols"]), _p(out["vals"])))
+        return out
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

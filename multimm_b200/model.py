@@ -132,6 +132,9 @@ class MultiMM:
         self.contacts_fine_file = None
         self.distances = None       # distance sums of the minimised structure (SAVE_DISTANCES)
         self.distances_file = None  # where finish() writes them; the ensemble driver points it outside run_<i>
+        # the same maps summed over the structures sampled during MD (MD_SAMPLE_STEP); written beside the
+        # files above, named by contacts.md_path
+        self.contacts_md = self.contacts_fine_md = self.distances_md = None
 
         # chrom_spin: chromosome id per bead; chrom_strength: indexed by POSITION in the (possibly
         # shuffled) order, not by chromosome id (model.py:158-162; appendix A, Q8)
@@ -372,7 +375,9 @@ class MultiMM:
         n_steps, every = int(a.SIM_N_STEPS), max(1, int(a.SIM_SAMPLING_STEP))
         dcd_every = max(1, n_steps // max(1, int(a.TRJ_FRAMES)))
         dcd = cif.DCDWriter(self.save_path + "metadata/MultiMM_annealing.dcd", a.N_BEADS, dt, dcd_every)
-        chunk = int(np.gcd(every, dcd_every))
+        sample_every = int(contact_setting(a, "MD_SAMPLE_STEP"))
+        sampling = self._configure_sampler() if sample_every > 0 else None
+        chunk = int(np.gcd.reduce([every, dcd_every] + ([sample_every] if sampling else [])))
         t0 = time.time()
         print('#"Step"\t"Potential Energy (kJ/mole)"\t"Kinetic Energy (kJ/mole)"\t"Total Energy (kJ/mole)"\t"Temperature (K)"')
         done = 0
@@ -394,8 +399,12 @@ class MultiMM:
                     cif.write_mmcif(10.0 * self.positions, self.chr_ends,
                                     self.save_path + f"md_frames/frame_{done // every}.cif", hetatm_ends=True,
                                     connections=False, decimals=4)
+                if sampling and done % sample_every == 0:
+                    self._sample(sampling)
         finally:
             dcd.close()
+        if sampling:
+            self._read_samples(sampling, sample_every)
         self.positions = self.engine.get_positions()
         cif.write_mmcif(10.0 * self.positions, self.chr_ends, self.save_path + "model/MultiMM_afterMD.cif",
                         hetatm_ends=True, connections=False, decimals=4)
@@ -460,6 +469,27 @@ class MultiMM:
         if self.args.SIM_RUN_MD:
             self.run_md()
 
+    def _contact_bins(self, fine: bool = False):
+        """Canonical bins of the contact map (fine: of the fine map, None when CONTACT_FINE_RESOLUTION is 0)."""
+        from . import contacts
+
+        a = self.args
+        if not fine:
+            return contacts.genome_bins(self.layout, int(contact_setting(a, "CONTACT_RESOLUTION")), n_beads=a.N_BEADS)
+        fine_res = int(contact_setting(a, "CONTACT_FINE_RESOLUTION"))
+        if fine_res <= 0:
+            return None
+        return contacts.genome_bins(self.layout, fine_res, n_beads=a.N_BEADS, max_bins=contacts.MAX_FINE_BINS)
+
+    def _distance_bins(self):
+        from . import contacts, distances
+
+        res = int(contact_setting(self.args, "DISTANCE_RESOLUTION"))
+        try:
+            return contacts.genome_bins(self.layout, res, n_beads=self.args.N_BEADS, max_bins=distances.MAX_BINS)
+        except ValueError as e:
+            raise ValueError(f"DISTANCE_RESOLUTION={res}: {e}") from None
+
     def count_contacts(self):
         """Contacts of the minimised structure (SAVE_CONTACTS), counted by this member's own engine at the
         positions the minimisation left on the device, binned in canonical genomic coordinates."""
@@ -467,15 +497,14 @@ class MultiMM:
 
         t0 = time.time()
         a = self.args
-        gb = contacts.genome_bins(self.layout, int(contact_setting(a, "CONTACT_RESOLUTION")), n_beads=a.N_BEADS)
+        gb = self._contact_bins()
         rc = float(contact_setting(a, "CONTACT_RADIUS"))
         cmap, sep, pairs = self.engine.contacts(rc, gb.bins, gb.n_bins)
         self.contacts = contacts.result(cmap, sep, pairs, rc, gb, contacts.sep_pairs(self.chrom_spin))
         self.timings["contacts_s"] = time.time() - t0
-        fine_res = int(contact_setting(a, "CONTACT_FINE_RESOLUTION"))
-        if fine_res > 0:
+        fb = self._contact_bins(fine=True)
+        if fb is not None:
             t0 = time.time()
-            fb = contacts.genome_bins(self.layout, fine_res, n_beads=a.N_BEADS, max_bins=contacts.MAX_FINE_BINS)
             rows, cols, vals, pairs = self.engine.contacts_sparse(rc, fb.bins, fb.n_bins)
             self.contacts_fine = contacts.fine_result(rows, cols, vals, pairs, rc, fb)
             self.timings["contacts_fine_s"] = time.time() - t0
@@ -487,15 +516,55 @@ class MultiMM:
         from . import contacts, distances
 
         t0 = time.time()
-        a = self.args
-        res = int(contact_setting(a, "DISTANCE_RESOLUTION"))
-        try:
-            gb = contacts.genome_bins(self.layout, res, n_beads=a.N_BEADS, max_bins=distances.MAX_BINS)
-        except ValueError as e:
-            raise ValueError(f"DISTANCE_RESOLUTION={res}: {e}") from None
+        gb = self._distance_bins()
         dsum, d2sum = self.engine.distance_map(gb.bins, gb.n_bins)
         self.distances = distances.result(dsum, d2sum, gb, self.engine.get_positions(), self.mass_center)
         self.timings["distances_s"] = time.time() - t0
+
+    def _configure_sampler(self) -> dict:
+        """MD_SAMPLE_STEP: set up the engine's sampler with the maps that are on (SAVE_CONTACTS with its fine map,
+        SAVE_DISTANCES), binned as the minimised structure's.  Returns the bins and the host-side radial sums."""
+        a = self.args
+        st = dict(rc=float(contact_setting(a, "CONTACT_RADIUS")), gb=None, fb=None, db=None)
+        if contact_setting(a, "SAVE_CONTACTS"):
+            st["gb"], st["fb"] = self._contact_bins(), self._contact_bins(fine=True)
+        if contact_setting(a, "SAVE_DISTANCES"):
+            db = st["db"] = self._distance_bins()
+            st["radial"] = [np.zeros(db.n_bins, np.uint64), np.zeros(db.n_bins, np.uint64)]
+        gb, fb, db = st["gb"], st["fb"], st["db"]
+        self.engine.sampler_configure(st["rc"], None if gb is None else gb.bins, 0 if gb is None else gb.n_bins,
+                                      None if fb is None else fb.bins, 0 if fb is None else fb.n_bins,
+                                      None if db is None else db.bins, 0 if db is None else db.n_bins)
+        return st
+
+    def _sample(self, st: dict):
+        """Add the structure on the device to the trajectory maps; the radial sums (O(N)) on the host."""
+        from . import distances
+
+        self.engine.sample()
+        if st["db"] is not None:
+            rs, r2s = distances.radial_sums(self.engine.get_positions(), self.mass_center, st["db"].bins,
+                                            st["db"].n_bins)
+            st["radial"][0] += rs
+            st["radial"][1] += r2s
+
+    def _read_samples(self, st: dict, sample_every: int):
+        from . import contacts, distances
+
+        r = self.engine.sampler_read()
+        s = r["samples"]
+        logger.info(f"trajectory maps: {s} structures sampled every {sample_every} MD steps "
+                    f"({r['device_ms']:.1f} ms on the device)")
+        if s == 0:
+            return
+        if st["gb"] is not None:
+            self.contacts_md = contacts.result(r["counts"], r["sep"], r["pairs"], st["rc"], st["gb"],
+                                               np.uint64(s) * contacts.sep_pairs(self.chrom_spin), members=s)
+        if st["fb"] is not None:
+            self.contacts_fine_md = contacts.fine_result(r["rows"], r["cols"], r["vals"], r["pairs"], st["rc"],
+                                                         st["fb"], members=s)
+        if st["db"] is not None:
+            self.distances_md = distances.sampled_result(r["dist_sum"], r["dist2_sum"], st["db"], *st["radial"], s)
 
     def finish(self):
         """Structure files, per-chromosome files, reports, parameters.  Host work (the report's device
@@ -505,23 +574,21 @@ class MultiMM:
             self.save_chromosomes()  # the minimised structure, as model.py:1222-1224 (before MD)
         if self.args.SAVE_PLOTS:
             self.make_reports()
-        if self.contacts is not None:
-            from . import contacts
+        from . import contacts, distances
 
-            if self.contacts_file is None:
-                contacts.save_dense(os.path.join(self.save_path, "analysis", "contacts.npz"), self.contacts)
-            else:
-                contacts.save_member(self.contacts_file, self.contacts)
-        if self.contacts_fine is not None:
-            from . import contacts
-
-            path = self.contacts_fine_file or os.path.join(self.save_path, "analysis", "contacts_fine.npz")
-            contacts.save_fine(path, self.contacts_fine)
-        if self.distances is not None:
-            from . import distances
-
-            distances.save(self.distances_file or os.path.join(self.save_path, "analysis", "distances.npz"),
-                           self.distances)
+        dense_path = self.contacts_file or os.path.join(self.save_path, "analysis", "contacts.npz")
+        fine_path = self.contacts_fine_file or os.path.join(self.save_path, "analysis", "contacts_fine.npz")
+        dist_path = self.distances_file or os.path.join(self.save_path, "analysis", "distances.npz")
+        save_dense = contacts.save_dense if self.contacts_file is None else contacts.save_member
+        for d, md_path in ((self.contacts, dense_path), (self.contacts_md, contacts.md_path(dense_path))):
+            if d is not None:
+                save_dense(md_path, d)
+        for d, path in ((self.contacts_fine, fine_path), (self.contacts_fine_md, contacts.md_path(fine_path))):
+            if d is not None:
+                contacts.save_fine(path, d)
+        for d, path in ((self.distances, dist_path), (self.distances_md, contacts.md_path(dist_path))):
+            if d is not None:
+                distances.save(path, d)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

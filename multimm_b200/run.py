@@ -201,6 +201,27 @@ def args_tests(args):
                          f"(supported: {', '.join(_lib.MD_INTEGRATORS)})")
     check_contact_fields(args)
     check_distance_fields(args)
+    check_md_sample_fields(args)
+
+
+def check_md_sample_fields(args):
+    """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES), and the
+    MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps, must reach the first
+    sample."""
+    step = int(contact_setting(args, "MD_SAMPLE_STEP"))
+    if step < 0:
+        raise ValueError(f"MD_SAMPLE_STEP={step} must be >= 0 (0 = no trajectory maps)")
+    if step == 0:
+        return
+    if not args.SIM_RUN_MD:
+        raise ValueError(f"MD_SAMPLE_STEP={step} samples the MD run, but SIM_RUN_MD is off")
+    if not (contact_setting(args, "SAVE_CONTACTS") or contact_setting(args, "SAVE_DISTANCES")):
+        raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES")
+    every = max(1, int(args.SIM_SAMPLING_STEP))
+    steps = (int(args.SIM_N_STEPS) // every) * every
+    if step > steps:
+        raise ValueError(f"MD_SAMPLE_STEP={step} exceeds the {steps} MD steps that run "
+                         "((SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP): no structure would be sampled")
 
 
 def check_distance_fields(args):
@@ -418,45 +439,63 @@ def member_distances_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "distances", f"member_{i}.npz")
 
 
+def _sampled_md(args) -> bool:
+    """The run writes trajectory maps (MD_SAMPLE_STEP with MD on)."""
+    return bool(args.SIM_RUN_MD) and int(contact_setting(args, "MD_SAMPLE_STEP")) > 0
+
+
 def write_ensemble_distances(args, results: list[dict]) -> str | None:
     """SAVE_DISTANCES: OUT_PATH/ensemble_distances.npz, the sum of the distance files of the members that
-    succeeded (exact integer sums: the same bits whichever GPU ran which member)."""
+    succeeded (exact integer sums: the same bits whichever GPU ran which member); with MD_SAMPLE_STEP also
+    ensemble_distances_md.npz, the sum of their trajectory maps."""
     if not contact_setting(args, "SAVE_DISTANCES") or not results:
         return None
-    from . import distances
+    from . import contacts, distances
 
-    paths = [member_distances_path(args.OUT_PATH, r["replica"]) for r in sorted(results, key=lambda r: r["replica"])]
-    agg = distances.aggregate(paths)
-    out = os.path.join(args.OUT_PATH, "ensemble_distances.npz")
-    distances.save(out, agg)
-    logger.info(f"ensemble distances: {int(agg['members'])} members, {len(agg['bin_beads'])} bins at "
-                f"{int(agg['resolution_bp'])} bp -> {out}")
+    out = None
+    for md in (False, True) if _sampled_md(args) else (False,):
+        name = contacts.md_path if md else (lambda p: p)
+        paths = [name(member_distances_path(args.OUT_PATH, r["replica"]))
+                 for r in sorted(results, key=lambda r: r["replica"])]
+        agg = distances.aggregate(paths)
+        path = name(os.path.join(args.OUT_PATH, "ensemble_distances.npz"))
+        distances.save(path, agg)
+        logger.info(f"ensemble distances{' (MD samples)' if md else ''}: {int(agg['members'])} "
+                    f"{'structures' if md else 'members'}, {len(agg['bin_beads'])} bins at "
+                    f"{int(agg['resolution_bp'])} bp -> {path}")
+        out = out or path
     return out
 
 
 def write_ensemble_contacts(args, results: list[dict]) -> str | None:
     """SAVE_CONTACTS: OUT_PATH/ensemble_contacts.npz, the sum of the contact files of the members that
-    succeeded (exact integer sums: the same bits whichever GPU ran which member)."""
+    succeeded (exact integer sums: the same bits whichever GPU ran which member); with MD_SAMPLE_STEP also
+    ensemble_contacts_md.npz (and _fine_md), the sum of their trajectory maps."""
     if not contact_setting(args, "SAVE_CONTACTS") or not results:
         return None
     from . import contacts
 
-    paths = [member_contacts_path(args.OUT_PATH, r["replica"]) for r in sorted(results, key=lambda r: r["replica"])]
-    agg = contacts.aggregate(paths)
-    out = os.path.join(args.OUT_PATH, "ensemble_contacts.npz")
-    contacts.save_dense(out, agg)
-    logger.info(f"ensemble contacts: {int(agg['members'])} members, {agg['counts'].shape[0]} bins at "
-                f"{int(agg['resolution_bp'])} bp, {int(agg['pairs'])} contacts (rc = {float(agg['radius_nm'])} nm) "
-                f"-> {out}")
-    if int(contact_setting(args, "CONTACT_FINE_RESOLUTION")) > 0:
-        paths = [member_contacts_fine_path(args.OUT_PATH, r["replica"])
-                 for r in sorted(results, key=lambda r: r["replica"])]
-        fine = contacts.aggregate_fine(paths)
-        out_fine = os.path.join(args.OUT_PATH, "ensemble_contacts_fine.npz")
-        contacts.save_fine(out_fine, fine)
-        logger.info(f"ensemble fine contacts: {int(fine['members'])} members, {int(fine['n_bins'])} bins at "
-                    f"{int(fine['resolution_bp'])} bp, {len(fine['vals'])} entries, {int(fine['pairs'])} contacts "
-                    f"-> {out_fine}")
+    out = None
+    members = sorted(results, key=lambda r: r["replica"])
+    for md in (False, True) if _sampled_md(args) else (False,):
+        name = contacts.md_path if md else (lambda p: p)
+        what, unit = (" (MD samples)", "structures") if md else ("", "members")
+        paths = [name(member_contacts_path(args.OUT_PATH, r["replica"])) for r in members]
+        agg = contacts.aggregate(paths)
+        path = name(os.path.join(args.OUT_PATH, "ensemble_contacts.npz"))
+        contacts.save_dense(path, agg)
+        logger.info(f"ensemble contacts{what}: {int(agg['members'])} {unit}, {agg['counts'].shape[0]} bins at "
+                    f"{int(agg['resolution_bp'])} bp, {int(agg['pairs'])} contacts (rc = {float(agg['radius_nm'])} nm) "
+                    f"-> {path}")
+        out = out or path
+        if int(contact_setting(args, "CONTACT_FINE_RESOLUTION")) > 0:
+            paths = [name(member_contacts_fine_path(args.OUT_PATH, r["replica"])) for r in members]
+            fine = contacts.aggregate_fine(paths)
+            out_fine = name(os.path.join(args.OUT_PATH, "ensemble_contacts_fine.npz"))
+            contacts.save_fine(out_fine, fine)
+            logger.info(f"ensemble fine contacts{what}: {int(fine['members'])} {unit}, {int(fine['n_bins'])} bins at "
+                        f"{int(fine['resolution_bp'])} bp, {len(fine['vals'])} entries, {int(fine['pairs'])} contacts "
+                        f"-> {out_fine}")
     return out
 
 
