@@ -325,6 +325,40 @@ int mmm_sampler_read(mmm_handle h, int64_t *samples_out, uint64_t *contact_map_o
  * succeeds.  MMM_ERR_STATE as mmm_sample. */
 int mmm_sampler_read_fine(mmm_handle h, int32_t *rows_out, int32_t *cols_out, uint64_t *vals_out);
 
+/* ---- loop readout (per-loop contact frequency and anchor distance, aggregate peak analysis of the loops of
+ * the input table, summed over structures; not in the reference, whose loops enter only as bonds,
+ * model.py:650-665) ------------------------------------------------------------------------------------- */
+/* Sets up the loop accumulator of this handle and clears its sums: the contact radius, the APA window W
+ * (0 <= window <= 25) and n_loops >= 0 rows (int32, group int8, each array of length n_loops): anchor beads
+ * bead_lo < bead_hi, the chromosome block [first_lo, end_lo) that holds bead_lo and [first_hi, end_hi) that
+ * holds bead_hi, group 0 (enforced) or 1 (held out).  MMM_ERR_ARG for rc <= 0 or not finite, a window outside
+ * [0, 25], a block that is empty or outside [0, N), a bead outside its block, bead_lo >= bead_hi or a group
+ * outside {0, 1}.  The buffers are the accumulator's own (allocated here, freed with the handle). */
+int mmm_loops_configure(mmm_handle h, double rc_nm, int32_t window, int32_t n_loops, const int32_t *bead_lo,
+                        const int32_t *bead_hi, const int32_t *first_lo, const int32_t *end_lo,
+                        const int32_t *first_hi, const int32_t *end_hi, const int8_t *group);
+/* Adds the structure at the current positions.  With d2 = (dx*dx + dy*dy) + dz*dz in FP64 on the master
+ * positions (as mmm_contacts), qd = rint(sqrt(d2) * 2^24) and qd2 = rint(d2 * 2^24) (as mmm_distance_map):
+ *   per row r at (lo, hi): contacts[r] += (d2 < rc^2), dist_sum[r] += qd, dist2_sum[r] += qd2;
+ *   per group g and offset (a, b) in [-W, W]^2, over the rows of g with first_lo <= lo + a < end_lo,
+ *   first_hi <= hi + b < end_hi and lo + a < hi + b, at (lo + a, hi + b):
+ *   apa_contacts[g][a][b] += (d2 < rc^2), apa_dist_sum[g][a][b] += qd.
+ * Integer sums: exact and independent of order, so K adds equal the sum of K single-structure reads.  The
+ * int64 guard is cumulative: MMM_ERR_ARG, with every sum left as it was, when max(n_loops, 1) x (largest
+ * quantised distance, from the beads' bounding box as in mmm_distance_map) would take the sum of the bounds of
+ * the structures already added to 2^63, or when the positions are not finite.  MMM_ERR_STATE before
+ * mmm_loops_configure or before positions are set.  Changes no state an evaluation, a minimisation, an MD step,
+ * mmm_last_result or the trajectory sampler reads; synchronises with the host. */
+int mmm_loops_add(mmm_handle h);
+/* The sums of the structures added since mmm_loops_configure: samples_out, the number of structures;
+ * contacts_out, dist_sum_out, dist2_sum_out (uint64[n_loops], in units of 2^-24 nm and nm^2);
+ * apa_contacts_out, apa_dist_sum_out (uint64[2][2W+1][2W+1]: group, a + W, b + W); device_ms_out, the device
+ * time of all mmm_loops_add calls (CUDA events on the handle's stream).  Any output may be NULL.
+ * MMM_ERR_STATE as mmm_loops_add. */
+int mmm_loops_read(mmm_handle h, int64_t *samples_out, uint64_t *contacts_out, uint64_t *dist_sum_out,
+                   uint64_t *dist2_sum_out, uint64_t *apa_contacts_out, uint64_t *apa_dist_sum_out,
+                   float *device_ms_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

@@ -204,13 +204,20 @@ DISTANCE_FIELDS: dict[str, tuple[Any, Any]] = {
 MD_SAMPLE_FIELDS: dict[str, tuple[Any, Any]] = {
     "MD_SAMPLE_STEP": (int, 0),           # MD steps between two structures added to the trajectory maps; 0 = off
 }
-EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS}
+# Loop readout (multimm_b200.loops), kept the same way: per-loop contact frequencies and anchor distances and
+# aggregate peak analysis of the rows of LOOPS_PATH; the contact test uses CONTACT_RADIUS, and MD_SAMPLE_STEP
+# also samples it.
+LOOP_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_LOOPS": (B, False),             # measure the input loops in the minimised structure (analysis/loops.npz; ensembles: ensemble_loops.npz)
+    "LOOP_APA_WINDOW": (int, 10),         # beads on each side of an anchor in the APA window, in [0, 25]
+}
+EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS, **LOOP_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
-    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS or MD_SAMPLE_FIELDS setting of `args`, its
-    default where it was not given."""
+    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS or LOOP_FIELDS setting of
+    `args`, its default where it was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

@@ -136,10 +136,7 @@ __global__ void __launch_bounds__(CT_WARPS * 32) k_contacts(
         const int jstart = tb == a ? lane + 1 : 0;  // i < j inside the diagonal tile
         if (ireal && jn > jstart) ncand += (unsigned long long)(jn - jstart);
         for (int jj = 0; jj < jn; ++jj) {  // every lane runs every step: the votes below see the whole warp
-          const double dx = __dadd_rn(xi, -s_x[w][0][jj]);
-          const double dy = __dadd_rn(yi, -s_x[w][1][jj]);
-          const double dz = __dadd_rn(zi, -s_x[w][2][jj]);
-          const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+          const double d2 = mmm_pair_d2(xi, yi, zi, s_x[w][0][jj], s_x[w][1][jj], s_x[w][2][jj]);
           const bool hit = ireal && jj >= jstart && d2 < rc2;
           if (!__any_sync(full, hit)) continue;
           const int bj = s_bin[w][jj];

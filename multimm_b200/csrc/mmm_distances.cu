@@ -32,7 +32,6 @@ constexpr int DM_WARPS = 8;          // warps per CTA
 constexpr int DM_CHUNK = 8;          // consecutive tile pairs per work item
 constexpr int DM_MAX_BINS = 4096;    // two dense maps of 128 MB each
 constexpr int DM_BOX_BLOCKS = 256;   // partial bounding boxes
-constexpr double DM_SCALE = 0x1p24;  // 1 / Q
 
 // first tile pair of row a: rows 0 .. a-1 hold ntr, ntr - 1, ..., ntr - a + 1 pairs
 __device__ __forceinline__ long long dm_row_start(long long a, long long ntr) { return a * ntr - a * (a - 1) / 2; }
@@ -126,13 +125,10 @@ __global__ void __launch_bounds__(DM_WARPS * 32) k_distance_map(const double* __
           sd = sd2 = 0;
           run = bj;
         }
-        const double dx = __dadd_rn(xi, -s_x[w][0][jj]);
-        const double dy = __dadd_rn(yi, -s_x[w][1][jj]);
-        const double dz = __dadd_rn(zi, -s_x[w][2][jj]);
-        const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+        const double d2 = mmm_pair_d2(xi, yi, zi, s_x[w][0][jj], s_x[w][1][jj], s_x[w][2][jj]);
         if (ireal && jj >= jstart && bi >= 0 && bj >= 0) {
-          sd += (unsigned long long)__double2ll_rn(__dmul_rn(__dsqrt_rn(d2), DM_SCALE));
-          sd2 += (unsigned long long)__double2ll_rn(__dmul_rn(d2, DM_SCALE));
+          sd += mmm_quantise(__dsqrt_rn(d2));
+          sd2 += mmm_quantise(d2);
         }
       }
       if (++b == ntr) {
@@ -170,12 +166,11 @@ __global__ void __launch_bounds__(256) k_dm_bbox(const double* __restrict__ x, i
 
 }  // namespace
 
-// Overflow guard of the distance sums: *bound = (pairs of the fullest bin pair) x (largest quantised value of
-// one pair), occ = beads per bin.  D bounds every pair distance: the diagonal of the beads' FP64 bounding box,
-// padded for rounding.  MMM_ERR_ARG (message prefixed by who) when the positions are not finite or when
-// prior + *bound reaches 2^63: the one-shot map passes prior = 0, the trajectory sampler the bounds of the
-// structures it has already summed.  Launches one kernel and synchronises; writes nothing else.
-int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t>& occ, double prior, double* bound) {
+// The quantised-distance bound of the current positions: *dpad bounds every bead pair's distance (the diagonal
+// of the beads' FP64 bounding box, padded for the rounding of d2 and d) and *qmax the quantised distance and
+// squared distance of every pair.  MMM_ERR_ARG (message prefixed by who) when the positions are not finite.
+// Launches one kernel and synchronises; writes nothing else.  The distance maps and mmm_loops_add guard with it.
+int mmm_distance_qmax(mmm_system* h, const char* who, double* dpad, double* qmax) {
   const int n = (int)h->n;
   int rc;
   if ((rc = mmm_reserve(h, h->d_dm_box, (size_t)DM_BOX_BLOCKS * 6, "distance-map boxes"))) return rc;
@@ -199,6 +194,20 @@ int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t
   }
   if (!std::isfinite(d2max))
     return mmm_fail(h, MMM_ERR_ARG, std::string(who) + ": positions are not finite (no distance can be quantised)");
+  *dpad = sqrt(d2max) * (1.0 + 0x1p-40) + 0x1p-60;  // D, padded for the rounding of d2 and d
+  *qmax = ceil(MMM_DIST_SCALE * std::max(*dpad * *dpad, *dpad)) + 1.0;  // bounds qd and qd2 of every pair
+  return MMM_OK;
+}
+
+// Overflow guard of the distance sums: *bound = (pairs of the fullest bin pair) x (largest quantised value of
+// one pair, mmm_distance_qmax), occ = beads per bin.  MMM_ERR_ARG (message prefixed by who) when the positions
+// are not finite or when prior + *bound reaches 2^63: the one-shot map passes prior = 0, the trajectory
+// sampler the bounds of the structures it has already summed.  Launches one kernel and synchronises; writes
+// nothing else.
+int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t>& occ, double prior, double* bound) {
+  double dpad, qmax;
+  int rc;
+  if ((rc = mmm_distance_qmax(h, who, &dpad, &qmax))) return rc;
   double pmax = 0.0, top1 = 0.0, top2 = 0.0;  // pairs of the fullest bin pair: a diagonal one or the two fullest bins
   for (int64_t c : occ) {
     const double v = (double)c;
@@ -211,8 +220,6 @@ int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t
     }
   }
   pmax = std::max(pmax, top1 * top2);
-  const double dpad = sqrt(d2max) * (1.0 + 0x1p-40) + 0x1p-60;  // D, padded for the rounding of d2 and d
-  const double qmax = ceil(DM_SCALE * std::max(dpad * dpad, dpad)) + 1.0;  // bounds qd and qd2 of every pair
   *bound = pmax * qmax;
   if (prior + *bound >= 0x1p63)
     return mmm_fail(h, MMM_ERR_ARG,

@@ -103,6 +103,29 @@ struct CellGrid {
   int dim, bits;       // cells per axis, key bits per axis
 };
 
+// One valid row of the loop table (mmm_loops.cu): anchor beads lo < hi, the chromosome block [first, end)
+// of each anchor, group 0 (enforced) or 1 (held out).
+struct LoopRow {
+  int lo, hi, first_lo, end_lo, first_hi, end_hi, group, pad;
+};
+
+// ---------------------------------------------------------------------------------------
+// the FP64 pair arithmetic of the analysis passes (mmm_contacts, mmm_distance_map, mmm_loops)
+// ---------------------------------------------------------------------------------------
+// d2 = (dx*dx + dy*dy) + dz*dz rounded operation by operation (no FMA contraction), so that a numpy
+// evaluation of the same expression gives the same bits; a pair is a contact when d2 < rc^2.
+__device__ __forceinline__ double mmm_pair_d2(double xi, double yi, double zi, double xj, double yj, double zj) {
+  const double dx = __dadd_rn(xi, -xj);
+  const double dy = __dadd_rn(yi, -yj);
+  const double dz = __dadd_rn(zi, -zj);
+  return __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+}
+constexpr double MMM_DIST_SCALE = 0x1p24;  // 1 / Q: distances are summed in units of Q = 2^-24 nm (nm^2)
+// rint(v / Q), half to even (the scaling is exact): v = d (correctly rounded sqrt of d2) or d2
+__device__ __forceinline__ unsigned long long mmm_quantise(double v) {
+  return (unsigned long long)__double2ll_rn(__dmul_rn(v, MMM_DIST_SCALE));
+}
+
 // ---------------------------------------------------------------------------------------
 // device memory
 // ---------------------------------------------------------------------------------------
@@ -333,6 +356,18 @@ struct mmm_system {
   DevBuf<unsigned long long> d_sp_acc_key[2], d_sp_acc_val[2];
   DevBuf<long long> d_sp_mpart;                        // merge partition, then run offsets of the merge
   int64_t sp_fine_n = 0;                               // accumulated fine entries
+
+  // loop readout (mmm_loops.cu): per-row and APA sums over structures, on the device until read
+  bool lp_configured = false;
+  double lp_rc = 0.0;
+  int lp_w = 0;                            // APA window: offsets [-lp_w, lp_w] on each anchor
+  int64_t lp_rows = 0;
+  int64_t lp_samples = 0;
+  double lp_bound = 0.0;                   // summed per-structure bounds of the sums (overflow guard)
+  float lp_ms = 0.f;                       // device time of all adds
+  cudaEvent_t lp_ev0 = nullptr, lp_ev1 = nullptr;
+  DevBuf<LoopRow> d_lp_row;                // [rows]
+  DevBuf<unsigned long long> d_lp_sum;     // [3][rows] contacts, dist_sum, dist2_sum; [2 sums][2 groups][(2W+1)^2] APA
 };
 
 // the sorted keys of one sparse pass (mmm_contacts_sparse_pass)
@@ -436,6 +471,7 @@ int mmm_contacts_sparse_pass(mmm_system* h, double rc_nm, const int* d_bin, int3
 int mmm_contacts_fine_accumulate(mmm_system* h);  // the sampler's fine map += the current structure's
 int mmm_contacts_fine_read(mmm_system* h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out);
 // mmm_distances.cu
+int mmm_distance_qmax(mmm_system* h, const char* who, double* dpad, double* qmax);
 int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t>& occ, double prior, double* bound);
 int mmm_distance_pass(mmm_system* h, const int* d_bin, int32_t n_bins, unsigned long long* dmap,
                       unsigned long long* d2map, bool clear);

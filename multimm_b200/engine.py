@@ -280,6 +280,38 @@ class Engine:
             self._ck(self._lib.mmm_sampler_read_fine(self._h, _p(out["rows"]), _p(out["cols"]), _p(out["vals"])))
         return out
 
+    # -- loop readout (per-loop sums and APA over many structures) -------------------------------------
+    def loops_configure(self, rc_nm: float, window: int, bead_lo, bead_hi, first_lo, end_lo, first_hi, end_hi,
+                        group):
+        """Clear the loop accumulator and set its rows (mmm_loops_configure): anchor beads ``bead_lo`` <
+        ``bead_hi``, the chromosome block [first, end) of each, ``group`` 0 (enforced) or 1 (held out); the
+        contact radius and the APA window W in [0, 25].  loops.device_rows gives these for a member."""
+        cols = [_arr(a, np.int32) for a in (bead_lo, bead_hi, first_lo, end_lo, first_hi, end_hi)]
+        grp = _arr(group, np.int8)
+        r = len(cols[0])
+        if any(c.shape != (r,) for c in cols) or grp.shape != (r,):
+            raise ValueError("loop rows: every array must have the same length")
+        self._ck(self._lib.mmm_loops_configure(self._h, float(rc_nm), int(window), r, *(_p(c) for c in cols), _p(grp)))
+        self._loops = (r, int(window))
+
+    def loops_add(self):
+        """Add the structure at the current positions to the loop sums (mmm_loops_add)."""
+        self._ck(self._lib.mmm_loops_add(self._h))
+
+    def loops_read(self) -> dict:
+        """The loop sums (mmm_loops_read): ``samples``; ``contacts``, ``dist_sum``, ``dist2_sum`` uint64[rows];
+        ``apa_contacts``, ``apa_dist_sum`` uint64 [2][2W+1][2W+1]; ``device_ms`` of all adds."""
+        r, w = getattr(self, "_loops", (0, 0))
+        span = 2 * w + 1
+        out = {k: np.zeros(r, np.uint64) for k in ("contacts", "dist_sum", "dist2_sum")}
+        out.update(apa_contacts=np.zeros((2, span, span), np.uint64), apa_dist_sum=np.zeros((2, span, span), np.uint64))
+        samples, ms = C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_loops_read(self._h, C.byref(samples), _p(out["contacts"]), _p(out["dist_sum"]),
+                                          _p(out["dist2_sum"]), _p(out["apa_contacts"]), _p(out["apa_dist_sum"]),
+                                          C.byref(ms)))
+        out.update(samples=int(samples.value), device_ms=float(ms.value))
+        return out
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

@@ -139,30 +139,9 @@ def import_mns_from_bedpe(bedpe_file, N_beads, coords=None, chrom=None, threshol
     np.random.seed(seed)
     df = pd.read_csv(bedpe_file, header=None, sep="\t")
     idxs, ends = _chrom_layout(chrom, shuffle, n_chroms)
-    if chrom is not None:
-        df = df[(df[0] == chrom) & (df[1] > coords[0]) & (df[2] < coords[1]) & (df[4] > coords[0])
-                & (df[5] < coords[1])].reset_index(drop=True)
-    c = [df[k].to_numpy(dtype=np.int64).copy() for k in (1, 2, 4, 5)]
+    df = loop_rows(df, chrom, coords).reset_index(drop=True)
     counts_raw = df[6].to_numpy(dtype=np.float64)
-    if chrom is None:
-        n0, n3 = df[0].to_numpy(), df[3].to_numpy()
-        for count, ci in enumerate(idxs):
-            name = CHROM_NAMES[int(ci)]
-            s0, s3 = n0 == name, n3 == name
-            c[0][s0] += ends[count]
-            c[1][s0] += ends[count]
-            c[2][s3] += ends[count]
-            c[3][s3] += ends[count]
-        resolution = int(np.max(c[3])) // N_beads
-    else:
-        resolution = (coords[1] - coords[0]) // N_beads
-        for a in c:
-            a -= coords[0]
-    chr_ends = ends // resolution
-    chr_ends[-1] = N_beads
-    c = [a // resolution for a in c]
-    ms = (c[0] + c[1]) // 2
-    ns = (c[2] + c[3]) // 2
+    ms, ns, resolution, chr_ends = loop_anchor_beads(df, idxs, ends, N_beads, chrom, coords)
     # mean count per (m, n); unique columns in lexicographic order, first occurrence wins
     pair = np.stack([ms, ns], axis=1)
     uniq, first, inv = np.unique(pair, axis=0, return_index=True, return_inverse=True)
@@ -198,6 +177,45 @@ def import_mns_from_bedpe(bedpe_file, N_beads, coords=None, chrom=None, threshol
                       chrom_idxs=idxs.astype(np.int64), start_bp=int(coords[0]) if chrom is not None else 0,
                       stop_bp=int(coords[1]) if chrom is not None else None)
     return ms.astype(int), ns.astype(int), ds, chr_ends.astype(int), idxs.astype(int)
+
+
+def loop_rows(df, chrom=None, coords=None):
+    """The rows of a bedpe table (columns 0..6) that import_mns_from_bedpe reads, in file order and with the
+    file's row index: all of them genome-wide; in a chromosome, region or gene run those whose first anchor is
+    on ``chrom`` and whose four coordinates lie inside ``coords`` (the second anchor's chromosome is not
+    checked)."""
+    if chrom is None:
+        return df
+    return df[(df[0] == chrom) & (df[1] > coords[0]) & (df[2] < coords[1]) & (df[4] > coords[0])
+              & (df[5] < coords[1])]
+
+
+def loop_anchor_beads(df, idxs, ends, N_beads, chrom=None, coords=None):
+    """The loader's bp -> bead arithmetic for every row of ``df`` (rows of loop_rows), with the chromosome
+    layout ``idxs``, ``ends`` of _chrom_layout: (m, n, resolution, chr_ends), m and n the bead midpoints
+    ``(a // res + b // res) // 2`` of the two anchors, not yet clamped to N - 1.  Genome-wide an anchor is
+    offset by its chromosome's block start ``ends[k]``; an anchor on a chromosome that is not modelled keeps
+    its raw coordinates (SURVEY appendix A, Q5).  In a region run every coordinate is taken relative to
+    ``coords[0]``."""
+    c = [df[k].to_numpy(dtype=np.int64).copy() for k in (1, 2, 4, 5)]
+    if chrom is None:
+        n0, n3 = df[0].to_numpy(), df[3].to_numpy()
+        for count, ci in enumerate(idxs):
+            name = CHROM_NAMES[int(ci)]
+            s0, s3 = n0 == name, n3 == name
+            c[0][s0] += ends[count]
+            c[1][s0] += ends[count]
+            c[2][s3] += ends[count]
+            c[3][s3] += ends[count]
+        resolution = int(np.max(c[3])) // N_beads
+    else:
+        resolution = (coords[1] - coords[0]) // N_beads
+        for a in c:
+            a -= coords[0]
+    chr_ends = ends // resolution
+    chr_ends[-1] = N_beads
+    c = [a // resolution for a in c]
+    return (c[0] + c[1]) // 2, (c[2] + c[3]) // 2, resolution, chr_ends
 
 
 def _minmax_raw(x):

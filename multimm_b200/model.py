@@ -65,6 +65,11 @@ def resolve_platform(name) -> str:
 
 
 class MultiMM:
+    # the loop readout (SAVE_LOOPS): the loop table and how this member measures it (built in __init__ from the
+    # loader's inputs), the sums of the minimised structure and of the MD samples, and where finish() writes
+    # them (the ensemble driver points loops_file outside run_<i>)
+    loop_table = loop_rows = loops = loops_md = loops_file = None
+
     def __init__(self, args, device: int | None = None):
         self.args = args
         self.ms = self.ns = self.ds = self.chr_ends = self.Cs = None
@@ -135,6 +140,11 @@ class MultiMM:
         # the same maps summed over the structures sampled during MD (MD_SAMPLE_STEP); written beside the
         # files above, named by contacts.md_path
         self.contacts_md = self.contacts_fine_md = self.distances_md = None
+        if contact_setting(args, "SAVE_LOOPS"):
+            from . import loops
+
+            self.loop_table = loops.table(args.LOOPS_PATH, chrom, coords)
+            self.loop_rows = loops.member_rows(self.loop_table, self.layout, args.N_BEADS, self.ms, self.ns, chrom)
 
         # chrom_spin: chromosome id per bead; chrom_strength: indexed by POSITION in the (possibly
         # shuffled) order, not by chromosome id (model.py:158-162; appendix A, Q8)
@@ -376,8 +386,12 @@ class MultiMM:
         dcd_every = max(1, n_steps // max(1, int(a.TRJ_FRAMES)))
         dcd = cif.DCDWriter(self.save_path + "metadata/MultiMM_annealing.dcd", a.N_BEADS, dt, dcd_every)
         sample_every = int(contact_setting(a, "MD_SAMPLE_STEP"))
-        sampling = self._configure_sampler() if sample_every > 0 else None
-        chunk = int(np.gcd.reduce([every, dcd_every] + ([sample_every] if sampling else [])))
+        maps = contact_setting(a, "SAVE_CONTACTS") or contact_setting(a, "SAVE_DISTANCES")
+        sampling = self._configure_sampler() if sample_every > 0 and maps else None
+        loop_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_LOOPS"))
+        if loop_sampling:
+            self._configure_loops()
+        chunk = int(np.gcd.reduce([every, dcd_every] + ([sample_every] if sampling or loop_sampling else [])))
         t0 = time.time()
         print('#"Step"\t"Potential Energy (kJ/mole)"\t"Kinetic Energy (kJ/mole)"\t"Total Energy (kJ/mole)"\t"Temperature (K)"')
         done = 0
@@ -401,10 +415,14 @@ class MultiMM:
                                     connections=False, decimals=4)
                 if sampling and done % sample_every == 0:
                     self._sample(sampling)
+                if loop_sampling and done % sample_every == 0:
+                    self.engine.loops_add()
         finally:
             dcd.close()
         if sampling:
             self._read_samples(sampling, sample_every)
+        if loop_sampling:
+            self._read_loops(md=True)
         self.positions = self.engine.get_positions()
         cif.write_mmcif(10.0 * self.positions, self.chr_ends, self.save_path + "model/MultiMM_afterMD.cif",
                         hetatm_ends=True, connections=False, decimals=4)
@@ -466,6 +484,8 @@ class MultiMM:
             self.count_contacts()
         if contact_setting(self.args, "SAVE_DISTANCES"):
             self.count_distances()
+        if contact_setting(self.args, "SAVE_LOOPS"):
+            self.measure_loops()
         if self.args.SIM_RUN_MD:
             self.run_md()
 
@@ -520,6 +540,40 @@ class MultiMM:
         dsum, d2sum = self.engine.distance_map(gb.bins, gb.n_bins)
         self.distances = distances.result(dsum, d2sum, gb, self.engine.get_positions(), self.mass_center)
         self.timings["distances_s"] = time.time() - t0
+
+    def _configure_loops(self):
+        """Set up the engine's loop accumulator with this member's valid rows (SAVE_LOOPS)."""
+        from . import loops
+
+        a = self.args
+        self.engine.loops_configure(float(contact_setting(a, "CONTACT_RADIUS")), int(contact_setting(a, "LOOP_APA_WINDOW")),
+                                    **loops.device_rows(self.loop_rows))
+
+    def _read_loops(self, md: bool = False):
+        from . import loops
+
+        a = self.args
+        r = self.engine.loops_read()
+        if md:
+            logger.info(f"loop readout: {r['samples']} MD structures ({r['device_ms']:.1f} ms on the device)")
+            if r["samples"] == 0:
+                return
+        d = loops.result(self.loop_table, self.loop_rows, r, float(contact_setting(a, "CONTACT_RADIUS")),
+                         int(contact_setting(a, "LOOP_APA_WINDOW")), r["samples"])
+        if md:
+            self.loops_md = d
+        else:
+            self.loops = d
+
+    def measure_loops(self):
+        """The loop readout of the minimised structure (SAVE_LOOPS): per-row sums and APA of the rows of the loop
+        table that are valid for this member, measured by its own engine at the positions the minimisation
+        left on the device."""
+        t0 = time.time()
+        self._configure_loops()
+        self.engine.loops_add()
+        self._read_loops()
+        self.timings["loops_s"] = time.time() - t0
 
     def _configure_sampler(self) -> dict:
         """MD_SAMPLE_STEP: set up the engine's sampler with the maps that are on (SAVE_CONTACTS with its fine map,
@@ -589,6 +643,13 @@ class MultiMM:
         for d, path in ((self.distances, dist_path), (self.distances_md, contacts.md_path(dist_path))):
             if d is not None:
                 distances.save(path, d)
+        if self.loops is not None or self.loops_md is not None:
+            from . import loops
+
+            loop_path = self.loops_file or os.path.join(self.save_path, "analysis", "loops.npz")
+            for d, path in ((self.loops, loop_path), (self.loops_md, contacts.md_path(loop_path))):
+                if d is not None:
+                    loops.save(path, d)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

@@ -201,13 +201,23 @@ def args_tests(args):
                          f"(supported: {', '.join(_lib.MD_INTEGRATORS)})")
     check_contact_fields(args)
     check_distance_fields(args)
+    check_loop_fields(args)
     check_md_sample_fields(args)
 
 
+def check_loop_fields(args):
+    """LOOP_APA_WINDOW in [0, loops.MAX_WINDOW]."""
+    from . import loops
+
+    w = int(contact_setting(args, "LOOP_APA_WINDOW"))
+    if not 0 <= w <= loops.MAX_WINDOW:
+        raise ValueError(f"LOOP_APA_WINDOW={w} must be in [0, {loops.MAX_WINDOW}] beads")
+
+
 def check_md_sample_fields(args):
-    """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES), and the
-    MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps, must reach the first
-    sample."""
+    """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES, or the loop
+    readout SAVE_LOOPS), and the MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps,
+    must reach the first sample."""
     step = int(contact_setting(args, "MD_SAMPLE_STEP"))
     if step < 0:
         raise ValueError(f"MD_SAMPLE_STEP={step} must be >= 0 (0 = no trajectory maps)")
@@ -215,8 +225,9 @@ def check_md_sample_fields(args):
         return
     if not args.SIM_RUN_MD:
         raise ValueError(f"MD_SAMPLE_STEP={step} samples the MD run, but SIM_RUN_MD is off")
-    if not (contact_setting(args, "SAVE_CONTACTS") or contact_setting(args, "SAVE_DISTANCES")):
-        raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES")
+    if not any(contact_setting(args, k) for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS")):
+        raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES "
+                         "(or SAVE_LOOPS)")
     every = max(1, int(args.SIM_SAMPLING_STEP))
     steps = (int(args.SIM_N_STEPS) // every) * every
     if step > steps:
@@ -423,6 +434,7 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     md.contacts_file = member_contacts_path(params["OUT_PATH"], i)
     md.contacts_fine_file = member_contacts_fine_path(params["OUT_PATH"], i)
     md.distances_file = member_distances_path(params["OUT_PATH"], i)
+    md.loops_file = member_loops_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
@@ -437,6 +449,10 @@ def member_contacts_fine_path(out_path: str, i: int) -> str:
 
 def member_distances_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "distances", f"member_{i}.npz")
+
+
+def member_loops_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "loops", f"member_{i}.npz")
 
 
 def _sampled_md(args) -> bool:
@@ -463,6 +479,27 @@ def write_ensemble_distances(args, results: list[dict]) -> str | None:
         logger.info(f"ensemble distances{' (MD samples)' if md else ''}: {int(agg['members'])} "
                     f"{'structures' if md else 'members'}, {len(agg['bin_beads'])} bins at "
                     f"{int(agg['resolution_bp'])} bp -> {path}")
+        out = out or path
+    return out
+
+
+def write_ensemble_loops(args, results: list[dict]) -> str | None:
+    """SAVE_LOOPS: OUT_PATH/ensemble_loops.npz, the sum of the loops files of the members that succeeded (exact
+    integer sums: the same bits whichever GPU ran which member); with MD_SAMPLE_STEP also ensemble_loops_md.npz,
+    the sum of their MD samples."""
+    if not contact_setting(args, "SAVE_LOOPS") or not results:
+        return None
+    from . import contacts, loops
+
+    out = None
+    for md in (False, True) if _sampled_md(args) else (False,):
+        name = contacts.md_path if md else (lambda p: p)
+        paths = [name(member_loops_path(args.OUT_PATH, r["replica"])) for r in sorted(results, key=lambda r: r["replica"])]
+        agg = loops.aggregate(paths)
+        path = name(os.path.join(args.OUT_PATH, "ensemble_loops.npz"))
+        loops.save(path, agg)
+        logger.info(f"ensemble loops{' (MD samples)' if md else ''}: {int(agg['members'])} structures, "
+                    f"{len(agg['row'])} rows, APA window {int(agg['apa_window'])} beads -> {path}")
         out = out or path
     return out
 
@@ -700,6 +737,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         results = [p for kind, p in got if kind == "ok"]
         write_ensemble_contacts(args, results)
         write_ensemble_distances(args, results)
+        write_ensemble_loops(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
         check_archives(results)
@@ -737,6 +775,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
                 p.join()
     write_ensemble_contacts(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_distances(args, [r for r in results if r.get("replica", -1) >= 0])
+    write_ensemble_loops(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
