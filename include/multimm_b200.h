@@ -359,6 +359,37 @@ int mmm_loops_read(mmm_handle h, int64_t *samples_out, uint64_t *contacts_out, u
                    uint64_t *dist2_sum_out, uint64_t *apa_contacts_out, uint64_t *apa_dist_sum_out,
                    float *device_ms_out);
 
+/* ---- three-way contact map (simulated multi-way chromatin capture: bead triples in mutual contact, summed over
+ * structures; not in the reference, whose analysis is pairwise, model.py:1069-1213) -------------------------- */
+/* Sets up the three-way accumulator of this handle and clears its sums: the contact radius, the bin table
+ * bin_of_bead (int32[N], -1 = the bead is left out, uploaded once) of 1 <= n_bins <= 2^20 bins, and
+ * max_chunk_keys, the most binned triples of one structure sorted at a time (0 = 2^26, 1 GiB of sort buffers;
+ * a chunk holds one bead's triples at least).  MMM_ERR_ARG for rc <= 0 or not finite, n_bins outside
+ * [1, 2^20], a NULL table, a bin id outside [-1, n_bins) or max_chunk_keys < 0.  The buffers are the
+ * accumulator's own (allocated here and as adds need, freed with the handle). */
+int mmm_triplets_configure(mmm_handle h, double rc_nm, const int32_t *bin_of_bead, int32_t n_bins,
+                           int64_t max_chunk_keys);
+/* Adds the structure at the current positions: every unordered bead triple i < j < k whose three pairs are
+ * contacts of mmm_contacts (d2 = (dx*dx + dy*dy) + dz*dz in FP64 on the master positions, d2 < rc^2), counted
+ * once.  A triple with a bead left out counts only in `triples`; otherwise its bins sorted into p <= q <= r
+ * add 1 to the entry of key (p * n_bins + q) * n_bins + r.  uint64 integer sums: exact and independent of
+ * schedule and max_chunk_keys, so K adds equal the sum of K single-structure reads.  No overflow guard: one
+ * structure adds at most N^3 / 6 to any count.  Scratch O(N + contacts + max_chunk_keys), never O(triples).
+ * MMM_ERR_STATE before mmm_triplets_configure or before positions are set; after any other error the
+ * accumulator must be configured again.  Changes no state an evaluation, a minimisation, an MD step,
+ * mmm_last_result, mmm_contacts_sparse_read, the trajectory sampler or the loop readout reads; synchronises
+ * with the host (twice per chunk and more). */
+int mmm_triplets_add(mmm_handle h);
+/* Of the structures added since mmm_triplets_configure: samples_out, their number; triples_out, all three-way
+ * contacts, binned or not; entries_out, the distinct keys (for mmm_triplets_read_entries); chunks_out, the
+ * chunks the adds sorted; device_ms_out, the device time of all adds (CUDA events on the handle's stream, host
+ * waits included).  Any output may be NULL.  MMM_ERR_STATE as mmm_triplets_add. */
+int mmm_triplets_read(mmm_handle h, int64_t *samples_out, uint64_t *triples_out, int64_t *entries_out,
+                      int64_t *chunks_out, float *device_ms_out);
+/* The entries, sorted by key, counts > 0: keys_out, vals_out uint64[entries]; either may be NULL, and 0
+ * entries succeeds.  MMM_ERR_STATE as mmm_triplets_add. */
+int mmm_triplets_read_entries(mmm_handle h, uint64_t *keys_out, uint64_t *vals_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

@@ -35,7 +35,7 @@ EXPORTS = (
     "mmm_minimize",
     "mmm_launch_count", "mmm_set_graph", "mmm_set_chb_surrogate", "mmm_set_pair_kernel", "mmm_pair_kernel_in_use", "mmm_last_pair_kernel_ms", "mmm_get_cell_list", "mmm_get_cell_grid", "mmm_measure_fp32_peak",
     "mmm_dist_unique_id", "mmm_dist_init", "mmm_dist_emulate", "mmm_dist_last_exchange_ms", "mmm_dist_queue_mode",
-    "mmm_mean_pair_distance", "mmm_contact_map", "mmm_contacts", "mmm_contacts_sparse", "mmm_contacts_sparse_read", "mmm_contacts_stats", "mmm_distance_map", "mmm_sampler_configure", "mmm_sample", "mmm_sampler_read", "mmm_sampler_read_fine", "mmm_loops_configure", "mmm_loops_add", "mmm_loops_read", "mmm_md_configure", "mmm_md_set_amd", "mmm_set_velocities_to_temperature", "mmm_set_velocities", "mmm_get_velocities", "mmm_md_run",
+    "mmm_mean_pair_distance", "mmm_contact_map", "mmm_contacts", "mmm_contacts_sparse", "mmm_contacts_sparse_read", "mmm_contacts_stats", "mmm_distance_map", "mmm_sampler_configure", "mmm_sample", "mmm_sampler_read", "mmm_sampler_read_fine", "mmm_loops_configure", "mmm_loops_add", "mmm_loops_read", "mmm_triplets_configure", "mmm_triplets_add", "mmm_triplets_read", "mmm_triplets_read_entries", "mmm_md_configure", "mmm_md_set_amd", "mmm_set_velocities_to_temperature", "mmm_set_velocities", "mmm_get_velocities", "mmm_md_run",
 )
 
 
@@ -130,6 +130,11 @@ def load():
         "mmm_loops_configure": (i32, [vp, dbl, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
         "mmm_loops_add": (i32, [vp]),
         "mmm_loops_read": (i32, [vp, C.POINTER(i64), vp, vp, vp, vp, vp, C.POINTER(C.c_float)]),
+        "mmm_triplets_configure": (i32, [vp, dbl, vp, i32, i64]),
+        "mmm_triplets_add": (i32, [vp]),
+        "mmm_triplets_read": (i32, [vp, C.POINTER(i64), C.POINTER(C.c_uint64), C.POINTER(i64), C.POINTER(i64),
+                                    C.POINTER(C.c_float)]),
+        "mmm_triplets_read_entries": (i32, [vp, vp, vp]),
         "mmm_md_configure": (i32, [vp, i32, dbl, dbl, dbl, dbl, C.c_uint64]),
         "mmm_md_set_amd": (i32, [vp, dbl, dbl]),
         "mmm_set_velocities_to_temperature": (i32, [vp, dbl, C.c_uint64]),

@@ -211,13 +211,20 @@ LOOP_FIELDS: dict[str, tuple[Any, Any]] = {
     "SAVE_LOOPS": (B, False),             # measure the input loops in the minimised structure (analysis/loops.npz; ensembles: ensemble_loops.npz)
     "LOOP_APA_WINDOW": (int, 10),         # beads on each side of an anchor in the APA window, in [0, 25]
 }
-EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS, **LOOP_FIELDS}
+# Three-way contact maps (multimm_b200.triplets), kept the same way: bead triples in mutual contact, binned in
+# genomic coordinates; the contact test uses CONTACT_RADIUS, and MD_SAMPLE_STEP also samples them.
+TRIPLET_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_TRIPLETS": (B, False),          # three-way contacts of the minimised structure (analysis/triplets.npz; ensembles: ensemble_triplets.npz)
+    "TRIPLET_RESOLUTION": (int, 0),       # bp per bin of the three-way map; 0 = about 1000 bins, at most 2^20 bins
+}
+EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS, **LOOP_FIELDS,
+                **TRIPLET_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
-    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS or LOOP_FIELDS setting of
-    `args`, its default where it was not given."""
+    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS, LOOP_FIELDS or
+    TRIPLET_FIELDS setting of `args`, its default where it was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

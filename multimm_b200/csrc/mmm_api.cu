@@ -122,7 +122,7 @@ int mmm_destroy(mmm_handle h) {
   if (h->h_done) cudaFreeHost(h->h_done);
   for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
   for (cudaEvent_t e : {h->ev_a, h->ev_b, h->ev_c0, h->ev_c1, h->ct_ev0, h->ct_ev1, h->dm_ev0, h->dm_ev1,
-                        h->sp_ev0, h->sp_ev1, h->lp_ev0, h->lp_ev1})
+                        h->sp_ev0, h->sp_ev1, h->lp_ev0, h->lp_ev1, h->tp_ev0, h->tp_ev1})
     if (e) cudaEventDestroy(e);
   if (h->stream) cudaStreamDestroy(h->stream);
   delete h;  // the device buffers free themselves

@@ -428,6 +428,8 @@ __global__ void __launch_bounds__(MG_THREADS) k_merge(const unsigned long long* 
   }
 }
 
+}  // namespace
+
 // exclusive scan of a[0, len) in place; part: ceil(len / CS_CHUNK) + 1 entries, the last receives the total
 void cs_scan(mmm_system* h, long long* a, long long len, long long* part) {
   const int nparts = (int)std::max<long long>(1, (len + CS_CHUNK - 1) / CS_CHUNK);
@@ -440,6 +442,38 @@ void cs_scan(mmm_system* h, long long* a, long long len, long long* part) {
 long long cs_blocks(long long nkeys) { return std::max<long long>(1, (nkeys + CS_CHUNK - 1) / CS_CHUNK); }
 // sort table (digit x chunk) followed by the partial sums of its scan
 size_t cs_table_len(long long nkeys) { return (size_t)(CS_DIGITS * cs_blocks(nkeys)) * 17 / 16 + 2; }
+
+int cs_key_bits(unsigned long long kmax) {
+  int bits = 0;
+  while (bits < 64 && (kmax >> bits)) ++bits;
+  return bits;
+}
+
+long long* cs_run_total(long long* table, long long nkeys) {
+  const long long nblocks = cs_blocks(nkeys);
+  return table + nblocks + cs_blocks(nblocks);
+}
+
+int cs_sort_runs(mmm_system* h, DevBuf<unsigned long long>* keys, long long m, int bits, long long* table) {
+  const int nblocks = (int)cs_blocks(m);
+  long long* table_part = table + (size_t)CS_DIGITS * nblocks;
+  int src = 0;
+  for (int shift = 0; shift < bits; shift += CS_DIGIT_BITS) {
+    k_rs_hist<<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, shift, table, nblocks);
+    cs_scan(h, table, (long long)CS_DIGITS * nblocks, table_part);
+    k_rs_scatter<<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, shift, table, nblocks, keys[1 - src]);
+    h->launches += 2;
+    src = 1 - src;
+  }
+  // entries: heads per chunk -> offsets (the first nblocks slots of the table, kept for the read)
+  k_rle<kCount><<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, table, nullptr, 0u, nullptr, nullptr, nullptr,
+                                                       nullptr, nullptr);
+  h->launches++;
+  cs_scan(h, table, nblocks, table + nblocks);
+  return src;
+}
+
+namespace {
 
 // the argument checks of mmm_contacts and mmm_contacts_sparse (max_bins: 4096 for the dense map)
 int ct_check_args(mmm_system* h, const char* who, double rc_nm, const int32_t* bin_of_bead, int32_t n_bins, int max_bins,
@@ -525,38 +559,20 @@ int mmm_contacts_sparse_pass(mmm_system* h, double rc_nm, const int* d_bin, int3
       (rc = mmm_reserve(h, table, cs_table_len(m), "contact sort table")))
     return rc;
   long long* tab = table;
-  const int nblocks = (int)cs_blocks(m);
-  long long* table_part = tab + (size_t)CS_DIGITS * nblocks;
   k_contacts<kKeys><<<ctas, CT_WARPS * 32, 0, h->stream>>>(
       h->d_x, h->d_type, d_bin, h->d_tiles, h->d_ct_stage, n, ntr, nst, rc_nm * rc_nm, rcm2, n_bins, nullptr,
       nullptr, cnt, tile, keys[0]);
   h->launches++;
   // keys < n_bins^2: sort on ceil(log2(n_bins^2)) bits, 8 per pass
-  int bits = 0;
-  const unsigned long long kmax = (unsigned long long)n_bins * (unsigned long long)n_bins - 1ull;
-  while (bits < 64 && (kmax >> bits)) ++bits;
+  const int bits = cs_key_bits((unsigned long long)n_bins * (unsigned long long)n_bins - 1ull);
   int src = 0;
-  if (m > 0) {
-    for (int shift = 0; shift < bits; shift += CS_DIGIT_BITS) {
-      k_rs_hist<<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, shift, tab, nblocks);
-      cs_scan(h, tab, (long long)CS_DIGITS * nblocks, table_part);
-      k_rs_scatter<<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, shift, tab, nblocks, keys[1 - src]);
-      h->launches += 2;
-      src = 1 - src;
-    }
-    // entries: heads per chunk -> offsets (the first nblocks slots of the table, kept for the read)
-    k_rle<kCount><<<nblocks, CS_THREADS, 0, h->stream>>>(keys[src], m, tab, nullptr, 0u, nullptr, nullptr, nullptr,
-                                                         nullptr, nullptr);
-    h->launches++;
-    cs_scan(h, tab, nblocks, tab + nblocks);
-  }
+  if (m > 0) src = cs_sort_runs(h, keys, m, bits, tab);
   MMM_CUDA(h, cudaGetLastError());
   if (ev1) MMM_CUDA(h, cudaEventRecord(ev1, h->stream));
   long long entries = 0;
   MMM_CUDA(h, cudaMemcpyAsync(out->cnt, cnt, sizeof(out->cnt), cudaMemcpyDeviceToHost, h->stream));
   if (m > 0)
-    MMM_CUDA(h, cudaMemcpyAsync(&entries, tab + nblocks + cs_blocks(nblocks), sizeof(entries), cudaMemcpyDeviceToHost,
-                                h->stream));
+    MMM_CUDA(h, cudaMemcpyAsync(&entries, cs_run_total(tab, m), sizeof(entries), cudaMemcpyDeviceToHost, h->stream));
   MMM_CUDA(h, cudaStreamSynchronize(h->stream));
   out->keys = m;
   out->entries = entries;
@@ -573,35 +589,33 @@ static size_t sp_capacity(long long n) {
   return ((size_t)n + step - 1) / step * step;
 }
 
-// The trajectory sampler's fine map: this structure's sparse map, reduced to a sorted unique (key, count) list
-// in the spare sort buffer and d_sp_sval, merged with the accumulated list d_sp_acc_*[0] into d_sp_acc_*[1],
-// and equal keys added back into d_sp_acc_*[0].  Work and memory O(accumulated + this structure's entries).
-int mmm_contacts_fine_accumulate(mmm_system* h) {
-  CsSorted srt;
-  int rc = mmm_contacts_sparse_pass(h, h->sp_rc, h->d_sp_fine_bin, h->sp_fine_bins, h->d_sp_tile, h->d_sp_keys,
-                                    h->d_sp_table, h->d_sp_cnt + 2, nullptr, nullptr, &srt);
-  if (rc) return rc;
-  const long long nb = srt.entries, na = h->sp_fine_n, nm = na + nb;
+// Adds the sorted keys[0, m) to the list acc: the runs of equal keys (off: their offsets per 4096-key chunk, as
+// cs_sort_runs leaves them; entries of them) become a sorted unique (key, count) list in spare (>= entries
+// slots) and acc.sval, which is merged with acc's entries [0] into [1], and equal keys (at most two, adjacent)
+// are added back into [0].  Work and memory O(acc.n + entries).
+int mmm_list_accumulate(mmm_system* h, const unsigned long long* keys, long long m, const long long* off,
+                        long long entries, unsigned long long* spare, KeyCountList& acc) {
+  const long long nb = entries, na = acc.n, nm = na + nb;
   if (nb == 0) return MMM_OK;
-  unsigned long long* skey = h->d_sp_keys[1 - srt.src];  // free after the sort; keys >= entries slots
-  if ((rc = mmm_reserve(h, h->d_sp_sval, sp_capacity(nb), "sampler fine counts")) ||
-      (rc = mmm_reserve(h, h->d_sp_acc_key[1], sp_capacity(nm), "sampler fine keys")) ||
-      (rc = mmm_reserve(h, h->d_sp_acc_val[1], sp_capacity(nm), "sampler fine counts")))
+  int rc;
+  if ((rc = mmm_reserve(h, acc.sval, sp_capacity(nb), "sorted list counts")) ||
+      (rc = mmm_reserve(h, acc.key[1], sp_capacity(nm), "sorted list keys")) ||
+      (rc = mmm_reserve(h, acc.val[1], sp_capacity(nm), "sorted list counts")))
     return rc;
-  MMM_CUDA(h, cudaMemsetAsync(h->d_sp_sval, 0, sizeof(unsigned long long) * (size_t)nb, h->stream));
-  k_rle<kKeyVals><<<(int)cs_blocks(srt.keys), CS_THREADS, 0, h->stream>>>(
-      h->d_sp_keys[srt.src], srt.keys, nullptr, h->d_sp_table, 0u, nullptr, h->d_sp_sval, skey, nullptr, nullptr);
+  MMM_CUDA(h, cudaMemsetAsync(acc.sval, 0, sizeof(unsigned long long) * (size_t)nb, h->stream));
+  k_rle<kKeyVals><<<(int)cs_blocks(m), CS_THREADS, 0, h->stream>>>(keys, m, nullptr, off, 0u, nullptr, acc.sval, spare,
+                                                                   nullptr, nullptr);
   const int nparts = (int)((nm + MG_TILE - 1) / MG_TILE);
   const long long nchunks = cs_blocks(nm);
-  if ((rc = mmm_reserve(h, h->d_sp_mpart, sp_capacity(std::max<long long>(nparts + 1, nchunks + cs_blocks(nchunks) + 1)),
-                        "sampler merge table")))
+  if ((rc = mmm_reserve(h, acc.part, sp_capacity(std::max<long long>(nparts + 1, nchunks + cs_blocks(nchunks) + 1)),
+                        "sorted list merge table")))
     return rc;
-  long long* part = h->d_sp_mpart;
-  k_merge_part<<<(nparts + 1 + 255) / 256, 256, 0, h->stream>>>(h->d_sp_acc_key[0], na, skey, nb, nparts, part);
-  k_merge<<<nparts, MG_THREADS, 0, h->stream>>>(h->d_sp_acc_key[0], h->d_sp_acc_val[0], na, skey, h->d_sp_sval, nb,
-                                                part, h->d_sp_acc_key[1], h->d_sp_acc_val[1]);
+  long long* part = acc.part;
+  k_merge_part<<<(nparts + 1 + 255) / 256, 256, 0, h->stream>>>(acc.key[0], na, spare, nb, nparts, part);
+  k_merge<<<nparts, MG_THREADS, 0, h->stream>>>(acc.key[0], acc.val[0], na, spare, acc.sval, nb, part, acc.key[1],
+                                                acc.val[1]);
   // equal keys -> one entry: heads per chunk, their offsets, then keys and summed counts
-  k_rle<kCount><<<(int)nchunks, CS_THREADS, 0, h->stream>>>(h->d_sp_acc_key[1], nm, part, nullptr, 0u, nullptr, nullptr,
+  k_rle<kCount><<<(int)nchunks, CS_THREADS, 0, h->stream>>>(acc.key[1], nm, part, nullptr, 0u, nullptr, nullptr,
                                                             nullptr, nullptr, nullptr);
   h->launches += 4;
   cs_scan(h, part, nchunks, part + nchunks);
@@ -609,17 +623,27 @@ int mmm_contacts_fine_accumulate(mmm_system* h) {
   long long ne = 0;
   MMM_CUDA(h, cudaMemcpyAsync(&ne, part + nchunks + cs_blocks(nchunks), sizeof(ne), cudaMemcpyDeviceToHost, h->stream));
   MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  if ((rc = mmm_reserve(h, h->d_sp_acc_key[0], sp_capacity(ne), "sampler fine keys")) ||
-      (rc = mmm_reserve(h, h->d_sp_acc_val[0], sp_capacity(ne), "sampler fine counts")))
+  if ((rc = mmm_reserve(h, acc.key[0], sp_capacity(ne), "sorted list keys")) ||
+      (rc = mmm_reserve(h, acc.val[0], sp_capacity(ne), "sorted list counts")))
     return rc;
-  MMM_CUDA(h, cudaMemsetAsync(h->d_sp_acc_val[0], 0, sizeof(unsigned long long) * (size_t)ne, h->stream));
-  k_rle<kKeyVals><<<(int)nchunks, CS_THREADS, 0, h->stream>>>(h->d_sp_acc_key[1], nm, nullptr, part, 0u,
-                                                              h->d_sp_acc_val[1], h->d_sp_acc_val[0],
-                                                              h->d_sp_acc_key[0], nullptr, nullptr);
+  MMM_CUDA(h, cudaMemsetAsync(acc.val[0], 0, sizeof(unsigned long long) * (size_t)ne, h->stream));
+  k_rle<kKeyVals><<<(int)nchunks, CS_THREADS, 0, h->stream>>>(acc.key[1], nm, nullptr, part, 0u, acc.val[1], acc.val[0],
+                                                              acc.key[0], nullptr, nullptr);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
-  h->sp_fine_n = ne;
+  acc.n = ne;
   return MMM_OK;
+}
+
+// The trajectory sampler's fine map: this structure's sparse map added to the accumulated list h->sp_fine.
+int mmm_contacts_fine_accumulate(mmm_system* h) {
+  CsSorted srt;
+  int rc = mmm_contacts_sparse_pass(h, h->sp_rc, h->d_sp_fine_bin, h->sp_fine_bins, h->d_sp_tile, h->d_sp_keys,
+                                    h->d_sp_table, h->d_sp_cnt + 2, nullptr, nullptr, &srt);
+  if (rc) return rc;
+  // the spare sort buffer (free after the sort, keys >= entries slots) takes this structure's list
+  return mmm_list_accumulate(h, h->d_sp_keys[srt.src], srt.keys, h->d_sp_table, srt.entries,
+                             h->d_sp_keys[1 - srt.src], h->sp_fine);
 }
 
 namespace {
@@ -634,15 +658,15 @@ __global__ void __launch_bounds__(256) k_split_keys(const unsigned long long* __
 }  // namespace
 
 int mmm_contacts_fine_read(mmm_system* h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out) {
-  const long long e = h->sp_fine_n;
+  const long long e = h->sp_fine.n;
   if (e == 0) return MMM_OK;
   if (vals_out)
-    MMM_CUDA(h, cudaMemcpyAsync(vals_out, h->d_sp_acc_val[0], sizeof(uint64_t) * (size_t)e, cudaMemcpyDeviceToHost,
+    MMM_CUDA(h, cudaMemcpyAsync(vals_out, h->sp_fine.val[0], sizeof(uint64_t) * (size_t)e, cudaMemcpyDeviceToHost,
                                 h->stream));
   if (rows_out || cols_out) {  // rows then cols as int32 in the free merge buffer (>= e slots of 8 B)
-    int* rows = reinterpret_cast<int*>(h->d_sp_acc_key[1].get());
+    int* rows = reinterpret_cast<int*>(h->sp_fine.key[1].get());
     int* cols = rows + e;
-    k_split_keys<<<(unsigned)((e + 255) / 256), 256, 0, h->stream>>>(h->d_sp_acc_key[0], e, (unsigned)h->sp_fine_bins,
+    k_split_keys<<<(unsigned)((e + 255) / 256), 256, 0, h->stream>>>(h->sp_fine.key[0], e, (unsigned)h->sp_fine_bins,
                                                                       rows, cols);
     h->launches++;
     MMM_CUDA(h, cudaGetLastError());

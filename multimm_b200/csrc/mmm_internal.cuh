@@ -163,6 +163,15 @@ class DevBuf {
   size_t cap_ = 0;
 };
 
+// A sorted unique (key, count) list summed over structures on the device (mmm_list_accumulate: the trajectory
+// sampler's fine map, the three-way contact map): key[0], val[0] hold the n entries; [1] receives the merge.
+struct KeyCountList {
+  DevBuf<unsigned long long> key[2], val[2];
+  DevBuf<unsigned long long> sval;   // counts of the list being added
+  DevBuf<long long> part;            // merge partition, then run offsets of the merge
+  int64_t n = 0;
+};
+
 // ---------------------------------------------------------------------------------------
 // the handle
 // ---------------------------------------------------------------------------------------
@@ -349,13 +358,10 @@ struct mmm_system {
   DevBuf<unsigned long long> d_sp_sep;     // [n] contacts by index separation
   DevBuf<unsigned long long> d_sp_cnt;     // [4] contacts, candidates (summed); the fine pass's own two
   DevBuf<unsigned long long> d_sp_dist;    // [2][n_bins^2] distance sums, squared-distance sums
-  // fine map: a sorted unique (key, count) list in d_sp_acc_*[0]; [1] receives the merge
+  // fine map: the sparse pass into these buffers, then its entries added to sp_fine
   DevBuf<long long> d_sp_tile, d_sp_table;             // the sparse pass's scratch (as d_cs_tile, d_cs_table)
   DevBuf<unsigned long long> d_sp_keys[2];             // the sparse pass's sort buffers
-  DevBuf<unsigned long long> d_sp_sval;                // counts of one structure's entries
-  DevBuf<unsigned long long> d_sp_acc_key[2], d_sp_acc_val[2];
-  DevBuf<long long> d_sp_mpart;                        // merge partition, then run offsets of the merge
-  int64_t sp_fine_n = 0;                               // accumulated fine entries
+  KeyCountList sp_fine;                                // accumulated fine entries
 
   // loop readout (mmm_loops.cu): per-row and APA sums over structures, on the device until read
   bool lp_configured = false;
@@ -368,6 +374,24 @@ struct mmm_system {
   cudaEvent_t lp_ev0 = nullptr, lp_ev1 = nullptr;
   DevBuf<LoopRow> d_lp_row;                // [rows]
   DevBuf<unsigned long long> d_lp_sum;     // [3][rows] contacts, dist_sum, dist2_sum; [2 sums][2 groups][(2W+1)^2] APA
+
+  // three-way contact map (mmm_triplets.cu): bead triples in mutual contact, summed over structures
+  bool tp_configured = false;
+  double tp_rc = 0.0;
+  int32_t tp_bins = 0;
+  int64_t tp_max_chunk = 0;                // keys per chunk of triples (a chunk holds one bead at least)
+  int64_t tp_samples = 0, tp_chunks = 0;
+  uint64_t tp_triples = 0;                 // all three-way contacts, binned or not
+  float tp_ms = 0.f;                       // device time of all adds
+  cudaEvent_t tp_ev0 = nullptr, tp_ev1 = nullptr;
+  DevBuf<int> d_tp_ident, d_tp_bin;        // [n] identity bins (the bead-level contact list), the caller's bins
+  DevBuf<long long> d_tp_tile, d_tp_table; // the sparse pass's scratch, then the chunks' sort table
+  DevBuf<unsigned long long> d_tp_adj[2];  // the sparse pass's sort buffers: forward adjacency i * n + j, i < j
+  DevBuf<unsigned long long> d_tp_cnt;     // [3] contacts, candidates, triples of the add
+  DevBuf<long long> d_tp_row;              // [n + 1] first adjacency entry of every bead
+  DevBuf<long long> d_tp_off;              // [n + 1 + scan parts] binned triples per bead -> their offsets
+  DevBuf<unsigned long long> d_tp_keys[2]; // one chunk's keys: the radix sort's buffers
+  KeyCountList tp_acc;                     // the accumulated (key, count) list
 };
 
 // the sorted keys of one sparse pass (mmm_contacts_sparse_pass)
@@ -468,6 +492,16 @@ int mmm_contacts_dense_pass(mmm_system* h, double rc_nm, const int* d_bin, int32
 int mmm_contacts_sparse_pass(mmm_system* h, double rc_nm, const int* d_bin, int32_t n_bins, DevBuf<long long>& tile,
                              DevBuf<unsigned long long>* keys, DevBuf<long long>& table, unsigned long long* cnt,
                              cudaEvent_t ev0, cudaEvent_t ev1, CsSorted* out);
+void cs_scan(mmm_system* h, long long* a, long long len, long long* part);  // exclusive, in place
+long long cs_blocks(long long nkeys);       // 4096-key chunks of the sort, scan and run kernels
+size_t cs_table_len(long long nkeys);       // the sort table of nkeys keys
+int cs_key_bits(unsigned long long kmax);   // significant bits of the largest key
+// LSD radix sort of keys[0][0, m) (< 2^bits) and the run offsets of the sorted keys in table[0, cs_blocks(m));
+// returns which buffer holds the sorted keys; the entry count lands at cs_run_total(table, m)
+int cs_sort_runs(mmm_system* h, DevBuf<unsigned long long>* keys, long long m, int bits, long long* table);
+long long* cs_run_total(long long* table, long long nkeys);
+int mmm_list_accumulate(mmm_system* h, const unsigned long long* keys, long long m, const long long* off,
+                        long long entries, unsigned long long* spare, KeyCountList& acc);
 int mmm_contacts_fine_accumulate(mmm_system* h);  // the sampler's fine map += the current structure's
 int mmm_contacts_fine_read(mmm_system* h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out);
 // mmm_distances.cu

@@ -110,7 +110,7 @@ extern "C" int mmm_sampler_configure(mmm_handle h, double rc_nm, const int32_t* 
   h->sp_samples = 0;
   h->sp_dm_bound = 0.0;
   h->sp_ms = 0.f;
-  h->sp_fine_n = 0;
+  h->sp_fine.n = 0;
   h->sp_configured = true;
   return MMM_OK;
 }
@@ -160,7 +160,7 @@ extern "C" int mmm_sampler_read(mmm_handle h, int64_t* samples_out, uint64_t* co
   MMM_CUDA(h, cudaStreamSynchronize(h->stream));
   if (samples_out) *samples_out = h->sp_samples;
   if (h->sp_ct_bins && pairs_out) *pairs_out = (int64_t)cnt[0];
-  if (fine_entries_out) *fine_entries_out = h->sp_fine_n;
+  if (fine_entries_out) *fine_entries_out = h->sp_fine.n;
   if (device_ms_out) *device_ms_out = h->sp_ms;
   return MMM_OK;
 }

@@ -312,6 +312,37 @@ class Engine:
         out.update(samples=int(samples.value), device_ms=float(ms.value))
         return out
 
+    # -- three-way contact map (bead triples in mutual contact, summed over many structures) -----------
+    def triplets_configure(self, rc_nm: float, bin_of_bead, n_bins: int, max_chunk_keys: int = 0):
+        """Clear the three-way accumulator and set its bins (mmm_triplets_configure): ``bin_of_bead`` (int[N],
+        -1 = left out) of ``n_bins`` <= 2^20 bins, the contact radius, and the most binned triples of one
+        structure sorted at a time (0 = 2^26)."""
+        bins = _arr(bin_of_bead, np.int32)
+        if bins is not None and bins.shape != (self.n,):
+            raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        self._ck(self._lib.mmm_triplets_configure(self._h, float(rc_nm), _p(bins), int(n_bins), int(max_chunk_keys)))
+        self._triplet_bins = int(n_bins)
+
+    def triplets_add(self):
+        """Add the three-way contacts of the structure at the current positions (mmm_triplets_add)."""
+        self._ck(self._lib.mmm_triplets_add(self._h))
+
+    def triplets_read(self) -> dict:
+        """The three-way sums (mmm_triplets_read, mmm_triplets_read_entries): ``samples``; ``triples``, all
+        three-way contacts; ``p`` <= ``q`` <= ``r`` (int32) and ``vals`` (uint64), the entries sorted by key
+        (p * B + q) * B + r; ``chunks`` and ``device_ms`` of all adds."""
+        samples, triples, entries, chunks, ms = C.c_int64(), C.c_uint64(), C.c_int64(), C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_triplets_read(self._h, C.byref(samples), C.byref(triples), C.byref(entries),
+                                             C.byref(chunks), C.byref(ms)))
+        e = int(entries.value)
+        keys, vals = np.empty(e, np.uint64), np.empty(e, np.uint64)
+        self._ck(self._lib.mmm_triplets_read_entries(self._h, _p(keys), _p(vals)))
+        b = np.uint64(getattr(self, "_triplet_bins", 1))
+        pq, r = keys // b, keys % b
+        return dict(samples=int(samples.value), triples=int(triples.value), chunks=int(chunks.value),
+                    device_ms=float(ms.value), p=(pq // b).astype(np.int32), q=(pq % b).astype(np.int32),
+                    r=r.astype(np.int32), vals=vals)
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

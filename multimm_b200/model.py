@@ -69,6 +69,9 @@ class MultiMM:
     # loader's inputs), the sums of the minimised structure and of the MD samples, and where finish() writes
     # them (the ensemble driver points loops_file outside run_<i>)
     loop_table = loop_rows = loops = loops_md = loops_file = None
+    # the three-way contact map (SAVE_TRIPLETS): the sums of the minimised structure and of the MD samples, and
+    # where finish() writes them (the ensemble driver points triplets_file outside run_<i>)
+    triplets = triplets_md = triplets_file = None
 
     def __init__(self, args, device: int | None = None):
         self.args = args
@@ -391,7 +394,10 @@ class MultiMM:
         loop_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_LOOPS"))
         if loop_sampling:
             self._configure_loops()
-        chunk = int(np.gcd.reduce([every, dcd_every] + ([sample_every] if sampling or loop_sampling else [])))
+        triplet_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_TRIPLETS"))
+        tb = self._configure_triplets() if triplet_sampling else None
+        chunk = int(np.gcd.reduce([every, dcd_every] +
+                                  ([sample_every] if sampling or loop_sampling or triplet_sampling else [])))
         t0 = time.time()
         print('#"Step"\t"Potential Energy (kJ/mole)"\t"Kinetic Energy (kJ/mole)"\t"Total Energy (kJ/mole)"\t"Temperature (K)"')
         done = 0
@@ -417,12 +423,16 @@ class MultiMM:
                     self._sample(sampling)
                 if loop_sampling and done % sample_every == 0:
                     self.engine.loops_add()
+                if triplet_sampling and done % sample_every == 0:
+                    self.engine.triplets_add()
         finally:
             dcd.close()
         if sampling:
             self._read_samples(sampling, sample_every)
         if loop_sampling:
             self._read_loops(md=True)
+        if triplet_sampling:
+            self._read_triplets(tb, md=True)
         self.positions = self.engine.get_positions()
         cif.write_mmcif(10.0 * self.positions, self.chr_ends, self.save_path + "model/MultiMM_afterMD.cif",
                         hetatm_ends=True, connections=False, decimals=4)
@@ -486,6 +496,8 @@ class MultiMM:
             self.count_distances()
         if contact_setting(self.args, "SAVE_LOOPS"):
             self.measure_loops()
+        if contact_setting(self.args, "SAVE_TRIPLETS"):
+            self.count_triplets()
         if self.args.SIM_RUN_MD:
             self.run_md()
 
@@ -575,6 +587,43 @@ class MultiMM:
         self._read_loops()
         self.timings["loops_s"] = time.time() - t0
 
+    def _configure_triplets(self):
+        """Set up the engine's three-way accumulator with the canonical bins of TRIPLET_RESOLUTION; returns them."""
+        from . import contacts, triplets
+
+        a = self.args
+        res = int(contact_setting(a, "TRIPLET_RESOLUTION"))
+        try:
+            gb = contacts.genome_bins(self.layout, res, n_beads=a.N_BEADS, max_bins=triplets.MAX_BINS)
+        except ValueError as e:
+            raise ValueError(f"TRIPLET_RESOLUTION={res}: {e}") from None
+        self.engine.triplets_configure(float(contact_setting(a, "CONTACT_RADIUS")), gb.bins, gb.n_bins)
+        return gb
+
+    def _read_triplets(self, gb, md: bool = False):
+        from . import triplets
+
+        r = self.engine.triplets_read()
+        if md:
+            logger.info(f"three-way contacts: {r['samples']} MD structures ({r['device_ms']:.1f} ms on the device)")
+            if r["samples"] == 0:
+                return
+        d = triplets.result(r, float(contact_setting(self.args, "CONTACT_RADIUS")), gb, r["samples"])
+        if md:
+            self.triplets_md = d
+        else:
+            self.triplets = d
+
+    def count_triplets(self):
+        """Three-way contacts of the minimised structure (SAVE_TRIPLETS): bead triples in mutual contact,
+        enumerated by this member's own engine at the positions the minimisation left on the device, binned in
+        canonical genomic coordinates."""
+        t0 = time.time()
+        gb = self._configure_triplets()
+        self.engine.triplets_add()
+        self._read_triplets(gb)
+        self.timings["triplets_s"] = time.time() - t0
+
     def _configure_sampler(self) -> dict:
         """MD_SAMPLE_STEP: set up the engine's sampler with the maps that are on (SAVE_CONTACTS with its fine map,
         SAVE_DISTANCES), binned as the minimised structure's.  Returns the bins and the host-side radial sums."""
@@ -650,6 +699,13 @@ class MultiMM:
             for d, path in ((self.loops, loop_path), (self.loops_md, contacts.md_path(loop_path))):
                 if d is not None:
                     loops.save(path, d)
+        if self.triplets is not None or self.triplets_md is not None:
+            from . import triplets
+
+            tri_path = self.triplets_file or os.path.join(self.save_path, "analysis", "triplets.npz")
+            for d, path in ((self.triplets, tri_path), (self.triplets_md, contacts.md_path(tri_path))):
+                if d is not None:
+                    triplets.save(path, d)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

@@ -202,7 +202,24 @@ def args_tests(args):
     check_contact_fields(args)
     check_distance_fields(args)
     check_loop_fields(args)
+    check_triplet_fields(args)
     check_md_sample_fields(args)
+
+
+def check_triplet_fields(args):
+    """TRIPLET_RESOLUTION >= 0 and, where the modelled stretch is known from the config alone, at most
+    triplets.MAX_BINS bins."""
+    from . import contacts, triplets
+
+    res = int(contact_setting(args, "TRIPLET_RESOLUTION"))
+    if res < 0:
+        raise ValueError(f"TRIPLET_RESOLUTION={res} must be >= 0 (0 = automatic)")
+    sp = _modelled_spans(args)
+    if res > 0 and sp is not None:
+        nb = contacts.bin_count(sp, res)
+        if nb > triplets.MAX_BINS:
+            raise ValueError(f"TRIPLET_RESOLUTION={res} bp gives {nb} three-way map bins; at most {triplets.MAX_BINS} "
+                             "are supported (0 = automatic)")
 
 
 def check_loop_fields(args):
@@ -215,9 +232,9 @@ def check_loop_fields(args):
 
 
 def check_md_sample_fields(args):
-    """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES, or the loop
-    readout SAVE_LOOPS), and the MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps,
-    must reach the first sample."""
+    """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES, the loop
+    readout SAVE_LOOPS or the three-way map SAVE_TRIPLETS), and the MD loop, which runs
+    (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps, must reach the first sample."""
     step = int(contact_setting(args, "MD_SAMPLE_STEP"))
     if step < 0:
         raise ValueError(f"MD_SAMPLE_STEP={step} must be >= 0 (0 = no trajectory maps)")
@@ -225,9 +242,9 @@ def check_md_sample_fields(args):
         return
     if not args.SIM_RUN_MD:
         raise ValueError(f"MD_SAMPLE_STEP={step} samples the MD run, but SIM_RUN_MD is off")
-    if not any(contact_setting(args, k) for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS")):
+    if not any(contact_setting(args, k) for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS", "SAVE_TRIPLETS")):
         raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES "
-                         "(or SAVE_LOOPS)")
+                         "(or SAVE_LOOPS, SAVE_TRIPLETS)")
     every = max(1, int(args.SIM_SAMPLING_STEP))
     steps = (int(args.SIM_N_STEPS) // every) * every
     if step > steps:
@@ -435,6 +452,7 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     md.contacts_fine_file = member_contacts_fine_path(params["OUT_PATH"], i)
     md.distances_file = member_distances_path(params["OUT_PATH"], i)
     md.loops_file = member_loops_path(params["OUT_PATH"], i)
+    md.triplets_file = member_triplets_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
@@ -453,6 +471,10 @@ def member_distances_path(out_path: str, i: int) -> str:
 
 def member_loops_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "loops", f"member_{i}.npz")
+
+
+def member_triplets_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "triplets", f"member_{i}.npz")
 
 
 def _sampled_md(args) -> bool:
@@ -500,6 +522,28 @@ def write_ensemble_loops(args, results: list[dict]) -> str | None:
         loops.save(path, agg)
         logger.info(f"ensemble loops{' (MD samples)' if md else ''}: {int(agg['members'])} structures, "
                     f"{len(agg['row'])} rows, APA window {int(agg['apa_window'])} beads -> {path}")
+        out = out or path
+    return out
+
+
+def write_ensemble_triplets(args, results: list[dict]) -> str | None:
+    """SAVE_TRIPLETS: OUT_PATH/ensemble_triplets.npz, the sum of the triplets files of the members that succeeded
+    (exact integer sums: the same bits whichever GPU ran which member); with MD_SAMPLE_STEP also
+    ensemble_triplets_md.npz, the sum of their MD samples."""
+    if not contact_setting(args, "SAVE_TRIPLETS") or not results:
+        return None
+    from . import contacts, triplets
+
+    out = None
+    for md in (False, True) if _sampled_md(args) else (False,):
+        name = contacts.md_path if md else (lambda p: p)
+        paths = [name(member_triplets_path(args.OUT_PATH, r["replica"]))
+                 for r in sorted(results, key=lambda r: r["replica"])]
+        agg = triplets.aggregate(paths)
+        path = name(os.path.join(args.OUT_PATH, "ensemble_triplets.npz"))
+        triplets.save(path, agg)
+        logger.info(f"ensemble three-way contacts{' (MD samples)' if md else ''}: {int(agg['members'])} structures, "
+                    f"{int(agg['triples'])} triples, {len(agg['vals'])} entries -> {path}")
         out = out or path
     return out
 
@@ -738,6 +782,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         write_ensemble_contacts(args, results)
         write_ensemble_distances(args, results)
         write_ensemble_loops(args, results)
+        write_ensemble_triplets(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
         check_archives(results)
@@ -776,6 +821,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
     write_ensemble_contacts(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_distances(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_loops(args, [r for r in results if r.get("replica", -1) >= 0])
+    write_ensemble_triplets(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
