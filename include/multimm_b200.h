@@ -390,6 +390,56 @@ int mmm_triplets_read(mmm_handle h, int64_t *samples_out, uint64_t *triples_out,
  * entries succeeds.  MMM_ERR_STATE as mmm_triplets_add. */
 int mmm_triplets_read_entries(mmm_handle h, uint64_t *keys_out, uint64_t *vals_out);
 
+/* ---- locus dynamics (simulated live-cell imaging: mean squared displacements and loop lifetimes over an ordered
+ * run of structures, e.g. the samples of an MD run; not in the reference, which writes MD frames only,
+ * model.py:907-995) ---------------------------------------------------------------------------------------- */
+/* Sets up the dynamics accumulator of this handle and clears its sums and run states: the contact radius; the lag
+ * set lags[n_lags] (in structures; strictly increasing, in [1, 4096]; L = the largest); the bin table bin_of_bead
+ * (int32[N], -1 = the bead is left out; NULL = no per-bin MSD) of 1 <= n_bins <= 2^22 bins; n_rows >= 0 loop rows
+ * (int32, group int8): anchor beads bead_lo < bead_hi in [0, N), group 0 (enforced) or 1 (held out).  MMM_ERR_ARG
+ * for rc <= 0 or not finite, an empty or malformed lag set, n_bins outside its range, a bin id outside
+ * [-1, n_bins), a bad row, or neither bins nor rows.  The buffers are the accumulator's own (allocated here,
+ * freed with the handle), among them a ring of the last L structures' master positions (24 L N bytes); when they
+ * do not fit, the error of the allocation (MMM_ERR_NOMEM) and the accumulator stays unconfigured. */
+int mmm_dynamics_configure(mmm_handle h, double rc_nm, const int32_t *lags, int32_t n_lags,
+                           const int32_t *bin_of_bead, int32_t n_bins, int32_t n_rows, const int32_t *bead_lo,
+                           const int32_t *bead_hi, const int8_t *group);
+/* Adds the structure at the current positions as sample s (s = 0, 1, ... since configure).  In FP64 on the master
+ * positions, rounded operation by operation, for every lag tau <= s, against sample s - tau:
+ *   msd_sum[tau][bin_i] += rint(2^24 d2) per bead i with a bin, d2 = (dx*dx + dy*dy) + dz*dz of x_i(s) - x_i(s - tau)
+ *   (as mmm_contacts; no drift correction);
+ *   rel_msd_sum[tau][r] += rint(2^24 d2) per row, d2 = (ex*ex + ey*ey) + ez*ez of e = R(s) - R(s - tau),
+ *   R = x_hi - x_lo per component (the two-anchor MSD, free of drift).
+ * Per row, the row is closed at s when the anchors are a contact (d2 < rc^2, as mmm_loops_add) and open otherwise;
+ * when the state changes, the run that ends (length l samples) is complete if it began at a change: per row its
+ * count and length are added by state, per group and state a histogram over floor(log2 l) and the length;
+ * otherwise it is left-censored: per group and state its count and length.  The run in progress is kept per row.
+ * uint64 integer sums: exact and independent of order, and reads change nothing, so K adds equal K adds with reads
+ * in between.  The int64 guard is cumulative: with D the diagonal of the union of the bounding boxes of every
+ * structure added so far and this one, an add bounds a bin's cell by (beads of the fullest bin) x qmax(D) and a
+ * row's by qmax(2 D), qmax as in mmm_distance_map; MMM_ERR_ARG, with the sums, the ring and the run states left as
+ * they were, when either running total would reach 2^63 or when the positions are not finite.  MMM_ERR_STATE
+ * before mmm_dynamics_configure or before positions are set; after any other error the accumulator must be
+ * configured again.  Changes no state an evaluation, a minimisation, an MD step, mmm_last_result, the trajectory
+ * sampler, the loop readout or the three-way map reads; synchronises with the host twice (the guard's box, the
+ * end of the add). */
+int mmm_dynamics_add(mmm_handle h);
+/* Of the structures added since mmm_dynamics_configure: samples_out, their number S; msd_sum_out
+ * (uint64[n_lags][n_bins]) and rel_msd_sum_out (uint64[n_lags][n_rows]), in units of 2^-24 nm^2 (lag tau sums
+ * max(0, S - tau) sample pairs); device_ms_out, the device time of all adds (CUDA events on the handle's stream).
+ * Any output may be NULL.  MMM_ERR_STATE as mmm_dynamics_add. */
+int mmm_dynamics_read(mmm_handle h, int64_t *samples_out, uint64_t *msd_sum_out, uint64_t *rel_msd_sum_out,
+                      float *device_ms_out);
+/* The run statistics (state index k: 0 closed, 1 open): row_runs_out (uint64[4][n_rows]: complete closed runs,
+ * their summed length, complete open runs, their summed length); per row the run in progress: closed_out (int8, 1
+ * closed), length_out (int64, 0 before the first add), from_transition_out (int8, 1 when it began at a change);
+ * hist_out (uint64[2 groups][2 k][64], complete runs by floor(log2 length)), hist_len_out (uint64[2][2], their
+ * summed length), left_runs_out, left_len_out (uint64[2][2], left-censored runs and their summed length).  Any
+ * output may be NULL.  MMM_ERR_STATE as mmm_dynamics_add. */
+int mmm_dynamics_read_runs(mmm_handle h, uint64_t *row_runs_out, int8_t *closed_out, int64_t *length_out,
+                           int8_t *from_transition_out, uint64_t *hist_out, uint64_t *hist_len_out,
+                           uint64_t *left_runs_out, uint64_t *left_len_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

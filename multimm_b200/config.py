@@ -217,14 +217,22 @@ TRIPLET_FIELDS: dict[str, tuple[Any, Any]] = {
     "SAVE_TRIPLETS": (B, False),          # three-way contacts of the minimised structure (analysis/triplets.npz; ensembles: ensemble_triplets.npz)
     "TRIPLET_RESOLUTION": (int, 0),       # bp per bin of the three-way map; 0 = about 1000 bins, at most 2^20 bins
 }
+# Locus dynamics of MD runs (multimm_b200.dynamics), kept the same way: mean squared displacements per genomic bin
+# and of the loop anchors, and loop lifetimes, over the structures MD_SAMPLE_STEP samples; the loop state uses
+# CONTACT_RADIUS.
+DYNAMICS_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_DYNAMICS": (B, False),          # MSDs and loop lifetimes of the MD samples (analysis/dynamics.npz; ensembles: ensemble_dynamics.npz)
+    "DYNAMICS_RESOLUTION": (int, 0),      # bp per bin of the per-bin MSD; 0 = about 1000 bins, at most 2^22 bins
+    "DYNAMICS_MAX_LAG": (int, 64),        # largest lag in samples, a power of two in [1, 4096]; lags 1, 2, 4, ..., max
+}
 EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS, **LOOP_FIELDS,
-                **TRIPLET_FIELDS}
+                **TRIPLET_FIELDS, **DYNAMICS_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
-    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS, LOOP_FIELDS or
-    TRIPLET_FIELDS setting of `args`, its default where it was not given."""
+    """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS, LOOP_FIELDS,
+    TRIPLET_FIELDS or DYNAMICS_FIELDS setting of `args`, its default where it was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

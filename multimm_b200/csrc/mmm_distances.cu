@@ -166,11 +166,9 @@ __global__ void __launch_bounds__(256) k_dm_bbox(const double* __restrict__ x, i
 
 }  // namespace
 
-// The quantised-distance bound of the current positions: *dpad bounds every bead pair's distance (the diagonal
-// of the beads' FP64 bounding box, padded for the rounding of d2 and d) and *qmax the quantised distance and
-// squared distance of every pair.  MMM_ERR_ARG (message prefixed by who) when the positions are not finite.
-// Launches one kernel and synchronises; writes nothing else.  The distance maps and mmm_loops_add guard with it.
-int mmm_distance_qmax(mmm_system* h, const char* who, double* dpad, double* qmax) {
+// The FP64 bounding box of the current positions: box = {min x, min y, min z, max x, max y, max z}, NaN on an
+// axis where a coordinate is NaN.  Launches one kernel and synchronises; writes nothing else.
+int mmm_positions_box(mmm_system* h, double box[6]) {
   const int n = (int)h->n;
   int rc;
   if ((rc = mmm_reserve(h, h->d_dm_box, (size_t)DM_BOX_BLOCKS * 6, "distance-map boxes"))) return rc;
@@ -178,24 +176,46 @@ int mmm_distance_qmax(mmm_system* h, const char* who, double* dpad, double* qmax
   k_dm_bbox<<<box_blocks, 256, 0, h->stream>>>(h->d_x, n, h->d_dm_box);
   h->launches++;
   MMM_CUDA(h, cudaGetLastError());
-  std::vector<double> box((size_t)box_blocks * 6);
-  MMM_CUDA(h, cudaMemcpyAsync(box.data(), h->d_dm_box, sizeof(double) * box.size(), cudaMemcpyDeviceToHost, h->stream));
+  std::vector<double> part((size_t)box_blocks * 6);
+  MMM_CUDA(h, cudaMemcpyAsync(part.data(), h->d_dm_box, sizeof(double) * part.size(), cudaMemcpyDeviceToHost, h->stream));
   MMM_CUDA(h, cudaStreamSynchronize(h->stream));
-  double d2max = 0.0;
   for (int c = 0; c < 3; ++c) {
     double lo = INFINITY, hi = -INFINITY;
     for (int b = 0; b < box_blocks; ++b) {
-      lo = std::min(lo, box[(size_t)b * 6 + c]);
-      hi = std::max(hi, box[(size_t)b * 6 + 3 + c]);
-      if (std::isnan(box[(size_t)b * 6 + c]) || std::isnan(box[(size_t)b * 6 + 3 + c])) lo = hi = NAN;
+      lo = std::min(lo, part[(size_t)b * 6 + c]);
+      hi = std::max(hi, part[(size_t)b * 6 + 3 + c]);
+      if (std::isnan(part[(size_t)b * 6 + c]) || std::isnan(part[(size_t)b * 6 + 3 + c])) lo = hi = NAN;
     }
-    const double ext = n > 0 ? hi - lo : 0.0;
+    box[c] = lo;
+    box[3 + c] = hi;
+  }
+  return MMM_OK;
+}
+
+// *dpad: a distance of at most sqrt(d2max), padded for the rounding of d2 and d; *qmax bounds its quantised
+// value and that of its square.
+void mmm_qmax_of(double d2max, double* dpad, double* qmax) {
+  *dpad = sqrt(d2max) * (1.0 + 0x1p-40) + 0x1p-60;
+  *qmax = ceil(MMM_DIST_SCALE * std::max(*dpad * *dpad, *dpad)) + 1.0;
+}
+
+// The quantised-distance bound of the current positions: *dpad bounds every bead pair's distance (the diagonal
+// of the beads' FP64 bounding box, padded for the rounding of d2 and d) and *qmax the quantised distance and
+// squared distance of every pair.  MMM_ERR_ARG (message prefixed by who) when the positions are not finite.
+// Launches one kernel and synchronises; writes nothing else.  The distance maps and mmm_loops_add guard with it.
+int mmm_distance_qmax(mmm_system* h, const char* who, double* dpad, double* qmax) {
+  const int n = (int)h->n;
+  double box[6];
+  int rc;
+  if ((rc = mmm_positions_box(h, box))) return rc;
+  double d2max = 0.0;
+  for (int c = 0; c < 3; ++c) {
+    const double ext = n > 0 ? box[3 + c] - box[c] : 0.0;
     d2max += ext * ext;
   }
   if (!std::isfinite(d2max))
     return mmm_fail(h, MMM_ERR_ARG, std::string(who) + ": positions are not finite (no distance can be quantised)");
-  *dpad = sqrt(d2max) * (1.0 + 0x1p-40) + 0x1p-60;  // D, padded for the rounding of d2 and d
-  *qmax = ceil(MMM_DIST_SCALE * std::max(*dpad * *dpad, *dpad)) + 1.0;  // bounds qd and qd2 of every pair
+  mmm_qmax_of(d2max, dpad, qmax);  // D and the bound of qd and qd2 of every pair
   return MMM_OK;
 }
 

@@ -392,6 +392,25 @@ struct mmm_system {
   DevBuf<long long> d_tp_off;              // [n + 1 + scan parts] binned triples per bead -> their offsets
   DevBuf<unsigned long long> d_tp_keys[2]; // one chunk's keys: the radix sort's buffers
   KeyCountList tp_acc;                     // the accumulated (key, count) list
+
+  // locus dynamics (mmm_dynamics.cu): lagged displacements and loop-state runs over an ordered run of structures
+  bool dy_configured = false;
+  double dy_rc = 0.0;
+  std::vector<int> dy_lags;                // strictly increasing, in [1, 4096]; the ring holds the last lags.back()
+  int32_t dy_bins = 0;                     // 0: no per-bin MSD
+  int64_t dy_rows = 0;
+  int64_t dy_fullest = 0;                  // beads of the fullest bin (overflow guard)
+  int64_t dy_samples = 0;
+  double dy_box[6] = {0, 0, 0, 0, 0, 0};   // union of the bounding boxes of the structures added
+  double dy_bound_bins = 0.0, dy_bound_rows = 0.0;  // summed per-add bounds of one cell (overflow guard)
+  float dy_ms = 0.f;                       // device time of all adds
+  cudaEvent_t dy_ev0 = nullptr, dy_ev1 = nullptr;
+  DevBuf<double> d_dy_ring;                // [L][3n] master positions of the last L structures, slot s mod L
+  DevBuf<int> d_dy_bin;                    // [n]
+  DevBuf<int> d_dy_lag;                    // [n_lags]
+  DevBuf<int4> d_dy_row;                   // [rows] (lo, hi, group, 0)
+  DevBuf<long long> d_dy_state;            // [3][rows] closed, current run length, began at a transition
+  DevBuf<unsigned long long> d_dy_sum;     // msd [lags][bins], rel [lags][rows], runs [4][rows], groups (DY_GROUP_SUMS)
 };
 
 // the sorted keys of one sparse pass (mmm_contacts_sparse_pass)
@@ -505,6 +524,8 @@ int mmm_list_accumulate(mmm_system* h, const unsigned long long* keys, long long
 int mmm_contacts_fine_accumulate(mmm_system* h);  // the sampler's fine map += the current structure's
 int mmm_contacts_fine_read(mmm_system* h, int32_t* rows_out, int32_t* cols_out, uint64_t* vals_out);
 // mmm_distances.cu
+int mmm_positions_box(mmm_system* h, double box[6]);  // {min x, y, z, max x, y, z} of d_x; synchronises
+void mmm_qmax_of(double d2max, double* dpad, double* qmax);
 int mmm_distance_qmax(mmm_system* h, const char* who, double* dpad, double* qmax);
 int mmm_distance_guard(mmm_system* h, const char* who, const std::vector<int64_t>& occ, double prior, double* bound);
 int mmm_distance_pass(mmm_system* h, const int* d_bin, int32_t n_bins, unsigned long long* dmap,

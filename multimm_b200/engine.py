@@ -343,6 +343,54 @@ class Engine:
                     device_ms=float(ms.value), p=(pq // b).astype(np.int32), q=(pq % b).astype(np.int32),
                     r=r.astype(np.int32), vals=vals)
 
+    # -- locus dynamics (lagged displacements and loop-state runs over an ordered run of structures) ----
+    def dynamics_configure(self, rc_nm: float, lags, bin_of_bead=None, n_bins: int = 0, bead_lo=None, bead_hi=None,
+                           group=None):
+        """Clear the dynamics accumulator and set it up (mmm_dynamics_configure): the contact radius of the loop
+        state, the lag set (structures; strictly increasing, in [1, 4096]), the bins of the per-bead MSD
+        (``bin_of_bead`` int[N], -1 = left out, ``n_bins`` <= 2^22; None: off) and the loop rows (anchor beads
+        ``bead_lo`` < ``bead_hi``, ``group`` 0 enforced or 1 held out; None: no rows)."""
+        lags = _arr(lags, np.int32)
+        bins = _arr(bin_of_bead, np.int32)
+        if bins is not None and bins.shape != (self.n,):
+            raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        lo, hi = _arr(bead_lo, np.int32), _arr(bead_hi, np.int32)
+        grp = _arr(group, np.int8)
+        r = 0 if lo is None else len(lo)
+        if any(a is None or a.shape != (r,) for a in (lo, hi, grp)) and r:
+            raise ValueError("dynamics rows: bead_lo, bead_hi and group must have the same length")
+        self._ck(self._lib.mmm_dynamics_configure(self._h, float(rc_nm), _p(lags), len(lags), _p(bins), int(n_bins), r,
+                                                  _p(lo), _p(hi), _p(grp)))
+        self._dynamics = (len(lags), None if bins is None else int(n_bins), r)
+
+    def dynamics_add(self):
+        """Add the structure at the current positions as the next sample (mmm_dynamics_add)."""
+        self._ck(self._lib.mmm_dynamics_add(self._h))
+
+    def dynamics_read(self) -> dict:
+        """The dynamics sums (mmm_dynamics_read, mmm_dynamics_read_runs): ``samples``; ``msd_sum`` uint64
+        [lags][bins] (None without bins) and ``rel_msd_sum`` [lags][rows] in units of 2^-24 nm^2; per row
+        ``closed_runs``, ``closed_len``, ``open_runs``, ``open_len`` (complete runs) and the run in progress,
+        ``closed`` (bool), ``length`` (int64), ``from_transition`` (bool); per group and state (0 closed, 1 open)
+        ``hist`` uint64 [2][2][64] over floor(log2 length), ``hist_len``, ``left_runs``, ``left_len`` uint64
+        [2][2]; ``device_ms`` of all adds."""
+        nl, nb, r = getattr(self, "_dynamics", (0, None, 0))
+        msd = np.zeros((nl, nb), np.uint64) if nb else None
+        rel = np.zeros((nl, r), np.uint64)
+        runs = np.zeros((4, r), np.uint64)
+        closed, frm = np.zeros(r, np.int8), np.zeros(r, np.int8)
+        length = np.zeros(r, np.int64)
+        hist = np.zeros((2, 2, 64), np.uint64)
+        hist_len, left_runs, left_len = (np.zeros((2, 2), np.uint64) for _ in range(3))
+        samples, ms = C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_dynamics_read(self._h, C.byref(samples), _p(msd), _p(rel), C.byref(ms)))
+        self._ck(self._lib.mmm_dynamics_read_runs(self._h, _p(runs), _p(closed), _p(length), _p(frm), _p(hist),
+                                                  _p(hist_len), _p(left_runs), _p(left_len)))
+        return dict(samples=int(samples.value), msd_sum=msd, rel_msd_sum=rel, closed_runs=runs[0], closed_len=runs[1],
+                    open_runs=runs[2], open_len=runs[3], closed=closed.astype(bool), length=length,
+                    from_transition=frm.astype(bool), hist=hist, hist_len=hist_len, left_runs=left_runs,
+                    left_len=left_len, device_ms=float(ms.value))
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

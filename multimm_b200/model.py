@@ -72,6 +72,9 @@ class MultiMM:
     # the three-way contact map (SAVE_TRIPLETS): the sums of the minimised structure and of the MD samples, and
     # where finish() writes them (the ensemble driver points triplets_file outside run_<i>)
     triplets = triplets_md = triplets_file = None
+    # the locus dynamics of the MD samples (SAVE_DYNAMICS) and where finish() writes them (the ensemble driver
+    # points dynamics_file outside run_<i>)
+    dynamics = dynamics_file = None
 
     def __init__(self, args, device: int | None = None):
         self.args = args
@@ -143,7 +146,7 @@ class MultiMM:
         # the same maps summed over the structures sampled during MD (MD_SAMPLE_STEP); written beside the
         # files above, named by contacts.md_path
         self.contacts_md = self.contacts_fine_md = self.distances_md = None
-        if contact_setting(args, "SAVE_LOOPS"):
+        if contact_setting(args, "SAVE_LOOPS") or contact_setting(args, "SAVE_DYNAMICS"):
             from . import loops
 
             self.loop_table = loops.table(args.LOOPS_PATH, chrom, coords)
@@ -396,8 +399,9 @@ class MultiMM:
             self._configure_loops()
         triplet_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_TRIPLETS"))
         tb = self._configure_triplets() if triplet_sampling else None
+        dyn = self._configure_dynamics() if sample_every > 0 and contact_setting(a, "SAVE_DYNAMICS") else None
         chunk = int(np.gcd.reduce([every, dcd_every] +
-                                  ([sample_every] if sampling or loop_sampling or triplet_sampling else [])))
+                                  ([sample_every] if sampling or loop_sampling or triplet_sampling or dyn else [])))
         t0 = time.time()
         print('#"Step"\t"Potential Energy (kJ/mole)"\t"Kinetic Energy (kJ/mole)"\t"Total Energy (kJ/mole)"\t"Temperature (K)"')
         done = 0
@@ -425,6 +429,8 @@ class MultiMM:
                     self.engine.loops_add()
                 if triplet_sampling and done % sample_every == 0:
                     self.engine.triplets_add()
+                if dyn and done % sample_every == 0:
+                    self.engine.dynamics_add()
         finally:
             dcd.close()
         if sampling:
@@ -433,6 +439,8 @@ class MultiMM:
             self._read_loops(md=True)
         if triplet_sampling:
             self._read_triplets(tb, md=True)
+        if dyn:
+            self._read_dynamics(dyn, sample_every)
         self.positions = self.engine.get_positions()
         cif.write_mmcif(10.0 * self.positions, self.chr_ends, self.save_path + "model/MultiMM_afterMD.cif",
                         hetatm_ends=True, connections=False, decimals=4)
@@ -624,6 +632,34 @@ class MultiMM:
         self._read_triplets(gb)
         self.timings["triplets_s"] = time.time() - t0
 
+    def _configure_dynamics(self) -> dict:
+        """SAVE_DYNAMICS: set up the engine's dynamics accumulator with the canonical bins of DYNAMICS_RESOLUTION,
+        the lags 1, 2, ..., DYNAMICS_MAX_LAG and this member's valid loop rows.  Returns the bins and lags."""
+        from . import contacts, dynamics, loops
+
+        a = self.args
+        res = int(contact_setting(a, "DYNAMICS_RESOLUTION"))
+        try:
+            gb = contacts.genome_bins(self.layout, res, n_beads=a.N_BEADS, max_bins=dynamics.MAX_BINS)
+        except ValueError as e:
+            raise ValueError(f"DYNAMICS_RESOLUTION={res}: {e}") from None
+        lags = dynamics.lag_set(int(contact_setting(a, "DYNAMICS_MAX_LAG")))
+        rows = loops.device_rows(self.loop_rows)
+        self.engine.dynamics_configure(float(contact_setting(a, "CONTACT_RADIUS")), lags, gb.bins, gb.n_bins,
+                                       rows["bead_lo"], rows["bead_hi"], rows["group"])
+        return dict(gb=gb, lags=lags)
+
+    def _read_dynamics(self, st: dict, sample_every: int):
+        from . import dynamics
+
+        a = self.args
+        r = self.engine.dynamics_read()
+        logger.info(f"locus dynamics: {r['samples']} MD structures, lags up to {int(st['lags'][-1])} samples "
+                    f"({r['device_ms']:.1f} ms on the device)")
+        self.dynamics = dynamics.result(r, st["lags"], st["gb"], self.loop_table, self.loop_rows,
+                                        float(contact_setting(a, "CONTACT_RADIUS")), sample_every,
+                                        _f(a.SIM_INTEGRATOR_STEP))
+
     def _configure_sampler(self) -> dict:
         """MD_SAMPLE_STEP: set up the engine's sampler with the maps that are on (SAVE_CONTACTS with its fine map,
         SAVE_DISTANCES), binned as the minimised structure's.  Returns the bins and the host-side radial sums."""
@@ -706,6 +742,10 @@ class MultiMM:
             for d, path in ((self.triplets, tri_path), (self.triplets_md, contacts.md_path(tri_path))):
                 if d is not None:
                     triplets.save(path, d)
+        if self.dynamics is not None:
+            from . import dynamics
+
+            dynamics.save(self.dynamics_file or os.path.join(self.save_path, "analysis", "dynamics.npz"), self.dynamics)
         self.save_args_to_txt(self.args.OUT_PATH + "/metadata/parameters.txt")
         return self.report
 

@@ -203,6 +203,7 @@ def args_tests(args):
     check_distance_fields(args)
     check_loop_fields(args)
     check_triplet_fields(args)
+    check_dynamics_fields(args)
     check_md_sample_fields(args)
 
 
@@ -222,6 +223,35 @@ def check_triplet_fields(args):
                              "are supported (0 = automatic)")
 
 
+def check_dynamics_fields(args):
+    """DYNAMICS_RESOLUTION >= 0 and, where the modelled stretch is known from the config alone, at most
+    dynamics.MAX_BINS bins; DYNAMICS_MAX_LAG a power of two in [1, dynamics.MAX_LAG]; SAVE_DYNAMICS needs an MD
+    run that samples at least two structures (MD_SAMPLE_STEP)."""
+    from . import contacts, dynamics
+
+    res = int(contact_setting(args, "DYNAMICS_RESOLUTION"))
+    if res < 0:
+        raise ValueError(f"DYNAMICS_RESOLUTION={res} must be >= 0 (0 = automatic)")
+    sp = _modelled_spans(args)
+    if res > 0 and sp is not None:
+        nb = contacts.bin_count(sp, res)
+        if nb > dynamics.MAX_BINS:
+            raise ValueError(f"DYNAMICS_RESOLUTION={res} bp gives {nb} dynamics bins; at most {dynamics.MAX_BINS} "
+                             "are supported (0 = automatic)")
+    dynamics.lag_set(int(contact_setting(args, "DYNAMICS_MAX_LAG")))
+    if not contact_setting(args, "SAVE_DYNAMICS"):
+        return
+    step = int(contact_setting(args, "MD_SAMPLE_STEP"))
+    if not args.SIM_RUN_MD or step <= 0:
+        raise ValueError("SAVE_DYNAMICS follows the structures an MD run samples: it needs SIM_RUN_MD and "
+                         "MD_SAMPLE_STEP > 0")
+    every = max(1, int(args.SIM_SAMPLING_STEP))
+    samples = ((int(args.SIM_N_STEPS) // every) * every) // step
+    if samples < 2:
+        raise ValueError(f"SAVE_DYNAMICS needs at least two MD samples, but MD_SAMPLE_STEP={step} samples {samples} "
+                         "structures of the MD run")
+
+
 def check_loop_fields(args):
     """LOOP_APA_WINDOW in [0, loops.MAX_WINDOW]."""
     from . import loops
@@ -233,7 +263,7 @@ def check_loop_fields(args):
 
 def check_md_sample_fields(args):
     """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES, the loop
-    readout SAVE_LOOPS or the three-way map SAVE_TRIPLETS), and the MD loop, which runs
+    readout SAVE_LOOPS, the three-way map SAVE_TRIPLETS or the dynamics SAVE_DYNAMICS), and the MD loop, which runs
     (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps, must reach the first sample."""
     step = int(contact_setting(args, "MD_SAMPLE_STEP"))
     if step < 0:
@@ -242,9 +272,10 @@ def check_md_sample_fields(args):
         return
     if not args.SIM_RUN_MD:
         raise ValueError(f"MD_SAMPLE_STEP={step} samples the MD run, but SIM_RUN_MD is off")
-    if not any(contact_setting(args, k) for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS", "SAVE_TRIPLETS")):
+    if not any(contact_setting(args, k)
+               for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS", "SAVE_TRIPLETS", "SAVE_DYNAMICS")):
         raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES "
-                         "(or SAVE_LOOPS, SAVE_TRIPLETS)")
+                         "(or SAVE_LOOPS, SAVE_TRIPLETS, SAVE_DYNAMICS)")
     every = max(1, int(args.SIM_SAMPLING_STEP))
     steps = (int(args.SIM_N_STEPS) // every) * every
     if step > steps:
@@ -453,6 +484,7 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     md.distances_file = member_distances_path(params["OUT_PATH"], i)
     md.loops_file = member_loops_path(params["OUT_PATH"], i)
     md.triplets_file = member_triplets_path(params["OUT_PATH"], i)
+    md.dynamics_file = member_dynamics_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
@@ -475,6 +507,10 @@ def member_loops_path(out_path: str, i: int) -> str:
 
 def member_triplets_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "triplets", f"member_{i}.npz")
+
+
+def member_dynamics_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "dynamics", f"member_{i}.npz")
 
 
 def _sampled_md(args) -> bool:
@@ -546,6 +582,22 @@ def write_ensemble_triplets(args, results: list[dict]) -> str | None:
                     f"{int(agg['triples'])} triples, {len(agg['vals'])} entries -> {path}")
         out = out or path
     return out
+
+
+def write_ensemble_dynamics(args, results: list[dict]) -> str | None:
+    """SAVE_DYNAMICS: OUT_PATH/ensemble_dynamics.npz, the sum of the dynamics files of the members that succeeded
+    (exact integer sums: the same bits whichever GPU ran which member)."""
+    if not contact_setting(args, "SAVE_DYNAMICS") or not results:
+        return None
+    from . import dynamics
+
+    paths = [member_dynamics_path(args.OUT_PATH, r["replica"]) for r in sorted(results, key=lambda r: r["replica"])]
+    agg = dynamics.aggregate(paths)
+    path = os.path.join(args.OUT_PATH, "ensemble_dynamics.npz")
+    dynamics.save(path, agg)
+    logger.info(f"ensemble dynamics: {int(agg['members'])} members, {int(agg['samples'])} MD samples, lags up to "
+                f"{int(agg['lags'][-1])} samples, {len(agg['row'])} rows -> {path}")
+    return path
 
 
 def write_ensemble_contacts(args, results: list[dict]) -> str | None:
@@ -783,6 +835,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         write_ensemble_distances(args, results)
         write_ensemble_loops(args, results)
         write_ensemble_triplets(args, results)
+        write_ensemble_dynamics(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
         check_archives(results)
@@ -822,6 +875,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
     write_ensemble_distances(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_loops(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_triplets(args, [r for r in results if r.get("replica", -1) >= 0])
+    write_ensemble_dynamics(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
