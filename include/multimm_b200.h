@@ -440,6 +440,36 @@ int mmm_dynamics_read_runs(mmm_handle h, uint64_t *row_runs_out, int8_t *closed_
                            int8_t *from_transition_out, uint64_t *hist_out, uint64_t *hist_len_out,
                            uint64_t *left_runs_out, uint64_t *left_len_out);
 
+/* ---- distance distributions per genomic bin pair (simulated chromatin tracing: median distance maps and the
+ * contact probability at any radius, summed over structures; not in the reference, whose pairwise analysis
+ * model.py:1069-1213 and cdist heat maps plots.py:540 look at one structure's distances) ---------------------- */
+/* Sets up the distance-histogram accumulator of this handle and clears its sums: the bin table bin_of_bead
+ * (int32[N], -1 = the bead is left out, uploaded once) of n_bins >= 1 bins and the edges e_1 < ... < e_E in nm
+ * (1 <= E = n_edges <= 63), which give H = E + 1 cells.  The squares e2[k] = e_k * e_k are taken in FP64 here.
+ * MMM_ERR_ARG for a NULL or bad table (a bin id outside [-1, n_bins)), NULL edges, n_edges outside [1, 63], an
+ * edge that is not finite or not > 0, edges whose squares are not finite, > 0 and strictly increasing, or more
+ * than 2^27 counters (B (B + 1) / 2 x H, 1 GiB of uint64).  The buffers are the accumulator's own (allocated here,
+ * freed with the handle); the accumulator stays unconfigured after any error. */
+int mmm_disthist_configure(mmm_handle h, const int32_t *bin_of_bead, int32_t n_bins, const double *edges_nm,
+                           int32_t n_edges);
+/* Adds the structure at the current positions: for every unordered bead pair i < j whose beads both have a bin,
+ * d2 = (dx*dx + dy*dy) + dz*dz in FP64 on the master positions, rounded operation by operation (as mmm_contacts
+ * and mmm_distance_map), falls in the cell h = #{k : e2[k] <= d2} (cell 0 is [0, e_1), cell E is [e_E, inf)),
+ * and counts[tri(p, q)][h] += 1 with p <= q the two bins and tri the row-major upper-triangle order
+ * (numpy.triu_indices(n_bins)).  The pairs in cells < k are those with d2 < e_k^2: the contacts of mmm_contacts at
+ * rc = e_k.  uint64 integer sums: exact and independent of schedule, so K adds equal the sum of K
+ * single-structure reads.  The guard is cumulative: one add raises a count by at most P, the bead pairs of the
+ * fullest bin pair; MMM_ERR_ARG, with the sums left as they were, when the running total of P over the adds would
+ * reach 2^63, or when the positions are not finite.  MMM_ERR_STATE before mmm_disthist_configure or before
+ * positions are set; after any other error the accumulator must be configured again.  Changes no state an
+ * evaluation, a minimisation, an MD step, mmm_last_result, the trajectory sampler or the other readouts read;
+ * synchronises with the host (the positions' check, the end of the add). */
+int mmm_disthist_add(mmm_handle h);
+/* Of the structures added since mmm_disthist_configure: samples_out, their number; counts_out (uint64
+ * [n_bins (n_bins + 1) / 2][H], rows in numpy.triu_indices(n_bins) order); device_ms_out, the device time of all
+ * adds (CUDA events on the handle's stream).  Any output may be NULL.  MMM_ERR_STATE as mmm_disthist_add. */
+int mmm_disthist_read(mmm_handle h, int64_t *samples_out, uint64_t *counts_out, float *device_ms_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

@@ -225,14 +225,22 @@ DYNAMICS_FIELDS: dict[str, tuple[Any, Any]] = {
     "DYNAMICS_RESOLUTION": (int, 0),      # bp per bin of the per-bin MSD; 0 = about 1000 bins, at most 2^22 bins
     "DYNAMICS_MAX_LAG": (int, 64),        # largest lag in samples, a power of two in [1, 4096]; lags 1, 2, 4, ..., max
 }
+# Distance distributions per genomic bin pair (multimm_b200.disthist), kept the same way: bead pairs counted per
+# distance cell between the edges; MD_SAMPLE_STEP also samples them.
+DISTANCE_HIST_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_DISTANCE_HIST": (B, False),     # distance histograms of the minimised structure (analysis/distance_hist.npz; ensembles: ensemble_distance_hist.npz)
+    "DISTANCE_HIST_RESOLUTION": (int, 0), # bp per bin; 0 = about 1000 bins; B (B + 1) / 2 x (edges + 1) <= 2^27 counters
+    "DISTANCE_HIST_EDGES": (str, "0.1,0.15,0.2,0.3,0.5,0.7,1,1.5,2,3,5,7,10,15,20,30,50,70,100"),  # cell edges in nm, comma-separated, strictly increasing, 1 to 63
+}
 EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS, **LOOP_FIELDS,
-                **TRIPLET_FIELDS, **DYNAMICS_FIELDS}
+                **TRIPLET_FIELDS, **DYNAMICS_FIELDS, **DISTANCE_HIST_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
     """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS, LOOP_FIELDS,
-    TRIPLET_FIELDS or DYNAMICS_FIELDS setting of `args`, its default where it was not given."""
+    TRIPLET_FIELDS, DYNAMICS_FIELDS or DISTANCE_HIST_FIELDS setting of `args`, its default where it was not
+    given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

@@ -411,6 +411,18 @@ struct mmm_system {
   DevBuf<int4> d_dy_row;                   // [rows] (lo, hi, group, 0)
   DevBuf<long long> d_dy_state;            // [3][rows] closed, current run length, began at a transition
   DevBuf<unsigned long long> d_dy_sum;     // msd [lags][bins], rel [lags][rows], runs [4][rows], groups (DY_GROUP_SUMS)
+
+  // distance distributions (mmm_disthist.cu): per bin pair, bead pairs counted per distance cell over structures
+  bool dh_configured = false;
+  int32_t dh_bins = 0, dh_cells = 0;       // B, H = edges + 1
+  uint64_t dh_pmax = 0;                    // bead pairs of the fullest bin pair: one add's bound on a count
+  uint64_t dh_total = 0;                   // summed bounds of the structures added (overflow guard)
+  int64_t dh_samples = 0;
+  float dh_ms = 0.f;                       // device time of all adds
+  cudaEvent_t dh_ev0 = nullptr, dh_ev1 = nullptr;
+  DevBuf<int> d_dh_bin;                    // [n]
+  DevBuf<unsigned long long> d_dh_e2;      // [63] squared edges (nm^2) as the bits of their doubles, the first H - 1 used
+  DevBuf<unsigned long long> d_dh_cnt;     // [B (B + 1) / 2][H] counts
 };
 
 // the sorted keys of one sparse pass (mmm_contacts_sparse_pass)

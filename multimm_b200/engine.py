@@ -391,6 +391,35 @@ class Engine:
                     from_transition=frm.astype(bool), hist=hist, hist_len=hist_len, left_runs=left_runs,
                     left_len=left_len, device_ms=float(ms.value))
 
+    # -- distance distributions (bead pairs per bin pair and distance cell, summed over many structures) --
+    def disthist_configure(self, bin_of_bead, n_bins: int, edges_nm):
+        """Clear the distance-histogram accumulator and set its bins and edges (mmm_disthist_configure):
+        ``bin_of_bead`` (int[N], -1 = left out) of ``n_bins`` bins, and the strictly increasing edges in nm (1 to
+        63 of them, giving E + 1 cells)."""
+        bins = _arr(bin_of_bead, np.int32)
+        if bins is not None and bins.shape != (self.n,):
+            raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        edges = _arr(edges_nm, np.float64)
+        if edges is not None and edges.ndim != 1:
+            raise ValueError("edges_nm must be one-dimensional")
+        ne = 0 if edges is None else len(edges)
+        self._ck(self._lib.mmm_disthist_configure(self._h, _p(bins), int(n_bins), _p(edges), ne))
+        self._disthist = (int(n_bins), ne + 1)
+
+    def disthist_add(self):
+        """Count the bead pairs of the structure at the current positions (mmm_disthist_add)."""
+        self._ck(self._lib.mmm_disthist_add(self._h))
+
+    def disthist_read(self) -> dict:
+        """The distance histograms (mmm_disthist_read): ``samples``; ``counts`` uint64 [B (B + 1) / 2, H], rows in
+        ``np.triu_indices(B)`` order, cell h = pairs with e_h <= d < e_(h+1) (e_0 = 0, e_H = inf); ``device_ms``
+        of all adds."""
+        nb, nc = getattr(self, "_disthist", (0, 0))
+        counts = np.zeros((nb * (nb + 1) // 2, nc), np.uint64)
+        samples, ms = C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_disthist_read(self._h, C.byref(samples), _p(counts), C.byref(ms)))
+        return dict(samples=int(samples.value), counts=counts, device_ms=float(ms.value))
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

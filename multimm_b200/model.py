@@ -75,6 +75,9 @@ class MultiMM:
     # the locus dynamics of the MD samples (SAVE_DYNAMICS) and where finish() writes them (the ensemble driver
     # points dynamics_file outside run_<i>)
     dynamics = dynamics_file = None
+    # the distance histograms (SAVE_DISTANCE_HIST): the counts of the minimised structure and of the MD samples,
+    # and where finish() writes them (the ensemble driver points distance_hist_file outside run_<i>)
+    distance_hist = distance_hist_md = distance_hist_file = None
 
     def __init__(self, args, device: int | None = None):
         self.args = args
@@ -400,8 +403,11 @@ class MultiMM:
         triplet_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_TRIPLETS"))
         tb = self._configure_triplets() if triplet_sampling else None
         dyn = self._configure_dynamics() if sample_every > 0 and contact_setting(a, "SAVE_DYNAMICS") else None
+        hist_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_DISTANCE_HIST"))
+        hb = self._configure_distance_hist() if hist_sampling else None
         chunk = int(np.gcd.reduce([every, dcd_every] +
-                                  ([sample_every] if sampling or loop_sampling or triplet_sampling or dyn else [])))
+                                  ([sample_every] if sampling or loop_sampling or triplet_sampling or dyn or hist_sampling
+                                   else [])))
         t0 = time.time()
         print('#"Step"\t"Potential Energy (kJ/mole)"\t"Kinetic Energy (kJ/mole)"\t"Total Energy (kJ/mole)"\t"Temperature (K)"')
         done = 0
@@ -431,6 +437,8 @@ class MultiMM:
                     self.engine.triplets_add()
                 if dyn and done % sample_every == 0:
                     self.engine.dynamics_add()
+                if hist_sampling and done % sample_every == 0:
+                    self.engine.disthist_add()
         finally:
             dcd.close()
         if sampling:
@@ -441,6 +449,8 @@ class MultiMM:
             self._read_triplets(tb, md=True)
         if dyn:
             self._read_dynamics(dyn, sample_every)
+        if hist_sampling:
+            self._read_distance_hist(hb, md=True)
         self.positions = self.engine.get_positions()
         cif.write_mmcif(10.0 * self.positions, self.chr_ends, self.save_path + "model/MultiMM_afterMD.cif",
                         hetatm_ends=True, connections=False, decimals=4)
@@ -506,6 +516,8 @@ class MultiMM:
             self.measure_loops()
         if contact_setting(self.args, "SAVE_TRIPLETS"):
             self.count_triplets()
+        if contact_setting(self.args, "SAVE_DISTANCE_HIST"):
+            self.count_distance_hist()
         if self.args.SIM_RUN_MD:
             self.run_md()
 
@@ -632,6 +644,46 @@ class MultiMM:
         self._read_triplets(gb)
         self.timings["triplets_s"] = time.time() - t0
 
+    def _configure_distance_hist(self):
+        """Set up the engine's distance-histogram accumulator with the canonical bins of DISTANCE_HIST_RESOLUTION
+        and the edges of DISTANCE_HIST_EDGES; returns the bins and edges."""
+        from . import contacts, disthist
+
+        a = self.args
+        edges = disthist.parse_edges(contact_setting(a, "DISTANCE_HIST_EDGES"))
+        res = int(contact_setting(a, "DISTANCE_HIST_RESOLUTION"))
+        try:
+            gb = contacts.genome_bins(self.layout, res, n_beads=a.N_BEADS, max_bins=disthist.max_bins(len(edges)))
+        except ValueError as e:
+            raise ValueError(f"DISTANCE_HIST_RESOLUTION={res}: {e}") from None
+        self.engine.disthist_configure(gb.bins, gb.n_bins, edges)
+        return gb, edges
+
+    def _read_distance_hist(self, hb, md: bool = False):
+        from . import disthist
+
+        gb, edges = hb
+        r = self.engine.disthist_read()
+        if md:
+            logger.info(f"distance histograms: {r['samples']} MD structures ({r['device_ms']:.1f} ms on the device)")
+            if r["samples"] == 0:
+                return
+        d = disthist.result(r["counts"], edges, gb, r["samples"])
+        if md:
+            self.distance_hist_md = d
+        else:
+            self.distance_hist = d
+
+    def count_distance_hist(self):
+        """Distance histograms of the minimised structure (SAVE_DISTANCE_HIST): every bead pair counted per bin
+        pair and distance cell by this member's own engine at the positions the minimisation left on the device,
+        binned in canonical genomic coordinates."""
+        t0 = time.time()
+        hb = self._configure_distance_hist()
+        self.engine.disthist_add()
+        self._read_distance_hist(hb)
+        self.timings["distance_hist_s"] = time.time() - t0
+
     def _configure_dynamics(self) -> dict:
         """SAVE_DYNAMICS: set up the engine's dynamics accumulator with the canonical bins of DYNAMICS_RESOLUTION,
         the lags 1, 2, ..., DYNAMICS_MAX_LAG and this member's valid loop rows.  Returns the bins and lags."""
@@ -742,6 +794,13 @@ class MultiMM:
             for d, path in ((self.triplets, tri_path), (self.triplets_md, contacts.md_path(tri_path))):
                 if d is not None:
                     triplets.save(path, d)
+        if self.distance_hist is not None or self.distance_hist_md is not None:
+            from . import disthist
+
+            hist_path = self.distance_hist_file or os.path.join(self.save_path, "analysis", "distance_hist.npz")
+            for d, path in ((self.distance_hist, hist_path), (self.distance_hist_md, contacts.md_path(hist_path))):
+                if d is not None:
+                    disthist.save(path, d)
         if self.dynamics is not None:
             from . import dynamics
 

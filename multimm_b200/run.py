@@ -204,6 +204,7 @@ def args_tests(args):
     check_loop_fields(args)
     check_triplet_fields(args)
     check_dynamics_fields(args)
+    check_distance_hist_fields(args)
     check_md_sample_fields(args)
 
 
@@ -252,6 +253,24 @@ def check_dynamics_fields(args):
                          "structures of the MD run")
 
 
+def check_distance_hist_fields(args):
+    """DISTANCE_HIST_EDGES parse into 1 to disthist.MAX_EDGES strictly increasing, finite edges > 0;
+    DISTANCE_HIST_RESOLUTION >= 0 and, where the modelled stretch is known from the config alone, few enough bins
+    for the counters of the device (disthist.max_bins)."""
+    from . import contacts, disthist
+
+    edges = disthist.parse_edges(contact_setting(args, "DISTANCE_HIST_EDGES"))
+    res = int(contact_setting(args, "DISTANCE_HIST_RESOLUTION"))
+    if res < 0:
+        raise ValueError(f"DISTANCE_HIST_RESOLUTION={res} must be >= 0 (0 = automatic)")
+    sp = _modelled_spans(args)
+    if res > 0 and sp is not None:
+        nb, most = contacts.bin_count(sp, res), disthist.max_bins(len(edges))
+        if nb > most:
+            raise ValueError(f"DISTANCE_HIST_RESOLUTION={res} bp gives {nb} distance-histogram bins; with "
+                             f"{len(edges)} edges at most {most} are supported (0 = automatic)")
+
+
 def check_loop_fields(args):
     """LOOP_APA_WINDOW in [0, loops.MAX_WINDOW]."""
     from . import loops
@@ -263,8 +282,9 @@ def check_loop_fields(args):
 
 def check_md_sample_fields(args):
     """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES, the loop
-    readout SAVE_LOOPS, the three-way map SAVE_TRIPLETS or the dynamics SAVE_DYNAMICS), and the MD loop, which runs
-    (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps, must reach the first sample."""
+    readout SAVE_LOOPS, the three-way map SAVE_TRIPLETS, the dynamics SAVE_DYNAMICS or the distance histograms
+    SAVE_DISTANCE_HIST), and the MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps,
+    must reach the first sample."""
     step = int(contact_setting(args, "MD_SAMPLE_STEP"))
     if step < 0:
         raise ValueError(f"MD_SAMPLE_STEP={step} must be >= 0 (0 = no trajectory maps)")
@@ -273,9 +293,10 @@ def check_md_sample_fields(args):
     if not args.SIM_RUN_MD:
         raise ValueError(f"MD_SAMPLE_STEP={step} samples the MD run, but SIM_RUN_MD is off")
     if not any(contact_setting(args, k)
-               for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS", "SAVE_TRIPLETS", "SAVE_DYNAMICS")):
+               for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS", "SAVE_TRIPLETS", "SAVE_DYNAMICS",
+                         "SAVE_DISTANCE_HIST")):
         raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES "
-                         "(or SAVE_LOOPS, SAVE_TRIPLETS, SAVE_DYNAMICS)")
+                         "(or SAVE_LOOPS, SAVE_TRIPLETS, SAVE_DYNAMICS, SAVE_DISTANCE_HIST)")
     every = max(1, int(args.SIM_SAMPLING_STEP))
     steps = (int(args.SIM_N_STEPS) // every) * every
     if step > steps:
@@ -485,6 +506,7 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     md.loops_file = member_loops_path(params["OUT_PATH"], i)
     md.triplets_file = member_triplets_path(params["OUT_PATH"], i)
     md.dynamics_file = member_dynamics_path(params["OUT_PATH"], i)
+    md.distance_hist_file = member_distance_hist_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
@@ -511,6 +533,10 @@ def member_triplets_path(out_path: str, i: int) -> str:
 
 def member_dynamics_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "dynamics", f"member_{i}.npz")
+
+
+def member_distance_hist_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "distance_hist", f"member_{i}.npz")
 
 
 def _sampled_md(args) -> bool:
@@ -580,6 +606,28 @@ def write_ensemble_triplets(args, results: list[dict]) -> str | None:
         triplets.save(path, agg)
         logger.info(f"ensemble three-way contacts{' (MD samples)' if md else ''}: {int(agg['members'])} structures, "
                     f"{int(agg['triples'])} triples, {len(agg['vals'])} entries -> {path}")
+        out = out or path
+    return out
+
+
+def write_ensemble_distance_hist(args, results: list[dict]) -> str | None:
+    """SAVE_DISTANCE_HIST: OUT_PATH/ensemble_distance_hist.npz, the sum of the distance-histogram files of the
+    members that succeeded (exact integer sums: the same bits whichever GPU ran which member); with MD_SAMPLE_STEP
+    also ensemble_distance_hist_md.npz, the sum of their MD samples."""
+    if not contact_setting(args, "SAVE_DISTANCE_HIST") or not results:
+        return None
+    from . import contacts, disthist
+
+    out = None
+    for md in (False, True) if _sampled_md(args) else (False,):
+        name = contacts.md_path if md else (lambda p: p)
+        paths = [name(member_distance_hist_path(args.OUT_PATH, r["replica"]))
+                 for r in sorted(results, key=lambda r: r["replica"])]
+        agg = disthist.aggregate(paths)
+        path = name(os.path.join(args.OUT_PATH, "ensemble_distance_hist.npz"))
+        disthist.save(path, agg)
+        logger.info(f"ensemble distance histograms{' (MD samples)' if md else ''}: {int(agg['members'])} structures, "
+                    f"{len(agg['edges_nm'])} edges -> {path}")
         out = out or path
     return out
 
@@ -836,6 +884,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         write_ensemble_loops(args, results)
         write_ensemble_triplets(args, results)
         write_ensemble_dynamics(args, results)
+        write_ensemble_distance_hist(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
         check_archives(results)
@@ -876,6 +925,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
     write_ensemble_loops(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_triplets(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_dynamics(args, [r for r in results if r.get("replica", -1) >= 0])
+    write_ensemble_distance_hist(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
