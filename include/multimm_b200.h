@@ -470,6 +470,37 @@ int mmm_disthist_add(mmm_handle h);
  * adds (CUDA events on the handle's stream).  Any output may be NULL.  MMM_ERR_STATE as mmm_disthist_add. */
 int mmm_disthist_read(mmm_handle h, int64_t *samples_out, uint64_t *counts_out, float *device_ms_out);
 
+/* ---- genome architecture mapping (simulated GAM: random thin slices through each structure, locus
+ * co-segregation summed over structures; not in the reference, which has no slicing readout) ------------------ */
+/* Sets up the GAM accumulator of this handle and clears its sums: the bin table bin_of_bead (int32[N], -1 = the
+ * bead is left out, uploaded once) of n_bins >= 1 bins, and max_slices, the most slices one add may take.  The
+ * detection bitset (n_bins x ceil(max_slices / 32) uint32), the slice bitset, the plane table and the
+ * co-segregation triangle are allocated here, so a table that does not fit fails here.  MMM_ERR_ARG for a NULL
+ * or bad table (a bin id outside [-1, n_bins)), B (B + 1) / 2 > 2^27 bin pairs, or max_slices outside
+ * [1, 65536].  The buffers are the accumulator's own (freed with the handle); the accumulator stays
+ * unconfigured after any error. */
+int mmm_gam_configure(mmm_handle h, const int32_t *bin_of_bead, int32_t n_bins, int32_t max_slices);
+/* Slices the structure at the current positions with S = n_slices planes (planes: double[S][4], the normal
+ * nx, ny, nz and the offset o of each; the normal need not be unit length) and the common half-thickness
+ * h >= 0.  Bead i lies in slice k iff |s| <= h with s = ((nx*x + ny*y) + nz*z) - o in FP64 on the master
+ * positions, rounded operation by operation (a bead exactly on the boundary is inside); bin p is detected in
+ * slice k iff a bead of bin p lies in it.  Then counts[tri(p, q)] += #{k : p and q both detected in k} for
+ * p <= q, with tri the row-major upper-triangle order (numpy.triu_indices(n_bins)), so the diagonal holds each
+ * bin's detections; slices += S, empty += #{k : no bin detected in k}, structures += 1.  Integer sums: exact and
+ * independent of schedule, so K adds equal the sum of K single adds.  MMM_ERR_ARG, with the sums left as they
+ * were, when S is outside [1, max_slices], planes is NULL, a plane value is not finite, h is not finite or < 0,
+ * the positions are not finite, or the running slice total would reach 2^63.  MMM_ERR_STATE before
+ * mmm_gam_configure or before positions are set; after any other error the accumulator must be configured
+ * again.  Changes no state an evaluation, a minimisation, an MD step, mmm_last_result, the trajectory sampler or
+ * the other readouts read; synchronises with the host (the positions' check, the end of the add). */
+int mmm_gam_add(mmm_handle h, const double *planes, int32_t n_slices, double half_thickness);
+/* Of the adds since mmm_gam_configure: structures_out, their number; slices_out, the slices; empty_out, the
+ * slices in which no bin was detected; counts_out (uint64[n_bins (n_bins + 1) / 2], rows in
+ * numpy.triu_indices(n_bins) order); device_ms_out, the device time of all adds (CUDA events on the handle's
+ * stream).  Any output may be NULL.  MMM_ERR_STATE as mmm_gam_add. */
+int mmm_gam_read(mmm_handle h, int64_t *structures_out, int64_t *slices_out, int64_t *empty_out,
+                 uint64_t *counts_out, float *device_ms_out);
+
 /* ---- one system on several GPUs of one box (exact mode only) -------------------------------- */
 /* The reference has no multi-GPU path (DeviceIndex is never set, model.py:862-876).  Here the
  * O(N^2) pair work of ONE system is dealt to `world` handles, one per GPU / process, each holding

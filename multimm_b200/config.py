@@ -232,15 +232,23 @@ DISTANCE_HIST_FIELDS: dict[str, tuple[Any, Any]] = {
     "DISTANCE_HIST_RESOLUTION": (int, 0), # bp per bin; 0 = about 1000 bins; B (B + 1) / 2 x (edges + 1) <= 2^27 counters
     "DISTANCE_HIST_EDGES": (str, "0.1,0.15,0.2,0.3,0.5,0.7,1,1.5,2,3,5,7,10,15,20,30,50,70,100"),  # cell edges in nm, comma-separated, strictly increasing, 1 to 63
 }
+# Genome architecture mapping (multimm_b200.gam), kept the same way: bins co-detected in random thin slices of each
+# structure; MD_SAMPLE_STEP also samples it.
+GAM_FIELDS: dict[str, tuple[Any, Any]] = {
+    "SAVE_GAM": (B, False),               # GAM co-segregation of the minimised structure (analysis/gam.npz; ensembles: ensemble_gam.npz)
+    "GAM_RESOLUTION": (int, 0),           # bp per bin; 0 = about 1000 bins; B (B + 1) / 2 <= 2^27
+    "GAM_SLICES": (int, 1024),            # slices per structure, in [1, 65536]
+    "GAM_SLICE_FRACTION": (float, 0.025), # slice thickness over the envelope diameter, in (0, 1]
+}
 EXTRA_FIELDS = {**CONTACT_FIELDS, **CONTACT_FINE_FIELDS, **DISTANCE_FIELDS, **MD_SAMPLE_FIELDS, **LOOP_FIELDS,
-                **TRIPLET_FIELDS, **DYNAMICS_FIELDS, **DISTANCE_HIST_FIELDS}
+                **TRIPLET_FIELDS, **DYNAMICS_FIELDS, **DISTANCE_HIST_FIELDS, **GAM_FIELDS}
 _CONTACT_ADAPTERS = {name: TypeAdapter(ftype) for name, (ftype, _) in EXTRA_FIELDS.items()}
 
 
 def contact_setting(args, name: str):
     """Value of a CONTACT_FIELDS, CONTACT_FINE_FIELDS, DISTANCE_FIELDS, MD_SAMPLE_FIELDS, LOOP_FIELDS,
-    TRIPLET_FIELDS, DYNAMICS_FIELDS or DISTANCE_HIST_FIELDS setting of `args`, its default where it was not
-    given."""
+    TRIPLET_FIELDS, DYNAMICS_FIELDS, DISTANCE_HIST_FIELDS or GAM_FIELDS setting of `args`, its default where it
+    was not given."""
     extra = getattr(args, "__pydantic_extra__", None) or {}
     return extra.get(name, EXTRA_FIELDS[name][1])
 

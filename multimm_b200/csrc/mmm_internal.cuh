@@ -423,6 +423,18 @@ struct mmm_system {
   DevBuf<int> d_dh_bin;                    // [n]
   DevBuf<unsigned long long> d_dh_e2;      // [63] squared edges (nm^2) as the bits of their doubles, the first H - 1 used
   DevBuf<unsigned long long> d_dh_cnt;     // [B (B + 1) / 2][H] counts
+
+  // genome architecture mapping (mmm_gam.cu): per bin pair, slices in which both bins are detected, over structures
+  bool gm_configured = false;
+  int32_t gm_bins = 0, gm_max_slices = 0;  // B, the most slices of one add
+  int64_t gm_structures = 0, gm_slices = 0, gm_empty = 0;
+  float gm_ms = 0.f;                       // device time of all adds
+  cudaEvent_t gm_ev0 = nullptr, gm_ev1 = nullptr;
+  DevBuf<int> d_gm_bin;                    // [n]
+  DevBuf<double> d_gm_planes;              // [max_slices][4] nx, ny, nz, o of the add
+  DevBuf<unsigned> d_gm_x;                 // [B][ceil(S / 32)] detection bitset of the add
+  DevBuf<unsigned> d_gm_any;               // [ceil(S / 32)] slices in which any bin is detected
+  DevBuf<unsigned long long> d_gm_cnt;     // [B (B + 1) / 2] co-segregation counts
 };
 
 // the sorted keys of one sparse pass (mmm_contacts_sparse_pass)

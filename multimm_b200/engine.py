@@ -420,6 +420,36 @@ class Engine:
         self._ck(self._lib.mmm_disthist_read(self._h, C.byref(samples), _p(counts), C.byref(ms)))
         return dict(samples=int(samples.value), counts=counts, device_ms=float(ms.value))
 
+    # -- genome architecture mapping (bins co-detected in random slices, summed over many structures) --
+    def gam_configure(self, bin_of_bead, n_bins: int, max_slices: int):
+        """Clear the GAM accumulator and set its bins (mmm_gam_configure): ``bin_of_bead`` (int[N], -1 = left
+        out) of ``n_bins`` bins, and ``max_slices``, the most slices of one add (1 to 65536)."""
+        bins = _arr(bin_of_bead, np.int32)
+        if bins is not None and bins.shape != (self.n,):
+            raise ValueError(f"bin_of_bead must have shape ({self.n},)")
+        self._ck(self._lib.mmm_gam_configure(self._h, _p(bins), int(n_bins), int(max_slices)))
+        self._gam_bins = int(n_bins)
+
+    def gam_add(self, planes, half_thickness: float):
+        """Slice the structure at the current positions (mmm_gam_add): ``planes`` float64 [S, 4] (normal nx, ny, nz
+        and offset o of every slice), a bead lies in a slice iff |((nx*x + ny*y) + nz*z) - o| <= half_thickness."""
+        pl = _arr(planes, np.float64)
+        if pl is None or pl.ndim != 2 or pl.shape[1] != 4:
+            raise ValueError("planes must have shape (S, 4)")
+        self._ck(self._lib.mmm_gam_add(self._h, _p(pl), len(pl), float(half_thickness)))
+
+    def gam_read(self) -> dict:
+        """The GAM sums (mmm_gam_read): ``structures``, ``slices``, ``empty`` (slices without any detected bin);
+        ``counts`` uint64 [B (B + 1) / 2], rows in ``np.triu_indices(B)`` order, the slices in which both bins
+        are detected (the diagonal: each bin's detections); ``device_ms`` of all adds."""
+        nb = getattr(self, "_gam_bins", 0)
+        counts = np.zeros(nb * (nb + 1) // 2, np.uint64)
+        structures, slices, empty, ms = C.c_int64(), C.c_int64(), C.c_int64(), C.c_float()
+        self._ck(self._lib.mmm_gam_read(self._h, C.byref(structures), C.byref(slices), C.byref(empty), _p(counts),
+                                        C.byref(ms)))
+        return dict(structures=int(structures.value), slices=int(slices.value), empty=int(empty.value), counts=counts,
+                    device_ms=float(ms.value))
+
     # -- MD relaxation ----------------------------------------------------------------------------
     def md_configure(self, integrator="langevin", dt_ps=0.001, temperature_k=310.0, friction_per_ps=0.5,
                      mass_amu=16427.889, seed=0, amd_alpha=None, amd_e=None):

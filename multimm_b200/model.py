@@ -78,6 +78,9 @@ class MultiMM:
     # the distance histograms (SAVE_DISTANCE_HIST): the counts of the minimised structure and of the MD samples,
     # and where finish() writes them (the ensemble driver points distance_hist_file outside run_<i>)
     distance_hist = distance_hist_md = distance_hist_file = None
+    # GAM co-segregation (SAVE_GAM): the sums of the minimised structure and of the MD samples, and where finish()
+    # writes them (the ensemble driver points gam_file outside run_<i>)
+    gam = gam_md = gam_file = None
 
     def __init__(self, args, device: int | None = None):
         self.args = args
@@ -405,9 +408,11 @@ class MultiMM:
         dyn = self._configure_dynamics() if sample_every > 0 and contact_setting(a, "SAVE_DYNAMICS") else None
         hist_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_DISTANCE_HIST"))
         hb = self._configure_distance_hist() if hist_sampling else None
+        gam_sampling = sample_every > 0 and bool(contact_setting(a, "SAVE_GAM"))
+        gg = self._configure_gam() if gam_sampling else None
         chunk = int(np.gcd.reduce([every, dcd_every] +
                                   ([sample_every] if sampling or loop_sampling or triplet_sampling or dyn or hist_sampling
-                                   else [])))
+                                   or gam_sampling else [])))
         t0 = time.time()
         print('#"Step"\t"Potential Energy (kJ/mole)"\t"Kinetic Energy (kJ/mole)"\t"Total Energy (kJ/mole)"\t"Temperature (K)"')
         done = 0
@@ -439,6 +444,8 @@ class MultiMM:
                     self.engine.dynamics_add()
                 if hist_sampling and done % sample_every == 0:
                     self.engine.disthist_add()
+                if gam_sampling and done % sample_every == 0:
+                    self._gam_add(gg, done // sample_every)
         finally:
             dcd.close()
         if sampling:
@@ -451,6 +458,8 @@ class MultiMM:
             self._read_dynamics(dyn, sample_every)
         if hist_sampling:
             self._read_distance_hist(hb, md=True)
+        if gam_sampling:
+            self._read_gam(gg, md=True)
         self.positions = self.engine.get_positions()
         cif.write_mmcif(10.0 * self.positions, self.chr_ends, self.save_path + "model/MultiMM_afterMD.cif",
                         hetatm_ends=True, connections=False, decimals=4)
@@ -518,6 +527,8 @@ class MultiMM:
             self.count_triplets()
         if contact_setting(self.args, "SAVE_DISTANCE_HIST"):
             self.count_distance_hist()
+        if contact_setting(self.args, "SAVE_GAM"):
+            self.count_gam()
         if self.args.SIM_RUN_MD:
             self.run_md()
 
@@ -684,6 +695,58 @@ class MultiMM:
         self._read_distance_hist(hb)
         self.timings["distance_hist_s"] = time.time() - t0
 
+    def _configure_gam(self):
+        """Set up the engine's GAM accumulator with the canonical bins of GAM_RESOLUTION and room for GAM_SLICES
+        slices per add; returns the bins."""
+        from . import contacts, gam
+
+        a = self.args
+        res = int(contact_setting(a, "GAM_RESOLUTION"))
+        try:
+            gb = contacts.genome_bins(self.layout, res, n_beads=a.N_BEADS, max_bins=gam.MAX_BINS)
+        except ValueError as e:
+            raise ValueError(f"GAM_RESOLUTION={res}: {e}") from None
+        self.engine.gam_configure(gb.bins, gb.n_bins, int(contact_setting(a, "GAM_SLICES")))
+        return gb
+
+    def _gam_add(self, gb, k: int):
+        """Slice the structure on the device with GAM_SLICES random planes about the container centre, drawn from
+        the private stream default_rng([SHUFFLING_SEED, k]) (k = 0: the minimised structure, k = s: MD sample s),
+        never from numpy's global stream, whose order the ensemble driver keeps."""
+        from . import gam
+
+        a = self.args
+        rng = np.random.default_rng([int(a.SHUFFLING_SEED), int(k)])
+        planes, h = gam.slice_planes(self.engine.get_positions(), self.mass_center, gb.bins,
+                                     int(contact_setting(a, "GAM_SLICES")), float(contact_setting(a, "GAM_SLICE_FRACTION")),
+                                     rng)
+        self.engine.gam_add(planes, h)
+
+    def _read_gam(self, gb, md: bool = False):
+        from . import gam
+
+        r = self.engine.gam_read()
+        if md:
+            logger.info(f"GAM: {r['structures']} MD structures, {r['slices']} slices ({r['empty']} empty; "
+                        f"{r['device_ms']:.1f} ms on the device)")
+            if r["structures"] == 0:
+                return
+        d = gam.result(r, gb, float(contact_setting(self.args, "GAM_SLICE_FRACTION")))
+        if md:
+            self.gam_md = d
+        else:
+            self.gam = d
+
+    def count_gam(self):
+        """GAM co-segregation of the minimised structure (SAVE_GAM): GAM_SLICES random slices through the
+        positions the minimisation left on the device, bins co-detected counted by this member's own engine in
+        canonical genomic coordinates."""
+        t0 = time.time()
+        gb = self._configure_gam()
+        self._gam_add(gb, 0)
+        self._read_gam(gb)
+        self.timings["gam_s"] = time.time() - t0
+
     def _configure_dynamics(self) -> dict:
         """SAVE_DYNAMICS: set up the engine's dynamics accumulator with the canonical bins of DYNAMICS_RESOLUTION,
         the lags 1, 2, ..., DYNAMICS_MAX_LAG and this member's valid loop rows.  Returns the bins and lags."""
@@ -801,6 +864,13 @@ class MultiMM:
             for d, path in ((self.distance_hist, hist_path), (self.distance_hist_md, contacts.md_path(hist_path))):
                 if d is not None:
                     disthist.save(path, d)
+        if self.gam is not None or self.gam_md is not None:
+            from . import gam
+
+            gam_path = self.gam_file or os.path.join(self.save_path, "analysis", "gam.npz")
+            for d, path in ((self.gam, gam_path), (self.gam_md, contacts.md_path(gam_path))):
+                if d is not None:
+                    gam.save(path, d)
         if self.dynamics is not None:
             from . import dynamics
 

@@ -16,6 +16,7 @@ from __future__ import annotations
 import argparse
 import configparser
 import logging
+import math
 import multiprocessing as mp
 import os
 import shutil
@@ -205,6 +206,7 @@ def args_tests(args):
     check_triplet_fields(args)
     check_dynamics_fields(args)
     check_distance_hist_fields(args)
+    check_gam_fields(args)
     check_md_sample_fields(args)
 
 
@@ -271,6 +273,31 @@ def check_distance_hist_fields(args):
                              f"{len(edges)} edges at most {most} are supported (0 = automatic)")
 
 
+def check_gam_fields(args):
+    """GAM_RESOLUTION >= 0 and, where the modelled stretch is known from the config alone, at most gam.MAX_BINS
+    bins; GAM_SLICES in [1, gam.MAX_SLICES]; GAM_SLICE_FRACTION finite, in (0, 1]; with SAVE_GAM, a
+    SHUFFLING_SEED >= 0 (the slices are drawn from it)."""
+    from . import contacts, gam
+
+    res = int(contact_setting(args, "GAM_RESOLUTION"))
+    if res < 0:
+        raise ValueError(f"GAM_RESOLUTION={res} must be >= 0 (0 = automatic)")
+    sp = _modelled_spans(args)
+    if res > 0 and sp is not None:
+        nb = contacts.bin_count(sp, res)
+        if nb > gam.MAX_BINS:
+            raise ValueError(f"GAM_RESOLUTION={res} bp gives {nb} GAM bins; at most {gam.MAX_BINS} are supported "
+                             "(0 = automatic)")
+    slices = int(contact_setting(args, "GAM_SLICES"))
+    if not 1 <= slices <= gam.MAX_SLICES:
+        raise ValueError(f"GAM_SLICES={slices} must be in [1, {gam.MAX_SLICES}]")
+    frac = float(contact_setting(args, "GAM_SLICE_FRACTION"))
+    if not (math.isfinite(frac) and 0.0 < frac <= 1.0):
+        raise ValueError(f"GAM_SLICE_FRACTION={frac} must be in (0, 1]")
+    if contact_setting(args, "SAVE_GAM") and int(args.SHUFFLING_SEED) < 0:
+        raise ValueError(f"SAVE_GAM draws its slices from SHUFFLING_SEED, which must be >= 0 (got {args.SHUFFLING_SEED})")
+
+
 def check_loop_fields(args):
     """LOOP_APA_WINDOW in [0, loops.MAX_WINDOW]."""
     from . import loops
@@ -282,9 +309,9 @@ def check_loop_fields(args):
 
 def check_md_sample_fields(args):
     """MD_SAMPLE_STEP >= 0; when > 0, MD must run, a map must be on (SAVE_CONTACTS or SAVE_DISTANCES, the loop
-    readout SAVE_LOOPS, the three-way map SAVE_TRIPLETS, the dynamics SAVE_DYNAMICS or the distance histograms
-    SAVE_DISTANCE_HIST), and the MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) * SIM_SAMPLING_STEP steps,
-    must reach the first sample."""
+    readout SAVE_LOOPS, the three-way map SAVE_TRIPLETS, the dynamics SAVE_DYNAMICS, the distance histograms
+    SAVE_DISTANCE_HIST or GAM SAVE_GAM), and the MD loop, which runs (SIM_N_STEPS // SIM_SAMPLING_STEP) *
+    SIM_SAMPLING_STEP steps, must reach the first sample."""
     step = int(contact_setting(args, "MD_SAMPLE_STEP"))
     if step < 0:
         raise ValueError(f"MD_SAMPLE_STEP={step} must be >= 0 (0 = no trajectory maps)")
@@ -294,9 +321,9 @@ def check_md_sample_fields(args):
         raise ValueError(f"MD_SAMPLE_STEP={step} samples the MD run, but SIM_RUN_MD is off")
     if not any(contact_setting(args, k)
                for k in ("SAVE_CONTACTS", "SAVE_DISTANCES", "SAVE_LOOPS", "SAVE_TRIPLETS", "SAVE_DYNAMICS",
-                         "SAVE_DISTANCE_HIST")):
+                         "SAVE_DISTANCE_HIST", "SAVE_GAM")):
         raise ValueError(f"MD_SAMPLE_STEP={step} needs a map to sample: enable SAVE_CONTACTS or SAVE_DISTANCES "
-                         "(or SAVE_LOOPS, SAVE_TRIPLETS, SAVE_DYNAMICS, SAVE_DISTANCE_HIST)")
+                         "(or SAVE_LOOPS, SAVE_TRIPLETS, SAVE_DYNAMICS, SAVE_DISTANCE_HIST, SAVE_GAM)")
     every = max(1, int(args.SIM_SAMPLING_STEP))
     steps = (int(args.SIM_N_STEPS) // every) * every
     if step > steps:
@@ -507,6 +534,7 @@ def build_replica(params: dict, i: int, run_path: str, device: int):
     md.triplets_file = member_triplets_path(params["OUT_PATH"], i)
     md.dynamics_file = member_dynamics_path(params["OUT_PATH"], i)
     md.distance_hist_file = member_distance_hist_path(params["OUT_PATH"], i)
+    md.gam_file = member_gam_path(params["OUT_PATH"], i)
     md.timings["ingest_s"] = time.time() - t0
     return md
 
@@ -537,6 +565,10 @@ def member_dynamics_path(out_path: str, i: int) -> str:
 
 def member_distance_hist_path(out_path: str, i: int) -> str:
     return os.path.join(out_path, "distance_hist", f"member_{i}.npz")
+
+
+def member_gam_path(out_path: str, i: int) -> str:
+    return os.path.join(out_path, "gam", f"member_{i}.npz")
 
 
 def _sampled_md(args) -> bool:
@@ -628,6 +660,27 @@ def write_ensemble_distance_hist(args, results: list[dict]) -> str | None:
         disthist.save(path, agg)
         logger.info(f"ensemble distance histograms{' (MD samples)' if md else ''}: {int(agg['members'])} structures, "
                     f"{len(agg['edges_nm'])} edges -> {path}")
+        out = out or path
+    return out
+
+
+def write_ensemble_gam(args, results: list[dict]) -> str | None:
+    """SAVE_GAM: OUT_PATH/ensemble_gam.npz, the sum of the GAM files of the members that succeeded (exact integer
+    sums: the same bits whichever GPU ran which member); with MD_SAMPLE_STEP also ensemble_gam_md.npz, the sum of
+    their MD samples."""
+    if not contact_setting(args, "SAVE_GAM") or not results:
+        return None
+    from . import contacts, gam
+
+    out = None
+    for md in (False, True) if _sampled_md(args) else (False,):
+        name = contacts.md_path if md else (lambda p: p)
+        paths = [name(member_gam_path(args.OUT_PATH, r["replica"])) for r in sorted(results, key=lambda r: r["replica"])]
+        agg = gam.aggregate(paths)
+        path = name(os.path.join(args.OUT_PATH, "ensemble_gam.npz"))
+        gam.save(path, agg)
+        logger.info(f"ensemble GAM{' (MD samples)' if md else ''}: {int(agg['structures'])} structures, "
+                    f"{int(agg['slices'])} slices ({int(agg['empty'])} empty) -> {path}")
         out = out or path
     return out
 
@@ -885,6 +938,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
         write_ensemble_triplets(args, results)
         write_ensemble_dynamics(args, results)
         write_ensemble_distance_hist(args, results)
+        write_ensemble_gam(args, results)
         if errors:
             raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
         check_archives(results)
@@ -926,6 +980,7 @@ def run_ensemble(args, devices: list[int] | None = None, archive: bool = True) -
     write_ensemble_triplets(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_dynamics(args, [r for r in results if r.get("replica", -1) >= 0])
     write_ensemble_distance_hist(args, [r for r in results if r.get("replica", -1) >= 0])
+    write_ensemble_gam(args, [r for r in results if r.get("replica", -1) >= 0])
     if errors:
         raise RuntimeError(f"{len(errors)} ensemble member(s) failed: {errors}")
     check_archives(results)
